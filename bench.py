@@ -20,6 +20,9 @@ Legs of the default run (every number in the JSON line is measured in this run u
                  ESS of every gamma_j, divided by the device time of burn-in + draws
   other_configs  BASELINE configs 2, 4, 5 on one GPU (N = 1 only): ms/sweep, chain-iterations/s, roofline fraction
   cpu_baseline   the reference's algorithm (NumPy/OpenBLAS port, Julia is absent) on the host cores (N = 1 only)
+
+--dump-outputs DIR writes what the K timed sweeps computed as DIR/<name>.npy.  Inputs and seeds are fixed, so two builds
+run with the same arguments can be compared output for output.
 """
 import os
 import sys
@@ -41,6 +44,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # bench.py writes nothing into the tree: no __pycache__ for what it imports from it
 
 CONFIGS = {
     # name: V, n, R, chains per GPU
@@ -197,12 +201,13 @@ def cpu_port_sample(X, y, R, chains, sweeps, warm):
 def run_reference(args, rank):
     """`--impl reference`: the reference's own CPU path (port) on all host cores, same config / metric / unit.
     One step = one sweep of the min(64, cores) chains that run concurrently (the bounded sample of the 64-chain
-    workload); exactly `steps` timed sweeps after `warmup` untimed ones are run and reported."""
+    workload); exactly `steps` timed sweeps (main() refuses more than --ref-max-sweeps) are run and reported, after
+    min(warmup, 3), at least 1, untimed ones."""
     if rank != 0:
         return
     X, y, dims = synth(args.config, args.dense)
     chains = CONFIGS[args.config]["chains"]
-    sweeps = max(1, min(args.steps, args.ref_max_sweeps))
+    sweeps = args.steps
     warm = max(1, min(args.warmup, 3))
     cpu, r = cpu_port_sample(X, y, dims["R"], chains, sweeps, warm)
     val = cpu["value"]
@@ -260,6 +265,29 @@ def time_sweeps(eng, K):
     return eng.last_run_ms()
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, eng, var_names, rank, world, chain_offset, rx, rg, status):
+    """--dump-outputs: what the timed sweeps hand to a caller -- every chain's state after the last sweep (Engine.get_state,
+    stacked over chains), the per-chain status bits and the split R-hat of the timed draws -- as float64 <name>.npy.
+    Beyond DUMP_BYTES in all, a fixed seeded sample of the chains is written; chain_ids.npy names the global chains kept.
+    With several ranks every rank writes its own chains under <name>_rank<r>.npy."""
+    per_chain = 8 * (2 + sum(int(np.prod(eng.var_shape(k))) for k in var_names))    # + status and chain id
+    room = DUMP_BYTES // world - 8 * (rx.size + rg.size) - (1 << 16)                  # 64 KB for the .npy headers
+    keep = max(1, min(eng.C, room // per_chain))
+    chains = np.arange(eng.C)
+    if keep < eng.C:
+        chains = np.sort(np.random.default_rng(0).choice(eng.C, keep, replace=False))
+    out = {"chain_ids": chain_offset + chains, "status": status[chains], "rhat_xi": rx, "rhat_gamma": rg}
+    for k in var_names:
+        out[k] = np.stack([eng.get_state(int(c), k) for c in chains])
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "_rank%d" % rank if world > 1 else ""
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + suffix + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -275,7 +303,7 @@ def main():
     ap.add_argument("--chain-groups", type=int, default=0, help="independent stream/graph groups per GPU (0 = library default)")
     ap.add_argument("--gamma-mode", default="auto", choices=["auto", "nform", "qform"])
     ap.add_argument("--dense", action="store_true", help="dense Gaussian X instead of sparse networks")
-    ap.add_argument("--ref-max-sweeps", type=int, default=200, help="reference arm: cap on the timed sweeps")
+    ap.add_argument("--ref-max-sweeps", type=int, default=200, help="reference arm: largest --steps it accepts")
     ap.add_argument("--cpu-sweeps", type=int, default=10, help="cpu_baseline leg of our arm: timed sweeps per chain")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-sweeps", type=int, default=5)
@@ -284,7 +312,16 @@ def main():
     ap.add_argument("--ess-max-lag", type=int, default=255)
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the timed sweeps computed (chain states after the last one, status, R-hat) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    if args.impl == "reference" and args.steps > args.ref_max_sweeps:
+        ap.error("--impl reference times exactly --steps sweeps: %d is above --ref-max-sweeps %d"
+                 % (args.steps, args.ref_max_sweeps))
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -357,6 +394,7 @@ def main():
     eng.run(Wm)
     eng.set_moment_window(Wm + 1, K)
     launches0 = eng.launch_count()
+    iter0 = eng.iteration
     barrier()
     sampler.mark()
     t0 = time.perf_counter()
@@ -367,6 +405,7 @@ def main():
     dev_ms = eng.last_run_ms()
     clocks = sampler.stop()
     launches = eng.launch_count() - launches0
+    assert eng.iteration - iter0 == K, "the timed run advanced %d sweeps, not --steps %d" % (eng.iteration - iter0, K)
     total_ms = max_over_ranks(dev_ms)          # collective: every rank calls it exactly once, here
     step_ms = total_ms / K
     value = world * chains * K / (total_ms * 1e-3)
@@ -385,6 +424,8 @@ def main():
     else:
         rx, rg = eng.rhat()
     status = eng.status()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, bnr.VAR, rank, world, rank * chains, rx, rg, status)
 
     # ---------------- per-phase CUDA-event profile of eager sweeps (roofline numerator) ----------------
     phases = {}

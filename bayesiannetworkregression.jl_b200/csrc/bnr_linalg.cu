@@ -506,8 +506,9 @@ k_trsm_dmma(const __grid_constant__ CUtensorMap tmL, const __grid_constant__ CUt
 // ------------------------------------------------------------------------------------------------------------
 // Blocked left-looking Cholesky, block size 128, of every chain's gdim x gdim matrix, with BOTH triangular solves
 // organised around it:
-//   * forward solve for free: the right-hand side r is stored as row m (the first padding row, m = n or q) of the
-//     matrix itself, with the diagonal entry d = 1 + |r|^2 / lmin (k_augment; lmin <= lambda_min(G)).  The bordered
+//   * forward solve for free: the right-hand side r (scaled by a power of two to |r| ~ 1) is stored as row m (the first
+//     padding row, m = n or q) of the matrix itself, with the diagonal entry d = 1 + |r|^2 / lmin (k_augment;
+//     lmin <= lambda_min(G)).  The bordered
 //     matrix [[G, r], [r', d]] is positive definite (r' G^-1 r <= |r|^2 / lambda_min < d), and row m of its Cholesky
 //     factor IS w' = (L^-1 r)': the DMMA update / panel-solve kernels below carry the solve along as one more row of
 //     the last row block.  (The corner entry sqrt(d - |w|^2) is never used.)
@@ -536,17 +537,20 @@ __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.a
 // row m of every G_c <- (r_c, 1 + |r_c|^2 / lmin_c), lmin_c a lower bound of the smallest eigenvalue of G_c, so that
 // the bordered matrix stays positive definite (r' G^-1 r <= |r|^2 / lambda_min):  n-form G = X D X' + I: lmin = 1;
 // q-form P = (X'X + D^-1)/tau2: lmin = 1 / (tau2 max_j S_j)  (S, tau2 given).  grid = C, block = 256.
+// The row holds r_c 2^-e with |r_c 2^-e| in [1/2, 1): the last pivot, 1 + |r|^2 / lmin - r' G^-1 r, is a difference of
+// two terms of size |r|^2, and unscaled its rounding (eps |r|^2) made it negative from |r| ~ 1e8 on when r is nearly
+// orthogonal to the range of X.  The row's arithmetic is linear in r, so the power-of-two scale is exact: k_bwd_stream
+// multiplies w by 2^e, which k_augment leaves in r_c[m] (the first padding entry of the right-hand side).
 __global__ void __launch_bounds__(256) k_augment(double* __restrict__ G, size_t chain_stride, int N, int m,
-                                                 const double* __restrict__ r, int r_stride,
+                                                 double* __restrict__ r, int r_stride,
                                                  const double* __restrict__ S, const double* __restrict__ tau2) {
-  __shared__ double red[8], redm[8];
+  __shared__ double red[8], redm[8], scale;
   const int c = blockIdx.x, tid = threadIdx.x;
   double* Gc = G + (size_t)c * chain_stride;
-  const double* rc = r + (size_t)c * r_stride;
+  double* rc = r + (size_t)c * r_stride;
   double s = 0.0, mx = 0.0;
   for (int k = tid; k < m; k += 256) {
     const double v = rc[k];
-    Gc[(size_t)k * N + m] = v;
     s += v * v;
     if (S) mx = fmax(mx, S[(size_t)c * r_stride + k]);
   }
@@ -560,9 +564,17 @@ __global__ void __launch_bounds__(256) k_augment(double* __restrict__ G, size_t 
   if (tid == 0) {
     double t = 0.0, mm = 0.0;
     for (int w = 0; w < 8; ++w) { t += red[w]; mm = fmax(mm, redm[w]); }
+    int e = 0;
+    frexp(sqrt(t), &e);
+    const double sc = ldexp(1.0, -e);
     const double inv_lmin = S ? tau2[c] * mm : 1.0;
-    Gc[(size_t)m * N + m] = 1.0 + t * inv_lmin;
+    Gc[(size_t)m * N + m] = 1.0 + t * sc * sc * inv_lmin;
+    rc[m] = ldexp(1.0, e);
+    scale = sc;
   }
+  __syncthreads();
+  const double sc = scale;
+  for (int k = tid; k < m; k += 256) Gc[(size_t)k * N + m] = rc[k] * sc;
 }
 
 // ---- warp-level 32 x 32 x 32 products on the FP64 tensor cores, operands column-major in shared memory ----
@@ -1177,8 +1189,9 @@ __global__ void __launch_bounds__(BW_THREADS) k_bwd_stream(const __grid_constant
     return;
   }
 
+  const double unscale = out[(size_t)c * out_stride + m];       // 2^e of k_augment (out is its right-hand side)
   for (int k = tid; k < N; k += 256)
-    x[k] = (k < m) ? Gc[(size_t)k * N + m] + (addz ? addz[(size_t)c * addz_stride + k] : 0.0) : 0.0;
+    x[k] = (k < m) ? Gc[(size_t)k * N + m] * unscale + (addz ? addz[(size_t)c * addz_stride + k] : 0.0) : 0.0;
   named_bar_sync(1, 256);
 
   int it = 0;
@@ -1370,9 +1383,11 @@ __global__ void k_splitk_reduce(const double* __restrict__ ws, double* __restric
   out[i] = s;
 }
 
+// k-splits of X v, X' a4 and X gamma.  The split count sets the summation order, so it depends on the handle's chain
+// count only: a chain group (a view with d.C < d.C_total) and an eager sweep over the whole handle add in the same order.
 static int x_times_splits(const Dims& d, int trans) {
   const int M = trans ? d.qp : d.np, K = trans ? d.np : d.qp;
-  const int tiles = ((M + XM_BM - 1) / XM_BM) * ((d.C + XM_BN - 1) / XM_BN);
+  const int tiles = ((M + XM_BM - 1) / XM_BM) * ((d.C_total + XM_BN - 1) / XM_BN);
   int ks = (2 * 148 + tiles - 1) / tiles;
   const int kmax = K / (4 * XM_BK) > 0 ? K / (4 * XM_BK) : 1;
   if (ks > kmax) ks = kmax;
@@ -1381,9 +1396,11 @@ static int x_times_splits(const Dims& d, int trans) {
   return ks;
 }
 
+// Every workspace (the handle's and each chain group's) holds splits x chains x rows partial sums for the handle's whole
+// chain count.  A launch uses splits x d.C x rows with the same splits and d.C <= d.C_total, so it always fits.
 size_t x_times_workspace_doubles(const Dims& d) {
   const int a = x_times_splits(d, 0), b = x_times_splits(d, 1);
-  const size_t wa = (size_t)a * d.C * d.np, wb = (size_t)b * d.C * d.qp;
+  const size_t wa = (size_t)a * d.C_total * d.np, wb = (size_t)b * d.C_total * d.qp;
   return wa > wb ? wa : wb;
 }
 

@@ -310,7 +310,9 @@ def test_lambda_pi(small):
                                               # edge cases: smallest network, single sample, n a multiple of 128
                                               # (extra padding block for the bordering row), R at its maximum
                                               (2, 1, 3, True, "nform"), (3, 2, 1, True, "nform"), (2, 1, 5, True, "qform"),
-                                              (6, 3, 128, True, "nform"), (4, 16, 30, True, "qform")])
+                                              (6, 3, 128, True, "nform"), (4, 16, 30, True, "qform"),
+                                              # the bordering row on the last row of the matrix (n + 1 = 128, 1024)
+                                              (6, 3, 127, True, "nform"), (6, 3, 1023, True, "nform")])
 def test_full_sweeps_injected(bnr, V, R, n, dense, mode):
     """bnr_run (production schedule, fused kernels) == oracle gibbs_sweep for consecutive sweeps; the larger
     cases span several 128-row tiles and 64-column Cholesky panels."""

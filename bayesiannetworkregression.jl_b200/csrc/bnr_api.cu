@@ -338,7 +338,11 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
   // the blocks above the diagonal of every inverted panel are exact zeros that k_potf2_inv never writes
   CK(cudaMemsetAsync(e.Linv, 0, sizeof(double) * C * (size_t)(d.gdim / TILE_N) * TILE_N * TILE_N, h->stream));
   e.syrk_ws = nullptr; e.syrk_ws_cap = 0;
-  if (d.gmode == BNR_GAMMA_NFORM) {
+  e.gram_planes = nullptr; e.gram_rscale = nullptr;
+  if (gram_i8_selected(d)) {
+    DA(e.gram_planes, C * gram_i8_plane_bytes(d));
+    DA(e.gram_rscale, C * d.np);
+  } else if (d.gmode == BNR_GAMMA_NFORM) {
     // few chains x tiles: the SYRK splits its contraction (see launch_syrk_G).  The split count is fixed per handle
     // from its total chain count, so the chain grouping never changes the summation order.
     const int smax = syrk_splits(d, d.C);
@@ -411,6 +415,10 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
     int ng_auto = d.C >= 6 ? 3 : (d.C >= 4 ? 4 : (d.C >= 2 ? 2 : 1));
     if (d.gmode == BNR_GAMMA_NFORM && d.C >= 4 && syrk_splits(d, d.C) > 1) ng_auto = 2;
     if (d.gmode == BNR_GAMMA_QFORM && d.C >= 2 && d.C < 24) ng_auto = 2;
+    // INT8 Gram path: a k_gram_i8 CTA is ~0.2 ms, so below 16 chains one group keeps the SMs busiest (measured on B200,
+    // config 3, 100-sweep runs: 8 chains 1 / 2 / 3 / 4 / 8 groups -> 1.61 / 1.78 / 1.72 / 1.73 / 1.77 ms; 12 chains ->
+    // 1.98 / 2.07 / 2.11 / 2.16 / 2.23 ms)
+    if (gram_i8_selected(d) && d.C < 16) ng_auto = 1;
     int ng = p->chain_groups > 0 ? p->chain_groups : ng_auto;
     if (ng > MAX_GROUPS) ng = MAX_GROUPS;
     if (ng > d.C) ng = d.C;
@@ -612,6 +620,7 @@ static Engine group_view(const bnr_handle* h, int c0, int Cg, long long* counter
   v.M += c * d.R * d.R; v.lambda += c * d.R; v.pi += c * 3 * d.R;
   v.xg += c * d.np; v.xv += c * d.np; v.rhs += c * d.np;
   v.G += c * d.gdim * d.gdim; if (v.syrk_ws) v.syrk_ws += c * (size_t)v.syrk_ws_cap * d.gdim * d.gdim; v.Linv += c * (size_t)(d.gdim / TILE_N) * TILE_N * TILE_N;
+  if (v.gram_planes) { v.gram_planes += c * gram_i8_plane_bytes(d); v.gram_rscale += c * d.np; }
   v.partials += c * d.nparts * (2 * MAX_R + 1);
   v.moments += c * 2 * (d.V + d.q) * 2;
   if (v.bmom) v.bmom += c * (size_t)v.bmom_nb * (d.V + d.q) * 2;

@@ -108,6 +108,8 @@ struct Engine {
   double* G;        // [C][gdim*gdim] col-major, lower triangle used
   double* syrk_ws;  // [C][syrk_ws_cap][gdim*gdim] partial Gram matrices of the k-split SYRK (nullptr: never split)
   int syrk_ws_cap;  // splits - 1, fixed per handle
+  signed char* gram_planes;  // [C][7][np][qp] int8 digit planes of X diag(sqrt(S_c)) (INT8 Gram path, else nullptr)
+  double* gram_rscale;       // [C][np] power-of-two row scales of the digit planes
   double* Linv;     // [C][gdim/128][128*128]  inverses of the 128 x 128 diagonal blocks of the factor (column-major)
   double* partials; // [C][nparts][2*MAX_R+1]  block partial sums: A_r, B_r (lambda), sum S
   double* tau2_part;      // [handle chains][2 * TAU2_MAX_BLOCKS] partial sums of the tau2 reduction (NOT offset per view)

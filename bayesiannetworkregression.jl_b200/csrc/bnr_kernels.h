@@ -43,6 +43,13 @@ void launch_x_times(const Engine& e, int trans, const double* in, double* out, d
 size_t x_times_workspace_doubles(const Dims& d);
 void launch_syrk_G(const Engine& e, cudaStream_t s);         // G_c = X diag(S_c) X' + I (lower tiles)
 int syrk_splits(const Dims& d, int C);                        // k-splits launch_syrk_G uses for a batch of C chains
+// launch_syrk_G computes the n-form Gram matrix on the INT8 tensor cores (Ozaki digit planes) for qp in
+// [GRAM_I8_QP_MIN, GRAM_I8_QP_MAX], on the FP64 DMMA SYRK otherwise.  The rule depends on the shape only, never on the
+// chain count: every chain grouping and graph / eager sweeps keep the same rounding.
+constexpr int GRAM_I8_QP_MIN = 1024;
+constexpr int GRAM_I8_QP_MAX = 18724;     // 7 qp 2^14 < 2^31: the int32 accumulators of the digit products are exact
+bool gram_i8_selected(const Dims& d);
+size_t gram_i8_plane_bytes(const Dims& d);                    // digit planes of one chain
 // optional second stream + events that let launch_cholesky run the off-diagonal panel updates next to the panel
 // factorisation (works eagerly and under stream capture, where it becomes a fork/join of the graph)
 struct ForkJoin {

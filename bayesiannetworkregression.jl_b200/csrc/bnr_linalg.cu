@@ -1421,10 +1421,15 @@ void launch_x_times(const Engine& e, int trans, const double* in, double* out, d
   }
 }
 
+__global__ void k_gram_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+                          const double* __restrict__ rscale, double* __restrict__ G, int np, int nvalid, int nkb);
+extern const size_t GI_SMEM_BYTES;
+
 void linalg_setup() {
   cudaFuncSetAttribute(k_xmma<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)XMMA_SMEM);
   cudaFuncSetAttribute(k_xmma<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)XMMA_SMEM);
   cudaFuncSetAttribute(k_gram_syrk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SYRK_SMEM);
+  cudaFuncSetAttribute(k_gram_i8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GI_SMEM_BYTES);
   cudaFuncSetAttribute(k_chol_update, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SYRK_SMEM);
   cudaFuncSetAttribute(k_trsm_dmma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SYRK_SMEM);
   cudaFuncSetAttribute(k_potf2_inv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)POTF2_SMEM);
@@ -1512,8 +1517,267 @@ int syrk_splits(const Dims& d, int C) {
   return s < 1 ? 1 : s;
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// n-form Gram matrix on the INT8 tensor cores (Ozaki scheme): G_c = A_c A_c' + I with A_c = X diag(sqrt(S_c)).
+//   k_gram_slice: row i of A_c is scaled by 2^p_i (row max in [2^53, 2^55)), rounded ONCE to an integer N (|N| < 2^55;
+//     the entries near the row max are integers already: exact) and N is written as 7 balanced base-256 digits
+//     N = sum_s D^(s) 2^(8(6-s)), s = 0 (top, |D| <= 127) .. 6 (each in [-128, 127]).  Planes [c][s][row][k] int8, k
+//     contiguous (the k-major boxes the UMMA reads), plus rscale[c][row] = 2^-p_i.  Rounding the scaled value to the
+//     nearest integer is unbiased, so the rounding errors of a row do not add up with one sign when X >= 0.
+//   k_gram_i8: C_g = sum_{s+t=g} D^(s) D^(t)' for g = 0..6 (28 digit products, the pairs with s + t > 6 weigh at most
+//     ~2^-56 of the row maxima and are dropped) in seven int32 TMEM accumulators of a 128 x 64 tile (448 of the 512
+//     columns), then G = 2^96 rscale_i rscale_j sum_g 2^-8g C_g, added in a fixed order (Horner from g = 6), + I.
+//     |D^(s) D^(t)| <= 2^14 and the largest group has 7 products per k, so int32 is exact while 7 qp 2^14 < 2^31:
+//     qp <= GRAM_I8_QP_MAX.  Larger qp stays on the FP64 SYRK (gram_i8_selected).
+// Warp roles of k_gram_i8 (192 threads, 1 CTA / SM): warp 4 lane 0 issues the TMA boxes (all 7 planes of the
+// 128-row and of the 64-row operand per k-block: one 3-D box each) into a GI_STAGES ring; warp 5 lane 0 issues the
+// tcgen05.mma and releases each stage with tcgen05.commit; warps 0-3 read the accumulators (TMEM lanes 32w..32w+31 =
+// rows of the tile) and store G.  Tiles: 128-row block ib x 64-column block jb <= 2 ib + 1, chains slowest, so the
+// CTAs of one chain run back to back while its planes are in L2.  The stored entries are exactly those the FP64 SYRK
+// stores (same 8 x 8 fragment rule), so the matrix the factorisation sees is the same up to the rounding.
+// ------------------------------------------------------------------------------------------------------------
+#ifndef BNR_GI_BK
+#define BNR_GI_BK 64
+#endif
+#ifndef BNR_GI_STAGES
+#define BNR_GI_STAGES 2
+#endif
+constexpr int GI_S = 7;                   // digit planes (and digit-sum groups)
+constexpr int GI_BM = 128, GI_BN = 64;    // tile
+constexpr int GI_BK = BNR_GI_BK;          // k-block in bytes (int8 elements) = swizzle width
+constexpr int GI_STAGES = BNR_GI_STAGES;
+constexpr int GI_A_PLANE = GI_BM * GI_BK, GI_B_PLANE = GI_BN * GI_BK;
+constexpr int GI_STAGE_BYTES = GI_S * (GI_A_PLANE + GI_B_PLANE);
+constexpr size_t GI_SMEM = (size_t)GI_STAGES * GI_STAGE_BYTES + 1024 + 256;   // + alignment slack + barriers
+const size_t GI_SMEM_BYTES = GI_SMEM;
+constexpr int GI_THREADS = 192;
+static_assert(GI_BK == 32 || GI_BK == 64 || GI_BK == 128, "k-block = swizzle width");
+static_assert(GI_S * GI_BN <= 512, "accumulators exceed tensor memory");
+
+// UMMA shared-memory descriptor of a K-major operand with GI_BK-byte swizzle: 8-row core groups GI_BK * 8 bytes apart
+__device__ __forceinline__ unsigned long long gi_desc(unsigned saddr) {
+  constexpr unsigned long long layout = GI_BK == 128 ? 2ull : (GI_BK == 64 ? 4ull : 6ull);
+  return (unsigned long long)((saddr & 0x3FFFF) >> 4) | (1ull << 16) | ((unsigned long long)((GI_BK * 8) >> 4) << 32) |
+         (1ull << 46) | (layout << 61);
+}
+// instruction descriptor: s32 accumulator, s8 x s8, both K-major, N = 64, M = 128
+constexpr unsigned GI_IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(GI_BN >> 3) << 17) | ((unsigned)(GI_BM >> 4) << 24);
+
+__device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* tm, int x, int y, int z, unsigned long long* bar) {
+  asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];\n" ::"r"(
+                   smem_u32(smem_dst)), "l"((unsigned long long)tm), "r"(x), "r"(y), "r"(z), "r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void umma_i8(unsigned tmem_d, unsigned long long adesc, unsigned long long bdesc, bool acc) {
+  asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n" ::"r"(tmem_d),
+               "l"(adesc), "l"(bdesc), "r"(GI_IDESC), "r"((int)acc));
+}
+__device__ __forceinline__ void umma_commit(unsigned long long* bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n" ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void tmem_ld8(unsigned taddr, int (&r)[8]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];\n"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) : "r"(taddr));
+}
+
+// grid = (np / 32, C), block = 256: 32 rows of one chain.  Lane = row (coalesced column reads of the column-major X),
+// warps split k; the digits of a 128-k chunk are gathered in shared memory and written as 4-byte words along k.
+__global__ void __launch_bounds__(256) k_gram_slice(const double* __restrict__ X, const double* __restrict__ S, int np,
+                                                    int q, int qp, signed char* __restrict__ planes,
+                                                    double* __restrict__ rscale) {
+  __shared__ unsigned buf[GI_S][32][33];
+  __shared__ double red[8][32];
+  const int c = blockIdx.y, r0 = blockIdx.x * 32, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int row = r0 + lane;
+  const double* Sc = S + (size_t)c * qp;
+  double m = 0.0;
+  for (int k = warp; k < q; k += 8) m = fmax(m, fabs(X[row + (size_t)np * k] * sqrt(Sc[k])));
+  red[warp][lane] = m;
+  __syncthreads();
+  m = 0.0;
+#pragma unroll
+  for (int w = 0; w < 8; ++w) m = fmax(m, red[w][lane]);
+  // 2^p m in [2^53 * 126/64, 2^54) or [2^54, 2^54 * 126/64]: the top digit stays within [-127, 127]
+  int p = 0;
+  if (m > 0.0) {
+    p = 54 - ilogb(m);
+    if (ldexp(m, p) > 126.0 * 0x1p48) --p;
+  }
+  if (warp == 0) rscale[(size_t)c * np + row] = ldexp(1.0, -p);
+  const int p1 = p > 1000 ? 1000 : p;
+  const double sc1 = ldexp(1.0, p1), sc2 = ldexp(1.0, p - p1);
+  signed char* out = planes + (size_t)c * GI_S * np * qp;
+  for (int k0 = 0; k0 < qp; k0 += 128) {
+#pragma unroll
+    for (int g = 0; g < 4; ++g) {
+      const int kw = warp * 4 + g;             // word of the chunk (4 k each)
+      unsigned w[GI_S] = {0, 0, 0, 0, 0, 0, 0};
+#pragma unroll
+      for (int b = 0; b < 4; ++b) {
+        const int k = k0 + kw * 4 + b;
+        if (k < q) {
+          long long N = __double2ll_rn(X[row + (size_t)np * k] * sqrt(Sc[k]) * sc1 * sc2);
+#pragma unroll
+          for (int s = GI_S - 1; s > 0; --s) {
+            const long long dg = ((N + 128) & 255) - 128;
+            w[s] |= ((unsigned)dg & 255u) << (8 * b);
+            N = (N - dg) >> 8;
+          }
+          w[0] |= ((unsigned)N & 255u) << (8 * b);
+        }
+      }
+#pragma unroll
+      for (int s = 0; s < GI_S; ++s) buf[s][lane][kw] = w[s];
+    }
+    __syncthreads();
+    for (int id = threadIdx.x; id < GI_S * 32 * 32; id += 256) {
+      const int s = id >> 10, rr = (id >> 5) & 31, kw = id & 31;
+      const int k = k0 + kw * 4;
+      if (k < qp) *reinterpret_cast<unsigned*>(out + ((size_t)s * np + r0 + rr) * qp + k) = buf[s][rr][kw];
+    }
+    __syncthreads();
+  }
+}
+
+__global__ void __launch_bounds__(GI_THREADS, 1)
+k_gram_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+          const double* __restrict__ rscale, double* __restrict__ G, int np, int nvalid, int nkb) {
+  extern __shared__ __align__(1024) unsigned char gsm_raw[];
+  unsigned char* gsm = reinterpret_cast<unsigned char*>(((size_t)gsm_raw + 1023) & ~(size_t)1023);
+  unsigned long long* full = reinterpret_cast<unsigned long long*>(gsm + (size_t)GI_STAGES * GI_STAGE_BYTES);
+  unsigned long long* empty = full + GI_STAGES;
+  unsigned long long* accf = empty + GI_STAGES;
+  unsigned* tmem_slot = reinterpret_cast<unsigned*>(accf + 1);
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int c = blockIdx.y;
+  int ib = 0;
+  while (2 * (ib + 1) * (ib + 2) / 2 <= (int)blockIdx.x) ++ib;       // row block ib holds 64-column blocks 0..2ib+1
+  const int jb = (int)blockIdx.x - ib * (ib + 1);
+  const int i0 = ib * GI_BM, j0 = jb * GI_BN;
+  const bool diag_block = (j0 / GI_BM) == ib;
+  // rows the FP64 SYRK stores: all rows of the diagonal 128-block; in a strictly lower block the 8-row fragments that
+  // hold a valid row, at least 4
+  int rows_st = GI_BM;
+  if (!diag_block) {
+    int nfv = (nvalid - i0 + 7) / 8;
+    if (nfv <= 0) return;                                             // block of padding rows only: nothing stored
+    rows_st = (nfv < 4 ? 4 : nfv) * 8;
+  }
+  if (tid == 0) {
+    for (int s = 0; s < GI_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
+    mbar_init(accf, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+  }
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;\n" ::"r"(smem_u32(tmem_slot)));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n");
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
+  const unsigned tmem = *tmem_slot;
+
+  if (warp == 4 && lane == 0) {
+    for (int kb = 0; kb < nkb; ++kb) {
+      const int st = kb % GI_STAGES;
+      mbar_wait(&empty[st], ((kb / GI_STAGES) & 1) ^ 1);
+      unsigned char* sa = gsm + (size_t)st * GI_STAGE_BYTES;
+      mbar_expect_tx(&full[st], GI_STAGE_BYTES);
+      tma_load_3d(sa, &tmA, kb * GI_BK, i0, c * GI_S, &full[st]);
+      tma_load_3d(sa + GI_S * GI_A_PLANE, &tmB, kb * GI_BK, j0, c * GI_S, &full[st]);
+    }
+  } else if (warp == 5 && lane == 0) {
+    for (int kb = 0; kb < nkb; ++kb) {
+      const int st = kb % GI_STAGES;
+      mbar_wait(&full[st], (kb / GI_STAGES) & 1);
+      asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
+      const unsigned sa = smem_u32(gsm + (size_t)st * GI_STAGE_BYTES), sb = sa + GI_S * GI_A_PLANE;
+#pragma unroll
+      for (int kk = 0; kk < GI_BK / 32; ++kk) {
+#pragma unroll
+        for (int s = 0; s < GI_S; ++s) {
+          const unsigned long long ad = gi_desc(sa + s * GI_A_PLANE + kk * 32);
+#pragma unroll
+          for (int t = 0; t < GI_S - s; ++t)
+            umma_i8(tmem + (unsigned)((s + t) * GI_BN), ad, gi_desc(sb + t * GI_B_PLANE + kk * 32), kb > 0 || kk > 0 || s > 0);
+        }
+      }
+      umma_commit(&empty[st]);
+    }
+    umma_commit(accf);
+  } else if (warp < 4) {
+    mbar_wait(accf, 0);
+    asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
+    const int r = warp * 32 + lane, i = i0 + r;
+    const double ri = rscale[(size_t)c * np + i] * 0x1p96;
+    double* Gc = G + (size_t)c * np * np;
+    const unsigned trow = tmem + ((unsigned)(warp * 32) << 16);
+    for (int j8 = 0; j8 < GI_BN; j8 += 8) {
+      int acc[GI_S][8];
+#pragma unroll
+      for (int g = 0; g < GI_S; ++g) tmem_ld8(trow + (unsigned)(g * GI_BN + j8), acc[g]);
+      asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory");
+#pragma unroll
+      for (int jj = 0; jj < 8; ++jj) {
+        const int j = j0 + j8 + jj;
+        double v = (double)acc[GI_S - 1][jj];
+#pragma unroll
+        for (int g = GI_S - 2; g >= 0; --g) v = (double)acc[g][jj] + v * 0x1p-8;
+        v = v * ri * rscale[(size_t)c * np + j];
+        if (i == j) v += 1.0;
+        if (r < rows_st && (i >> 3) >= (j >> 3)) Gc[(size_t)j * np + i] = v;
+      }
+    }
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
+  __syncthreads();
+  if (warp == 0) {
+    asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;\n" ::"r"(tmem));
+  }
+}
+
+bool gram_i8_selected(const Dims& d) { return d.gmode == 1 && d.qp >= GRAM_I8_QP_MIN && d.qp <= GRAM_I8_QP_MAX; }
+
+size_t gram_i8_plane_bytes(const Dims& d) { return (size_t)GI_S * d.np * d.qp; }
+
+// planes [C][7][np rows][qp] as a 3-D map {qp, np, 7 C}; a box is all 7 planes of box_rows rows x GI_BK k
+static CUresult encode_planes_map(CUtensorMap* m, const signed char* planes, const Dims& d, int C, uint32_t box_rows) {
+  memset(m, 0, sizeof(*m));
+  const cuuint64_t dims[3] = {(cuuint64_t)d.qp, (cuuint64_t)d.np, (cuuint64_t)GI_S * C};
+  const cuuint64_t strides[2] = {(cuuint64_t)d.qp, (cuuint64_t)d.qp * d.np};
+  const cuuint32_t box[3] = {(cuuint32_t)GI_BK, box_rows, (cuuint32_t)GI_S};
+  const cuuint32_t estr[3] = {1, 1, 1};
+  const CUtensorMapSwizzle sw = GI_BK == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
+                                             : (GI_BK == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+  if (!tmap_setup()) return CUDA_ERROR_NOT_SUPPORTED;
+  return g_tmap_encode(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<signed char*>(planes), dims, strides, box, estr,
+                       CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+}
+
+static void launch_gram_i8(const Engine& e, cudaStream_t s) {
+  const Dims& d = e.d;
+  CUtensorMap tmA, tmB;
+  if (encode_planes_map(&tmA, e.gram_planes, d, d.C, GI_BM) != CUDA_SUCCESS ||
+      encode_planes_map(&tmB, e.gram_planes, d, d.C, GI_BN) != CUDA_SUCCESS) {
+    fprintf(stderr, "[bnr] cuTensorMapEncodeTiled failed for the Gram digit planes (%d x %d)\n", d.np, d.qp);
+    abort();
+  }
+  ++g_launches; k_gram_slice<<<dim3(d.np / 32, d.C), 256, 0, s>>>(e.X, e.S, d.np, d.q, d.qp, e.gram_planes, e.gram_rscale);
+  const int T = d.np / GI_BM;
+  ++g_launches; k_gram_i8<<<dim3(T * (T + 1), d.C), GI_THREADS, GI_SMEM, s>>>(tmA, tmB, e.gram_rscale, e.G, d.np, d.n,
+                                                                             (d.qp + GI_BK - 1) / GI_BK);
+}
+
 void launch_syrk_G(const Engine& e, cudaStream_t s) {
   const Dims& d = e.d;
+  if (gram_i8_selected(d)) {
+    launch_gram_i8(e, s);
+    if (e.aux.G_copy) {
+      dim3 g2(d.np, d.C);
+      ++g_launches; k_copy_sym<<<g2, 256, 0, s>>>(e.G, (size_t)d.np * d.np, d.np, e.aux.G_copy);
+    }
+    return;
+  }
   const int T = d.np / SY_BT;
   const int nk = d.qp / SY_BK;
   const int ns = e.syrk_ws ? e.syrk_ws_cap + 1 : 1;   // fixed per handle: chain groups must not change the summation order

@@ -274,13 +274,21 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
   d.qp = (d.q + TILE_K - 1) / TILE_K * TILE_K;
   // gamma draw formulation (SURVEY 8d cost model): the q x q precision form costs q^3/3 + 4q^2 flops per
   // chain-iteration, the n x n Bhattacharya form (what the reference runs, src/gibbs.jl:429-436) n^2 q + n^3/3.
+  // AUTO: the rule of the 8192 limit (q-form iff cheaper and qp128 <= 8192) wherever its choice has a factored dimension
+  // <= 8192, so that no shape accepted then changes form; beyond, the cheaper of the forms that fit chol_max_dim().
   {
     const double qd = d.q, nd = d.n;
     const double cost_q = qd * qd * qd / 3.0 + 4.0 * qd * qd, cost_n = nd * nd * qd + nd * nd * nd / 3.0;
     const int qp128 = (d.q + 1 + TILE_N - 1) / TILE_N * TILE_N;
+    const int small = bwd_stream_max_dim(), large = chol_max_dim();
     int mode = p->gamma_mode;
-    if (mode != BNR_GAMMA_NFORM && mode != BNR_GAMMA_QFORM)
-      mode = (cost_q < cost_n && qp128 <= chol_max_dim()) ? BNR_GAMMA_QFORM : BNR_GAMMA_NFORM;
+    if (mode != BNR_GAMMA_NFORM && mode != BNR_GAMMA_QFORM) {
+      mode = (cost_q < cost_n && qp128 <= small) ? BNR_GAMMA_QFORM : BNR_GAMMA_NFORM;
+      if ((mode == BNR_GAMMA_QFORM ? qp128 : d.np) > small) {
+        const bool q_fits = qp128 <= large, n_fits = d.np <= large;
+        mode = (q_fits && (cost_q < cost_n || !n_fits)) ? BNR_GAMMA_QFORM : BNR_GAMMA_NFORM;
+      }
+    }
     d.gmode = mode;
     if (mode == BNR_GAMMA_QFORM) d.qp = qp128;       // q-padded vectors double as right-hand sides of the q x q solve
     d.gdim = mode == BNR_GAMMA_QFORM ? d.qp : d.np;
@@ -294,12 +302,19 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
   // dynamic shared memory of the per-chain kernels grows with V*R
   const size_t need = sizeof(double) * ((size_t)d.V * d.R + 2 * d.R * d.R + 2 + 4 * (2 * d.V + 2 * d.R * d.R + 3 * d.R));
   if (need > 200 * 1024 || d.gdim > chol_max_dim()) {
-    return fail(BNR_EINVAL, "problem too large for the per-chain shared-memory kernels (V*R > 200 KB of shared memory, or factored dimension > 8192)");
+    return fail(BNR_EINVAL, "problem too large for the per-chain shared-memory kernels (V*R > 200 KB of shared memory, or factored dimension > 32768: n <= 32767 in the n-form, V <= 255 in the q-form)");
   }
   CK(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
   CK(cudaEventCreate(&h->ev0));
   CK(cudaEventCreate(&h->ev1));
   linalg_setup();
+  {
+    // above 8192 the back solve is one cluster of 8 CTAs (~210 KB of shared memory each) per chain
+    const int clusters = bwd_cluster_capacity(d.gdim);
+    if (clusters < 0) return fail(BNR_ECUDA, "cudaOccupancyMaxActiveClusters failed for the cluster back solve");
+    if (clusters == 0)
+      return fail(BNR_ECUDA, "this device cannot co-schedule the back solve's cluster of 8 CTAs with ~210 KB of shared memory each (factored dimension > 8192)");
+  }
   if (!tmap_setup()) return fail(BNR_ECUDA, "cuTensorMapEncodeTiled is not available from this driver (TMA tensor maps are required)");
   small_kernels_setup();
 

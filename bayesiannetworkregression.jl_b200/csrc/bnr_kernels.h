@@ -67,6 +67,8 @@ void launch_chol_solve(const Engine& e, double* rhs, const double* addz, cudaStr
 void launch_xtx(const Dims& d, const double* XT, const double* ones, double* XtX, cudaStream_t s);   // X'X, once
 void launch_build_P(const Engine& e, cudaStream_t s);        // q-form: P_c = (X'X + diag(1/S_c)) / tau2_c
 int chol_max_dim();
+int bwd_stream_max_dim();                                     // above it the back solve runs on a CTA cluster per chain
+int bwd_cluster_capacity(int N);                              // resident back-solve clusters (0: none fits, < 0: error)
 bool tmaps_check(const Engine& e);                            // all tensor maps of this handle's geometry encode
 bool tmap_setup();                                            // resolves cuTensorMapEncodeTiled (false: driver without TMA maps)
 void linalg_setup();                                          // one-time cudaFuncSetAttribute calls

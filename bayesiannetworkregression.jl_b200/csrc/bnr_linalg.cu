@@ -2,7 +2,8 @@
 //   G_c = X diag(S_c) X' + I          -> k_gram_syrk : FP64 tensor-core (DMMA m8n8k4) SYRK, ring of TMA tensor-map boxes + mbarriers
 //   G_c = L_c L_c', w = L_c^-1 rhs    -> blocked left-looking Cholesky: k_augment / k_chol_update (DMMA) / k_potf2_inv /
 //                                        k_trsm_dmma (DMMA) / k_small_tile; the forward solve rides along as a bordering row
-//   a4  = L_c^-T w                    -> k_bwd_stream (the factor streamed once through a ring of TMA boxes)
+//   a4  = L_c^-T w                    -> k_bwd_stream (the factor streamed once through a ring of TMA boxes); above
+//                                        N = 8192 k_bwd_cluster (the same stream split over a cluster of 8 CTAs)
 //   X v, X' a4 (all chains at once)   -> k_xmma (tall-skinny DMMA GEMM, deterministic split-K)
 // tcgen05 has no FP64 kind, so the Blackwell tensor path for this contraction is the warp-level DMMA.
 #include <cstdio>
@@ -521,9 +522,14 @@ k_trsm_dmma(const __grid_constant__ CUtensorMap tmL, const __grid_constant__ CUt
 //       k_trsm_dmma   (DMMA): G[I, J] <- G[I, J] Linv_J' for I > J -- the panel solve is a GEMM
 //   * backward solve L' x = w (+ z): k_bwd_stream, one CTA per chain streams the factor once (tensor-map boxes of
 //     128 rows x 32 columns into a shared-memory ring), every step is a block mat-vec; the diagonal blocks use Linv.
+//     Above BWD_STREAM_MAX_DIM k_bwd_cluster spreads the same solve over a cluster of BWC_K CTAs per chain.
+// Index bound: N <= CHOL_MAX_DIM = 2^15, so N^2 = 2^30 and every in-matrix offset j * N + i fits an int; the kernels form
+// them in size_t anyway.  A tensor-map coordinate c * N + k (chain c) is an int: it needs C * N < 2^31, far above any
+// chain count whose factors fit in device memory (8.6 GB per chain at N = 32768).
 // ------------------------------------------------------------------------------------------------------------
 constexpr int PB = 128;            // panel / diagonal block size
-constexpr int CHOL_MAX_DIM = 8192; // largest factored dimension (the back solve keeps the solution vector in shared memory)
+constexpr int CHOL_MAX_DIM = 32768;        // largest factored dimension: N^2 fits an int, every grid fits its bound
+constexpr int BWD_STREAM_MAX_DIM = 8192;   // the one-CTA back solve keeps all of x in shared memory
 
 __device__ __forceinline__ void bulk_s2g(void* gdst, const void* ssrc, unsigned bytes) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;\n" ::"l"(gdst), "r"(smem_u32(ssrc)), "r"(bytes)
@@ -1247,6 +1253,228 @@ __global__ void __launch_bounds__(BW_THREADS) k_bwd_stream(const __grid_constant
   for (int k = tid; k < N; k += 256) out[(size_t)c * out_stride + k] = x[k];
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// backward solve above BWD_STREAM_MAX_DIM: one cluster of BWC_K CTAs per chain (the same solve as k_bwd_stream, over K
+// SMs' share of L2 bandwidth instead of one, and with x spread over K shared memories instead of held by one).
+//   ownership  CTA r owns the block rows I = r (mod K): it keeps b_I, overwritten by x_I, in its shared memory and
+//              streams the tiles L[I, J], I > J, of its own rows (and Linv_J of its own columns) through its own ring
+//              (tensor-map boxes, full / empty mbarriers, one producer lane: exactly k_bwd_stream's ring).
+//   column J   every CTA forms p_r = sum_{own I > J, I descending} L[I, J]' x_I with k_bwd_stream's mat-vec (warp per
+//              4 columns of a part, partial sums in registers).  A non-owner writes p_r into slot r of the owner's
+//              current slot set (DSMEM stores by lane 0 of each warp, then one release-arrive per warp, cluster scope, on
+//              the owner's "slot set full" mbarrier).  The owner waits for the K - 1 partials, forms
+//              b_J - p_0 - p_1 - ... - p_{K-1} in rank order, releases the slot set (a remote arrive on a "slot free"
+//              mbarrier in every other CTA) and computes x_J = Linv_J' b_J.  Only the owner waits: the x_I a CTA needs
+//              are the ones it solved itself, so the others run ahead up to BWC_SLOTS columns per owner.
+// K is a constant, so the summation order depends on N only: every chain count, chain grouping and device split adds
+// in the same order.  grid = C * K (cluster K x 1 x 1), block = 288 (8 consumer warps + the producer warp).
+// ------------------------------------------------------------------------------------------------------------
+constexpr int BWC_K = 8;           // CTAs per chain (the portable cluster size)
+constexpr int BWC_SLOTS = 2;       // slot sets per owner: a writer may run this many of the owner's columns ahead
+static int bwc_own_blocks(int N) { return (N / PB + BWC_K - 1) / BWC_K; }
+static size_t bwc_fixed_bytes(int N) {
+  return sizeof(double) * ((size_t)bwc_own_blocks(N) * PB + (size_t)BWC_SLOTS * BWC_K * PB) +
+         sizeof(unsigned long long) * (2 * BW_MAX_STAGES + BWC_SLOTS + BWC_K * BWC_SLOTS) + 128;
+}
+static int bwc_stages(int N) {
+  const size_t budget = 227 * 1024 - bwc_fixed_bytes(N);
+  const int ns = (int)(budget / (sizeof(double) * BW_STAGE_DBL));
+  return ns > BW_MAX_STAGES ? BW_MAX_STAGES : ns;
+}
+static size_t bwc_smem(int N) { return sizeof(double) * (size_t)bwc_stages(N) * BW_STAGE_DBL + bwc_fixed_bytes(N); }
+
+__device__ __forceinline__ unsigned cluster_ctarank() {
+  unsigned r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;\n" : "=r"(r));
+  return r;
+}
+// shared::cluster address of the same shared-memory offset in CTA `rank` of the cluster
+__device__ __forceinline__ unsigned mapa_rank(const void* p, unsigned rank) {
+  unsigned a;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;\n" : "=r"(a) : "r"(smem_u32(p)), "r"(rank));
+  return a;
+}
+__device__ __forceinline__ void st_cluster_f64(unsigned addr, double v) {
+  asm volatile("st.shared::cluster.f64 [%0], %1;\n" ::"r"(addr), "d"(v) : "memory");
+}
+// release at cluster scope: this thread's earlier (DSMEM) stores are visible to whoever acquires the phase
+__device__ __forceinline__ void mbar_arrive_remote(unsigned addr) {
+  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];\n" ::"r"(addr) : "memory");
+}
+__device__ __forceinline__ void mbar_wait_cluster(unsigned long long* bar, unsigned parity) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "WAIT_LOOP:\n"
+      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n"
+      "@p bra DONE;\n"
+      "bra WAIT_LOOP;\n"
+      "DONE:\n"
+      "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
+}
+__device__ __forceinline__ void cluster_sync_all() {
+  asm volatile("barrier.cluster.arrive.release;\nbarrier.cluster.wait.acquire;\n" ::: "memory");
+}
+
+__global__ void __launch_bounds__(BW_THREADS) k_bwd_cluster(const __grid_constant__ CUtensorMap tmG,
+                                                            const __grid_constant__ CUtensorMap tmL,
+                                                            const double* __restrict__ G, size_t chain_stride, int N, int m,
+                                                            double* __restrict__ out, int out_stride,
+                                                            const double* __restrict__ addz, int addz_stride, int nstages) {
+  extern __shared__ __align__(128) double sm[];
+  const int T = N / PB, nown = (T + BWC_K - 1) / BWC_K;
+  double* ring = sm;
+  double* xo = sm + (size_t)nstages * BW_STAGE_DBL;               // [nown][128] b_I, then x_I, of the own blocks I = r + K li
+  double* slot = xo + (size_t)nown * PB;                          // [BWC_SLOTS][BWC_K][128] partials of the other CTAs
+  unsigned long long* full = reinterpret_cast<unsigned long long*>(slot + (size_t)BWC_SLOTS * BWC_K * PB);
+  unsigned long long* empty = full + BW_MAX_STAGES;
+  unsigned long long* sfull = empty + BW_MAX_STAGES;              // [BWC_SLOTS] the K - 1 partials of a slot set are in
+  unsigned long long* sfree = sfull + BWC_SLOTS;                  // [owner][BWC_SLOTS] the owner has read that slot set
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int r = (int)cluster_ctarank(), c = (int)blockIdx.x / BWC_K;
+  const int Itop = (T - 1) - (T - 1 - r) % BWC_K;                 // the last own block row (T > K: every rank owns one)
+  const double* Gc = G + (size_t)c * chain_stride;
+  if (tid == 0) {
+    for (int s = 0; s < nstages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 8); }
+    for (int s = 0; s < BWC_SLOTS; ++s) mbar_init(&sfull[s], 8 * (BWC_K - 1));
+    for (int i = 0; i < BWC_K * BWC_SLOTS; ++i) mbar_init(&sfree[i], 1);
+    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+  }
+  __syncthreads();
+  cluster_sync_all();                                             // every barrier of the cluster exists before a remote arrive
+
+  if (warp == 8) {
+    // ---- producer: the parts in consumption order (J down; own I from the top down to J + 1; Linv_J if J is own) ----
+    if (lane == 0) {
+      int p = 0;
+      for (int J = T - 1; J >= 0; --J) {
+        // own rows I > J of block column J, then (own column) the inverse of the diagonal block: I == J
+        const int Ilast = (J % BWC_K == r) ? J : J + 1;
+        for (int I = Itop; I >= Ilast; I -= BWC_K) {
+          for (int h = 0; h < BW_NH; ++h, ++p) {
+            const int stage = p % nstages;
+            mbar_wait(&empty[stage], ((p / nstages) & 1) ^ 1);
+            mbar_expect_tx(&full[stage], BW_STAGE_DBL * 8u);
+            double* dst = ring + (size_t)stage * BW_STAGE_DBL;
+            if (I == J) tma_load_2d(dst, &tmL, 0, (c * T + J) * PB + h * BW_COLS, &full[stage]);
+            else tma_load_2d(dst, &tmG, I * PB, c * N + J * PB + h * BW_COLS, &full[stage]);
+          }
+        }
+      }
+    }
+  } else {
+    const double unscale = out[(size_t)c * out_stride + m];       // 2^e of k_augment (out is its right-hand side)
+    for (int id = tid; id < nown * PB; id += 256) {
+      const int I = r + BWC_K * (id / PB), k = I * PB + id % PB;
+      xo[id] = (I < T && k < m) ? Gc[(size_t)k * N + m] * unscale + (addz ? addz[(size_t)c * addz_stride + k] : 0.0) : 0.0;
+    }
+    named_bar_sync(1, 256);
+
+    int it = 0;
+    for (int J = T - 1; J >= 0; --J) {
+      const int o = J % BWC_K, u = (T - 1 - J) / BWC_K;            // owner of column J, and its use count of the slots
+      const int s = u % BWC_SLOTS;
+      const unsigned par = (u / BWC_SLOTS) & 1;
+      double pr[BW_NH][BW_CPW];
+#pragma unroll
+      for (int h = 0; h < BW_NH; ++h)
+#pragma unroll
+        for (int q = 0; q < BW_CPW; ++q) pr[h][q] = 0.0;
+      for (int I = Itop; I > J; I -= BWC_K) {
+        const double* v = xo + (size_t)(I / BWC_K) * PB;
+        const double v0 = v[lane], v1 = v[lane + 32], v2 = v[lane + 64], v3 = v[lane + 96];
+#pragma unroll
+        for (int h = 0; h < BW_NH; ++h, ++it) {
+          const int stage = it % nstages;
+          mbar_wait(&full[stage], (it / nstages) & 1);
+          const double* B = ring + (size_t)stage * BW_STAGE_DBL + (size_t)(warp * BW_CPW) * PB + lane;
+          double acc[BW_CPW];
+#pragma unroll
+          for (int q = 0; q < BW_CPW; ++q)
+            acc[q] = B[q * PB] * v0 + B[q * PB + 32] * v1 + B[q * PB + 64] * v2 + B[q * PB + 96] * v3;
+#pragma unroll
+          for (int q = 0; q < BW_CPW; ++q) {
+#pragma unroll
+            for (int o2 = 16; o2 > 0; o2 >>= 1) acc[q] += __shfl_xor_sync(0xffffffffu, acc[q], o2);
+            pr[h][q] += acc[q];
+          }
+          // released after the shuffles have consumed every lane's loads (DESIGN section 4, rule 4)
+          __syncwarp();
+          if (lane == 0) mbar_arrive(&empty[stage]);
+        }
+      }
+      if (o != r) {
+        if (lane == 0) {
+          mbar_wait_cluster(&sfree[o * BWC_SLOTS + s], par ^ 1);   // the owner has read this slot set's previous use
+          const unsigned dst = mapa_rank(slot + ((size_t)s * BWC_K + r) * PB, (unsigned)o);
+#pragma unroll
+          for (int h = 0; h < BW_NH; ++h)
+#pragma unroll
+            for (int q = 0; q < BW_CPW; ++q) st_cluster_f64(dst + 8u * (h * BW_COLS + warp * BW_CPW + q), pr[h][q]);
+          mbar_arrive_remote(mapa_rank(&sfull[s], (unsigned)o));
+        }
+        __syncwarp();
+        continue;
+      }
+      double* bJ = xo + (size_t)(J / BWC_K) * PB;
+      if (lane == 0) {
+        mbar_wait_cluster(&sfull[s], par);
+        const double* sl = slot + (size_t)s * BWC_K * PB;
+#pragma unroll
+        for (int h = 0; h < BW_NH; ++h)
+#pragma unroll
+          for (int q = 0; q < BW_CPW; ++q) {
+            const int col = h * BW_COLS + warp * BW_CPW + q;
+            double t = bJ[col];
+#pragma unroll
+            for (int rr = 0; rr < BWC_K; ++rr) t -= (rr == r) ? pr[h][q] : sl[rr * PB + col];
+            bJ[col] = t;
+          }
+      }
+      __syncwarp();
+      named_bar_sync(1, 256);                  // b_J is complete; every read of the slot set has gone into it
+      if (tid == 0) {
+        for (int rr = 0; rr < BWC_K; ++rr)
+          if (rr != r) mbar_arrive_remote(mapa_rank(&sfree[r * BWC_SLOTS + s], (unsigned)rr));
+      }
+      const double v0 = bJ[lane], v1 = bJ[lane + 32], v2 = bJ[lane + 64], v3 = bJ[lane + 96];
+      double xn[BW_NH][BW_CPW];
+#pragma unroll
+      for (int h = 0; h < BW_NH; ++h, ++it) {
+        const int stage = it % nstages;
+        mbar_wait(&full[stage], (it / nstages) & 1);
+        const double* B = ring + (size_t)stage * BW_STAGE_DBL + (size_t)(warp * BW_CPW) * PB + lane;
+        double acc[BW_CPW];
+#pragma unroll
+        for (int q = 0; q < BW_CPW; ++q)
+          acc[q] = B[q * PB] * v0 + B[q * PB + 32] * v1 + B[q * PB + 64] * v2 + B[q * PB + 96] * v3;
+#pragma unroll
+        for (int q = 0; q < BW_CPW; ++q) {
+#pragma unroll
+          for (int o2 = 16; o2 > 0; o2 >>= 1) acc[q] += __shfl_xor_sync(0xffffffffu, acc[q], o2);
+          xn[h][q] = acc[q];
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&empty[stage]);
+      }
+      named_bar_sync(1, 256);                  // everybody has read b_J
+      if (lane == 0) {
+#pragma unroll
+        for (int h = 0; h < BW_NH; ++h)
+#pragma unroll
+          for (int q = 0; q < BW_CPW; ++q) bJ[h * BW_COLS + warp * BW_CPW + q] = xn[h][q];
+      }
+      __syncwarp();
+      named_bar_sync(1, 256);                  // x_J is visible
+    }
+    for (int id = tid; id < nown * PB; id += 256) {
+      const int I = r + BWC_K * (id / PB);
+      if (I < T) out[(size_t)c * out_stride + (size_t)I * PB + id % PB] = xo[id];
+    }
+  }
+  cluster_sync_all();                          // no CTA leaves while another may still write its slots or barriers
+}
+
 // symmetric copy of G (lower -> full) into the aux buffer, for the parity tests.  grid = (np, C)
 __global__ void k_copy_sym(const double* __restrict__ G, size_t chain_stride, int np, double* __restrict__ out) {
   const int c = blockIdx.y, j = blockIdx.x;
@@ -1434,6 +1662,7 @@ void linalg_setup() {
   cudaFuncSetAttribute(k_trsm_dmma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SYRK_SMEM);
   cudaFuncSetAttribute(k_potf2_inv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)POTF2_SMEM);
   cudaFuncSetAttribute(k_bwd_stream, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  cudaFuncSetAttribute(k_bwd_cluster, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   cudaFuncSetAttribute(k_small_tile<1, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_tile_smem(32));
   cudaFuncSetAttribute(k_small_tile<2, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_tile_smem(32));
   cudaFuncSetAttribute(k_small_tile<1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_tile_smem(16));
@@ -2018,10 +2247,45 @@ void launch_chol_solve(const Engine& e, double* out, const double* addz, cudaStr
   const int stride = d.gmode == 2 ? d.qp : d.np;
   const CUtensorMap tmG = make_map(e.G, N, (uint64_t)N * d.C, N, PB, BW_COLS);
   const CUtensorMap tmL = make_map(e.Linv, PB, (uint64_t)PB * (N / PB) * d.C, PB, PB, BW_COLS);
-  ++g_launches; k_bwd_stream<<<d.C, BW_THREADS, bwd_smem(N), s>>>(tmG, tmL, e.G, (size_t)N * N, N, m, out, stride, addz, stride,
-                                                               bwd_stages(N));
+  if (N <= BWD_STREAM_MAX_DIM) {
+    ++g_launches; k_bwd_stream<<<d.C, BW_THREADS, bwd_smem(N), s>>>(tmG, tmL, e.G, (size_t)N * N, N, m, out, stride, addz,
+                                                                 stride, bwd_stages(N));
+    return;
+  }
+  cudaLaunchConfig_t cfg = {};
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = BWC_K; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  cfg.gridDim = dim3(d.C * BWC_K);
+  cfg.blockDim = dim3(BW_THREADS);
+  cfg.dynamicSmemBytes = bwc_smem(N);
+  cfg.stream = s;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  ++g_launches;
+  cudaLaunchKernelEx(&cfg, k_bwd_cluster, tmG, tmL, (const double*)e.G, (size_t)N * N, N, m, out, stride, addz, stride,
+                     bwc_stages(N));
+}
+
+// clusters of the back solve that can be resident at once for factored dimension N (0: the cluster cannot be placed,
+// < 0: the query failed); N <= BWD_STREAM_MAX_DIM runs the one-CTA kernel, which needs no check
+int bwd_cluster_capacity(int N) {
+  if (N <= BWD_STREAM_MAX_DIM) return 1;
+  cudaLaunchConfig_t cfg = {};
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = BWC_K; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  cfg.gridDim = dim3(BWC_K);
+  cfg.blockDim = dim3(BW_THREADS);
+  cfg.dynamicSmemBytes = bwc_smem(N);
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  int n = 0;
+  if (cudaOccupancyMaxActiveClusters(&n, k_bwd_cluster, &cfg) != cudaSuccess) return -1;
+  return n;
 }
 
 int chol_max_dim() { return CHOL_MAX_DIM; }
+int bwd_stream_max_dim() { return BWD_STREAM_MAX_DIM; }
 
 }  // namespace bnr

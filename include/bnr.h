@@ -137,9 +137,11 @@ typedef struct bnr_params {
 
 #define BNR_MAX_R 16
 /* Size limits (bnr_create returns BNR_EINVAL beyond them; the reference has none): R <= 16; the factored dimension --
- * n + 1 for the n x n form, q + 1 for the q x q form, rounded up to a multiple of 128 -- at most 8192 (the back solve
- * keeps the solution vector in shared memory); V * R doubles + a few R x R blocks must fit 200 KB of shared memory. */
-#define BNR_MAX_FACTOR_DIM 8192
+ * n + 1 for the n x n form, q + 1 for the q x q form, rounded up to a multiple of 128 -- at most 32768 (n <= 32767 in
+ * the n-form, V <= 255 in the q-form; above 8192 the back solve runs on a cluster of 8 CTAs per chain); V * R doubles +
+ * a few R x R blocks must fit 200 KB of shared memory.  AUTO keeps the choice it made under the former 8192 limit
+ * wherever that choice fits 8192, and otherwise picks the cheaper of the forms that fit 32768. */
+#define BNR_MAX_FACTOR_DIM 32768
 
 int bnr_version(void);
 const char* bnr_last_error(void);

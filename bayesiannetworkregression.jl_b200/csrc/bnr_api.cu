@@ -430,10 +430,9 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
     int ng_auto = d.C >= 6 ? 3 : (d.C >= 4 ? 4 : (d.C >= 2 ? 2 : 1));
     if (d.gmode == BNR_GAMMA_NFORM && d.C >= 4 && syrk_splits(d, d.C) > 1) ng_auto = 2;
     if (d.gmode == BNR_GAMMA_QFORM && d.C >= 2 && d.C < 24) ng_auto = 2;
-    // INT8 Gram path: a k_gram_i8 CTA is ~0.2 ms, so below 16 chains one group keeps the SMs busiest (measured on B200,
-    // config 3, 100-sweep runs: 8 chains 1 / 2 / 3 / 4 / 8 groups -> 1.61 / 1.78 / 1.72 / 1.73 / 1.77 ms; 12 chains ->
-    // 1.98 / 2.07 / 2.11 / 2.16 / 2.23 ms)
-    if (gram_i8_selected(d) && d.C < 16) ng_auto = 1;
+    // INT8 Gram path: below 12 chains one group keeps the SMs busiest (measured on B200 at 1000 W, config 3, 100-sweep
+    // runs: 8 chains 1 / 2 / 3 groups -> 1.36 / 1.44 / 1.41 ms; 12 chains -> 1.76 / 1.70 / 1.70 ms)
+    if (gram_i8_selected(d) && d.C < 12) ng_auto = 1;
     int ng = p->chain_groups > 0 ? p->chain_groups : ng_auto;
     if (ng > MAX_GROUPS) ng = MAX_GROUPS;
     if (ng > d.C) ng = d.C;

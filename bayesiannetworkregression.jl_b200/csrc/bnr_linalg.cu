@@ -1764,6 +1764,7 @@ int syrk_splits(const Dims& d, int C) {
 // rows of the tile) and store G.  Tiles: 128-row block ib x 64-column block jb <= 2 ib + 1, chains slowest, so the
 // CTAs of one chain run back to back while its planes are in L2.  The stored entries are exactly those the FP64 SYRK
 // stores (same 8 x 8 fragment rule), so the matrix the factorisation sees is the same up to the rounding.
+// GI_LAB_LOADS_ONLY / GI_LAB_MMA_ONLY are defined only by the diagnostic builds of tools/lab/gram_i8_lab.cu.
 // ------------------------------------------------------------------------------------------------------------
 #ifndef BNR_GI_BK
 #define BNR_GI_BK 64
@@ -1789,16 +1790,19 @@ __device__ __forceinline__ unsigned long long gi_desc(unsigned saddr) {
   return (unsigned long long)((saddr & 0x3FFFF) >> 4) | (1ull << 16) | ((unsigned long long)((GI_BK * 8) >> 4) << 32) |
          (1ull << 46) | (layout << 61);
 }
-// instruction descriptor: s32 accumulator, s8 x s8, both K-major, N = 64, M = 128
-constexpr unsigned GI_IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(GI_BN >> 3) << 17) | ((unsigned)(GI_BM >> 4) << 24);
+// instruction descriptor: s32 accumulator, s8 x s8, both K-major, M = 128, N = n (n % 16 == 0, n <= 256)
+__host__ __device__ constexpr unsigned gi_idesc(int n) {
+  return (2u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(n >> 3) << 17) | ((unsigned)(GI_BM >> 4) << 24);
+}
 
 __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* tm, int x, int y, int z, unsigned long long* bar) {
   asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];\n" ::"r"(
                    smem_u32(smem_dst)), "l"((unsigned long long)tm), "r"(x), "r"(y), "r"(z), "r"(smem_u32(bar)) : "memory");
 }
-__device__ __forceinline__ void umma_i8(unsigned tmem_d, unsigned long long adesc, unsigned long long bdesc, bool acc) {
+__device__ __forceinline__ void umma_i8(unsigned tmem_d, unsigned long long adesc, unsigned long long bdesc, unsigned idesc,
+                                        bool acc) {
   asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n" ::"r"(tmem_d),
-               "l"(adesc), "l"(bdesc), "r"(GI_IDESC), "r"((int)acc));
+               "l"(adesc), "l"(bdesc), "r"(idesc), "r"((int)acc));
 }
 __device__ __forceinline__ void umma_commit(unsigned long long* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n" ::"r"(smem_u32(bar)) : "memory");
@@ -1810,6 +1814,7 @@ __device__ __forceinline__ void tmem_ld8(unsigned taddr, int (&r)[8]) {
 
 // grid = (np / 32, C), block = 256: 32 rows of one chain.  Lane = row (coalesced column reads of the column-major X),
 // warps split k; the digits of a 128-k chunk are gathered in shared memory and written as 4-byte words along k.
+// Every lane of a warp needs the same sqrt(S_k): lane l takes the root of one k and the warp shares it by shuffle.
 __global__ void __launch_bounds__(256) k_gram_slice(const double* __restrict__ X, const double* __restrict__ S, int np,
                                                     int q, int qp, signed char* __restrict__ planes,
                                                     double* __restrict__ rscale) {
@@ -1819,7 +1824,12 @@ __global__ void __launch_bounds__(256) k_gram_slice(const double* __restrict__ X
   const int row = r0 + lane;
   const double* Sc = S + (size_t)c * qp;
   double m = 0.0;
-  for (int k = warp; k < q; k += 8) m = fmax(m, fabs(X[row + (size_t)np * k] * sqrt(Sc[k])));
+  for (int k0 = warp; k0 < q; k0 += 8 * 32) {
+    const int kl = k0 + 8 * lane;
+    const double sq = kl < q ? sqrt(Sc[kl]) : 0.0;
+    const int nk = (q - k0 + 7) / 8 < 32 ? (q - k0 + 7) / 8 : 32;
+    for (int j = 0; j < nk; ++j) m = fmax(m, fabs(X[row + (size_t)np * (k0 + 8 * j)] * __shfl_sync(0xffffffffu, sq, j)));
+  }
   red[warp][lane] = m;
   __syncthreads();
   m = 0.0;
@@ -1836,6 +1846,8 @@ __global__ void __launch_bounds__(256) k_gram_slice(const double* __restrict__ X
   const double sc1 = ldexp(1.0, p1), sc2 = ldexp(1.0, p - p1);
   signed char* out = planes + (size_t)c * GI_S * np * qp;
   for (int k0 = 0; k0 < qp; k0 += 128) {
+    const int kl = k0 + warp * 16 + (lane & 15);   // the 16 k of this warp in the chunk
+    const double sq = kl < q ? sqrt(Sc[kl]) : 0.0;
 #pragma unroll
     for (int g = 0; g < 4; ++g) {
       const int kw = warp * 4 + g;             // word of the chunk (4 k each)
@@ -1843,15 +1855,16 @@ __global__ void __launch_bounds__(256) k_gram_slice(const double* __restrict__ X
 #pragma unroll
       for (int b = 0; b < 4; ++b) {
         const int k = k0 + kw * 4 + b;
+        const double sqk = __shfl_sync(0xffffffffu, sq, g * 4 + b);
         if (k < q) {
-          long long N = __double2ll_rn(X[row + (size_t)np * k] * sqrt(Sc[k]) * sc1 * sc2);
+          // balanced digits: with the bias B = 128 (1 + 2^8 + ... + 2^40), byte i of N + B is D^(6-i) + 128 for i < 6
+          // and (N + B) >> 48 is the top digit D^(0)
+          const long long M = __double2ll_rn(X[row + (size_t)np * k] * sqk * sc1 * sc2) + 0x808080808080ll;
+          const unsigned lo = (unsigned)M ^ 0x80808080u, hi = (unsigned)(M >> 32) ^ 0x8080u;
 #pragma unroll
-          for (int s = GI_S - 1; s > 0; --s) {
-            const long long dg = ((N + 128) & 255) - 128;
-            w[s] |= ((unsigned)dg & 255u) << (8 * b);
-            N = (N - dg) >> 8;
-          }
-          w[0] |= ((unsigned)N & 255u) << (8 * b);
+          for (int i = 0; i < 4; ++i) w[GI_S - 1 - i] |= ((lo >> (8 * i)) & 255u) << (8 * b);
+#pragma unroll
+          for (int i = 0; i < 3; ++i) w[2 - i] |= ((hi >> (8 * i)) & 255u) << (8 * b);
         }
       }
 #pragma unroll
@@ -1906,7 +1919,11 @@ k_gram_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
   const unsigned tmem = *tmem_slot;
 
   if (warp == 4 && lane == 0) {
+#if defined(GI_LAB_MMA_ONLY)
+    for (int kb = 0; kb < GI_STAGES && kb < nkb; ++kb) {
+#else
     for (int kb = 0; kb < nkb; ++kb) {
+#endif
       const int st = kb % GI_STAGES;
       mbar_wait(&empty[st], ((kb / GI_STAGES) & 1) ^ 1);
       unsigned char* sa = gsm + (size_t)st * GI_STAGE_BYTES;
@@ -1917,17 +1934,32 @@ k_gram_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
   } else if (warp == 5 && lane == 0) {
     for (int kb = 0; kb < nkb; ++kb) {
       const int st = kb % GI_STAGES;
+#if defined(GI_LAB_MMA_ONLY)
+      if (kb < GI_STAGES) mbar_wait(&full[st], 0);
+#else
       mbar_wait(&full[st], (kb / GI_STAGES) & 1);
+#endif
       asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
+#if defined(GI_LAB_LOADS_ONLY)
+      umma_commit(&empty[st]);
+      continue;
+#endif
       const unsigned sa = smem_u32(gsm + (size_t)st * GI_STAGE_BYTES), sb = sa + GI_S * GI_A_PLANE;
+      // A plane s times the B planes t = 0..6-s, which lie back to back in the stage (one K-major operand of 64 (7-s)
+      // rows, the same 8-row group stride) and accumulate into the adjacent columns 64 (s+t): one MMA of N = 64 (7-s),
+      // cut at N = 256.  10 instructions per 32-byte k-step; only the s = 0 pair of the first k-step (all 448
+      // columns) overwrites.
 #pragma unroll
       for (int kk = 0; kk < GI_BK / 32; ++kk) {
 #pragma unroll
         for (int s = 0; s < GI_S; ++s) {
           const unsigned long long ad = gi_desc(sa + s * GI_A_PLANE + kk * 32);
 #pragma unroll
-          for (int t = 0; t < GI_S - s; ++t)
-            umma_i8(tmem + (unsigned)((s + t) * GI_BN), ad, gi_desc(sb + t * GI_B_PLANE + kk * 32), kb > 0 || kk > 0 || s > 0);
+          for (int t0 = 0; t0 < GI_S - s; t0 += 4) {
+            const int nt = GI_S - s - t0 < 4 ? GI_S - s - t0 : 4;
+            umma_i8(tmem + (unsigned)((s + t0) * GI_BN), ad, gi_desc(sb + t0 * GI_B_PLANE + kk * 32), gi_idesc(nt * GI_BN),
+                    kb > 0 || kk > 0 || s > 0);
+          }
         }
       }
       umma_commit(&empty[st]);
@@ -1983,7 +2015,8 @@ static CUresult encode_planes_map(CUtensorMap* m, const signed char* planes, con
                        CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 }
 
-static void launch_gram_i8(const Engine& e, cudaStream_t s) {
+// k_gram_i8 alone (the digit planes of e's chains are in place)
+static void launch_gram_i8_products(const Engine& e, cudaStream_t s) {
   const Dims& d = e.d;
   CUtensorMap tmA, tmB;
   if (encode_planes_map(&tmA, e.gram_planes, d, d.C, GI_BM) != CUDA_SUCCESS ||
@@ -1991,10 +2024,15 @@ static void launch_gram_i8(const Engine& e, cudaStream_t s) {
     fprintf(stderr, "[bnr] cuTensorMapEncodeTiled failed for the Gram digit planes (%d x %d)\n", d.np, d.qp);
     abort();
   }
-  ++g_launches; k_gram_slice<<<dim3(d.np / 32, d.C), 256, 0, s>>>(e.X, e.S, d.np, d.q, d.qp, e.gram_planes, e.gram_rscale);
   const int T = d.np / GI_BM;
   ++g_launches; k_gram_i8<<<dim3(T * (T + 1), d.C), GI_THREADS, GI_SMEM, s>>>(tmA, tmB, e.gram_rscale, e.G, d.np, d.n,
                                                                              (d.qp + GI_BK - 1) / GI_BK);
+}
+
+static void launch_gram_i8(const Engine& e, cudaStream_t s) {
+  const Dims& d = e.d;
+  ++g_launches; k_gram_slice<<<dim3(d.np / 32, d.C), 256, 0, s>>>(e.X, e.S, d.np, d.q, d.qp, e.gram_planes, e.gram_rscale);
+  launch_gram_i8_products(e, s);
 }
 
 void launch_syrk_G(const Engine& e, cudaStream_t s) {

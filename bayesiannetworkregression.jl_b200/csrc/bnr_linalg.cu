@@ -1812,72 +1812,152 @@ __device__ __forceinline__ void tmem_ld8(unsigned taddr, int (&r)[8]) {
                : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) : "r"(taddr));
 }
 
-// grid = (np / 32, C), block = 256: 32 rows of one chain.  Lane = row (coalesced column reads of the column-major X),
-// warps split k; the digits of a 128-k chunk are gathered in shared memory and written as 4-byte words along k.
-// Every lane of a warp needs the same sqrt(S_k): lane l takes the root of one k and the warp shares it by shuffle.
-__global__ void __launch_bounds__(256) k_gram_slice(const double* __restrict__ X, const double* __restrict__ S, int np,
-                                                    int q, int qp, signed char* __restrict__ planes,
-                                                    double* __restrict__ rscale) {
-  __shared__ unsigned buf[GI_S][32][33];
-  __shared__ double red[8][32];
-  const int c = blockIdx.y, r0 = blockIdx.x * 32, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int row = r0 + lane;
-  const double* Sc = S + (size_t)c * qp;
-  double m = 0.0;
-  for (int k0 = warp; k0 < q; k0 += 8 * 32) {
-    const int kl = k0 + 8 * lane;
-    const double sq = kl < q ? sqrt(Sc[kl]) : 0.0;
-    const int nk = (q - k0 + 7) / 8 < 32 ? (q - k0 + 7) / 8 : 32;
-    for (int j = 0; j < nk; ++j) m = fmax(m, fabs(X[row + (size_t)np * (k0 + 8 * j)] * __shfl_sync(0xffffffffu, sq, j)));
+// k_gram_slice: a CTA takes GS_ROWS rows x GS_CB chains of the launch (the last chain block may be partial) over all k,
+// so each X element it loads serves GS_CB chains, in both passes (row maximum, then the digits).  Lane l of a warp
+// takes row l & 15 and the 16 k at 16 (l >> 4) of a 32-k block; the 8 warps take the 32-k blocks of a GS_TK-wide
+// window in turn.  The roots sqrt(S_ck) of a window are taken once per CTA into shared memory (both passes: the roots of
+// all k would not fit beside a resident k_gram_i8 CTA).  A thread's 16 k of one row are 16 contiguous bytes of each
+// plane: the bytes of 4 elements are transposed into 4 words with __byte_perm and each plane is one 16-byte store, so a
+// warp store covers 16 rows x 32 B, whole sectors.  Every element is computed as before, so the planes and rscale are
+// the same bits for any GS_CB.  GS_LAB_NO_STORES / GS_LAB_NO_DIGITS are defined only by the diagnostic builds of
+// tools/lab/gram_i8_lab.cu.
+constexpr int GS_ROWS = 16, GS_CB = 4, GS_THREADS = 256, GS_TK = 512;
+constexpr int GS_TKP = GS_TK + GS_TK / 8;   // 2 pad doubles per 16 k: the two half-warps read different banks
+__device__ __forceinline__ int gs_tidx(int kk) { return kk + 2 * (kk >> 4); }
+
+// sqrt(S_ck) for the window [t0, t0 + GS_TK) of the block's chains (0 for k >= q and for chains past the launch's)
+__device__ __forceinline__ void gs_roots(double (*sq)[GS_TKP], const double* __restrict__ S, int qp, int q, int ncb, int t0) {
+  for (int id = threadIdx.x; id < GS_CB * GS_TK; id += GS_THREADS) {
+    const int cb = id / GS_TK, kk = id % GS_TK, k = t0 + kk;
+    sq[cb][gs_tidx(kk)] = cb < ncb && k < q ? sqrt(S[(size_t)cb * qp + k]) : 0.0;
   }
-  red[warp][lane] = m;
-  __syncthreads();
-  m = 0.0;
+}
+
+__device__ __forceinline__ void gs_load_x(double (&x)[16], const double* __restrict__ X, int np, int q, int row, int k0) {
+  const bool full = k0 + 16 <= q;
 #pragma unroll
-  for (int w = 0; w < 8; ++w) m = fmax(m, red[w][lane]);
-  // 2^p m in [2^53 * 126/64, 2^54) or [2^54, 2^54 * 126/64]: the top digit stays within [-127, 127]
-  int p = 0;
-  if (m > 0.0) {
-    p = 54 - ilogb(m);
-    if (ldexp(m, p) > 126.0 * 0x1p48) --p;
-  }
-  if (warp == 0) rscale[(size_t)c * np + row] = ldexp(1.0, -p);
-  const int p1 = p > 1000 ? 1000 : p;
-  const double sc1 = ldexp(1.0, p1), sc2 = ldexp(1.0, p - p1);
-  signed char* out = planes + (size_t)c * GI_S * np * qp;
-  for (int k0 = 0; k0 < qp; k0 += 128) {
-    const int kl = k0 + warp * 16 + (lane & 15);   // the 16 k of this warp in the chunk
-    const double sq = kl < q ? sqrt(Sc[kl]) : 0.0;
+  for (int j = 0; j < 16; ++j) x[j] = full || k0 + j < q ? X[row + (size_t)np * (k0 + j)] : 0.0;
+}
+
+__global__ void __launch_bounds__(GS_THREADS, 2) k_gram_slice(const double* __restrict__ X, const double* __restrict__ S,
+                                                            int np, int q, int qp, int C, signed char* __restrict__ planes,
+                                                            double* __restrict__ rscale) {
+  __shared__ __align__(16) double sq[GS_CB][GS_TKP];
+  __shared__ double red[GS_THREADS / 32][GS_CB][GS_ROWS];
+  __shared__ double2 scl[GS_CB][GS_ROWS];   // (2^p1, 2^(p - p1)) per chain and row
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, rr = lane & 15, h = lane >> 4;
+  const int r0 = blockIdx.x * GS_ROWS, row = r0 + rr, c0 = blockIdx.y * GS_CB;
+  const int ncb = C - c0 < GS_CB ? C - c0 : GS_CB;
+  const double* Sb = S + (size_t)c0 * qp;
+  constexpr int NW = GS_THREADS / 32, BPW = GS_TK / 32 / NW;   // warps, 32-k blocks per warp and window
+  double x[16];
+
+  // pass 1: row maxima of |A| over k < q
+  double m[GS_CB];
 #pragma unroll
-    for (int g = 0; g < 4; ++g) {
-      const int kw = warp * 4 + g;             // word of the chunk (4 k each)
-      unsigned w[GI_S] = {0, 0, 0, 0, 0, 0, 0};
+  for (int cb = 0; cb < GS_CB; ++cb) m[cb] = 0.0;
+  for (int t0 = 0; t0 < q; t0 += GS_TK) {
+    __syncthreads();
+    gs_roots(sq, Sb, qp, q, ncb, t0);
+    __syncthreads();
 #pragma unroll
-      for (int b = 0; b < 4; ++b) {
-        const int k = k0 + kw * 4 + b;
-        const double sqk = __shfl_sync(0xffffffffu, sq, g * 4 + b);
-        if (k < q) {
-          // balanced digits: with the bias B = 128 (1 + 2^8 + ... + 2^40), byte i of N + B is D^(6-i) + 128 for i < 6
-          // and (N + B) >> 48 is the top digit D^(0)
-          const long long M = __double2ll_rn(X[row + (size_t)np * k] * sqk * sc1 * sc2) + 0x808080808080ll;
-          const unsigned lo = (unsigned)M ^ 0x80808080u, hi = (unsigned)(M >> 32) ^ 0x8080u;
+    for (int i = 0; i < BPW; ++i) {
+      const int kk = 32 * (warp + NW * i) + 16 * h;
+      if (t0 + kk >= q) continue;
+      gs_load_x(x, X, np, q, row, t0 + kk);
 #pragma unroll
-          for (int i = 0; i < 4; ++i) w[GI_S - 1 - i] |= ((lo >> (8 * i)) & 255u) << (8 * b);
+      for (int cb = 0; cb < GS_CB; ++cb) {
+        if (cb >= ncb) break;
 #pragma unroll
-          for (int i = 0; i < 3; ++i) w[2 - i] |= ((hi >> (8 * i)) & 255u) << (8 * b);
+        for (int j = 0; j < 16; j += 2) {
+          const double2 s2 = *reinterpret_cast<const double2*>(&sq[cb][gs_tidx(kk + j)]);
+          m[cb] = fmax(m[cb], fabs(x[j] * s2.x));
+          m[cb] = fmax(m[cb], fabs(x[j + 1] * s2.y));
         }
       }
-#pragma unroll
-      for (int s = 0; s < GI_S; ++s) buf[s][lane][kw] = w[s];
     }
-    __syncthreads();
-    for (int id = threadIdx.x; id < GI_S * 32 * 32; id += 256) {
-      const int s = id >> 10, rr = (id >> 5) & 31, kw = id & 31;
-      const int k = k0 + kw * 4;
-      if (k < qp) *reinterpret_cast<unsigned*>(out + ((size_t)s * np + r0 + rr) * qp + k) = buf[s][rr][kw];
-    }
-    __syncthreads();
   }
+#pragma unroll
+  for (int cb = 0; cb < GS_CB; ++cb) {
+    const double o = __shfl_xor_sync(0xffffffffu, m[cb], 16);
+    if (h == 0) red[warp][cb][rr] = fmax(m[cb], o);
+  }
+  __syncthreads();
+  if (threadIdx.x < GS_CB * GS_ROWS) {
+    const int cb = threadIdx.x / GS_ROWS, i = threadIdx.x % GS_ROWS;
+    double mx = 0.0;
+#pragma unroll
+    for (int w = 0; w < NW; ++w) mx = fmax(mx, red[w][cb][i]);
+    // 2^p m in [2^53 * 126/64, 2^54) or [2^54, 2^54 * 126/64]: the top digit stays within [-127, 127]
+    int p = 0;
+    if (mx > 0.0) {
+      p = 54 - ilogb(mx);
+      if (ldexp(mx, p) > 126.0 * 0x1p48) --p;
+    }
+    if (cb < ncb) rscale[(size_t)(c0 + cb) * np + r0 + i] = ldexp(1.0, -p);
+    const int p1 = p > 1000 ? 1000 : p;
+    scl[cb][i] = make_double2(ldexp(1.0, p1), ldexp(1.0, p - p1));
+  }
+
+  // pass 2: the digits.  With the bias B = 128 (1 + 2^8 + ... + 2^40), byte i of N + B is D^(6-i) + 128 for i < 6 and
+  // byte 6 is the top digit D^(0); (N + B) ^ (128 (1 + ... + 2^40)) holds D^(6-i) in byte i.
+#if defined(GS_LAB_NO_STORES)
+  unsigned sink = 0;
+#endif
+  for (int t0 = 0; t0 < qp; t0 += GS_TK) {
+    __syncthreads();
+    gs_roots(sq, Sb, qp, q, ncb, t0);
+    __syncthreads();
+#pragma unroll 1
+    for (int i = 0; i < BPW; ++i) {
+      const int kk = 32 * (warp + NW * i) + 16 * h;
+      if (t0 + kk >= qp) continue;
+      gs_load_x(x, X, np, q, row, t0 + kk);
+#pragma unroll 1
+      for (int cb = 0; cb < ncb; ++cb) {
+        const double2 sc = scl[cb][rr];
+        uint4 w[GI_S];
+#pragma unroll
+        for (int g = 0; g < 4; ++g) {
+          unsigned lo[4], hi[4];
+#pragma unroll
+          for (int b = 0; b < 4; ++b) {
+            const int j = 4 * g + b;
+#if defined(GS_LAB_NO_DIGITS)
+            lo[b] = __double2loint(x[j]) + j; hi[b] = __double2hiint(x[j]) + cb;
+#else
+            const double sqk = sq[cb][gs_tidx(kk + j)];
+            const unsigned long long M = (unsigned long long)__double2ll_rn(x[j] * sqk * sc.x * sc.y) + 0x808080808080ull;
+            lo[b] = (unsigned)M; hi[b] = (unsigned)(M >> 32);
+#endif
+          }
+          // 4 x 4 byte transpose: word s holds byte (6 - s) of the 4 elements, element b in byte b
+          const unsigned a0 = __byte_perm(lo[0], lo[1], 0x5140), a1 = __byte_perm(lo[0], lo[1], 0x7362);
+          const unsigned a2 = __byte_perm(lo[2], lo[3], 0x5140), a3 = __byte_perm(lo[2], lo[3], 0x7362);
+          const unsigned b0 = __byte_perm(hi[0], hi[1], 0x5140), b1 = __byte_perm(hi[0], hi[1], 0x7362);
+          const unsigned b2 = __byte_perm(hi[2], hi[3], 0x5140), b3 = __byte_perm(hi[2], hi[3], 0x7362);
+          const unsigned v[GI_S] = {__byte_perm(b1, b3, 0x5410), __byte_perm(b0, b2, 0x7632) ^ 0x80808080u,
+                                    __byte_perm(b0, b2, 0x5410) ^ 0x80808080u, __byte_perm(a1, a3, 0x7632) ^ 0x80808080u,
+                                    __byte_perm(a1, a3, 0x5410) ^ 0x80808080u, __byte_perm(a0, a2, 0x7632) ^ 0x80808080u,
+                                    __byte_perm(a0, a2, 0x5410) ^ 0x80808080u};
+#pragma unroll
+          for (int s = 0; s < GI_S; ++s) (&w[s].x)[g] = v[s];
+        }
+        signed char* out = planes + ((size_t)(c0 + cb) * GI_S * np + row) * qp + t0 + kk;
+#pragma unroll
+        for (int s = 0; s < GI_S; ++s) {
+#if defined(GS_LAB_NO_STORES)
+          sink ^= w[s].x ^ w[s].y ^ w[s].z ^ w[s].w;
+#else
+          *reinterpret_cast<uint4*>(out + (size_t)s * np * qp) = w[s];
+#endif
+        }
+      }
+    }
+  }
+#if defined(GS_LAB_NO_STORES)
+  if (sink == 0x9e3779b9u) planes[0] = 1;   // keeps the digit math live
+#endif
 }
 
 __global__ void __launch_bounds__(GI_THREADS, 1)
@@ -2029,9 +2109,15 @@ static void launch_gram_i8_products(const Engine& e, cudaStream_t s) {
                                                                              (d.qp + GI_BK - 1) / GI_BK);
 }
 
-static void launch_gram_i8(const Engine& e, cudaStream_t s) {
+// k_gram_slice: the digit planes and row scales of e's chains
+static void launch_gram_slice(const Engine& e, cudaStream_t s) {
   const Dims& d = e.d;
-  ++g_launches; k_gram_slice<<<dim3(d.np / 32, d.C), 256, 0, s>>>(e.X, e.S, d.np, d.q, d.qp, e.gram_planes, e.gram_rscale);
+  ++g_launches; k_gram_slice<<<dim3(d.np / GS_ROWS, (d.C + GS_CB - 1) / GS_CB), GS_THREADS, 0, s>>>(
+      e.X, e.S, d.np, d.q, d.qp, d.C, e.gram_planes, e.gram_rscale);
+}
+
+static void launch_gram_i8(const Engine& e, cudaStream_t s) {
+  launch_gram_slice(e, s);
   launch_gram_i8_products(e, s);
 }
 

@@ -49,6 +49,7 @@ AUX = dict(tau2_params=0, sigma_inv=1, sigma_chol=2, mu_t=3, log_odds=4, W=5, G=
            theta_params=11, delta_params=12, m_params=13, mu_params=14, lambda_logw=15, lambda_weights=16,
            pi_alpha=17, gig_used=18)
 GAMMA_MODE = dict(auto=0, nform=1, qform=2)
+PRED_MEAN, PRED_PREDICTIVE = 0, 1
 STATUS_BITS = dict(jitter=1, sigma_notpd=2, g_notpd=4, gig_cap=8, inj_exhausted=16, nan=32, psi_notpd=64)
 
 _H = C.c_void_p
@@ -99,6 +100,11 @@ PROTOTYPES = {
     "bnr_ess_stream_finish": (C.c_int, [_H]),
     "bnr_ess_stream_window": (C.c_int, [_H, C.c_int32, C.c_int64, C.c_int64]),
     "bnr_chain_groups": (C.c_int, [_H, C.POINTER(C.c_int32)]),
+    "bnr_set_predictors": (C.c_int, [_H, C.c_int32, _DP, C.c_int64, C.c_int32]),
+    "bnr_get_prediction_trace": (C.c_int, [_H, C.c_int32, C.c_int64, C.c_int64, _DP]),
+    "bnr_export_predictions": (C.c_int, [_H, C.c_int64, C.c_int64, C.c_void_p]),
+    "bnr_prediction_summary": (C.c_int, [C.c_int, C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_int64, _DP, _DP,
+                                         _DP]),
     "bnr_device_copy": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int64]),
     "bnr_fit_default_params": (None, [C.POINTER(FitParams)]),
     "bnr_fit_last_error": (C.c_char_p, []),
@@ -110,6 +116,8 @@ PROTOTYPES = {
     "bnr_fit_state": (C.c_int, [_H, C.c_int32, _DP]),
     "bnr_fit_handle": (C.c_int, [_H, C.c_int32, C.POINTER(_H)]),
     "bnr_fit_free": (C.c_int, [_H]),
+    "bnr_fit_predict": (C.c_int, [C.POINTER(FitParams), _DP, _DP, C.c_int32, _DP, C.c_int32, C.POINTER(_H)]),
+    "bnr_fit_prediction": (C.c_int, [_H, _DP, _DP, _DP]),
     "bnr_fit_plan": (C.c_int, [C.POINTER(FitParams), _DP, C.c_int32, _I64P, C.c_int64, _I64P, C.POINTER(FitInfo)]),
     "bnr_gamma_mode": (C.c_int, [_H, C.POINTER(C.c_int32)]),
     "bnr_launch_count": (C.c_int, [_H, _I64P]),

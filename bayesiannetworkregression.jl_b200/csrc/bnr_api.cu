@@ -607,6 +607,20 @@ static void enqueue_sweep(Engine& e, double* ws, const ForkJoin& fj, cudaStream_
   { NvtxRange r("u, xi"); launch_uxi(e, s); }
   std::swap(e.u, e.u_alt);          // u now holds the new draw (pointer swap is baked per captured sweep)
   { NvtxRange r("gamma + D (GIG)"); run_gamma(e, ws, fj, s, 3, fork_syrk); }
+  // predictions for new networks: X_new gamma depends on gamma only, so it runs on the side stream next to the scalar
+  // conditionals and joins before k_pred_record, which needs the new mu (and tau2)
+  const bool fork_pred = e.pred_m > 0 && fj.side != nullptr;
+  if (e.pred_m > 0) {
+    NvtxRange r("predictions: X_new gamma");
+    if (fork_pred) {
+      cudaEventRecord(fj.fork, s);
+      cudaStreamWaitEvent(fj.side, fj.fork, 0);
+      launch_pred_product(e, fj.side);
+      cudaEventRecord(fj.join, fj.side);
+    } else {
+      launch_pred_product(e, s);
+    }
+  }
   {
     NvtxRange r("theta, Delta, M, mu, Lambda, pi");
     launch_x_times(e, 0, e.gamma, e.xg, ws, s);
@@ -616,6 +630,10 @@ static void enqueue_sweep(Engine& e, double* ws, const ForkJoin& fj, cudaStream_
   NvtxRange r("record");
   launch_record(e, 1, s);
   if (e.ess_ring) launch_ess_stream(e, s);
+  if (e.pred_m > 0) {
+    if (fork_pred) cudaStreamWaitEvent(s, fj.join, 0);
+    launch_pred_record(e, 1, s);
+  }
   launch_advance(e, 1, s);
 }
 
@@ -653,6 +671,10 @@ static Engine group_view(const bnr_handle* h, int c0, int Cg, long long* counter
   v.trace_full_chains = tfc;
   if (v.tr_full) v.tr_full += c * v.trace_rows * v.rowlen_full;
   if (tfc == 0) v.tr_full = nullptr;
+  if (v.pred) {
+    v.pred += c * (size_t)v.pred_rows * v.pred_m;
+    v.pred_ws += c * (size_t)v.pred_splits * v.pred_mp;
+  }
   v.iter = counters; v.trace_row = counters + 1; v.mom_window = mom_window;
   v.inj = nullptr; v.inj_stride = 0;
   memset(&v.aux, 0, sizeof(v.aux));
@@ -695,6 +717,10 @@ extern "C" int bnr_init_state(bnr_handle* h) {
   CK(cudaMemsetAsync(e.status, 0, sizeof(int) * e.d.C, h->stream));
   launch_init(e, h->stream);
   launch_record(e, 0, h->stream);
+  if (e.pred_m > 0) {
+    launch_pred_product(e, h->stream);
+    launch_pred_record(e, 0, h->stream);
+  }
   launch_advance(e, 0, h->stream);
   h->xg_valid = false;
   CK(cudaGetLastError());
@@ -800,18 +826,22 @@ extern "C" int bnr_copy_trace_rows(bnr_handle* h, int64_t dst, int64_t src, int6
   if (!h || dst < 0 || src < 0 || count < 0) return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
   Engine& e = h->e;
-  if (e.trace_rows == 0 || (!e.tr_full && !e.tr_gx)) return BNR_OK;     // this handle records no traces: nothing to move
-  if (dst + count > e.trace_rows || src + count > e.trace_rows) return fail(BNR_EINVAL, "rows out of range");
+  const bool traces = e.trace_rows > 0 && (e.tr_full || e.tr_gx), preds = e.pred_m > 0;
+  if (!traces && !preds) return BNR_OK;     // this handle records no traces and no predictions: nothing to move
+  if (traces && (dst + count > e.trace_rows || src + count > e.trace_rows)) return fail(BNR_EINVAL, "rows out of range");
+  if (preds && (dst + count > e.pred_rows || src + count > e.pred_rows))
+    return fail(BNR_EINVAL, "rows beyond the prediction table");
   if (count == 0 || dst == src) return BNR_OK;
   // rows are contiguous per chain; regions may overlap -> stage through one temporary (stream order keeps the chains apart)
   const bool overlap = !(dst + count <= src || src + count <= dst);
-  const size_t max_row = (size_t)(e.tr_full ? e.rowlen_full : 0) > (size_t)(e.d.V + e.d.q) ? (size_t)e.rowlen_full
-                                                                                           : (size_t)(e.d.V + e.d.q);
+  size_t max_row = (size_t)(e.tr_full ? e.rowlen_full : 0) > (size_t)(e.d.V + e.d.q) ? (size_t)e.rowlen_full
+                                                                                     : (size_t)(e.d.V + e.d.q);
+  if (preds && (size_t)e.pred_m > max_row) max_row = (size_t)e.pred_m;
   Scratch sc(h->p.device, overlap ? (size_t)count * max_row * sizeof(double) : 256);
   if (overlap && !sc.p) return fail(BNR_ENOMEM, "device scratch allocation failed");
-  auto move = [&](double* base, size_t rowlen, int chains) -> int {
+  auto move = [&](double* base, size_t rowlen, int chains, long long table_rows) -> int {
     for (int c = 0; c < chains; ++c) {
-      double* b = base + (size_t)c * e.trace_rows * rowlen;
+      double* b = base + (size_t)c * table_rows * rowlen;
       const size_t bytes = (size_t)count * rowlen * sizeof(double);
       if (!overlap) {
         CK(cudaMemcpyAsync(b + (size_t)dst * rowlen, b + (size_t)src * rowlen, bytes, cudaMemcpyDeviceToDevice, h->stream));
@@ -822,8 +852,9 @@ extern "C" int bnr_copy_trace_rows(bnr_handle* h, int64_t dst, int64_t src, int6
     }
     return 0;
   };
-  if (e.tr_full) { int r = move(e.tr_full, e.rowlen_full, e.trace_full_chains); if (r) return r; }
-  if (e.tr_gx) { int r = move(e.tr_gx, e.d.V + e.d.q, e.trace_gx_chains); if (r) return r; }
+  if (traces && e.tr_full) { int r = move(e.tr_full, e.rowlen_full, e.trace_full_chains, e.trace_rows); if (r) return r; }
+  if (traces && e.tr_gx) { int r = move(e.tr_gx, e.d.V + e.d.q, e.trace_gx_chains, e.trace_rows); if (r) return r; }
+  if (preds) { int r = move(e.pred, e.pred_m, e.d.C, e.pred_rows); if (r) return r; }
   CK(cudaStreamSynchronize(h->stream));
   return BNR_OK;
 }
@@ -1264,6 +1295,10 @@ extern "C" int bnr_finish_sweep(bnr_handle* h) {
   CK(cudaSetDevice(h->p.device));
   launch_record(h->e, 1, h->stream);
   if (h->e.ess_ring) launch_ess_stream(h->e, h->stream);
+  if (h->e.pred_m > 0) {
+    launch_pred_product(h->e, h->stream);
+    launch_pred_record(h->e, 1, h->stream);
+  }
   launch_advance(h->e, 1, h->stream);
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
@@ -1632,5 +1667,109 @@ extern "C" int bnr_profile_sweep(bnr_handle* h, float* ms) {
   for (int i = 0; i < 8; ++i) CK(cudaEventElapsedTime(&ms[i], ev[i], ev[i + 1]));
   for (int i = 0; i < 9; ++i) cudaEventDestroy(ev[i]);
   CK(cudaGetLastError());
+  return BNR_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Predictions for new networks: every recorded row of every chain also gets mu + X_new gamma (+ noise) per new network
+// ---------------------------------------------------------------------------------------------------------
+static void drop_predictors(bnr_handle* h) {
+  Engine& e = h->e;
+  release_alloc(h, const_cast<double*>(e.Xp));
+  release_alloc(h, e.pred);
+  release_alloc(h, e.pred_ws);
+  e.Xp = nullptr; e.pred = nullptr; e.pred_ws = nullptr;
+  e.pred_m = e.pred_mp = e.pred_mode = e.pred_splits = 0;
+  e.pred_rows = 0;
+}
+
+extern "C" int bnr_set_predictors(bnr_handle* h, int32_t m, const double* X_new, int64_t rows, int32_t mode) {
+  if (!h) return fail(BNR_EINVAL, "null handle");
+  if (m < 0) return fail(BNR_EINVAL, "m must be >= 0");
+  if (mode != BNR_PRED_MEAN && mode != BNR_PRED_PREDICTIVE) return fail(BNR_EINVAL, "unknown prediction mode");
+  if (m > 0 && !X_new) return fail(BNR_EINVAL, "null X_new");
+  if (m > 0 && rows < 1) return fail(BNR_EINVAL, "the prediction table needs rows >= 1");
+  CK(cudaSetDevice(h->p.device));
+  CK(cudaStreamSynchronize(h->stream));
+  drop_graph(h);                       // the captured sweeps gain or lose the prediction nodes
+  drop_predictors(h);
+  if (m == 0) return BNR_OK;
+  Engine& e = h->e;
+  const Dims& d = e.d;
+  const int mp = (m + TILE_N - 1) / TILE_N * TILE_N;
+  const int ks = pred_splits(d, mp);
+  double *xp = nullptr, *pred = nullptr, *ws = nullptr;
+  int r = dalloc(h, &xp, (size_t)d.qp * mp);
+  if (!r) r = dalloc(h, &pred, (size_t)d.C * rows * m, false);
+  if (!r) r = dalloc(h, &ws, (size_t)ks * d.C * mp, false);
+  if (r) {
+    cudaGetLastError();                // a refused cudaMalloc must not surface in a later call
+    release_alloc(h, xp); release_alloc(h, pred); release_alloc(h, ws);
+    return fail(r, "prediction buffers (" + std::to_string(8.0 * ((double)d.qp * mp + (double)d.C * rows * m +
+                                                                   (double)ks * d.C * mp)) +
+                       " bytes): " + g_err);
+  }
+  // X_new: m x q column-major host -> columns padded to mp rows (zeros beyond m and beyond q, like X)
+  CK(cudaMemcpy2DAsync(xp, (size_t)mp * sizeof(double), X_new, (size_t)m * sizeof(double), (size_t)m * sizeof(double),
+                       (size_t)d.q, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemsetAsync(pred, 0xff, sizeof(double) * (size_t)d.C * rows * m, h->stream));   // NaN: rows never written
+  CK(cudaStreamSynchronize(h->stream));
+  e.Xp = xp; e.pred = pred; e.pred_ws = ws;
+  e.pred_m = m; e.pred_mp = mp; e.pred_mode = mode; e.pred_splits = ks; e.pred_rows = rows;
+  return BNR_OK;
+}
+
+extern "C" int bnr_get_prediction_trace(bnr_handle* h, int32_t chain, int64_t first, int64_t last, double* out) {
+  if (!h || !out || chain < 0 || chain >= h->e.d.C || first < 0 || last < first) return fail(BNR_EINVAL, "bad arguments");
+  const Engine& e = h->e;
+  if (e.pred_m == 0) return fail(BNR_ESTATE, "no predictors set (bnr_set_predictors)");
+  if (last > e.pred_rows) return fail(BNR_EINVAL, "rows beyond the prediction table");
+  CK(cudaSetDevice(h->p.device));
+  const size_t count = (size_t)(last - first), m = (size_t)e.pred_m;
+  if (count == 0) return BNR_OK;
+  std::vector<double> tmp(count * m);
+  CK(cudaMemcpyAsync(tmp.data(), e.pred + ((size_t)chain * e.pred_rows + first) * m, sizeof(double) * tmp.size(),
+                     cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  for (size_t r = 0; r < count; ++r)
+    for (size_t j = 0; j < m; ++j) out[r + count * j] = tmp[r * m + j];
+  return BNR_OK;
+}
+
+extern "C" int bnr_export_predictions(bnr_handle* h, int64_t first_row, int64_t nrows, double* dev_dst) {
+  if (!h || !dev_dst || first_row < 0 || nrows < 0) return fail(BNR_EINVAL, "bad arguments");
+  const Engine& e = h->e;
+  if (e.pred_m == 0) return fail(BNR_ESTATE, "no predictors set (bnr_set_predictors)");
+  if (first_row + nrows > e.pred_rows) return fail(BNR_EINVAL, "rows beyond the prediction table");
+  CK(cudaSetDevice(h->p.device));
+  if (nrows == 0) return BNR_OK;
+  const size_t rowb = sizeof(double) * (size_t)e.pred_m;
+  CK(cudaMemcpy2DAsync(dev_dst, rowb * nrows, e.pred + (size_t)first_row * e.pred_m, rowb * e.pred_rows, rowb * nrows,
+                       (size_t)e.d.C, cudaMemcpyDeviceToDevice, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  return BNR_OK;
+}
+
+extern "C" int bnr_prediction_summary(int device, const double* dev_rows, int64_t count, int32_t m, int64_t rank_lo,
+                                      int64_t rank_hi, double* mean, double* lo, double* hi) {
+  if (!dev_rows || count < 1 || m < 1) return fail(BNR_EINVAL, "bad arguments (need rows, count >= 1, m >= 1)");
+  if (rank_lo < 1 || rank_hi < 1 || rank_lo > count || rank_hi > count)
+    return fail(BNR_EINVAL, "order-statistic ranks must lie in 1..count");
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+    return fail(BNR_ENODEV, "no CUDA device visible: libbnr has no CPU fallback");
+  if (device < 0 || device >= ndev) return fail(BNR_EINVAL, "device ordinal out of range");
+  CK(cudaSetDevice(device));
+  const size_t outb = sizeof(double) * 3 * (size_t)m;
+  Scratch sc(device, pred_select_ws_bytes(count, m) + outb);
+  if (!sc.p) return fail(BNR_ENOMEM, "device scratch allocation failed");
+  double* o = (double*)sc.p;
+  launch_pred_select(dev_rows, count, m, rank_lo, rank_hi, o, o + m, o + 2 * m, o + 3 * m, 0);
+  std::vector<double> host((size_t)3 * m);
+  CK(cudaMemcpy(host.data(), o, outb, cudaMemcpyDeviceToHost));
+  CK(cudaGetLastError());
+  if (mean) memcpy(mean, host.data(), sizeof(double) * m);
+  if (lo) memcpy(lo, host.data() + m, sizeof(double) * m);
+  if (hi) memcpy(hi, host.data() + 2 * m, sizeof(double) * m);
   return BNR_OK;
 }

@@ -96,6 +96,124 @@ void launch_summary_select(const double* rows, size_t rowlen, int off, int nelem
 }
 
 // ------------------------------------------------------------------------------------------------------------
+// Pooled predictions: mean and two exact order statistics of every column j of rows[N][m] (N = all retained draws of
+// all chains: millions of rows, m ~ 100 columns).  k_summary_select's one-block-per-8-columns grid would leave most SMs
+// idle here, so the rows are split over blocks too: per 8-bit digit pass (MSB first, the order key of k_summary_select)
+//   k_pred_hist : grid (ceil(m / 8), RB), block 256 = 8 columns x 32 row lanes over rows [by * per, (by + 1) * per):
+//                 a shared histogram of the digit among the keys that match the prefix picked so far, added into the
+//                 global [2][m][256] integer histogram (order-free); pass 0 also writes the block's column sums
+//   k_pred_pick : thread per (rank, column): walks the 256 bins, extends the prefix, clears the histogram
+// and k_pred_mean adds the RB block sums of each column in block order.  RB depends on (N, m) only.
+// ------------------------------------------------------------------------------------------------------------
+constexpr int PS_EPB = 8;
+constexpr long long PS_MIN_ROWS = 1024;    // rows per block at least
+
+static int pred_select_row_blocks(long long N, int m) {
+  const long long gx = (m + PS_EPB - 1) / PS_EPB;
+  long long rb = (4 * 148 + gx - 1) / gx;
+  const long long by_rows = (N + PS_MIN_ROWS - 1) / PS_MIN_ROWS;
+  if (rb > by_rows) rb = by_rows;
+  if (rb > 65535) rb = 65535;
+  return rb < 1 ? 1 : (int)rb;
+}
+
+__global__ void __launch_bounds__(256) k_pred_hist(const double* __restrict__ rows, long long N, int m, long long per,
+                                                   int pass, unsigned long long* __restrict__ hist,
+                                                   const unsigned long long* __restrict__ prefix,
+                                                   double* __restrict__ psum) {
+  __shared__ unsigned int h[2][PS_EPB][256];
+  __shared__ double ps[32][PS_EPB];
+  const int tid = threadIdx.x, e = tid % PS_EPB, lane = tid / PS_EPB;
+  const int el = blockIdx.x * PS_EPB + e;
+  const bool live = el < m;
+  const long long r0 = (long long)blockIdx.y * per, r1 = min(N, r0 + per);
+  for (int i = tid; i < 2 * PS_EPB * 256; i += 256) (&h[0][0][0])[i] = 0u;
+  __syncthreads();
+  const int shift = 56 - 8 * pass;
+  const unsigned long long p0 = (pass && live) ? prefix[el] : 0ull, p1 = (pass && live) ? prefix[m + el] : 0ull;
+  double s = 0.0;
+  if (live) {
+    for (long long r = r0 + lane; r < r1; r += 32) {
+      const double x = rows[(size_t)r * m + el];
+      if (pass == 0) s += x;
+      const unsigned long long k = order_key(x);
+      const unsigned long long hi = pass == 0 ? 0ull : (k >> (shift + 8));
+      const int dg = (int)((k >> shift) & 0xffull);
+      if (hi == p0) atomicAdd(&h[0][e][dg], 1u);
+      if (hi == p1) atomicAdd(&h[1][e][dg], 1u);
+    }
+  }
+  __syncthreads();
+  for (int i = tid; i < 2 * PS_EPB * 256; i += 256) {
+    const int t = i / (PS_EPB * 256), ee = (i / 256) % PS_EPB, b = i % 256;
+    const unsigned int v = (&h[0][0][0])[i];
+    const int col = blockIdx.x * PS_EPB + ee;
+    if (v && col < m) atomicAdd(&hist[((size_t)t * m + col) * 256 + b], (unsigned long long)v);
+  }
+  if (pass == 0) {
+    ps[lane][e] = s;
+    __syncthreads();
+    if (tid < PS_EPB && blockIdx.x * PS_EPB + tid < m) {
+      double tot = 0.0;
+      for (int l = 0; l < 32; ++l) tot += ps[l][tid];
+      psum[(size_t)blockIdx.y * m + blockIdx.x * PS_EPB + tid] = tot;
+    }
+  }
+}
+
+__global__ void k_pred_pick(int m, int pass, long long rank_lo, long long rank_hi, unsigned long long* __restrict__ hist,
+                            unsigned long long* __restrict__ prefix, long long* __restrict__ remain) {
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;      // (rank t, column j) = (idx / m, idx % m)
+  if (idx >= 2 * m) return;
+  unsigned long long* hb = hist + (size_t)idx * 256;
+  long long rem = pass == 0 ? (idx < m ? rank_lo : rank_hi) : remain[idx];
+  int b = 0;
+  for (; b < 255; ++b) {
+    const long long cnt = (long long)hb[b];
+    if (rem <= cnt) break;
+    rem -= cnt;
+  }
+  remain[idx] = rem;
+  prefix[idx] = ((pass == 0 ? 0ull : prefix[idx]) << 8) | (unsigned long long)b;
+  for (int i = 0; i < 256; ++i) hb[i] = 0ull;
+}
+
+__global__ void k_pred_mean(int m, int rb, long long N, const double* __restrict__ psum,
+                            const unsigned long long* __restrict__ prefix, double* __restrict__ mean,
+                            double* __restrict__ lo, double* __restrict__ hi) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= m) return;
+  double tot = 0.0;
+  for (int b = 0; b < rb; ++b) tot += psum[(size_t)b * m + j];
+  mean[j] = tot / (double)N;
+  lo[j] = key_to_double(prefix[j]);
+  hi[j] = key_to_double(prefix[m + j]);
+}
+
+// scratch: hist [2][m][256] | prefix [2][m] | remain [2][m] | psum [RB][m]
+size_t pred_select_ws_bytes(long long N, int m) {
+  return sizeof(unsigned long long) * ((size_t)2 * m * 256 + 4 * (size_t)m) +
+         sizeof(double) * (size_t)pred_select_row_blocks(N, m) * m;
+}
+
+void launch_pred_select(const double* rows, long long N, int m, long long rank_lo, long long rank_hi, double* mean,
+                        double* lo, double* hi, void* ws, cudaStream_t s) {
+  const int rb = pred_select_row_blocks(N, m);
+  const long long per = (N + rb - 1) / rb;
+  unsigned long long* hist = (unsigned long long*)ws;
+  unsigned long long* prefix = hist + (size_t)2 * m * 256;
+  long long* remain = (long long*)(prefix + 2 * (size_t)m);
+  double* psum = (double*)(remain + 2 * (size_t)m);
+  cudaMemsetAsync(hist, 0, sizeof(unsigned long long) * (size_t)2 * m * 256, s);
+  const dim3 grid((m + PS_EPB - 1) / PS_EPB, rb);
+  for (int pass = 0; pass < 8; ++pass) {
+    ++g_launches; k_pred_hist<<<grid, 256, 0, s>>>(rows, N, m, per, pass, hist, prefix, psum);
+    ++g_launches; k_pred_pick<<<(2 * m + 127) / 128, 128, 0, s>>>(m, pass, rank_lo, rank_hi, hist, prefix, remain);
+  }
+  ++g_launches; k_pred_mean<<<(m + 127) / 128, 128, 0, s>>>(m, rb, N, psum, prefix, mean, lo, hi);
+}
+
+// ------------------------------------------------------------------------------------------------------------
 // ESS.  tr: [C][trace_rows][P] rows of (xi, gamma); window = rows [first, first + N).
 //   k_chain_mean : cmean[c][p]                       grid = (ceil(P/128), C), block = 128
 //   k_acov_sum   : acov[l][p] = sum_c 1/N sum_t (x_t - m_c)(x_{t+l} - m_c), l = 0 .. L (biased, per-chain centred)

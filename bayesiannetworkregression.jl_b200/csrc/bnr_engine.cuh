@@ -134,6 +134,14 @@ struct Engine {
   double* tr_full;  // [trace_full_chains][rows][rowlen_full]
   double* tr_gx;    // [trace_gx_chains][rows][V+q]  (xi then gamma)
   int rowlen_full;
+  // predictions for new networks (bnr_set_predictors; pred_m == 0: off).  Every recorded row r of chain c gets
+  // pred[c][r][j] = mu_c + X_new[j,:] gamma_c (+ sqrt(tau2_c) z_j in the predictive mode), written at *trace_row
+  const double* Xp;       // [qp][pred_mp] X_new columns padded to pred_mp rows (a multiple of 128; zeros beyond m, q)
+  int pred_m, pred_mp, pred_mode, pred_splits;   // m, padded m, BNR_PRED_*, k-splits of the product X_new gamma
+  long long pred_rows;    // rows of each chain's prediction table
+  double* pred;           // [C][pred_rows][pred_m]
+  double* pred_ws;        // split-K partials of X_new gamma, [pred_splits][C][pred_mp]; a chain group's view uses
+                          // [pred_splits][Cg][pred_mp] at offset c0 * pred_splits * pred_mp
   // injection
   const double* inj;  // [C][inj_stride] or nullptr
   long long inj_stride;

@@ -286,6 +286,11 @@ struct bnr_fit_result {
   Outcome out;
   std::vector<double> rhat_xi, rhat_gamma, s_mean, s_lo, s_hi, s_xi, ess_xi, ess_gamma;
   bool summary_ok = false, ess_ok = false;
+  // predictions for new networks (bnr_fit_predict; pm == 0: none)
+  int pm = 0, pmode = 0;
+  std::vector<double*> pexp;           // per device: the retained rows of its chains, [chain][row][m]
+  std::vector<double> p_mean, p_lo, p_hi;
+  bool pred_ok = false;
   int gamma_mode = 0;
   int status_or = 0;
   const char* exchange = "none";
@@ -293,6 +298,7 @@ struct bnr_fit_result {
     for (size_t d = 0; d < h.size(); ++d) {
       if (d < dev.size()) cudaSetDevice(dev[d]);
       if (d < gbuf.size() && gbuf[d]) cudaFree(gbuf[d]);
+      if (d < pexp.size() && pexp[d]) cudaFree(pexp[d]);
       if (d < xs.size() && xs[d]) cudaStreamDestroy(xs[d]);
     }
     if (xbuf) { cudaSetDevice(dev[0]); cudaFree(xbuf); }
@@ -319,8 +325,10 @@ enum { PH_CREATE = 0, PH_INIT, PH_RUN, PH_COPY, PH_PSRF, PH_SUMMARY, PH_ESS, PH_
 struct DeviceOps : Ops {
   bnr_fit_result& R;
   const double* X; const double* y;
+  const double* X_new;
   PhaseClock clk;
-  explicit DeviceOps(bnr_fit_result& r, const double* X_, const double* y_) : R(r), X(X_), y(y_) {}
+  explicit DeviceOps(bnr_fit_result& r, const double* X_, const double* y_, const double* X_new_)
+      : R(r), X(X_), y(y_), X_new(X_new_) {}
   int total_chains() const { return R.C * (int)R.h.size() * (R.p.ext_world > 1 ? R.p.ext_world : 1); }
 
   int create(long long rows, bool gx_all, int full) override {
@@ -363,6 +371,68 @@ struct DeviceOps : Ops {
         R.exchange = "peer-copy";
       }
     }
+    if (R.pm > 0) return create_predictions(rows);
+    return 0;
+  }
+
+  // prediction tables of `rows` rows on every handle, the export buffers and the pooled buffers of the all-gather,
+  // all before the first sweep: a fit that cannot hold its predictions fails here, not after the sampling
+  int create_predictions(long long rows) {
+    const int nd = (int)R.h.size(), world = R.p.ext_world > 1 ? R.p.ext_world : 1;
+    for (auto* h : R.h) BN(bnr_set_predictors(h, R.pm, X_new, rows, R.pmode));
+    const size_t local = (size_t)R.C * rows * R.pm;
+    auto refuse = [&](const char* what, size_t doubles) {
+      cudaGetLastError();
+      return ffail(BNR_ENOMEM, std::string("cannot allocate the ") + what + " of the predictions (" +
+                                   std::to_string(doubles * sizeof(double)) + " bytes)");
+    };
+    R.pexp.assign(nd, nullptr);
+    for (int d = 0; d < nd; ++d) {
+      CKF(cudaSetDevice(R.dev[d]));
+      if (cudaMalloc((void**)&R.pexp[d], local * sizeof(double)) != cudaSuccess) { R.pexp[d] = nullptr; return refuse("export buffer", local); }
+    }
+    if (nd > 1 || world > 1) {
+      // gather_local / gather_ext reuse these buffers (they only grow)
+      for (int d = 0; d < nd; ++d) {
+        CKF(cudaSetDevice(R.dev[d]));
+        if (R.gbuf[d]) CKF(cudaFree(R.gbuf[d]));
+        R.gbuf[d] = nullptr;
+        if (cudaMalloc((void**)&R.gbuf[d], local * nd * sizeof(double)) != cudaSuccess) {
+          R.gbuf[d] = nullptr; R.gbuf_doubles = 0;
+          return refuse("pooled buffer", local * nd);
+        }
+      }
+      R.gbuf_doubles = local * nd;
+      if (world > 1) {
+        CKF(cudaSetDevice(R.dev[0]));
+        if (cudaMalloc((void**)&R.xbuf, local * nd * world * sizeof(double)) != cudaSuccess) {
+          R.xbuf = nullptr;
+          return refuse("pooled buffer", local * nd * world);
+        }
+        R.xbuf_doubles = local * nd * world;
+      }
+    }
+    return 0;
+  }
+
+  // the retained rows of every chain in global-chain order on device 0, then their pooled mean and order statistics
+  int predictions(const Outcome& o) {
+    const long long N = (long long)total_chains() * o.sampled;
+    const double lower = (100 - (R.p.interval > 0 ? R.p.interval : 95)) / 200.0;
+    const long long lw = jround(N * lower), hi = jround(N * (1.0 - lower));
+    if (o.sampled < 1 || lw < 1 || hi > N) return 0;
+    const int nd = (int)R.h.size();
+    for (int d = 0; d < nd; ++d) BN(bnr_export_predictions(R.h[d], o.burn_in, o.sampled, R.pexp[d]));
+    const size_t cnt = (size_t)R.C * o.sampled * R.pm;
+    const double* all = R.pexp[0];
+    if (nd > 1 || R.p.ext_world > 1) {
+      std::vector<const double*> src(R.pexp.begin(), R.pexp.end());
+      if (int r = gather_local(src, cnt)) return r;
+      if (int r = gather_ext(cnt * nd, &all)) return r;
+    }
+    R.p_mean.assign(R.pm, 0); R.p_lo.assign(R.pm, 0); R.p_hi.assign(R.pm, 0);
+    BN(bnr_prediction_summary(R.dev[0], all, N, R.pm, lw, hi, R.p_mean.data(), R.p_lo.data(), R.p_hi.data()));
+    R.pred_ok = true;
     return 0;
   }
   int init() override { PhaseClock::Scope sc(clk, PH_INIT); for (auto* h : R.h) BN(bnr_init_state(h)); return 0; }
@@ -567,7 +637,9 @@ extern "C" int bnr_fit_plan(const bnr_fit_params* p, const double* psrf_max, int
   return BNR_OK;
 }
 
-extern "C" int bnr_fit(const bnr_fit_params* p, const double* X, const double* y, bnr_fit_result** res_out) {
+// bnr_fit and bnr_fit_predict (m > 0: predictions for the m rows of X_new)
+static int fit_body(const bnr_fit_params* p, const double* X, const double* y, int32_t m, const double* X_new,
+                    int32_t mode, bnr_fit_result** res_out) {
   if (int r = check_params(p)) return r;
   if (!X || !y || !res_out) return ffail(BNR_EINVAL, "null argument");
   if (p->base.nu < p->base.R)
@@ -576,7 +648,8 @@ extern "C" int bnr_fit(const bnr_fit_params* p, const double* X, const double* y
     return ffail(BNR_EINVAL, "nu must not be smaller than R");
   bnr_fit_result* R = new bnr_fit_result();
   R->p = *p;
-  DeviceOps o(*R, X, y);
+  R->pm = m; R->pmode = mode;
+  DeviceOps o(*R, X, y, X_new);
   const double t_start = PhaseClock::now();
   int rc = fit_loops(o, *p, R->out);
   if (!rc) {
@@ -592,6 +665,7 @@ extern "C" int bnr_fit(const bnr_fit_params* p, const double* X, const double* y
       else rc = ffail(BNR_ECUDA, std::string("bnr_summary: ") + bnr_last_error());
     }
   }
+  if (!rc && m > 0) rc = o.predictions(R->out);
   if (!rc) rc = o.ess(R->out);
   if (!rc) {
     std::vector<int32_t> st(R->C);
@@ -611,6 +685,29 @@ extern "C" int bnr_fit(const bnr_fit_params* p, const double* X, const double* y
     return rc;
   }
   *res_out = R;
+  return BNR_OK;
+}
+
+extern "C" int bnr_fit(const bnr_fit_params* p, const double* X, const double* y, bnr_fit_result** res_out) {
+  return fit_body(p, X, y, 0, nullptr, BNR_PRED_MEAN, res_out);
+}
+
+extern "C" int bnr_fit_predict(const bnr_fit_params* p, const double* X, const double* y, int32_t m,
+                               const double* X_new, int32_t mode, bnr_fit_result** res_out) {
+  if (m < 0) return ffail(BNR_EINVAL, "m must be >= 0");
+  if (m > 0 && !X_new) return ffail(BNR_EINVAL, "null X_new");
+  if (mode != BNR_PRED_MEAN && mode != BNR_PRED_PREDICTIVE) return ffail(BNR_EINVAL, "unknown prediction mode");
+  return fit_body(p, X, y, m, X_new, mode, res_out);
+}
+
+extern "C" int bnr_fit_prediction(const bnr_fit_result* r, double* mean, double* lo, double* hi) {
+  if (!r) return ffail(BNR_EINVAL, "null result");
+  if (!r->pred_ok)
+    return ffail(BNR_ESTATE, r->pm > 0 ? "too few retained draws for the prediction interval"
+                                       : "the fit was run without X_new (bnr_fit_predict)");
+  if (mean) memcpy(mean, r->p_mean.data(), sizeof(double) * r->pm);
+  if (lo) memcpy(lo, r->p_lo.data(), sizeof(double) * r->pm);
+  if (hi) memcpy(hi, r->p_hi.data(), sizeof(double) * r->pm);
   return BNR_OK;
 }
 

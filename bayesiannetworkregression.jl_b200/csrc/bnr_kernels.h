@@ -40,7 +40,16 @@ void launch_rng_dump(const Dims& d, int chain, long long iteration, int site, in
 // out[c][m] = sum_k A(m,k) v[c][k];  trans=0: A = X (np x qp), out = e.xv-like [C][np], in [C][qp]
 //                                     trans=1: A = X' (qp x np), out [C][qp], in [C][np]
 void launch_x_times(const Engine& e, int trans, const double* in, double* out, double* splitk_ws, cudaStream_t s);
+// the same product with any operand A (lda >= M, K = qp for trans 0); out == nullptr leaves the k-split partial products
+// [splits][d.C][M] in splitk_ws without adding them (a single split included)
+void launch_x_times(const Dims& d, int trans, const double* A, int lda, int M, int K, const double* in, double* out,
+                    double* splitk_ws, cudaStream_t s);
 size_t x_times_workspace_doubles(const Dims& d);
+// predictions: partials of X_new gamma for every chain of the view into e.pred_ws (k_xmma<0>, pred_splits(d, mp) splits)
+int pred_splits(const Dims& d, int mp);
+void launch_pred_product(const Engine& e, cudaStream_t s);
+// adds the partials in split order, mu_c and (predictive mode) sqrt(tau2_c) z_j, and stores the row at *e.trace_row
+void launch_pred_record(const Engine& e, int sweep_done, cudaStream_t s);
 void launch_syrk_G(const Engine& e, cudaStream_t s);         // G_c = X diag(S_c) X' + I (lower tiles)
 int syrk_splits(const Dims& d, int C);                        // k-splits launch_syrk_G uses for a batch of C chains
 // launch_syrk_G computes the n-form Gram matrix on the INT8 tensor cores (Ozaki digit planes) for qp in
@@ -86,6 +95,11 @@ void launch_acov_sum(const double* tr, long long trace_rows, int P, int C, long 
 // launch_acov_sum / launch_chain_mean produce (acov [L+1][P] summed over the local chains, chain means [C][P])
 void launch_ess_stream(const Engine& e, cudaStream_t s);
 void launch_ess_stream_finalize(const Engine& e, long long N, double* acov, double* cmean, cudaStream_t s);
+// pooled predictions: mean and the exact order statistics (1-based ranks) of each of the m columns of rows[N][m];
+// ws: pred_select_ws_bytes(N, m) bytes of device scratch
+size_t pred_select_ws_bytes(long long N, int m);
+void launch_pred_select(const double* rows, long long N, int m, long long rank_lo, long long rank_hi, double* mean,
+                        double* lo, double* hi, void* ws, cudaStream_t s);
 void launch_ess_finish(const double* acov_parts, int nparts, const double* cmeans, int chains, int P, long long N,
                        int L, double* ess, double* lag_used, cudaStream_t s);
 

@@ -1611,11 +1611,11 @@ __global__ void k_splitk_reduce(const double* __restrict__ ws, double* __restric
   out[i] = s;
 }
 
-// k-splits of X v, X' a4 and X gamma.  The split count sets the summation order, so it depends on the handle's chain
-// count only: a chain group (a view with d.C < d.C_total) and an eager sweep over the whole handle add in the same order.
-static int x_times_splits(const Dims& d, int trans) {
-  const int M = trans ? d.qp : d.np, K = trans ? d.np : d.qp;
-  const int tiles = ((M + XM_BM - 1) / XM_BM) * ((d.C_total + XM_BN - 1) / XM_BN);
+// k-splits of X v, X' a4, X gamma and X_new gamma (M x K operand).  The split count sets the summation order, so it
+// depends on the handle's chain count only: a chain group (a view with d.C < d.C_total) and an eager sweep over the whole
+// handle add in the same order.
+static int x_times_splits(int M, int K, int C_total) {
+  const int tiles = ((M + XM_BM - 1) / XM_BM) * ((C_total + XM_BN - 1) / XM_BN);
   int ks = (2 * 148 + tiles - 1) / tiles;
   const int kmax = K / (4 * XM_BK) > 0 ? K / (4 * XM_BK) : 1;
   if (ks > kmax) ks = kmax;
@@ -1627,26 +1627,36 @@ static int x_times_splits(const Dims& d, int trans) {
 // Every workspace (the handle's and each chain group's) holds splits x chains x rows partial sums for the handle's whole
 // chain count.  A launch uses splits x d.C x rows with the same splits and d.C <= d.C_total, so it always fits.
 size_t x_times_workspace_doubles(const Dims& d) {
-  const int a = x_times_splits(d, 0), b = x_times_splits(d, 1);
+  const int a = x_times_splits(d.np, d.qp, d.C_total), b = x_times_splits(d.qp, d.np, d.C_total);
   const size_t wa = (size_t)a * d.C_total * d.np, wb = (size_t)b * d.C_total * d.qp;
   return wa > wb ? wa : wb;
 }
 
-void launch_x_times(const Engine& e, int trans, const double* in, double* out, double* ws, cudaStream_t s) {
-  const Dims& d = e.d;
-  const int M = trans ? d.qp : d.np, K = trans ? d.np : d.qp, N = d.C;
-  const int ldin = trans ? d.np : d.qp, ldout = trans ? d.qp : d.np;
-  const int ks = x_times_splits(d, trans);
+int pred_splits(const Dims& d, int mp) { return x_times_splits(mp, d.qp, d.C_total); }
+
+void launch_x_times(const Dims& d, int trans, const double* A, int lda, int M, int K, const double* in, double* out,
+                    double* ws, cudaStream_t s) {
+  const int N = d.C, ldin = K, ldout = M;
+  const int ks = x_times_splits(M, K, d.C_total);
   const int kper = ((K + ks - 1) / ks + XM_BK - 1) / XM_BK * XM_BK;
   dim3 grid((M + XM_BM - 1) / XM_BM, (N + XM_BN - 1) / XM_BN, ks);
-  double* dst = ks == 1 ? out : ws;
+  double* dst = (ks == 1 && out) ? out : ws;
   ++g_launches;
-  if (trans) k_xmma<1><<<grid, 256, XMMA_SMEM, s>>>(e.X, d.np, M, K, N, in, ldin, dst, ldout, kper);
-  else k_xmma<0><<<grid, 256, XMMA_SMEM, s>>>(e.X, d.np, M, K, N, in, ldin, dst, ldout, kper);
-  if (ks > 1) {
+  if (trans) k_xmma<1><<<grid, 256, XMMA_SMEM, s>>>(A, lda, M, K, N, in, ldin, dst, ldout, kper);
+  else k_xmma<0><<<grid, 256, XMMA_SMEM, s>>>(A, lda, M, K, N, in, ldin, dst, ldout, kper);
+  if (ks > 1 && out) {
     const size_t count = (size_t)N * ldout;
     ++g_launches; k_splitk_reduce<<<(unsigned)((count + 255) / 256), 256, 0, s>>>(ws, out, count, ks);
   }
+}
+
+void launch_x_times(const Engine& e, int trans, const double* in, double* out, double* ws, cudaStream_t s) {
+  const Dims& d = e.d;
+  launch_x_times(d, trans, e.X, d.np, trans ? d.qp : d.np, trans ? d.np : d.qp, in, out, ws, s);
+}
+
+void launch_pred_product(const Engine& e, cudaStream_t s) {
+  launch_x_times(e.d, 0, e.Xp, e.pred_mp, e.pred_mp, e.d.qp, e.gamma, nullptr, e.pred_ws, s);
 }
 
 __global__ void k_gram_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,

@@ -13,6 +13,7 @@ namespace bnr {
 enum Site : uint32_t {
   SITE_TAU2 = 1, SITE_UXI = 2, SITE_GAMMA_Z1 = 3, SITE_GAMMA_Z2 = 4, SITE_S = 5, SITE_THETA = 6,
   SITE_DELTA = 7, SITE_M = 8, SITE_MU = 9, SITE_LAMBDA = 10, SITE_PI = 11,
+  SITE_PRED = 12,   // predictive noise of the predictions for new networks (k_pred_record); not an injected site
   SITE_INIT_S = 20, SITE_INIT_PI = 21, SITE_INIT_LAMBDA = 22, SITE_INIT_XI = 23, SITE_INIT_M = 24,
   SITE_INIT_U = 25, SITE_INIT_GAMMA = 26
 };

@@ -809,6 +809,25 @@ __global__ void __launch_bounds__(256) k_record(Engine e, int sweep_done /* 1: s
   }
 }
 
+// one prediction row per chain: pred[c][row][j] = mu_c + sum_z partial_z[c][j] (z in split order) (+ sqrt(tau2_c) z_j,
+// z_j from the SITE_PRED stream of element j at the row's sweep).  grid = (ceil(m / 256), C)
+__global__ void __launch_bounds__(256) k_pred_record(Engine e, int sweep_done /* 1: state belongs to sweep iter+1 */) {
+  const int c = blockIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x;
+  const long long row = *e.trace_row;
+  if (j >= e.pred_m || row >= e.pred_rows) return;
+  const size_t stride = (size_t)e.d.C * e.pred_mp;
+  const double* w = e.pred_ws + (size_t)c * e.pred_mp + j;
+  double s = 0.0;
+  for (int z = 0; z < e.pred_splits; ++z) s += w[z * stride];
+  double v = e.mu[c] + s;
+  if (e.pred_mode == 1) {
+    const long long sweep = *e.iter + (sweep_done ? 1 : 0);
+    DrawStream st(chain_key(e.d, c), (uint32_t)sweep, SITE_PRED, (uint32_t)j);
+    v += sqrt(e.tau2[c]) * st.normal();
+  }
+  e.pred[((size_t)c * e.pred_rows + row) * e.pred_m + j] = v;
+}
+
 __global__ void k_advance(Engine e, int inc_iter) {
   if (threadIdx.x == 0 && blockIdx.x == 0) {
     if (inc_iter) *e.iter += 1;
@@ -906,6 +925,10 @@ void launch_init(const Engine& e, cudaStream_t s) {
 void launch_record(const Engine& e, int sweep_done, cudaStream_t s) {
   dim3 grid((e.d.V + e.d.q + 255) / 256, e.d.C);
   ++g_launches; k_record<<<grid, 256, 0, s>>>(e, sweep_done);
+}
+void launch_pred_record(const Engine& e, int sweep_done, cudaStream_t s) {
+  dim3 grid((e.pred_m + 255) / 256, e.d.C);
+  ++g_launches; k_pred_record<<<grid, 256, 0, s>>>(e, sweep_done);
 }
 void launch_advance(const Engine& e, int inc_iter, cudaStream_t s) { k_advance<<<1, 32, 0, s>>>(e, inc_iter); }
 void launch_rhat(const double* mom, int chains, int nparams, long long h, double* out, cudaStream_t s) {

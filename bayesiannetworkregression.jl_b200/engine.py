@@ -3,7 +3,7 @@ import ctypes as C
 
 import numpy as np
 
-from .capi import lib, check, Params, VAR, COND, AUX, GAMMA_MODE
+from .capi import lib, check, Params, VAR, COND, AUX, GAMMA_MODE, PRED_MEAN, PRED_PREDICTIVE
 
 _DP = C.POINTER(C.c_double)
 
@@ -43,6 +43,7 @@ class Engine:
         p.chain_groups = int(chain_groups)
         p.trace_gamma_xi_chains = int(trace_gamma_xi_chains)
         self.params = p
+        self.pred_m = 0
         self.device = int(device)
         self.trace_rows = int(trace_rows)
         Xf = np.asfortranarray(X)
@@ -223,6 +224,41 @@ class Engine:
         ms = (C.c_float * 8)()
         check(self._L.bnr_profile_sweep(self._h, ms))
         return dict(zip(self.PHASES, [float(x) for x in ms]))
+
+    # -- predictions for new networks ------------------------------------------------------------------
+    def set_predictors(self, X_new, rows=0, predictive=False):
+        """Record mu + X_new gamma (+ sqrt(tau2) z with predictive=True) for the m rows of X_new (m x q, laid out like
+        X) at every recorded row of every chain, in a table of `rows` (>= 1) rows per chain.  X_new=None switches it
+        off (rows is then not needed)."""
+        if X_new is None:
+            check(self._L.bnr_set_predictors(self._h, 0, None, 0, PRED_MEAN))
+            self.pred_m = 0
+            return
+        Xn = np.asfortranarray(X_new, dtype=np.float64)
+        if Xn.ndim != 2 or Xn.shape[1] != self.q:
+            raise ValueError("X_new must be m x q with q = %d" % self.q)
+        check(self._L.bnr_set_predictors(self._h, Xn.shape[0], _dp(Xn), int(rows),
+                                         PRED_PREDICTIVE if predictive else PRED_MEAN))
+        self.pred_m = Xn.shape[0]
+
+    def prediction_trace(self, chain, first, last):
+        """Rows [first, last) of one chain's prediction table as an array of shape (last - first, m)."""
+        rows = int(last) - int(first)
+        out = np.empty(rows * self.pred_m)
+        check(self._L.bnr_get_prediction_trace(self._h, int(chain), int(first), int(last), _dp(out)))
+        return out.reshape((rows, self.pred_m), order="F")
+
+    def export_predictions(self, first_row, nrows, dev_ptr):
+        """Rows [first_row, first_row + nrows) of every chain into device memory at dev_ptr as [chain][row][m]."""
+        check(self._L.bnr_export_predictions(self._h, int(first_row), int(nrows), C.c_void_p(dev_ptr)))
+
+    def prediction_summary(self, dev_ptr, count, m, rank_lo, rank_hi):
+        """(mean, sort[rank_lo], sort[rank_hi]) of each of the m columns of `count` rows at a device pointer; ranks are
+        1-based."""
+        mean, lo, hi = np.empty(m), np.empty(m), np.empty(m)
+        check(self._L.bnr_prediction_summary(self.device, C.c_void_p(dev_ptr), int(count), int(m), int(rank_lo),
+                                             int(rank_hi), _dp(mean), _dp(lo), _dp(hi)))
+        return mean, lo, hi
 
     # -- state / traces in reference layout ------------------------------------------------------------
     def var_shape(self, var):

@@ -12,7 +12,8 @@ import random
 
 import numpy as np
 
-from .capi import lib, check, check_fit, FitParams, FitInfo, ALLGATHER_FN, STATE, VAR, GAMMA_MODE
+from .capi import lib, check, check_fit, FitParams, FitInfo, ALLGATHER_FN, STATE, VAR, GAMMA_MODE, PRED_MEAN, \
+    PRED_PREDICTIVE
 
 _DP = C.POINTER(C.c_double)
 
@@ -84,6 +85,31 @@ class BNRSummary:
                                                                 e["lower_bound"][i], e["upper_bound"][i]))
         lines.append("Node Probabilities")
         lines.extend(" %4d  %.3f" % (i + 1, p) for i, p in enumerate(self.prob_nodes["probability"]))
+        return "\n".join(lines)
+
+
+class BNRPrediction:
+    """Predict's table: per new network (1-based `sample`) the posterior mean of the prediction and the order-statistic
+    bounds of its interval (a dict of columns, like BNRSummary.edge_coef)."""
+
+    def __init__(self, table, ci_level, predictive):
+        self.table = table
+        self.ci_level = ci_level
+        self.predictive = predictive
+
+    def __repr__(self):
+        t = self.table
+        kind = "posterior predictive" if self.predictive else "credible"
+        lines = ["", "Predicted Responses (%d%% %s intervals)" % (self.ci_level, kind),
+                 " sample  estimate  lower_bound  upper_bound"]
+        n = len(t["sample"])
+        show = list(range(n)) if n <= 20 else list(range(10)) + [None] + list(range(n - 10, n))
+        for i in show:
+            if i is None:
+                lines.append("   ...")
+            else:
+                lines.append(" %6d  %8.3f  %11.3f  %11.3f" % (t["sample"][i], t["estimate"][i], t["lower_bound"][i],
+                                                             t["upper_bound"][i]))
         return "\n".join(lines)
 
 
@@ -171,8 +197,10 @@ _ALLGATHER = ALLGATHER_FN(_torch_allgather)
 
 def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsamp=0, mingen=0, maxgen=0,
                 psrf_cutoff=1.01, purge_burn=None, num_chains=2, seed=0, device=0, return_state="full", verbose=False,
-                chain_offset=0, n_devices=1, ess_max_lag=0, interval=95, gamma_mode="auto", chain_groups=0):
-    """One bnr_fit call (include/bnr.h): chain generation, purge ring, PSRF loop, R-hat, Summary statistics on the GPU."""
+                chain_offset=0, n_devices=1, ess_max_lag=0, interval=95, gamma_mode="auto", chain_groups=0, X_new=None,
+                predictive=False):
+    """One bnr_fit call (include/bnr.h): chain generation, purge ring, PSRF loop, R-hat, Summary statistics on the GPU.
+    With X_new (m x q, already vectorised) the call is bnr_fit_predict, which also pools the predictions."""
     L = lib()
     Xf = np.asfortranarray(Xn, dtype=np.float64)
     y = np.ascontiguousarray(y, dtype=np.float64)
@@ -197,7 +225,15 @@ def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsa
     if world > 1:
         p.ext_world, p.ext_rank, p.allgather = world, rank, _ALLGATHER
     res = C.c_void_p()
-    check_fit(L.bnr_fit(C.byref(p), Xf.ctypes.data_as(_DP), y.ctypes.data_as(_DP), C.byref(res)))
+    if X_new is None:
+        check_fit(L.bnr_fit(C.byref(p), Xf.ctypes.data_as(_DP), y.ctypes.data_as(_DP), C.byref(res)))
+    else:
+        Xp = np.asfortranarray(X_new, dtype=np.float64)
+        if Xp.ndim != 2 or Xp.shape[1] != q:
+            raise ValueError("X_new must hold networks like X (%d edge columns after setup_X)" % q)
+        check_fit(L.bnr_fit_predict(C.byref(p), Xf.ctypes.data_as(_DP), y.ctypes.data_as(_DP), Xp.shape[0],
+                                    Xp.ctypes.data_as(_DP), PRED_PREDICTIVE if predictive else PRED_MEAN,
+                                    C.byref(res)))
     try:
         info = FitInfo()
         check_fit(L.bnr_fit_get_info(res, C.byref(info)))
@@ -213,6 +249,17 @@ def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsa
             ex, eg = np.empty(V), np.empty(q)
             check_fit(L.bnr_fit_ess(res, ex.ctypes.data_as(_DP), eg.ctypes.data_as(_DP)))
             ess = dict(xi=ex, gamma=eg, max_lag=ess_max_lag)
+        prediction = None
+        if X_new is not None:
+            m = Xp.shape[0]
+            pm, pl, ph = np.empty(m), np.empty(m), np.empty(m)
+            rc = L.bnr_fit_prediction(res, *(a.ctypes.data_as(_DP) for a in (pm, pl, ph)))
+            if rc == -4:                      # BNR_ESTATE: too few pooled draws for the interval's ranks
+                pm = pl = ph = None
+            else:
+                check_fit(rc)
+            prediction = dict(interval=interval, mean=pm, lower=pl, upper=ph, predictive=bool(predictive), m=m,
+                              draws=int(info.total_chains) * int(info.sampled))
         st = Table()
         rows = int(info.rows)
         shapes = {"tau2": (1, 1), "u": (R, V), "xi": (V, 1), "gamma": (q, 1), "S": (q, 1), "theta": (1, 1),
@@ -235,6 +282,8 @@ def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsa
                      rhat_streamed=bool(info.streamed), n_psrf=int(info.n_psrf), total_chains=int(info.total_chains),
                      n_devices=int(info.n_devices), exchange={0: "none", 1: "nccl", 2: "peer-copy"}[int(info.exchange)],
                      ess=ess)
+        if prediction is not None:
+            extra["prediction"] = prediction
         return Results(st, rx, rg, int(info.burn_in), int(info.sampled), extra)
     finally:
         L.bnr_fit_free(res)
@@ -244,14 +293,17 @@ def Fit(X, y, R, *, η=None, V=30, ζ=None, ι=None, aΔ=None, bΔ=None, ν=None
         mingen=0, maxgen=0, psrf_cutoff=1.01, x_transform=True, suppress_timer=False, num_chains=2, seed=None,
         purge_burn=None, filename="parameters.log", eta=None, zeta=None, iota=None, a_delta=None, b_delta=None,
         nu=None, device=0, return_state="full", verbose=False, chain_offset=0, n_devices=1, ess_max_lag=0,
-        gamma_mode="auto", chain_groups=0):
+        gamma_mode="auto", chain_groups=0, X_new=None, predictive=False):
     """Drop-in for `Fit!(X, y, R; ...)` (src/gibbs.jl:725-751).  Greek keyword names are accepted as in the
     reference; ASCII aliases (eta, zeta, iota, a_delta, b_delta, nu) are equivalent.  Engine-only keywords: device,
     n_devices (GPUs of this process to shard the chains over; num_chains is the count PER GPU), return_state
     ("full" | "gamma_xi" | "none": how much of chain 1's table is copied back), ess_max_lag (> 0: gamma / xi ESS of the
     retained draws in res.extra["ess"]), chain_offset (global id of the first chain), gamma_mode, chain_groups.
     Inside a torch.distributed job every rank calls Fit with its own share of the chains; the R-hat tables then cover
-    the chains of all ranks."""
+    the chains of all ranks.
+    X_new (new networks, in the form of X; vectorised by setup_X with the same x_transform): every chain also records
+    mu + X_new gamma at every sweep (plus sqrt(tau2) N(0,1) noise with predictive=True, the posterior predictive), and
+    the retained draws of all chains are pooled on the GPU into res.extra["prediction"] (see Predict)."""
     def pick(greek, ascii_, default):
         return default if (greek is None and ascii_ is None) else (greek if greek is not None else ascii_)
 
@@ -282,10 +334,14 @@ def Fit(X, y, R, *, η=None, V=30, ζ=None, ι=None, aΔ=None, bΔ=None, ν=None
               psrf_cutoff=psrf_cutoff, x_transform=x_transform, num_chains=num_chains, seed=seed,
               purge_burn=purge_burn, device=device, return_state=return_state, verbose=verbose,
               chain_offset=chain_offset, n_devices=n_devices, ess_max_lag=ess_max_lag, gamma_mode=gamma_mode,
-              chain_groups=chain_groups)
+              chain_groups=chain_groups, X_new=X_new, predictive=predictive)
     if mingen > 0 and maxgen > 0:
         return generate_samples_dbl(X, y, R, mingen=mingen, maxgen=maxgen, **kw)
     return generate_samples(X, y, R, nburn=nburn, nsamp=nsamples, **kw)
+
+
+def _prepare_new(X_new, x_transform):
+    return None if X_new is None else setup_X(X_new, x_transform)
 
 
 def _prepare(X, y, R, nu, x_transform):
@@ -305,6 +361,7 @@ def generate_samples(X, y, R, *, eta=1.01, zeta=1.0, iota=1.0, a_delta=1.0, b_de
     """The "traditional" scheme (generate_samples!, src/gibbs.jl:897-1020; maxburn = nburn + nsamp as Fit! passes it):
     the control loop runs inside libbnr (bnr_fit)."""
     Xn, y = _prepare(X, y, R, nu, x_transform)
+    kw["X_new"] = _prepare_new(kw.get("X_new"), x_transform)
     seed = random.randint(1, 55555) if seed is None else seed
     return _native_fit(Xn, y, R, eta=eta, zeta=zeta, iota=iota, a_delta=a_delta, b_delta=b_delta, nu=nu, nburn=nburn,
                        nsamp=nsamp, psrf_cutoff=psrf_cutoff, purge_burn=purge_burn, num_chains=num_chains, seed=seed, **kw)
@@ -315,6 +372,7 @@ def generate_samples_dbl(X, y, R, *, eta=1.01, zeta=1.0, iota=1.0, a_delta=1.0, 
                          purge_burn=None, **kw):
     """The "doubling generation" scheme (generate_samples_dbl!, src/gibbs.jl:1051-1198), inside libbnr (bnr_fit)."""
     Xn, y = _prepare(X, y, R, nu, x_transform)
+    kw["X_new"] = _prepare_new(kw.get("X_new"), x_transform)
     seed = random.randint(1, 55555) if seed is None else seed
     return _native_fit(Xn, y, R, eta=eta, zeta=zeta, iota=iota, a_delta=a_delta, b_delta=b_delta, nu=nu, mingen=mingen,
                        maxgen=maxgen, psrf_cutoff=psrf_cutoff, purge_burn=purge_burn, num_chains=num_chains, seed=seed,
@@ -355,3 +413,22 @@ def Summary(results, interval=95, digits=3):
                 lower_bound=np.round(lo, digits), upper_bound=np.round(up, digits))
     nodes = dict(probability=np.round(xm, digits))
     return BNRSummary(edge, nodes, interval)
+
+
+def Predict(results, interval=95, digits=3):
+    """Predicted responses for the networks passed to Fit as X_new: per network the posterior mean of the prediction
+    and the exact order statistics lw, hi of the draws of ALL chains (on every GPU and rank), lw / hi the Julia-rounded
+    ranks of Summary applied to the pooled count.  The statistics are reduced on the GPU at the end of Fit for the
+    95 % interval; only the rounding happens here."""
+    pred = (getattr(results, "extra", None) or {}).get("prediction")
+    if pred is None:
+        raise ValueError("Predict needs a fit with new networks: call Fit(..., X_new=...)")
+    if pred["interval"] != interval:
+        raise ValueError("the prediction interval was reduced on the GPU for interval=%s only, not %s"
+                         % (pred["interval"], interval))
+    if pred["mean"] is None:
+        raise IndexError("BoundsError: %d pooled draws are too few for a %d%% interval" % (pred["draws"], interval))
+    m = int(pred["m"])
+    table = dict(sample=np.arange(1, m + 1, dtype=np.int64), estimate=np.round(pred["mean"], digits),
+                 lower_bound=np.round(pred["lower"], digits), upper_bound=np.round(pred["upper"], digits))
+    return BNRPrediction(table, interval, bool(pred["predictive"]))

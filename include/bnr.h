@@ -246,6 +246,27 @@ int bnr_ess_stream_begin(bnr_handle* h, int32_t max_lag, int64_t ndraws);
 int bnr_ess_stream_window(bnr_handle* h, int32_t max_lag, int64_t first_sweep, int64_t ndraws);
 int bnr_ess_stream_finish(bnr_handle* h);
 
+/* Predictions for new networks (posterior predictive of the response y).  X_new is m x q column-major, built like X
+ * (setup_X!).  Every recorded row of every chain -- row 0 by bnr_init_state, then one per sweep at the current trace
+ * row, moved by bnr_copy_trace_rows like the traces -- also writes m doubles to the chain's prediction table:
+ *   BNR_PRED_MEAN        mu + X_new[j,:] gamma                       (credible interval of E[y | x_j])
+ *   BNR_PRED_PREDICTIVE  mu + X_new[j,:] gamma + sqrt(tau2) z_j      (posterior predictive interval), z_j ~ N(0,1)
+ *                        from its own Philox draw site (element j, the row's sweep number)
+ * with the row's own state.  Predictions only read the state: the chains are bit-identical with and without them.
+ * Rows never written hold NaN.  The table has its own capacity, so handles without traces can predict too. */
+#define BNR_PRED_MEAN 0
+#define BNR_PRED_PREDICTIVE 1
+/* X_new: m x q column-major; rows: capacity of each chain's prediction table; m = 0 switches predictions off */
+int bnr_set_predictors(bnr_handle* h, int32_t m, const double* X_new, int64_t rows, int32_t mode);
+/* rows [first, last) of one local chain, iteration-fastest: out[(r - first) + (last - first) * j] */
+int bnr_get_prediction_trace(bnr_handle* h, int32_t chain, int64_t first, int64_t last, double* out);
+/* rows [first_row, first_row + nrows) of every local chain into caller-owned DEVICE memory as [chain][row][m] */
+int bnr_export_predictions(bnr_handle* h, int64_t first_row, int64_t nrows, double* dev_dst);
+/* pooled mean and order statistics over `count` rows of m doubles at a DEVICE pointer; outputs are HOST arrays.  Ranks
+ * are 1-based and exact (radix select, no interpolation); the result does not depend on how the rows were produced. */
+int bnr_prediction_summary(int device, const double* dev_rows, int64_t count, int32_t m, int64_t rank_lo,
+                           int64_t rank_hi, double* mean, double* lo, double* hi);
+
 /* chain groups (independent streams / CUDA graphs) the handle runs */
 int bnr_chain_groups(bnr_handle* h, int32_t* groups);
 /* which gamma formulation the handle runs (BNR_GAMMA_NFORM / BNR_GAMMA_QFORM; AUTO is resolved at create) */
@@ -265,8 +286,9 @@ int bnr_profile_sweep(bnr_handle* h, float* ms);
  *
  * Chains: base.num_chains chains PER DEVICE on n_devices GPUs of this process (devices base.device, base.device + 1,
  * ...); global chain ids (RNG keys) are base.chain_offset + (ext_rank * n_devices + d) * num_chains + local id.  The only
- * data that crosses NVLink are the split-half moments (32 (V + q) bytes per chain) and the ESS statistics, exchanged
- * with ncclAllGather inside the library (libnccl.so.2 is loaded at run time; without it, peer copies).  Several
+ * data that crosses NVLink are the split-half moments (32 (V + q) bytes per chain), the ESS statistics and, with
+ * bnr_fit_predict, the retained predictions (8 m bytes per chain and draw), exchanged with ncclAllGather inside the
+ * library (libnccl.so.2 is loaded at run time; without it, peer copies).  Several
  * PROCESSES can fit a share each (ext_world > 1): the library then calls `allgather` to exchange across processes.
  * --------------------------------------------------------------------------------------------------------------- */
 #define BNR_STATE_NONE 0       /* no table of chain 1 is kept for bnr_fit_state */
@@ -320,6 +342,16 @@ int bnr_fit_state(bnr_fit_result* r, int32_t var, double* out);
 /* the engine handle of one of the result's devices (valid until bnr_fit_free), e.g. for bnr_status / bnr_get_trace */
 int bnr_fit_handle(bnr_fit_result* r, int32_t device_index, bnr_handle** h);
 int bnr_fit_free(bnr_fit_result* r);
+/* bnr_fit plus predictions for m new networks (X_new: m x q column-major, mode BNR_PRED_*); bnr_fit itself is unchanged
+ * and issues exactly the same operations.  Every chain of every device and process keeps a prediction table of the
+ * fit's row capacity; the retained rows of all chains are all-gathered in global-chain order (the same exchange as the
+ * moments) and reduced on device 0.  The tables and the pooled buffer (total_chains x rows x m doubles) are allocated
+ * before the first sweep: a fit that cannot hold them fails at once with BNR_ENOMEM. */
+int bnr_fit_predict(const bnr_fit_params* p, const double* X, const double* y, int32_t m, const double* X_new,
+                    int32_t mode, bnr_fit_result** out);
+/* per new network: the mean and the order statistics of ranks round(N (100 - interval) / 200) and
+ * round(N (1 - (100 - interval) / 200)) (Julia round) of the N = total_chains x sampled pooled draws; [m] each */
+int bnr_fit_prediction(const bnr_fit_result* r, double* mean, double* lo, double* hi);
 /* The control flow of bnr_fit as a pure host function (no GPU): the engine operations a fit would issue when its k-th
  * PSRF evaluation returns psrf_max[k] as the maximum R-hat of both xi and gamma (NaN allowed; 0 beyond n_psrf).
  * ops: [cap_ops][4] = (op, a, b, c) with op  0 create(trace rows, all chains traced, full-state chains)  1 init

@@ -45,25 +45,40 @@ const VARS = ((:τ², 0), (:u, 1), (:ξ, 2), (:γ, 3), (:S, 4), (:θ, 5), (:Δ, 
 fit_error() = unsafe_string(ccall((:bnr_fit_last_error, libbnr), Cstring, ()))
 check(rc) = rc == 0 || error("libbnr error $rc: " * fit_error())
 
-"""
-    fit_b200(X_new, y, R; η, ζ, ι, aΔ, bΔ, ν, nburn, nsamp, mingen, maxgen, psrf_cutoff, num_chains, seed, purge_burn,
-             n_devices = 1) -> (state::Table, rhatξ::Vector, rhatγ::Vector, burn_in, sampled)
+const PRED_MEAN = Int32(0)
+const PRED_PREDICTIVE = Int32(1)
 
-Drop-in for the body of generate_samples! / generate_samples_dbl! after `setup_X!`: `X_new` is the n x q
+"""
+    fit_b200(Xv, y, R; η, ζ, ι, aΔ, bΔ, ν, nburn, nsamp, mingen, maxgen, psrf_cutoff, num_chains, seed, purge_burn,
+             n_devices = 1, X_new = nothing, predictive = false)
+        -> (state::Table, rhatξ::Vector, rhatγ::Vector, burn_in, sampled, prediction)
+
+Drop-in for the body of generate_samples! / generate_samples_dbl! after `setup_X!`: `Xv` is the n x q
 `Matrix{Float64}`; the returned arrays have the reference's (iteration, d1, d2) layout, so
 `Results(state, Table(ξ = rhatξ), Table(γ = rhatγ), burn_in, sampled)` is the same object `Fit!` returns today.
 `num_chains` chains run on EACH of the `n_devices` GPUs (the reference runs one chain per Distributed.jl worker).
+`X_new` (m x q, new networks vectorised by `setup_X!` like `Xv`) runs `bnr_fit_predict`: `prediction` is then
+`(mean, lower, upper)` of μ + X_new γ (+ √τ² z with `predictive = true`) pooled over the retained draws of all chains
+(95 % interval), else `nothing`.
 """
-function fit_b200(X_new::Matrix{Float64}, y::Vector{Float64}, R::Integer; η = 1.01, ζ = 1.0, ι = 1.0, aΔ = 1.0, bΔ = 1.0,
+function fit_b200(Xv::Matrix{Float64}, y::Vector{Float64}, R::Integer; η = 1.01, ζ = 1.0, ι = 1.0, aΔ = 1.0, bΔ = 1.0,
                   ν = 10, nburn = 30000, nsamp = 20000, mingen = 0, maxgen = 0, psrf_cutoff = 1.01, num_chains = 2,
-                  seed = 1, purge_burn = nothing, n_devices = 1, device = 0, verbose = false)
-    n, q = size(X_new)
+                  seed = 1, purge_burn = nothing, n_devices = 1, device = 0, verbose = false,
+                  X_new::Union{Nothing,Matrix{Float64}} = nothing, predictive = false)
+    n, q = size(Xv)
     V = Int((-1 + sqrt(1 + 8q)) / 2)
     base = BnrParams(n, V, R, num_chains, 0, device, 1, 0, 0, UInt64(seed), η, ζ, ι, aΔ, bΔ, Float64(ν), 64, 0, 0, 1)
     p = Ref(BnrFitParams(base, nburn, nsamp, mingen, maxgen, psrf_cutoff, isnothing(purge_burn) ? 0 : purge_burn,
                          STATE_FULL, n_devices, 95, 0, verbose ? 1 : 0, 0, 0, C_NULL, C_NULL))
     res = Ref{Ptr{Cvoid}}(C_NULL)
-    check(ccall((:bnr_fit, libbnr), Cint, (Ref{BnrFitParams}, Ptr{Float64}, Ptr{Float64}, Ref{Ptr{Cvoid}}), p, X_new, y, res))
+    if X_new === nothing
+        check(ccall((:bnr_fit, libbnr), Cint, (Ref{BnrFitParams}, Ptr{Float64}, Ptr{Float64}, Ref{Ptr{Cvoid}}), p, Xv, y, res))
+    else
+        size(X_new, 2) == q || error("X_new must have the q = $q columns of Xv")
+        check(ccall((:bnr_fit_predict, libbnr), Cint,
+                    (Ref{BnrFitParams}, Ptr{Float64}, Ptr{Float64}, Int32, Ptr{Float64}, Int32, Ref{Ptr{Cvoid}}),
+                    p, Xv, y, Int32(size(X_new, 1)), X_new, predictive ? PRED_PREDICTIVE : PRED_MEAN, res))
+    end
     try
         info = Ref{BnrFitInfo}()
         check(ccall((:bnr_fit_get_info, libbnr), Cint, (Ptr{Cvoid}, Ref{BnrFitInfo}), res[], info))
@@ -80,7 +95,15 @@ function fit_b200(X_new::Matrix{Float64}, y::Vector{Float64}, R::Integer; η = 1
         check(ccall((:bnr_fit_rhat, libbnr), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}), res[], rξ, rγ))
         state = Table(τ² = cols[:τ²], u = cols[:u], ξ = cols[:ξ], γ = cols[:γ], S = cols[:S], θ = cols[:θ], Δ = cols[:Δ],
                       M = cols[:M], μ = cols[:μ], λ = cols[:λ], πᵥ = cols[:πᵥ])
-        return state, rξ, rγ, Int(info[].burn_in), Int(info[].sampled)
+        prediction = nothing
+        if X_new !== nothing
+            m = size(X_new, 1)
+            pm = Vector{Float64}(undef, m); pl = Vector{Float64}(undef, m); ph = Vector{Float64}(undef, m)
+            check(ccall((:bnr_fit_prediction, libbnr), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                        res[], pm, pl, ph))
+            prediction = (mean = pm, lower = pl, upper = ph)
+        end
+        return state, rξ, rγ, Int(info[].burn_in), Int(info[].sampled), prediction
     finally
         ccall((:bnr_fit_free, libbnr), Cint, (Ptr{Cvoid},), res[])
     end

@@ -105,6 +105,10 @@ PROTOTYPES = {
     "bnr_export_predictions": (C.c_int, [_H, C.c_int64, C.c_int64, C.c_void_p]),
     "bnr_prediction_summary": (C.c_int, [C.c_int, C.c_void_p, C.c_int64, C.c_int32, C.c_int64, C.c_int64, _DP, _DP,
                                          _DP]),
+    "bnr_set_loglik": (C.c_int, [_H, C.c_int64]),
+    "bnr_get_loglik_trace": (C.c_int, [_H, C.c_int32, C.c_int64, C.c_int64, _DP]),
+    "bnr_export_loglik": (C.c_int, [_H, C.c_int64, C.c_int64, C.c_void_p]),
+    "bnr_loo_summary": (C.c_int, [C.c_int, C.c_void_p, C.c_int64, C.c_int32, _DP, _DP, _DP, _DP, _DP]),
     "bnr_device_copy": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int64]),
     "bnr_fit_default_params": (None, [C.POINTER(FitParams)]),
     "bnr_fit_last_error": (C.c_char_p, []),
@@ -118,6 +122,8 @@ PROTOTYPES = {
     "bnr_fit_free": (C.c_int, [_H]),
     "bnr_fit_predict": (C.c_int, [C.POINTER(FitParams), _DP, _DP, C.c_int32, _DP, C.c_int32, C.POINTER(_H)]),
     "bnr_fit_prediction": (C.c_int, [_H, _DP, _DP, _DP]),
+    "bnr_fit_loo": (C.c_int, [C.POINTER(FitParams), _DP, _DP, C.c_int32, _DP, C.c_int32, C.POINTER(_H)]),
+    "bnr_fit_loo_pointwise": (C.c_int, [_H, _DP, _DP, _DP, _DP, _DP]),
     "bnr_fit_plan": (C.c_int, [C.POINTER(FitParams), _DP, C.c_int32, _I64P, C.c_int64, _I64P, C.POINTER(FitInfo)]),
     "bnr_gamma_mode": (C.c_int, [_H, C.POINTER(C.c_int32)]),
     "bnr_launch_count": (C.c_int, [_H, _I64P]),

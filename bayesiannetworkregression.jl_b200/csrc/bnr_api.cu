@@ -634,6 +634,7 @@ static void enqueue_sweep(Engine& e, double* ws, const ForkJoin& fj, cudaStream_
     if (fork_pred) cudaStreamWaitEvent(s, fj.join, 0);
     launch_pred_record(e, 1, s);
   }
+  if (e.ll) launch_loglik_record(e, s);
   launch_advance(e, 1, s);
 }
 
@@ -675,6 +676,7 @@ static Engine group_view(const bnr_handle* h, int c0, int Cg, long long* counter
     v.pred += c * (size_t)v.pred_rows * v.pred_m;
     v.pred_ws += c * (size_t)v.pred_splits * v.pred_mp;
   }
+  if (v.ll) v.ll += c * (size_t)v.ll_rows * d.n;
   v.iter = counters; v.trace_row = counters + 1; v.mom_window = mom_window;
   v.inj = nullptr; v.inj_stride = 0;
   memset(&v.aux, 0, sizeof(v.aux));
@@ -720,6 +722,10 @@ extern "C" int bnr_init_state(bnr_handle* h) {
   if (e.pred_m > 0) {
     launch_pred_product(e, h->stream);
     launch_pred_record(e, 0, h->stream);
+  }
+  if (e.ll) {
+    refresh_xg(h);                     // X gamma_0: the cache is not valid after launch_init
+    launch_loglik_record(e, h->stream);
   }
   launch_advance(e, 0, h->stream);
   h->xg_valid = false;
@@ -826,23 +832,31 @@ extern "C" int bnr_copy_trace_rows(bnr_handle* h, int64_t dst, int64_t src, int6
   if (!h || dst < 0 || src < 0 || count < 0) return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
   Engine& e = h->e;
-  const bool traces = e.trace_rows > 0 && (e.tr_full || e.tr_gx), preds = e.pred_m > 0;
-  if (!traces && !preds) return BNR_OK;     // this handle records no traces and no predictions: nothing to move
-  if (traces && (dst + count > e.trace_rows || src + count > e.trace_rows)) return fail(BNR_EINVAL, "rows out of range");
-  if (preds && (dst + count > e.pred_rows || src + count > e.pred_rows))
-    return fail(BNR_EINVAL, "rows beyond the prediction table");
+  // every per-chain table the record kernels write at *trace_row: traces, predictions, log-likelihood
+  struct Table { double* base; size_t rowlen; int chains; long long rows; const char* range_msg; };
+  Table tabs[4];
+  int nt = 0;
+  if (e.trace_rows > 0 && e.tr_full)
+    tabs[nt++] = {e.tr_full, (size_t)e.rowlen_full, e.trace_full_chains, e.trace_rows, "rows out of range"};
+  if (e.trace_rows > 0 && e.tr_gx)
+    tabs[nt++] = {e.tr_gx, (size_t)(e.d.V + e.d.q), e.trace_gx_chains, e.trace_rows, "rows out of range"};
+  if (e.pred_m > 0) tabs[nt++] = {e.pred, (size_t)e.pred_m, e.d.C, e.pred_rows, "rows beyond the prediction table"};
+  if (e.ll) tabs[nt++] = {e.ll, (size_t)e.d.n, e.d.C, e.ll_rows, "rows beyond the log-likelihood table"};
+  if (nt == 0) return BNR_OK;               // this handle records no per-row tables: nothing to move
+  size_t max_row = 0;
+  for (int t = 0; t < nt; ++t) {
+    if (dst + count > tabs[t].rows || src + count > tabs[t].rows) return fail(BNR_EINVAL, tabs[t].range_msg);
+    if (tabs[t].rowlen > max_row) max_row = tabs[t].rowlen;
+  }
   if (count == 0 || dst == src) return BNR_OK;
   // rows are contiguous per chain; regions may overlap -> stage through one temporary (stream order keeps the chains apart)
   const bool overlap = !(dst + count <= src || src + count <= dst);
-  size_t max_row = (size_t)(e.tr_full ? e.rowlen_full : 0) > (size_t)(e.d.V + e.d.q) ? (size_t)e.rowlen_full
-                                                                                     : (size_t)(e.d.V + e.d.q);
-  if (preds && (size_t)e.pred_m > max_row) max_row = (size_t)e.pred_m;
   Scratch sc(h->p.device, overlap ? (size_t)count * max_row * sizeof(double) : 256);
   if (overlap && !sc.p) return fail(BNR_ENOMEM, "device scratch allocation failed");
-  auto move = [&](double* base, size_t rowlen, int chains, long long table_rows) -> int {
-    for (int c = 0; c < chains; ++c) {
-      double* b = base + (size_t)c * table_rows * rowlen;
-      const size_t bytes = (size_t)count * rowlen * sizeof(double);
+  for (int t = 0; t < nt; ++t) {
+    const size_t rowlen = tabs[t].rowlen, bytes = (size_t)count * rowlen * sizeof(double);
+    for (int c = 0; c < tabs[t].chains; ++c) {
+      double* b = tabs[t].base + (size_t)c * tabs[t].rows * rowlen;
       if (!overlap) {
         CK(cudaMemcpyAsync(b + (size_t)dst * rowlen, b + (size_t)src * rowlen, bytes, cudaMemcpyDeviceToDevice, h->stream));
       } else {
@@ -850,11 +864,7 @@ extern "C" int bnr_copy_trace_rows(bnr_handle* h, int64_t dst, int64_t src, int6
         CK(cudaMemcpyAsync(b + (size_t)dst * rowlen, sc.p, bytes, cudaMemcpyDeviceToDevice, h->stream));
       }
     }
-    return 0;
-  };
-  if (traces && e.tr_full) { int r = move(e.tr_full, e.rowlen_full, e.trace_full_chains, e.trace_rows); if (r) return r; }
-  if (traces && e.tr_gx) { int r = move(e.tr_gx, e.d.V + e.d.q, e.trace_gx_chains, e.trace_rows); if (r) return r; }
-  if (preds) { int r = move(e.pred, e.pred_m, e.d.C, e.pred_rows); if (r) return r; }
+  }
   CK(cudaStreamSynchronize(h->stream));
   return BNR_OK;
 }
@@ -1298,6 +1308,10 @@ extern "C" int bnr_finish_sweep(bnr_handle* h) {
   if (h->e.pred_m > 0) {
     launch_pred_product(h->e, h->stream);
     launch_pred_record(h->e, 1, h->stream);
+  }
+  if (h->e.ll) {
+    if (!h->xg_valid) refresh_xg(h);
+    launch_loglik_record(h->e, h->stream);
   }
   launch_advance(h->e, 1, h->stream);
   CK(cudaGetLastError());
@@ -1771,5 +1785,90 @@ extern "C" int bnr_prediction_summary(int device, const double* dev_rows, int64_
   if (mean) memcpy(mean, host.data(), sizeof(double) * m);
   if (lo) memcpy(lo, host.data() + m, sizeof(double) * m);
   if (hi) memcpy(hi, host.data() + 2 * m, sizeof(double) * m);
+  return BNR_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Pointwise log-likelihood: every recorded row of every chain also gets log p(y_i | state) for every observation i,
+// the input of PSIS-LOO and WAIC (bnr_loo_summary)
+// ---------------------------------------------------------------------------------------------------------
+extern "C" int bnr_set_loglik(bnr_handle* h, int64_t rows) {
+  if (!h) return fail(BNR_EINVAL, "null handle");
+  if (rows < 0) return fail(BNR_EINVAL, "rows must be >= 0");
+  CK(cudaSetDevice(h->p.device));
+  CK(cudaStreamSynchronize(h->stream));
+  drop_graph(h);                       // the captured sweeps gain or lose the k_loglik_record node
+  Engine& e = h->e;
+  release_alloc(h, e.ll);
+  e.ll = nullptr; e.ll_rows = 0;
+  if (rows == 0) return BNR_OK;
+  const size_t count = (size_t)e.d.C * rows * e.d.n;
+  double* ll = nullptr;
+  if (int r = dalloc(h, &ll, count, false)) {
+    cudaGetLastError();                // a refused cudaMalloc must not surface in a later call
+    return fail(r, "log-likelihood table (" + std::to_string(8.0 * (double)count) + " bytes): " + g_err);
+  }
+  CK(cudaMemsetAsync(ll, 0xff, sizeof(double) * count, h->stream));   // NaN: rows never written
+  CK(cudaStreamSynchronize(h->stream));
+  e.ll = ll; e.ll_rows = rows;
+  return BNR_OK;
+}
+
+extern "C" int bnr_get_loglik_trace(bnr_handle* h, int32_t chain, int64_t first, int64_t last, double* out) {
+  if (!h || !out || chain < 0 || chain >= h->e.d.C || first < 0 || last < first) return fail(BNR_EINVAL, "bad arguments");
+  const Engine& e = h->e;
+  if (!e.ll) return fail(BNR_ESTATE, "no log-likelihood table (bnr_set_loglik)");
+  if (last > e.ll_rows) return fail(BNR_EINVAL, "rows beyond the log-likelihood table");
+  CK(cudaSetDevice(h->p.device));
+  const size_t count = (size_t)(last - first), n = (size_t)e.d.n;
+  if (count == 0) return BNR_OK;
+  std::vector<double> tmp(count * n);
+  CK(cudaMemcpyAsync(tmp.data(), e.ll + ((size_t)chain * e.ll_rows + first) * n, sizeof(double) * tmp.size(),
+                     cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  for (size_t r = 0; r < count; ++r)
+    for (size_t i = 0; i < n; ++i) out[r + count * i] = tmp[r * n + i];
+  return BNR_OK;
+}
+
+extern "C" int bnr_export_loglik(bnr_handle* h, int64_t first_row, int64_t nrows, double* dev_dst) {
+  if (!h || !dev_dst || first_row < 0 || nrows < 0) return fail(BNR_EINVAL, "bad arguments");
+  const Engine& e = h->e;
+  if (!e.ll) return fail(BNR_ESTATE, "no log-likelihood table (bnr_set_loglik)");
+  if (first_row + nrows > e.ll_rows) return fail(BNR_EINVAL, "rows beyond the log-likelihood table");
+  CK(cudaSetDevice(h->p.device));
+  if (nrows == 0) return BNR_OK;
+  const size_t rowb = sizeof(double) * (size_t)e.d.n;
+  CK(cudaMemcpy2DAsync(dev_dst, rowb * nrows, e.ll + (size_t)first_row * e.d.n, rowb * e.ll_rows, rowb * nrows,
+                       (size_t)e.d.C, cudaMemcpyDeviceToDevice, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  return BNR_OK;
+}
+
+extern "C" int bnr_loo_summary(int device, const double* dev_rows, int64_t N, int32_t n, double* elpd_loo,
+                               double* p_loo, double* pareto_k, double* elpd_waic, double* p_waic) {
+  if (!dev_rows || N < 2 || n < 1) return fail(BNR_EINVAL, "bad arguments (need rows, N >= 2 draws, n >= 1)");
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+    return fail(BNR_ENODEV, "no CUDA device visible: libbnr has no CPU fallback");
+  if (device < 0 || device >= ndev) return fail(BNR_EINVAL, "device ordinal out of range");
+  CK(cudaSetDevice(device));
+  const long long M = loo_tail_len(N), Mmax = loo_tail_max();
+  if (M > Mmax)
+    return fail(BNR_EINVAL, "the Pareto tail of " + std::to_string(N) + " draws (" + std::to_string(M) +
+                                " values) exceeds the " + std::to_string(Mmax) +
+                                " values one block's shared memory holds (at most about " +
+                                std::to_string((long long)((double)Mmax * Mmax / 9.0)) + " pooled draws)");
+  const size_t outb = sizeof(double) * 5 * (size_t)n;
+  Scratch sc(device, loo_ws_bytes(N, n) + outb);
+  if (!sc.p) return fail(BNR_ENOMEM, "device scratch allocation failed");
+  double* o = (double*)sc.p;
+  launch_loo(dev_rows, N, n, o, o + 5 * (size_t)n, 0);
+  std::vector<double> host((size_t)5 * n);
+  CK(cudaMemcpy(host.data(), o, outb, cudaMemcpyDeviceToHost));
+  CK(cudaGetLastError());
+  double* dst[5] = {elpd_loo, p_loo, pareto_k, elpd_waic, p_waic};
+  for (int k = 0; k < 5; ++k)
+    if (dst[k]) memcpy(dst[k], host.data() + (size_t)k * n, sizeof(double) * n);
   return BNR_OK;
 }

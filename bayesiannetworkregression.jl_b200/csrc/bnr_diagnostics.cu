@@ -214,6 +214,274 @@ void launch_pred_select(const double* rows, long long N, int m, long long rank_l
 }
 
 // ------------------------------------------------------------------------------------------------------------
+// Pooled PSIS-LOO and WAIC of every column i of ll[N][n] (N pooled draws of the pointwise log-likelihood), as the R
+// package loo 2.x computes them with r_eff = 1: log ratios -ll, shifted so that the largest is 0 (lw = min ll - ll); the
+// tail is the M = ceil(min(0.2 N, 3 sqrt N)) largest lw, i.e. the M smallest ll; the generalised Pareto fit of
+// Zhang & Stephens (gpdfit) replaces the tail by its quantiles; weights are truncated at 0.
+//   launch_pred_select : ranks a = ll_(M), b = ll_(M+1) (the cutoff) and the column mean
+//   k_loo_pass         : rows split over blocks like k_pred_hist (8 columns x 32 row lanes); per block and column the
+//                        logsumexp partial of ll, sum (ll - mean)^2 and the non-tail weight sum sum_{ll > a} exp(b - ll);
+//                        values below a are compacted into the column's tail through an integer cursor, values equal
+//                        to a are counted
+//   k_loo_tail         : block per column: the tail (cursor entries, then copies of a) sorted in shared memory, the
+//                        GPD fit, smoothing, truncation and the block partials added in block order
+// Every floating-point sum has a fixed order; the tail is sorted before use, so its compaction order does not matter.
+// ------------------------------------------------------------------------------------------------------------
+constexpr int LOO_TB = 512;     // threads of k_loo_tail
+
+long long loo_tail_len(long long N) {
+  const double S = (double)N;
+  return (long long)ceil(fmin(0.2 * S, 3.0 * sqrt(S)));
+}
+
+// dynamic shared memory of k_loo_tail: tail [M] | reduction scratch [32] | broadcast [8] | theta [G] | l(theta) [G]
+__host__ __device__ static int loo_grid(long long M) { return 30 + (int)floor(sqrt((double)M)); }
+static size_t loo_tail_smem(long long M) { return sizeof(double) * ((size_t)M + 40 + 2 * (size_t)loo_grid(M)); }
+
+long long loo_tail_max() {
+  int dev = 0, optin = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+  long long M = optin / 8 - 40 - 2 * loo_grid(optin / 8);
+  while (M > 0 && loo_tail_smem(M) > (size_t)optin) --M;
+  return M;
+}
+
+__global__ void __launch_bounds__(256) k_loo_pass(const double* __restrict__ rows, long long N, int n, long long per,
+                                                  long long M, const double* __restrict__ mean,
+                                                  const double* __restrict__ av, const double* __restrict__ bv,
+                                                  double* __restrict__ part, unsigned long long* __restrict__ cnt,
+                                                  double* __restrict__ tail) {
+  __shared__ double red[4][32][PS_EPB];
+  const int tid = threadIdx.x, e = tid % PS_EPB, lane = tid / PS_EPB;
+  const int col = blockIdx.x * PS_EPB + e;
+  const bool live = col < n;
+  const long long r0 = (long long)blockIdx.y * per, r1 = min(N, r0 + per);
+  double mx = -INFINITY, se = 0.0, sq = 0.0, w = 0.0;
+  unsigned long long eq = 0;
+  if (live) {
+    const double mu = mean[col], a = av[col], b = bv[col];
+    double* tl = tail + (size_t)col * M;
+    for (long long r = r0 + lane; r < r1; r += 32) {
+      const double x = rows[(size_t)r * n + col];
+      if (x > mx) { se = se * exp(mx - x) + 1.0; mx = x; }
+      else se += exp(x - mx);
+      const double dv = x - mu;
+      sq += dv * dv;
+      if (x > a) w += exp(b - x);
+      else if (x < a) tl[atomicAdd(&cnt[col], 1ull)] = x;
+      else ++eq;
+    }
+    if (eq) atomicAdd(&cnt[n + col], eq);
+  }
+  red[0][lane][e] = mx; red[1][lane][e] = se; red[2][lane][e] = sq; red[3][lane][e] = w;
+  __syncthreads();
+  if (tid < PS_EPB && blockIdx.x * PS_EPB + tid < n) {
+    double m = -INFINITY, s = 0.0, q = 0.0, ww = 0.0;
+    for (int l = 0; l < 32; ++l) {
+      const double m2 = red[0][l][tid], s2 = red[1][l][tid];
+      if (s2 > 0.0) {
+        if (m2 > m) { s = s * exp(m - m2) + s2; m = m2; }
+        else s += s2 * exp(m2 - m);
+      }
+      q += red[2][l][tid];
+      ww += red[3][l][tid];
+    }
+    double* p = part + ((size_t)blockIdx.y * n + blockIdx.x * PS_EPB + tid) * 4;
+    p[0] = m; p[1] = s; p[2] = q; p[3] = ww;
+  }
+}
+
+// the same value on every thread: warp trees, then the warps in order
+__device__ double loo_block_sum(double v, double* red) {
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double t = 0.0;
+  for (int i = 0; i < (int)(blockDim.x >> 5); ++i) t += red[i];
+  return t;
+}
+__device__ double loo_block_max(double v, double* red) {
+  for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_down_sync(0xffffffffu, v, o));
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double t = -INFINITY;
+  for (int i = 0; i < (int)(blockDim.x >> 5); ++i) t = fmax(t, red[i]);
+  return t;
+}
+
+// out[k * n + col]: k = 0 elpd_loo, 1 p_loo, 2 pareto_k, 3 elpd_waic, 4 p_waic
+__global__ void __launch_bounds__(LOO_TB) k_loo_tail(long long N, int n, long long M, int rb,
+                                                     const double* __restrict__ part,
+                                                     const unsigned long long* __restrict__ cnt,
+                                                     const double* __restrict__ av, const double* __restrict__ bv,
+                                                     const double* __restrict__ tail, double* __restrict__ out) {
+  extern __shared__ double sm[];
+  const int G = loo_grid(M);
+  double* v = sm;              // the tail's ll values, sorted ascending
+  double* red = v + M;
+  double* bc = red + 32;
+  double* th = bc + 8;
+  double* lt = th + G;
+  const int col = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
+  const long long below = (long long)cnt[col], eq = (long long)cnt[n + col];
+  const double a = av[col], b = bv[col];
+  for (long long i = tid; i < M; i += nt) v[i] = i < below ? tail[(size_t)col * M + i] : a;
+  __syncthreads();
+  // bitonic sort of M values without storing the padding to a power of two: every compare-exchange puts the larger
+  // value at the higher index, so virtual +inf beyond M never moves and pairs reaching past M are skipped
+  long long P = 1;
+  while (P < M) P <<= 1;
+  for (long long k = 2; k <= P; k <<= 1) {
+    for (long long t = tid; t < P / 2; t += nt) {
+      const long long h = k >> 1, blk = t / h, off = t % h;
+      const long long i = blk * k + off, j = blk * k + k - 1 - off;
+      if (j < M && v[i] > v[j]) { const double x = v[i]; v[i] = v[j]; v[j] = x; }
+    }
+    __syncthreads();
+    for (long long d = k >> 2; d >= 1; d >>= 1) {
+      for (long long t = tid; t < P / 2; t += nt) {
+        const long long blk = t / d, off = t % d;
+        const long long i = blk * 2 * d + off, j = i + d;
+        if (j < M && v[i] > v[j]) { const double x = v[i]; v[i] = v[j]; v[j] = x; }
+      }
+      __syncthreads();
+    }
+  }
+  // log weight of the tail value of ascending rank j (0-based): lw_j = min ll - ll_(M-1-j); cutoff = min ll - b
+  const double mn = v[0], cut = mn - b, ec = exp(cut);
+  const double Md = (double)M;
+  double kh = INFINITY, sigma = 0.0;
+  if (M >= 5 && v[0] != v[M - 1]) {
+    const double xM = exp(mn - v[0]) - ec;
+    const long long qi = (long long)floor(Md / 4.0 + 0.5) - 1;
+    const double xs = exp(mn - v[M - 1 - qi]) - ec;
+    for (int j = tid; j < G; j += nt) th[j] = 1.0 / xM + (1.0 - sqrt((double)G / (j + 0.5))) / (3.0 * xs);
+    __syncthreads();
+    for (int g = 0; g < G; ++g) {
+      const double t = th[g];
+      double s = 0.0;
+      for (long long i = tid; i < M; i += nt) s += log1p(-t * (exp(mn - v[i]) - ec));
+      s = loo_block_sum(s, red);
+      if (tid == 0) {
+        const double kk = s / Md;
+        lt[g] = Md * (log(-t / kk) - kk - 1.0);
+      }
+    }
+    __syncthreads();
+    if (tid == 0) {
+      double lm = -INFINITY;
+      for (int g = 0; g < G; ++g) lm = fmax(lm, lt[g]);
+      double z = 0.0;
+      for (int g = 0; g < G; ++g) z += exp(lt[g] - lm);
+      const double lse = lm + log(z);
+      double thh = 0.0;
+      for (int g = 0; g < G; ++g) thh += th[g] * exp(lt[g] - lse);
+      bc[0] = thh;
+    }
+    __syncthreads();
+    const double thh = bc[0];
+    double s = 0.0;
+    for (long long i = tid; i < M; i += nt) s += log1p(-thh * (exp(mn - v[i]) - ec));
+    s = loo_block_sum(s, red);
+    const double k0 = s / Md;
+    sigma = -k0 / thh;
+    kh = (Md * k0 + 5.0) / (Md + 10.0);
+    if (isnan(kh)) kh = INFINITY;
+  }
+  const bool smooth = isfinite(kh);
+  // smoothed, truncated log weight s_j of rank j and its raw lw_j
+  auto smoothed = [&](long long j, double& lwr) {
+    lwr = mn - v[M - 1 - j];
+    double s = lwr;
+    if (smooth) {
+      const double p = ((double)j + 0.5) / Md;
+      const double qq = kh == 0.0 ? -sigma * log1p(-p) : sigma * expm1(-kh * log1p(-p)) / kh;
+      s = log(qq + ec);
+    }
+    return s > 0.0 ? 0.0 : s;
+  };
+  // lse(lw + ll) = mn + lse(t) with t_j = s_j - lw_j in the tail and t = 0 for the N - M others;
+  // lse(lw) over the tail's s_j and the non-tail term cut + log W, W = sum_{ll > a} exp(b - ll) + (copies of a outside)
+  double mt = 0.0, ms = -INFINITY;
+  for (long long j = tid; j < M; j += nt) {
+    double lwr;
+    const double s = smoothed(j, lwr);
+    mt = fmax(mt, s - lwr);
+    ms = fmax(ms, s);
+  }
+  mt = loo_block_max(mt, red);
+  ms = loo_block_max(ms, red);
+  double st = 0.0, ss = 0.0;
+  for (long long j = tid; j < M; j += nt) {
+    double lwr;
+    const double s = smoothed(j, lwr);
+    st += exp(s - lwr - mt);
+    ss += exp(s - ms);
+  }
+  st = loo_block_sum(st, red);
+  ss = loo_block_sum(ss, red);
+  if (tid == 0) {
+    double m = -INFINITY, se = 0.0, sq = 0.0, w = 0.0;
+    for (int y = 0; y < rb; ++y) {
+      const double* p = part + ((size_t)y * n + col) * 4;
+      if (p[1] > 0.0) {
+        if (p[0] > m) { se = se * exp(m - p[0]) + p[1]; m = p[0]; }
+        else se += p[1] * exp(p[0] - m);
+      }
+      sq += p[2];
+      w += p[3];
+    }
+    w += (double)(below + eq - M);
+    const double S = (double)N;
+    const double lse_a = mn + mt + log((S - Md) * exp(-mt) + st);
+    const double lnt = cut + log(w);
+    const double mm = fmax(lnt, ms);
+    const double lse_b = mm + log(exp(lnt - mm) + ss * exp(ms - mm));
+    const double elpd = lse_a - lse_b;
+    const double lpd = m + log(se) - log(S);
+    const double pw = sq / (S - 1.0);
+    out[col] = elpd;
+    out[n + col] = lpd - elpd;
+    out[2 * n + col] = kh;
+    out[3 * n + col] = lpd - pw;
+    out[4 * n + col] = pw;
+  }
+}
+
+// scratch: select | mean, a, b [3][n] | partials [RB][n][4] | counters [2][n] | tails [n][M]
+size_t loo_ws_bytes(long long N, int n) {
+  const size_t sel = (pred_select_ws_bytes(N, n) + 255) / 256 * 256;
+  return sel + sizeof(double) * ((size_t)3 * n + (size_t)pred_select_row_blocks(N, n) * n * 4) +
+         sizeof(unsigned long long) * 2 * (size_t)n + sizeof(double) * (size_t)n * loo_tail_len(N);
+}
+
+void launch_loo(const double* rows, long long N, int n, double* out, void* ws, cudaStream_t s) {
+  const long long M = loo_tail_len(N);
+  const int rb = pred_select_row_blocks(N, n);
+  const long long per = (N + rb - 1) / rb;
+  char* p = (char*)ws;
+  void* sel = p;
+  p += (pred_select_ws_bytes(N, n) + 255) / 256 * 256;
+  double* mean = (double*)p;
+  double* av = mean + n;
+  double* bv = av + n;
+  double* part = bv + n;
+  unsigned long long* cnt = (unsigned long long*)(part + (size_t)rb * n * 4);
+  double* tail = (double*)(cnt + 2 * (size_t)n);
+  launch_pred_select(rows, N, n, M, M + 1, mean, av, bv, sel, s);
+  cudaMemsetAsync(cnt, 0, sizeof(unsigned long long) * 2 * (size_t)n, s);
+  ++g_launches;
+  k_loo_pass<<<dim3((n + PS_EPB - 1) / PS_EPB, rb), 256, 0, s>>>(rows, N, n, per, M, mean, av, bv, part, cnt, tail);
+  const size_t smem = loo_tail_smem(M);
+  cudaFuncSetAttribute(k_loo_tail, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  ++g_launches;
+  k_loo_tail<<<n, LOO_TB, smem, s>>>(N, n, M, rb, part, cnt, av, bv, tail, out);
+}
+
+// ------------------------------------------------------------------------------------------------------------
 // ESS.  tr: [C][trace_rows][P] rows of (xi, gamma); window = rows [first, first + N).
 //   k_chain_mean : cmean[c][p]                       grid = (ceil(P/128), C), block = 128
 //   k_acov_sum   : acov[l][p] = sum_c 1/N sum_t (x_t - m_c)(x_{t+l} - m_c), l = 0 .. L (biased, per-chain centred)

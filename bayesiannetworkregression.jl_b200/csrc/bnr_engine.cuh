@@ -142,6 +142,10 @@ struct Engine {
   double* pred;           // [C][pred_rows][pred_m]
   double* pred_ws;        // split-K partials of X_new gamma, [pred_splits][C][pred_mp]; a chain group's view uses
                           // [pred_splits][Cg][pred_mp] at offset c0 * pred_splits * pred_mp
+  // pointwise log-likelihood (bnr_set_loglik; ll == nullptr: off).  Every recorded row r of chain c gets
+  // ll[c][r][i] = log N(y_i | mu_c + (X gamma_c)_i, tau2_c) of the row's own state, written at *trace_row
+  long long ll_rows;      // rows of each chain's log-likelihood table
+  double* ll;             // [C][ll_rows][n]
   // injection
   const double* inj;  // [C][inj_stride] or nullptr
   long long inj_stride;

@@ -291,6 +291,11 @@ struct bnr_fit_result {
   std::vector<double*> pexp;           // per device: the retained rows of its chains, [chain][row][m]
   std::vector<double> p_mean, p_lo, p_hi;
   bool pred_ok = false;
+  // PSIS-LOO / WAIC (bnr_fit_loo)
+  bool loo = false;
+  std::vector<double*> lexp;           // per device: the retained log-likelihood rows of its chains, [chain][row][n]
+  std::vector<double> l_pw[5];         // elpd_loo, p_loo, pareto_k, elpd_waic, p_waic per observation
+  bool loo_ok = false;
   int gamma_mode = 0;
   int status_or = 0;
   const char* exchange = "none";
@@ -299,6 +304,7 @@ struct bnr_fit_result {
       if (d < dev.size()) cudaSetDevice(dev[d]);
       if (d < gbuf.size() && gbuf[d]) cudaFree(gbuf[d]);
       if (d < pexp.size() && pexp[d]) cudaFree(pexp[d]);
+      if (d < lexp.size() && lexp[d]) cudaFree(lexp[d]);
       if (d < xs.size() && xs[d]) cudaStreamDestroy(xs[d]);
     }
     if (xbuf) { cudaSetDevice(dev[0]); cudaFree(xbuf); }
@@ -371,26 +377,42 @@ struct DeviceOps : Ops {
         R.exchange = "peer-copy";
       }
     }
-    if (R.pm > 0) return create_predictions(rows);
+    if (R.pm > 0 || R.loo) return create_tables(rows);
     return 0;
   }
 
-  // prediction tables of `rows` rows on every handle, the export buffers and the pooled buffers of the all-gather,
-  // all before the first sweep: a fit that cannot hold its predictions fails here, not after the sampling
-  int create_predictions(long long rows) {
+  // prediction and log-likelihood tables of `rows` rows on every handle, their export buffers and the pooled buffers
+  // of the all-gather (sized for the wider of the two), all before the first sweep: a fit that cannot hold them fails
+  // here, not after the sampling
+  int create_tables(long long rows) {
     const int nd = (int)R.h.size(), world = R.p.ext_world > 1 ? R.p.ext_world : 1;
-    for (auto* h : R.h) BN(bnr_set_predictors(h, R.pm, X_new, rows, R.pmode));
-    const size_t local = (size_t)R.C * rows * R.pm;
-    auto refuse = [&](const char* what, size_t doubles) {
+    const char* what = "predictions";
+    auto refuse = [&](const char* buf, size_t doubles) {
       cudaGetLastError();
-      return ffail(BNR_ENOMEM, std::string("cannot allocate the ") + what + " of the predictions (" +
+      return ffail(BNR_ENOMEM, std::string("cannot allocate the ") + buf + " of the " + what + " (" +
                                    std::to_string(doubles * sizeof(double)) + " bytes)");
     };
-    R.pexp.assign(nd, nullptr);
-    for (int d = 0; d < nd; ++d) {
-      CKF(cudaSetDevice(R.dev[d]));
-      if (cudaMalloc((void**)&R.pexp[d], local * sizeof(double)) != cudaSuccess) { R.pexp[d] = nullptr; return refuse("export buffer", local); }
+    auto exports = [&](std::vector<double*>& buf, size_t local) -> int {
+      buf.assign(nd, nullptr);
+      for (int d = 0; d < nd; ++d) {
+        CKF(cudaSetDevice(R.dev[d]));
+        if (cudaMalloc((void**)&buf[d], local * sizeof(double)) != cudaSuccess) { buf[d] = nullptr; return refuse("export buffer", local); }
+      }
+      return 0;
+    };
+    int width = 0;
+    if (R.pm > 0) {
+      for (auto* h : R.h) BN(bnr_set_predictors(h, R.pm, X_new, rows, R.pmode));
+      if (int r = exports(R.pexp, (size_t)R.C * rows * R.pm)) return r;
+      width = R.pm;
     }
+    if (R.loo) {
+      what = "log-likelihood";
+      for (auto* h : R.h) BN(bnr_set_loglik(h, rows));
+      if (int r = exports(R.lexp, (size_t)R.C * rows * R.p.base.n)) return r;
+      if (R.p.base.n > width) width = R.p.base.n;
+    }
+    const size_t local = (size_t)R.C * rows * width;
     if (nd > 1 || world > 1) {
       // gather_local / gather_ext reuse these buffers (they only grow)
       for (int d = 0; d < nd; ++d) {
@@ -433,6 +455,26 @@ struct DeviceOps : Ops {
     R.p_mean.assign(R.pm, 0); R.p_lo.assign(R.pm, 0); R.p_hi.assign(R.pm, 0);
     BN(bnr_prediction_summary(R.dev[0], all, N, R.pm, lw, hi, R.p_mean.data(), R.p_lo.data(), R.p_hi.data()));
     R.pred_ok = true;
+    return 0;
+  }
+
+  // the retained log-likelihood rows of every chain in global-chain order on device 0, then PSIS-LOO and WAIC
+  int loo(const Outcome& o) {
+    const long long N = (long long)total_chains() * o.sampled;
+    if (N < 2) return 0;
+    const int nd = (int)R.h.size(), n = R.p.base.n;
+    for (int d = 0; d < nd; ++d) BN(bnr_export_loglik(R.h[d], o.burn_in, o.sampled, R.lexp[d]));
+    const size_t cnt = (size_t)R.C * o.sampled * n;
+    const double* all = R.lexp[0];
+    if (nd > 1 || R.p.ext_world > 1) {
+      std::vector<const double*> src(R.lexp.begin(), R.lexp.end());
+      if (int r = gather_local(src, cnt)) return r;
+      if (int r = gather_ext(cnt * nd, &all)) return r;
+    }
+    for (auto& v : R.l_pw) v.assign(n, 0);
+    BN(bnr_loo_summary(R.dev[0], all, N, n, R.l_pw[0].data(), R.l_pw[1].data(), R.l_pw[2].data(), R.l_pw[3].data(),
+                       R.l_pw[4].data()));
+    R.loo_ok = true;
     return 0;
   }
   int init() override { PhaseClock::Scope sc(clk, PH_INIT); for (auto* h : R.h) BN(bnr_init_state(h)); return 0; }
@@ -637,9 +679,9 @@ extern "C" int bnr_fit_plan(const bnr_fit_params* p, const double* psrf_max, int
   return BNR_OK;
 }
 
-// bnr_fit and bnr_fit_predict (m > 0: predictions for the m rows of X_new)
+// bnr_fit, bnr_fit_predict (m > 0: predictions for the m rows of X_new) and bnr_fit_loo (loo: PSIS-LOO and WAIC)
 static int fit_body(const bnr_fit_params* p, const double* X, const double* y, int32_t m, const double* X_new,
-                    int32_t mode, bnr_fit_result** res_out) {
+                    int32_t mode, bool loo, bnr_fit_result** res_out) {
   if (int r = check_params(p)) return r;
   if (!X || !y || !res_out) return ffail(BNR_EINVAL, "null argument");
   if (p->base.nu < p->base.R)
@@ -648,7 +690,7 @@ static int fit_body(const bnr_fit_params* p, const double* X, const double* y, i
     return ffail(BNR_EINVAL, "nu must not be smaller than R");
   bnr_fit_result* R = new bnr_fit_result();
   R->p = *p;
-  R->pm = m; R->pmode = mode;
+  R->pm = m; R->pmode = mode; R->loo = loo;
   DeviceOps o(*R, X, y, X_new);
   const double t_start = PhaseClock::now();
   int rc = fit_loops(o, *p, R->out);
@@ -666,6 +708,7 @@ static int fit_body(const bnr_fit_params* p, const double* X, const double* y, i
     }
   }
   if (!rc && m > 0) rc = o.predictions(R->out);
+  if (!rc && loo) rc = o.loo(R->out);
   if (!rc) rc = o.ess(R->out);
   if (!rc) {
     std::vector<int32_t> st(R->C);
@@ -689,7 +732,7 @@ static int fit_body(const bnr_fit_params* p, const double* X, const double* y, i
 }
 
 extern "C" int bnr_fit(const bnr_fit_params* p, const double* X, const double* y, bnr_fit_result** res_out) {
-  return fit_body(p, X, y, 0, nullptr, BNR_PRED_MEAN, res_out);
+  return fit_body(p, X, y, 0, nullptr, BNR_PRED_MEAN, false, res_out);
 }
 
 extern "C" int bnr_fit_predict(const bnr_fit_params* p, const double* X, const double* y, int32_t m,
@@ -697,7 +740,27 @@ extern "C" int bnr_fit_predict(const bnr_fit_params* p, const double* X, const d
   if (m < 0) return ffail(BNR_EINVAL, "m must be >= 0");
   if (m > 0 && !X_new) return ffail(BNR_EINVAL, "null X_new");
   if (mode != BNR_PRED_MEAN && mode != BNR_PRED_PREDICTIVE) return ffail(BNR_EINVAL, "unknown prediction mode");
-  return fit_body(p, X, y, m, X_new, mode, res_out);
+  return fit_body(p, X, y, m, X_new, mode, false, res_out);
+}
+
+extern "C" int bnr_fit_loo(const bnr_fit_params* p, const double* X, const double* y, int32_t m, const double* X_new,
+                           int32_t pred_mode, bnr_fit_result** res_out) {
+  if (m < 0) return ffail(BNR_EINVAL, "m must be >= 0");
+  if (m > 0 && !X_new) return ffail(BNR_EINVAL, "null X_new");
+  if (pred_mode != BNR_PRED_MEAN && pred_mode != BNR_PRED_PREDICTIVE) return ffail(BNR_EINVAL, "unknown prediction mode");
+  return fit_body(p, X, y, m, X_new, pred_mode, true, res_out);
+}
+
+extern "C" int bnr_fit_loo_pointwise(const bnr_fit_result* r, double* elpd_loo, double* p_loo, double* pareto_k,
+                                     double* elpd_waic, double* p_waic) {
+  if (!r) return ffail(BNR_EINVAL, "null result");
+  if (!r->loo_ok)
+    return ffail(BNR_ESTATE, r->loo ? "fewer than 2 retained draws for PSIS-LOO"
+                                    : "the fit was run without the log-likelihood (bnr_fit_loo)");
+  double* dst[5] = {elpd_loo, p_loo, pareto_k, elpd_waic, p_waic};
+  for (int k = 0; k < 5; ++k)
+    if (dst[k]) memcpy(dst[k], r->l_pw[k].data(), sizeof(double) * r->l_pw[k].size());
+  return BNR_OK;
 }
 
 extern "C" int bnr_fit_prediction(const bnr_fit_result* r, double* mean, double* lo, double* hi) {

@@ -50,6 +50,8 @@ int pred_splits(const Dims& d, int mp);
 void launch_pred_product(const Engine& e, cudaStream_t s);
 // adds the partials in split order, mu_c and (predictive mode) sqrt(tau2_c) z_j, and stores the row at *e.trace_row
 void launch_pred_record(const Engine& e, int sweep_done, cudaStream_t s);
+// pointwise log-likelihood of the current state (needs e.xg == X gamma) into e.ll at *e.trace_row
+void launch_loglik_record(const Engine& e, cudaStream_t s);
 void launch_syrk_G(const Engine& e, cudaStream_t s);         // G_c = X diag(S_c) X' + I (lower tiles)
 int syrk_splits(const Dims& d, int C);                        // k-splits launch_syrk_G uses for a batch of C chains
 // launch_syrk_G computes the n-form Gram matrix on the INT8 tensor cores (Ozaki digit planes) for qp in
@@ -100,6 +102,12 @@ void launch_ess_stream_finalize(const Engine& e, long long N, double* acov, doub
 size_t pred_select_ws_bytes(long long N, int m);
 void launch_pred_select(const double* rows, long long N, int m, long long rank_lo, long long rank_hi, double* mean,
                         double* lo, double* hi, void* ws, cudaStream_t s);
+// pooled PSIS-LOO and WAIC of each of the n columns of rows[N][n] (loo 2.x psis / gpdfit, r_eff = 1); out: [5][n]
+// (elpd_loo, p_loo, pareto_k, elpd_waic, p_waic).  ws: loo_ws_bytes(N, n) bytes; loo_tail_max() bounds the tail length
+long long loo_tail_len(long long N);
+long long loo_tail_max();
+size_t loo_ws_bytes(long long N, int n);
+void launch_loo(const double* rows, long long N, int n, double* out, void* ws, cudaStream_t s);
 void launch_ess_finish(const double* acov_parts, int nparts, const double* cmeans, int chains, int P, long long N,
                        int L, double* ess, double* lag_used, cudaStream_t s);
 

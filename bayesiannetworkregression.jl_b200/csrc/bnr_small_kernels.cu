@@ -828,6 +828,17 @@ __global__ void __launch_bounds__(256) k_pred_record(Engine e, int sweep_done /*
   e.pred[((size_t)c * e.pred_rows + row) * e.pred_m + j] = v;
 }
 
+// one log-likelihood row per chain: ll[c][row][i] = -1/2 log(2 pi tau2_c) - (y_i - mu_c - (X gamma_c)_i)^2 / (2 tau2_c),
+// X gamma from the cache e.xg (valid for the new gamma once launch_finish ran).  grid = (ceil(n / 256), C)
+__global__ void __launch_bounds__(256) k_loglik_record(Engine e) {
+  const int c = blockIdx.y, i = blockIdx.x * blockDim.x + threadIdx.x;
+  const long long row = *e.trace_row;
+  if (i >= e.d.n || row >= e.ll_rows) return;
+  const double t2 = e.tau2[c];
+  const double r = e.y[i] - e.mu[c] - e.xg[(size_t)c * e.d.np + i];
+  e.ll[((size_t)c * e.ll_rows + row) * e.d.n + i] = -0.5 * log(6.283185307179586 * t2) - r * r / (2.0 * t2);
+}
+
 __global__ void k_advance(Engine e, int inc_iter) {
   if (threadIdx.x == 0 && blockIdx.x == 0) {
     if (inc_iter) *e.iter += 1;
@@ -929,6 +940,10 @@ void launch_record(const Engine& e, int sweep_done, cudaStream_t s) {
 void launch_pred_record(const Engine& e, int sweep_done, cudaStream_t s) {
   dim3 grid((e.pred_m + 255) / 256, e.d.C);
   ++g_launches; k_pred_record<<<grid, 256, 0, s>>>(e, sweep_done);
+}
+void launch_loglik_record(const Engine& e, cudaStream_t s) {
+  dim3 grid((e.d.n + 255) / 256, e.d.C);
+  ++g_launches; k_loglik_record<<<grid, 256, 0, s>>>(e);
 }
 void launch_advance(const Engine& e, int inc_iter, cudaStream_t s) { k_advance<<<1, 32, 0, s>>>(e, inc_iter); }
 void launch_rhat(const double* mom, int chains, int nparams, long long h, double* out, cudaStream_t s) {

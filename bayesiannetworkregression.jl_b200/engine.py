@@ -12,6 +12,16 @@ def _dp(a):
     return a.ctypes.data_as(_DP)
 
 
+LOO_FIELDS = ("elpd_loo", "p_loo", "pareto_k", "elpd_waic", "p_waic")
+
+
+def loo_summary(device, dev_ptr, N, n):
+    """bnr_loo_summary on a device table of N draws x n observations: dict of the five pointwise [n] arrays."""
+    out = [np.empty(int(n)) for _ in LOO_FIELDS]
+    check(lib().bnr_loo_summary(int(device), C.c_void_p(dev_ptr), int(N), int(n), *(_dp(a) for a in out)))
+    return dict(zip(LOO_FIELDS, out))
+
+
 class Engine:
     """`Engine(X, y, R, num_chains=...)` uploads the n x q design matrix once and owns every chain's state on
     the device.  X may be C- or F-ordered; it is passed to the library column-major like the reference's
@@ -259,6 +269,28 @@ class Engine:
         check(self._L.bnr_prediction_summary(self.device, C.c_void_p(dev_ptr), int(count), int(m), int(rank_lo),
                                              int(rank_hi), _dp(mean), _dp(lo), _dp(hi)))
         return mean, lo, hi
+
+    # -- pointwise log-likelihood (PSIS-LOO / WAIC) --------------------------------------------------------
+    def set_loglik(self, rows):
+        """Record log N(y_i | mu + (X gamma)_i, tau2) for every observation i at every recorded row of every chain, in
+        a table of `rows` rows per chain (C x rows x n doubles on the device).  rows=0 switches it off."""
+        check(self._L.bnr_set_loglik(self._h, int(rows)))
+
+    def loglik_trace(self, chain, first, last):
+        """Rows [first, last) of one chain's log-likelihood table as an array of shape (last - first, n)."""
+        rows = int(last) - int(first)
+        out = np.empty(rows * self.n)
+        check(self._L.bnr_get_loglik_trace(self._h, int(chain), int(first), int(last), _dp(out)))
+        return out.reshape((rows, self.n), order="F")
+
+    def export_loglik(self, first_row, nrows, dev_ptr):
+        """Rows [first_row, first_row + nrows) of every chain into device memory at dev_ptr as [chain][row][n]."""
+        check(self._L.bnr_export_loglik(self._h, int(first_row), int(nrows), C.c_void_p(dev_ptr)))
+
+    def loo_summary(self, dev_ptr, N, n):
+        """PSIS-LOO and WAIC of N pooled draws x n observations at a device pointer (row-major): a dict of the
+        pointwise arrays elpd_loo, p_loo, pareto_k, elpd_waic, p_waic."""
+        return loo_summary(self.device, dev_ptr, N, n)
 
     # -- state / traces in reference layout ------------------------------------------------------------
     def var_shape(self, var):

@@ -9,11 +9,13 @@ import ctypes as C
 import datetime
 import math
 import random
+import warnings
 
 import numpy as np
 
 from .capi import lib, check, check_fit, FitParams, FitInfo, ALLGATHER_FN, STATE, VAR, GAMMA_MODE, PRED_MEAN, \
     PRED_PREDICTIVE
+from .engine import LOO_FIELDS
 
 _DP = C.POINTER(C.c_double)
 
@@ -198,9 +200,10 @@ _ALLGATHER = ALLGATHER_FN(_torch_allgather)
 def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsamp=0, mingen=0, maxgen=0,
                 psrf_cutoff=1.01, purge_burn=None, num_chains=2, seed=0, device=0, return_state="full", verbose=False,
                 chain_offset=0, n_devices=1, ess_max_lag=0, interval=95, gamma_mode="auto", chain_groups=0, X_new=None,
-                predictive=False):
+                predictive=False, loo=False):
     """One bnr_fit call (include/bnr.h): chain generation, purge ring, PSRF loop, R-hat, Summary statistics on the GPU.
-    With X_new (m x q, already vectorised) the call is bnr_fit_predict, which also pools the predictions."""
+    With X_new (m x q, already vectorised) the call is bnr_fit_predict, which also pools the predictions; with loo=True
+    it is bnr_fit_loo, which also scores the fit by PSIS-LOO and WAIC."""
     L = lib()
     Xf = np.asfortranarray(Xn, dtype=np.float64)
     y = np.ascontiguousarray(y, dtype=np.float64)
@@ -225,12 +228,17 @@ def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsa
     if world > 1:
         p.ext_world, p.ext_rank, p.allgather = world, rank, _ALLGATHER
     res = C.c_void_p()
-    if X_new is None:
-        check_fit(L.bnr_fit(C.byref(p), Xf.ctypes.data_as(_DP), y.ctypes.data_as(_DP), C.byref(res)))
-    else:
+    if X_new is not None:
         Xp = np.asfortranarray(X_new, dtype=np.float64)
         if Xp.ndim != 2 or Xp.shape[1] != q:
             raise ValueError("X_new must hold networks like X (%d edge columns after setup_X)" % q)
+    if loo:
+        m, xp = (0, None) if X_new is None else (Xp.shape[0], Xp.ctypes.data_as(_DP))
+        check_fit(L.bnr_fit_loo(C.byref(p), Xf.ctypes.data_as(_DP), y.ctypes.data_as(_DP), m, xp,
+                                PRED_PREDICTIVE if predictive else PRED_MEAN, C.byref(res)))
+    elif X_new is None:
+        check_fit(L.bnr_fit(C.byref(p), Xf.ctypes.data_as(_DP), y.ctypes.data_as(_DP), C.byref(res)))
+    else:
         check_fit(L.bnr_fit_predict(C.byref(p), Xf.ctypes.data_as(_DP), y.ctypes.data_as(_DP), Xp.shape[0],
                                     Xp.ctypes.data_as(_DP), PRED_PREDICTIVE if predictive else PRED_MEAN,
                                     C.byref(res)))
@@ -260,6 +268,16 @@ def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsa
                 check_fit(rc)
             prediction = dict(interval=interval, mean=pm, lower=pl, upper=ph, predictive=bool(predictive), m=m,
                               draws=int(info.total_chains) * int(info.sampled))
+        loo_out = None
+        if loo:
+            pw = [np.empty(n) for _ in LOO_FIELDS]
+            rc = L.bnr_fit_loo_pointwise(res, *(a.ctypes.data_as(_DP) for a in pw))
+            if rc == -4:                      # BNR_ESTATE: fewer than 2 pooled draws
+                pw = None
+            else:
+                check_fit(rc)
+            loo_out = dict(pointwise=None if pw is None else dict(zip(LOO_FIELDS, pw)),
+                           draws=int(info.total_chains) * int(info.sampled), y=y.copy())
         st = Table()
         rows = int(info.rows)
         shapes = {"tau2": (1, 1), "u": (R, V), "xi": (V, 1), "gamma": (q, 1), "S": (q, 1), "theta": (1, 1),
@@ -284,6 +302,8 @@ def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsa
                      ess=ess)
         if prediction is not None:
             extra["prediction"] = prediction
+        if loo_out is not None:
+            extra["loo"] = loo_out
         return Results(st, rx, rg, int(info.burn_in), int(info.sampled), extra)
     finally:
         L.bnr_fit_free(res)
@@ -293,7 +313,7 @@ def Fit(X, y, R, *, η=None, V=30, ζ=None, ι=None, aΔ=None, bΔ=None, ν=None
         mingen=0, maxgen=0, psrf_cutoff=1.01, x_transform=True, suppress_timer=False, num_chains=2, seed=None,
         purge_burn=None, filename="parameters.log", eta=None, zeta=None, iota=None, a_delta=None, b_delta=None,
         nu=None, device=0, return_state="full", verbose=False, chain_offset=0, n_devices=1, ess_max_lag=0,
-        gamma_mode="auto", chain_groups=0, X_new=None, predictive=False):
+        gamma_mode="auto", chain_groups=0, X_new=None, predictive=False, loo=False):
     """Drop-in for `Fit!(X, y, R; ...)` (src/gibbs.jl:725-751).  Greek keyword names are accepted as in the
     reference; ASCII aliases (eta, zeta, iota, a_delta, b_delta, nu) are equivalent.  Engine-only keywords: device,
     n_devices (GPUs of this process to shard the chains over; num_chains is the count PER GPU), return_state
@@ -303,7 +323,10 @@ def Fit(X, y, R, *, η=None, V=30, ζ=None, ι=None, aΔ=None, bΔ=None, ν=None
     the chains of all ranks.
     X_new (new networks, in the form of X; vectorised by setup_X with the same x_transform): every chain also records
     mu + X_new gamma at every sweep (plus sqrt(tau2) N(0,1) noise with predictive=True, the posterior predictive), and
-    the retained draws of all chains are pooled on the GPU into res.extra["prediction"] (see Predict)."""
+    the retained draws of all chains are pooled on the GPU into res.extra["prediction"] (see Predict).
+    loo=True: every chain also records the pointwise log-likelihood log N(y_i | mu + (X gamma)_i, tau2) at every sweep,
+    and PSIS-LOO and WAIC of the retained draws of all chains are computed on the GPU into res.extra["loo"] (see Loo
+    and Compare)."""
     def pick(greek, ascii_, default):
         return default if (greek is None and ascii_ is None) else (greek if greek is not None else ascii_)
 
@@ -334,7 +357,7 @@ def Fit(X, y, R, *, η=None, V=30, ζ=None, ι=None, aΔ=None, bΔ=None, ν=None
               psrf_cutoff=psrf_cutoff, x_transform=x_transform, num_chains=num_chains, seed=seed,
               purge_burn=purge_burn, device=device, return_state=return_state, verbose=verbose,
               chain_offset=chain_offset, n_devices=n_devices, ess_max_lag=ess_max_lag, gamma_mode=gamma_mode,
-              chain_groups=chain_groups, X_new=X_new, predictive=predictive)
+              chain_groups=chain_groups, X_new=X_new, predictive=predictive, loo=loo)
     if mingen > 0 and maxgen > 0:
         return generate_samples_dbl(X, y, R, mingen=mingen, maxgen=maxgen, **kw)
     return generate_samples(X, y, R, nburn=nburn, nsamp=nsamples, **kw)
@@ -432,3 +455,115 @@ def Predict(results, interval=95, digits=3):
     table = dict(sample=np.arange(1, m + 1, dtype=np.int64), estimate=np.round(pred["mean"], digits),
                  lower_bound=np.round(pred["lower"], digits), upper_bound=np.round(pred["upper"], digits))
     return BNRPrediction(table, interval, bool(pred["predictive"]))
+
+
+# -- out-of-sample scoring (the R package loo: print.loo, loo_compare) ----------------------------------------------
+def _loo_pointwise(results):
+    lo = (getattr(results, "extra", None) or {}).get("loo")
+    if lo is None:
+        raise ValueError("Loo needs a fit scored out of sample: call Fit(..., loo=True)")
+    if lo["pointwise"] is None:
+        raise ValueError("PSIS-LOO needs at least 2 retained draws, the fit kept %d" % lo["draws"])
+    return lo
+
+
+def _estimate(x):
+    x = np.asarray(x, dtype=np.float64)
+    return float(x.sum()), float(math.sqrt(x.size * x.var(ddof=1))) if x.size > 1 else float("nan")
+
+
+class BNRLoo:
+    """Loo's result: `estimates` maps elpd_loo, p_loo, looic, elpd_waic, p_waic, waic to (estimate, SE) with
+    SE = sqrt(n var(pointwise)); `pointwise` holds the [n] arrays (looic / waic are -2 elpd); `n_high_k` counts the
+    observations whose Pareto k exceeds `k_threshold` = min(1 - 1 / log10(S), 0.7) for S pooled draws."""
+
+    NAMES = ("elpd_loo", "p_loo", "looic", "elpd_waic", "p_waic", "waic")
+
+    def __init__(self, pointwise, draws):
+        pw = {k: np.asarray(v, dtype=np.float64) for k, v in pointwise.items()}
+        pw["looic"] = -2.0 * pw["elpd_loo"]
+        pw["waic"] = -2.0 * pw["elpd_waic"]
+        self.pointwise = pw
+        self.draws = int(draws)
+        self.n = int(pw["elpd_loo"].size)
+        self.estimates = {k: _estimate(pw[k]) for k in self.NAMES}
+        self.k_threshold = min(1.0 - 1.0 / math.log10(self.draws), 0.7)
+        self.n_high_k = int(np.sum(pw["pareto_k"] > self.k_threshold))
+
+    def __repr__(self):
+        lines = ["", "Computed from %d by %d log-likelihood matrix." % (self.draws, self.n), "",
+                 "           Estimate      SE"]
+        for k in self.NAMES:
+            e, se = self.estimates[k]
+            lines.append("%-9s %9.1f %7.1f" % (k, e, se))
+        if self.n_high_k:
+            lines.append("")
+            lines.append("Warning: %d of %d Pareto k diagnostic values are above %.2f: PSIS-LOO is unreliable for "
+                         "these observations." % (self.n_high_k, self.n, self.k_threshold))
+        else:
+            lines.append("")
+            lines.append("All Pareto k estimates are good (k <= %.2f)." % self.k_threshold)
+        return "\n".join(lines)
+
+
+def Loo(results):
+    """PSIS-LOO and WAIC of a fit run with Fit(..., loo=True): estimates with standard errors, the pointwise arrays and
+    the Pareto k diagnostic.  The pointwise values were computed on the GPU from the retained draws of ALL chains;
+    only the sums happen here.  Warns (like loo's print method) when some Pareto k are too high."""
+    lo = _loo_pointwise(results)
+    out = BNRLoo(lo["pointwise"], lo["draws"])
+    if out.n_high_k:
+        warnings.warn("%d of %d Pareto k diagnostic values are above %.2f: PSIS-LOO is unreliable for these "
+                      "observations" % (out.n_high_k, out.n, out.k_threshold), stacklevel=2)
+    return out
+
+
+class BNRCompare:
+    """Compare's table: one row per fit, best first (a dict of columns like BNRSummary.edge_coef)."""
+
+    COLUMNS = ("elpd_diff", "se_diff", "elpd_loo", "se_elpd_loo", "p_loo", "se_p_loo", "looic", "se_looic")
+
+    def __init__(self, table):
+        self.table = table
+
+    def __repr__(self):
+        t = self.table
+        lines = ["", "%-10s" % "model" + "".join("%12s" % c for c in self.COLUMNS)]
+        for i, name in enumerate(t["model"]):
+            lines.append("%-10s" % name + "".join("%12.1f" % t[c][i] for c in self.COLUMNS))
+        return "\n".join(lines)
+
+
+def Compare(*results, names=None):
+    """loo_compare: the fits ranked by elpd_loo (best first); elpd_diff = elpd_loo - elpd_loo(best) and
+    se_diff = sqrt(n) sd(pointwise elpd_loo differences to the best), both 0 for the best.  The fits must have been
+    run on the same responses y."""
+    if len(results) < 2:
+        raise ValueError("Compare needs at least two fits")
+    names = list(names) if names is not None else ["model%d" % (i + 1) for i in range(len(results))]
+    if len(names) != len(results):
+        raise ValueError("one name per fit")
+    los = [_loo_pointwise(r) for r in results]
+    y0 = los[0]["y"]
+    for lo in los[1:]:
+        if lo["y"].shape != y0.shape or not np.array_equal(lo["y"], y0):
+            raise ValueError("Compare needs fits of the same responses y")
+    loos = [BNRLoo(lo["pointwise"], lo["draws"]) for lo in los]
+    elpd = np.array([lo.estimates["elpd_loo"][0] for lo in loos])
+    order = sorted(range(len(loos)), key=lambda i: -elpd[i])
+    best = loos[order[0]].pointwise["elpd_loo"]
+    n = best.size
+    table = {c: [] for c in ("model",) + BNRCompare.COLUMNS}
+    for i in order:
+        lo = loos[i]
+        d = lo.pointwise["elpd_loo"] - best
+        table["model"].append(names[i])
+        table["elpd_diff"].append(float(d.sum()))
+        table["se_diff"].append(float(math.sqrt(n) * d.std(ddof=1)) if n > 1 else 0.0)
+        for k in ("elpd_loo", "p_loo", "looic"):
+            e, se = lo.estimates[k]
+            table[k].append(e)
+            table["se_" + k].append(se)
+    for c in BNRCompare.COLUMNS:
+        table[c] = np.asarray(table[c])
+    return BNRCompare(table)

@@ -267,6 +267,24 @@ int bnr_export_predictions(bnr_handle* h, int64_t first_row, int64_t nrows, doub
 int bnr_prediction_summary(int device, const double* dev_rows, int64_t count, int32_t m, int64_t rank_lo,
                            int64_t rank_hi, double* mean, double* lo, double* hi);
 
+/* Pointwise log-likelihood (out-of-sample scoring: PSIS-LOO and WAIC).  Every recorded row of every chain -- row 0 by
+ * bnr_init_state, then one per sweep at the current trace row, moved by bnr_copy_trace_rows like the traces -- also
+ * writes n doubles to the chain's log-likelihood table:
+ *   ll[i] = -1/2 log(2 pi tau2) - (y_i - mu - (X gamma)_i)^2 / (2 tau2)
+ * with the row's own state.  It only reads the state: the chains are bit-identical with and without it.  Rows never
+ * written hold NaN.  rows: capacity of each chain's table (C x rows x n x 8 bytes); 0 switches it off. */
+int bnr_set_loglik(bnr_handle* h, int64_t rows);
+/* rows [first, last) of one local chain, iteration-fastest: out[(r - first) + (last - first) * i] */
+int bnr_get_loglik_trace(bnr_handle* h, int32_t chain, int64_t first, int64_t last, double* out);
+/* rows [first_row, first_row + nrows) of every local chain into caller-owned DEVICE memory as [chain][row][n] */
+int bnr_export_loglik(bnr_handle* h, int64_t first_row, int64_t nrows, double* dev_dst);
+/* PSIS-LOO and WAIC of N pooled draws x n observations at a DEVICE pointer (row-major [N][n]), as the R package loo 2.x
+ * computes them with r_eff = 1 (psis, gpdfit); outputs are HOST arrays of n.  The Pareto tail of ceil(min(0.2 N,
+ * 3 sqrt N)) draws is sorted in one block's shared memory: beyond about 8e7 draws on a B200 the call returns
+ * BNR_EINVAL.  Deterministic: the same table gives bit-identical results. */
+int bnr_loo_summary(int device, const double* dev_rows, int64_t N, int32_t n, double* elpd_loo, double* p_loo,
+                    double* pareto_k, double* elpd_waic, double* p_waic);
+
 /* chain groups (independent streams / CUDA graphs) the handle runs */
 int bnr_chain_groups(bnr_handle* h, int32_t* groups);
 /* which gamma formulation the handle runs (BNR_GAMMA_NFORM / BNR_GAMMA_QFORM; AUTO is resolved at create) */
@@ -287,8 +305,8 @@ int bnr_profile_sweep(bnr_handle* h, float* ms);
  * Chains: base.num_chains chains PER DEVICE on n_devices GPUs of this process (devices base.device, base.device + 1,
  * ...); global chain ids (RNG keys) are base.chain_offset + (ext_rank * n_devices + d) * num_chains + local id.  The only
  * data that crosses NVLink are the split-half moments (32 (V + q) bytes per chain), the ESS statistics and, with
- * bnr_fit_predict, the retained predictions (8 m bytes per chain and draw), exchanged with ncclAllGather inside the
- * library (libnccl.so.2 is loaded at run time; without it, peer copies).  Several
+ * bnr_fit_predict, the retained predictions (8 m bytes per chain and draw) and, with bnr_fit_loo, the retained
+ * log-likelihood rows (8 n bytes per chain and draw), exchanged with ncclAllGather inside the library (libnccl.so.2 is loaded at run time; without it, peer copies).  Several
  * PROCESSES can fit a share each (ext_world > 1): the library then calls `allgather` to exchange across processes.
  * --------------------------------------------------------------------------------------------------------------- */
 #define BNR_STATE_NONE 0       /* no table of chain 1 is kept for bnr_fit_state */
@@ -352,6 +370,17 @@ int bnr_fit_predict(const bnr_fit_params* p, const double* X, const double* y, i
 /* per new network: the mean and the order statistics of ranks round(N (100 - interval) / 200) and
  * round(N (1 - (100 - interval) / 200)) (Julia round) of the N = total_chains x sampled pooled draws; [m] each */
 int bnr_fit_prediction(const bnr_fit_result* r, double* mean, double* lo, double* hi);
+/* bnr_fit_predict (m = 0: no predictions) plus a pointwise log-likelihood table on every chain of every device and
+ * process; the retained rows of all chains are all-gathered in global-chain order and reduced on device 0 by
+ * bnr_loo_summary.  The tables (C x rows x n doubles per device), the export buffers and the pooled buffer
+ * (total_chains x rows x n doubles) are allocated before the first sweep: a fit that cannot hold them fails at once
+ * with BNR_ENOMEM.  All other outputs equal those of bnr_fit_predict with the same arguments. */
+int bnr_fit_loo(const bnr_fit_params* p, const double* X, const double* y, int32_t m, const double* X_new,
+                int32_t pred_mode, bnr_fit_result** out);
+/* per observation [n]: elpd_loo, p_loo, Pareto k, elpd_waic, p_waic over the N = total_chains x sampled pooled draws;
+ * BNR_ESTATE when the fit ran without bnr_fit_loo or kept fewer than 2 draws */
+int bnr_fit_loo_pointwise(const bnr_fit_result* r, double* elpd_loo, double* p_loo, double* pareto_k,
+                          double* elpd_waic, double* p_waic);
 /* The control flow of bnr_fit as a pure host function (no GPU): the engine operations a fit would issue when its k-th
  * PSRF evaluation returns psrf_max[k] as the maximum R-hat of both xi and gamma (NaN allowed; 0 beyond n_psrf).
  * ops: [cap_ops][4] = (op, a, b, c) with op  0 create(trace rows, all chains traced, full-state chains)  1 init

@@ -50,8 +50,8 @@ const PRED_PREDICTIVE = Int32(1)
 
 """
     fit_b200(Xv, y, R; η, ζ, ι, aΔ, bΔ, ν, nburn, nsamp, mingen, maxgen, psrf_cutoff, num_chains, seed, purge_burn,
-             n_devices = 1, X_new = nothing, predictive = false)
-        -> (state::Table, rhatξ::Vector, rhatγ::Vector, burn_in, sampled, prediction)
+             n_devices = 1, X_new = nothing, predictive = false, loo = false)
+        -> (state::Table, rhatξ::Vector, rhatγ::Vector, burn_in, sampled, prediction, loo)
 
 Drop-in for the body of generate_samples! / generate_samples_dbl! after `setup_X!`: `Xv` is the n x q
 `Matrix{Float64}`; the returned arrays have the reference's (iteration, d1, d2) layout, so
@@ -59,22 +59,30 @@ Drop-in for the body of generate_samples! / generate_samples_dbl! after `setup_X
 `num_chains` chains run on EACH of the `n_devices` GPUs (the reference runs one chain per Distributed.jl worker).
 `X_new` (m x q, new networks vectorised by `setup_X!` like `Xv`) runs `bnr_fit_predict`: `prediction` is then
 `(mean, lower, upper)` of μ + X_new γ (+ √τ² z with `predictive = true`) pooled over the retained draws of all chains
-(95 % interval), else `nothing`.
+(95 % interval), else `nothing`.  `loo = true` runs `bnr_fit_loo` (with or without `X_new`): `loo` is then the
+pointwise `(elpd_loo, p_loo, pareto_k, elpd_waic, p_waic)` (vectors of n) of PSIS-LOO and WAIC over the retained draws
+of all chains (`nothing` when fewer than 2 draws were kept), else `nothing`.
 """
 function fit_b200(Xv::Matrix{Float64}, y::Vector{Float64}, R::Integer; η = 1.01, ζ = 1.0, ι = 1.0, aΔ = 1.0, bΔ = 1.0,
                   ν = 10, nburn = 30000, nsamp = 20000, mingen = 0, maxgen = 0, psrf_cutoff = 1.01, num_chains = 2,
                   seed = 1, purge_burn = nothing, n_devices = 1, device = 0, verbose = false,
-                  X_new::Union{Nothing,Matrix{Float64}} = nothing, predictive = false)
+                  X_new::Union{Nothing,Matrix{Float64}} = nothing, predictive = false, loo = false)
     n, q = size(Xv)
     V = Int((-1 + sqrt(1 + 8q)) / 2)
     base = BnrParams(n, V, R, num_chains, 0, device, 1, 0, 0, UInt64(seed), η, ζ, ι, aΔ, bΔ, Float64(ν), 64, 0, 0, 1)
     p = Ref(BnrFitParams(base, nburn, nsamp, mingen, maxgen, psrf_cutoff, isnothing(purge_burn) ? 0 : purge_burn,
                          STATE_FULL, n_devices, 95, 0, verbose ? 1 : 0, 0, 0, C_NULL, C_NULL))
     res = Ref{Ptr{Cvoid}}(C_NULL)
-    if X_new === nothing
+    X_new === nothing || size(X_new, 2) == q || error("X_new must have the q = $q columns of Xv")
+    if loo
+        m = X_new === nothing ? 0 : size(X_new, 1)
+        check(ccall((:bnr_fit_loo, libbnr), Cint,
+                    (Ref{BnrFitParams}, Ptr{Float64}, Ptr{Float64}, Int32, Ptr{Float64}, Int32, Ref{Ptr{Cvoid}}),
+                    p, Xv, y, Int32(m), X_new === nothing ? Ptr{Float64}(C_NULL) : X_new,
+                    predictive ? PRED_PREDICTIVE : PRED_MEAN, res))
+    elseif X_new === nothing
         check(ccall((:bnr_fit, libbnr), Cint, (Ref{BnrFitParams}, Ptr{Float64}, Ptr{Float64}, Ref{Ptr{Cvoid}}), p, Xv, y, res))
     else
-        size(X_new, 2) == q || error("X_new must have the q = $q columns of Xv")
         check(ccall((:bnr_fit_predict, libbnr), Cint,
                     (Ref{BnrFitParams}, Ptr{Float64}, Ptr{Float64}, Int32, Ptr{Float64}, Int32, Ref{Ptr{Cvoid}}),
                     p, Xv, y, Int32(size(X_new, 1)), X_new, predictive ? PRED_PREDICTIVE : PRED_MEAN, res))
@@ -103,7 +111,15 @@ function fit_b200(Xv::Matrix{Float64}, y::Vector{Float64}, R::Integer; η = 1.01
                         res[], pm, pl, ph))
             prediction = (mean = pm, lower = pl, upper = ph)
         end
-        return state, rξ, rγ, Int(info[].burn_in), Int(info[].sampled), prediction
+        pointwise = nothing
+        if loo
+            pw = ntuple(_ -> Vector{Float64}(undef, n), 5)
+            rc = ccall((:bnr_fit_loo_pointwise, libbnr), Cint,
+                       (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}), res[], pw...)
+            rc == -4 || check(rc)           # BNR_ESTATE: fewer than 2 retained draws
+            rc == 0 && (pointwise = (elpd_loo = pw[1], p_loo = pw[2], pareto_k = pw[3], elpd_waic = pw[4], p_waic = pw[5]))
+        end
+        return state, rξ, rγ, Int(info[].burn_in), Int(info[].sampled), prediction, pointwise
     finally
         ccall((:bnr_fit_free, libbnr), Cint, (Ptr{Cvoid},), res[])
     end

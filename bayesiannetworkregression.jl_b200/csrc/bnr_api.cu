@@ -194,6 +194,16 @@ static int dalloc(bnr_handle* h, T** ptr, size_t count, bool zero = true) {
   *ptr = (T*)p;
   return 0;
 }
+// the buffer of a row table whose shape is set; nan_fill: rows never written read as NaN.  A refusal names the table and
+// its size and is cleared, so that it does not surface in a later call
+static int alloc_table(bnr_handle* h, RowTable& t, bool nan_fill, const char* what) {
+  if (int r = dalloc(h, &t.base, t.doubles(), false)) {
+    cudaGetLastError();
+    return fail(r, std::string(what) + " (" + std::to_string(8.0 * (double)t.doubles()) + " bytes): " + g_err);
+  }
+  if (nan_fill) CK(cudaMemsetAsync(t.base, 0xff, sizeof(double) * t.doubles(), h->stream));
+  return BNR_OK;
+}
 #define DA(ptr, count)                          \
   do {                                          \
     int _r = dalloc(h, &(ptr), (count));        \
@@ -396,24 +406,17 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
   DA(h->d_esswin, 4);
   DA(h->ws, x_times_workspace_doubles(d));
   DA(h->d_rhat, (size_t)(d.V + d.q));
-  e.trace_full_chains = p->trace_rows > 0 ? (p->trace_full_chains < d.C ? p->trace_full_chains : d.C) : 0;
-  if (e.trace_full_chains < 0) e.trace_full_chains = 0;
-  e.trace_gx_chains = 0;
-  if (p->trace_rows > 0) {
-    if (p->trace_gamma_xi_all) e.trace_gx_chains = d.C;
-    else if (p->trace_gamma_xi_chains > 0) e.trace_gx_chains = p->trace_gamma_xi_chains < d.C ? p->trace_gamma_xi_chains : d.C;
+  const long long trace_rows = p->trace_rows > 0 ? p->trace_rows : 0;
+  e.tr_full = {nullptr, trace_rows, 4 + d.V * d.R + d.V + 2 * d.q + d.R * d.R + d.R + 3 * d.R, 0};
+  e.tr_gx = {nullptr, trace_rows, d.V + d.q, 0};
+  if (trace_rows > 0) {
+    e.tr_full.chains = p->trace_full_chains < 0 ? 0 : (p->trace_full_chains < d.C ? p->trace_full_chains : d.C);
+    if (p->trace_gamma_xi_all) e.tr_gx.chains = d.C;
+    else if (p->trace_gamma_xi_chains > 0) e.tr_gx.chains = p->trace_gamma_xi_chains < d.C ? p->trace_gamma_xi_chains : d.C;
   }
-  e.trace_rows = p->trace_rows > 0 ? p->trace_rows : 0;
-  e.rowlen_full = 4 + d.V * d.R + d.V + 2 * d.q + d.R * d.R + d.R + 3 * d.R;
-  e.tr_full = nullptr; e.tr_gx = nullptr;
-  if (e.trace_full_chains > 0) {
-    int r = dalloc(h, &e.tr_full, (size_t)e.trace_full_chains * e.trace_rows * e.rowlen_full, false);
-    if (r) return r;
-  }
-  if (e.trace_gx_chains > 0) {
-    int r = dalloc(h, &e.tr_gx, (size_t)e.trace_gx_chains * e.trace_rows * (d.V + d.q), false);
-    if (r) return r;
-  }
+  // traces are not NaN-filled: a memset of a multi-GB trace would cost time at every create
+  if (e.tr_full.chains > 0) if (int r = alloc_table(h, e.tr_full, false, "full-state trace")) return r;
+  if (e.tr_gx.chains > 0) if (int r = alloc_table(h, e.tr_gx, false, "gamma/xi trace")) return r;
   {
     // chain groups (see ChainGroup): 2 by default once there are enough chains to split
     // default: 2 groups once the SYRK of half the chains fills the GPU for several waves; 4 when the chains are few
@@ -609,8 +612,8 @@ static void enqueue_sweep(Engine& e, double* ws, const ForkJoin& fj, cudaStream_
   { NvtxRange r("gamma + D (GIG)"); run_gamma(e, ws, fj, s, 3, fork_syrk); }
   // predictions for new networks: X_new gamma depends on gamma only, so it runs on the side stream next to the scalar
   // conditionals and joins before k_pred_record, which needs the new mu (and tau2)
-  const bool fork_pred = e.pred_m > 0 && fj.side != nullptr;
-  if (e.pred_m > 0) {
+  const bool fork_pred = e.pred.base && fj.side != nullptr;
+  if (e.pred.base) {
     NvtxRange r("predictions: X_new gamma");
     if (fork_pred) {
       cudaEventRecord(fj.fork, s);
@@ -630,11 +633,11 @@ static void enqueue_sweep(Engine& e, double* ws, const ForkJoin& fj, cudaStream_
   NvtxRange r("record");
   launch_record(e, 1, s);
   if (e.ess_ring) launch_ess_stream(e, s);
-  if (e.pred_m > 0) {
+  if (e.pred.base) {
     if (fork_pred) cudaStreamWaitEvent(s, fj.join, 0);
     launch_pred_record(e, 1, s);
   }
-  if (e.ll) launch_loglik_record(e, s);
+  if (e.ll.base) launch_loglik_record(e, s);
   launch_advance(e, 1, s);
 }
 
@@ -662,21 +665,9 @@ static Engine group_view(const bnr_handle* h, int c0, int Cg, long long* counter
     v.ess_ring += c * (size_t)v.ess_cap * P; v.ess_head += c * (size_t)v.ess_L * P;
     v.ess_acc += c * (size_t)(v.ess_L + 1) * P; v.ess_sum += c * 2 * P;
   }
-  int tgc = h->e.trace_gx_chains - c0;
-  tgc = tgc < 0 ? 0 : (tgc > Cg ? Cg : tgc);
-  v.trace_gx_chains = tgc;
-  if (v.tr_gx) v.tr_gx += c * v.trace_rows * (d.V + d.q);
-  if (tgc == 0) v.tr_gx = nullptr;
-  int tfc = h->e.trace_full_chains - c0;
-  tfc = tfc < 0 ? 0 : (tfc > Cg ? Cg : tfc);
-  v.trace_full_chains = tfc;
-  if (v.tr_full) v.tr_full += c * v.trace_rows * v.rowlen_full;
-  if (tfc == 0) v.tr_full = nullptr;
-  if (v.pred) {
-    v.pred += c * (size_t)v.pred_rows * v.pred_m;
-    v.pred_ws += c * (size_t)v.pred_splits * v.pred_mp;
-  }
-  if (v.ll) v.ll += c * (size_t)v.ll_rows * d.n;
+  v.tr_full = v.tr_full.view(c0, Cg); v.tr_gx = v.tr_gx.view(c0, Cg);
+  v.pred = v.pred.view(c0, Cg); v.ll = v.ll.view(c0, Cg);
+  if (v.pred_ws) v.pred_ws += c * (size_t)v.pred_splits * v.pred_mp;
   v.iter = counters; v.trace_row = counters + 1; v.mom_window = mom_window;
   v.inj = nullptr; v.inj_stride = 0;
   memset(&v.aux, 0, sizeof(v.aux));
@@ -719,11 +710,11 @@ extern "C" int bnr_init_state(bnr_handle* h) {
   CK(cudaMemsetAsync(e.status, 0, sizeof(int) * e.d.C, h->stream));
   launch_init(e, h->stream);
   launch_record(e, 0, h->stream);
-  if (e.pred_m > 0) {
+  if (e.pred.base) {
     launch_pred_product(e, h->stream);
     launch_pred_record(e, 0, h->stream);
   }
-  if (e.ll) {
+  if (e.ll.base) {
     refresh_xg(h);                     // X gamma_0: the cache is not valid after launch_init
     launch_loglik_record(e, h->stream);
   }
@@ -832,36 +823,33 @@ extern "C" int bnr_copy_trace_rows(bnr_handle* h, int64_t dst, int64_t src, int6
   if (!h || dst < 0 || src < 0 || count < 0) return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
   Engine& e = h->e;
-  // every per-chain table the record kernels write at *trace_row: traces, predictions, log-likelihood
-  struct Table { double* base; size_t rowlen; int chains; long long rows; const char* range_msg; };
-  Table tabs[4];
-  int nt = 0;
-  if (e.trace_rows > 0 && e.tr_full)
-    tabs[nt++] = {e.tr_full, (size_t)e.rowlen_full, e.trace_full_chains, e.trace_rows, "rows out of range"};
-  if (e.trace_rows > 0 && e.tr_gx)
-    tabs[nt++] = {e.tr_gx, (size_t)(e.d.V + e.d.q), e.trace_gx_chains, e.trace_rows, "rows out of range"};
-  if (e.pred_m > 0) tabs[nt++] = {e.pred, (size_t)e.pred_m, e.d.C, e.pred_rows, "rows beyond the prediction table"};
-  if (e.ll) tabs[nt++] = {e.ll, (size_t)e.d.n, e.d.C, e.ll_rows, "rows beyond the log-likelihood table"};
-  if (nt == 0) return BNR_OK;               // this handle records no per-row tables: nothing to move
-  size_t max_row = 0;
-  for (int t = 0; t < nt; ++t) {
-    if (dst + count > tabs[t].rows || src + count > tabs[t].rows) return fail(BNR_EINVAL, tabs[t].range_msg);
-    if (tabs[t].rowlen > max_row) max_row = tabs[t].rowlen;
+  // every row table of the engine: the record kernels write all of them at *trace_row
+  const struct { const RowTable& t; const char* range_msg; } all[] = {
+      {e.tr_full, "rows out of range"}, {e.tr_gx, "rows out of range"},
+      {e.pred, "rows beyond the prediction table"}, {e.ll, "rows beyond the log-likelihood table"}};
+  bool any = false;
+  int max_row = 0;
+  for (const auto& a : all) {
+    if (!a.t.base) continue;
+    if (dst + count > a.t.rows || src + count > a.t.rows) return fail(BNR_EINVAL, a.range_msg);
+    if (a.t.width > max_row) max_row = a.t.width;
+    any = true;
   }
+  if (!any) return BNR_OK;                  // this handle records no per-row tables: nothing to move
   if (count == 0 || dst == src) return BNR_OK;
   // rows are contiguous per chain; regions may overlap -> stage through one temporary (stream order keeps the chains apart)
   const bool overlap = !(dst + count <= src || src + count <= dst);
   Scratch sc(h->p.device, overlap ? (size_t)count * max_row * sizeof(double) : 256);
   if (overlap && !sc.p) return fail(BNR_ENOMEM, "device scratch allocation failed");
-  for (int t = 0; t < nt; ++t) {
-    const size_t rowlen = tabs[t].rowlen, bytes = (size_t)count * rowlen * sizeof(double);
-    for (int c = 0; c < tabs[t].chains; ++c) {
-      double* b = tabs[t].base + (size_t)c * tabs[t].rows * rowlen;
+  for (const auto& a : all) {
+    if (!a.t.base) continue;
+    const size_t bytes = (size_t)count * a.t.width * sizeof(double);
+    for (int c = 0; c < a.t.chains; ++c) {
       if (!overlap) {
-        CK(cudaMemcpyAsync(b + (size_t)dst * rowlen, b + (size_t)src * rowlen, bytes, cudaMemcpyDeviceToDevice, h->stream));
+        CK(cudaMemcpyAsync(a.t.row(c, dst), a.t.row(c, src), bytes, cudaMemcpyDeviceToDevice, h->stream));
       } else {
-        CK(cudaMemcpyAsync(sc.p, b + (size_t)src * rowlen, bytes, cudaMemcpyDeviceToDevice, h->stream));
-        CK(cudaMemcpyAsync(b + (size_t)dst * rowlen, sc.p, bytes, cudaMemcpyDeviceToDevice, h->stream));
+        CK(cudaMemcpyAsync(sc.p, a.t.row(c, src), bytes, cudaMemcpyDeviceToDevice, h->stream));
+        CK(cudaMemcpyAsync(a.t.row(c, dst), sc.p, bytes, cudaMemcpyDeviceToDevice, h->stream));
       }
     }
   }
@@ -967,14 +955,13 @@ extern "C" int bnr_rhat_from_moments(int device, const double* dev_moments, int3
 
 // two-pass split-half moments of rows [first_row, first_row + nrows) of the gamma/xi traces (what
 // return_psrf_VOI + rhat see, src/gibbs.jl:771-789).  grid = (ceil((V+q)/128), C, 2)
-__global__ void k_moments_from_trace(const double* __restrict__ tr, long long trace_rows, int nparam, long long first,
-                                     long long nrows, double* __restrict__ mom) {
-  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+__global__ void k_moments_from_trace(RowTable tr, long long first, long long nrows, double* __restrict__ mom) {
+  const int nparam = tr.width, p = blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= nparam) return;
   const int c = blockIdx.y, half = blockIdx.z;
   const long long h = nrows / 2;
   const long long r0 = first + (half == 0 ? 0 : nrows - h);
-  const double* base = tr + ((size_t)c * trace_rows + r0) * nparam + p;
+  const double* __restrict__ base = tr.row(c, r0) + p;
   double s = 0.0;
   for (long long r = 0; r < h; ++r) s += base[(size_t)r * nparam];
   const double mean = s / (double)h;
@@ -988,14 +975,13 @@ extern "C" int bnr_moments_from_trace(bnr_handle* h, int64_t first_row, int64_t 
   if (!h || first_row < 0 || nrows < 0) return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
   Engine& e = h->e;
-  if (!e.tr_gx || e.trace_gx_chains < e.d.C)
+  if (!e.tr_gx.base || e.tr_gx.chains < e.d.C)
     return fail(BNR_ESTATE, "gamma/xi traces of every chain are needed (trace_gamma_xi_all = 0): use the streaming "
                             "moments of bnr_set_moment_window instead");
-  if (first_row + nrows > e.trace_rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
+  if (first_row + nrows > e.tr_gx.rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
   if (nrows / 2 < 2) return fail(BNR_EINVAL, "need at least 4 rows");
-  const int np_ = e.d.V + e.d.q;
-  dim3 grid((np_ + 127) / 128, e.d.C, 2);
-  k_moments_from_trace<<<grid, 128, 0, h->stream>>>(e.tr_gx, e.trace_rows, np_, first_row, nrows, e.moments);
+  dim3 grid((e.tr_gx.width + 127) / 128, e.d.C, 2);
+  k_moments_from_trace<<<grid, 128, 0, h->stream>>>(e.tr_gx, first_row, nrows, e.moments);
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
   h->mom_half = nrows / 2;
@@ -1092,27 +1078,28 @@ __global__ void k_gather_trace(const double* __restrict__ rows, size_t rowlen, i
   out[idx] = rows[(size_t)(first + it) * rowlen + off + src];
 }
 
+// the trace table that holds variable `var` of `chain` and the variable's offset in its rows (nullptr: not traced)
+static const RowTable* traced(const Engine& e, int chain, int var, int* off) {
+  if (e.tr_full.holds(chain, 0)) { *off = row_offset(e.d, var); return &e.tr_full; }
+  if (e.tr_gx.holds(chain, 0) && (var == BNR_VAR_XI || var == BNR_VAR_GAMMA)) {
+    *off = var == BNR_VAR_XI ? 0 : e.d.V;
+    return &e.tr_gx;
+  }
+  return nullptr;
+}
+
 extern "C" int bnr_get_trace(bnr_handle* h, int32_t chain, int32_t var, int64_t first, int64_t last, double* out) {
   if (!h || !out || chain < 0 || chain >= h->e.d.C || var < 0 || var >= BNR_NUM_VARS || first < 0 || last < first)
     return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
   Engine& e = h->e;
-  if (last > e.trace_rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
+  if (last > e.tr_full.rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
   const Dims& d = e.d;
-  const double* rows = nullptr;
-  size_t rowlen = 0;
   int off = 0;
-  if (chain < e.trace_full_chains && e.tr_full) {
-    rowlen = e.rowlen_full;
-    rows = e.tr_full + (size_t)chain * e.trace_rows * rowlen;
-    off = row_offset(d, var);
-  } else if (e.tr_gx && chain < e.trace_gx_chains && (var == BNR_VAR_XI || var == BNR_VAR_GAMMA)) {
-    rowlen = d.V + d.q;
-    rows = e.tr_gx + (size_t)chain * e.trace_rows * rowlen;
-    off = var == BNR_VAR_XI ? 0 : d.V;
-  } else {
-    return fail(BNR_ESTATE, "this variable of this chain is not traced (see trace_full_chains / trace_gamma_xi_all)");
-  }
+  const RowTable* t = traced(e, chain, var, &off);
+  if (!t) return fail(BNR_ESTATE, "this variable of this chain is not traced (see trace_full_chains / trace_gamma_xi_all)");
+  const double* rows = t->row(chain, 0);
+  const size_t rowlen = t->width;
   const int nelem = var_size(d, var);
   const long long count = last - first;
   if (count == 0) return BNR_OK;
@@ -1305,11 +1292,11 @@ extern "C" int bnr_finish_sweep(bnr_handle* h) {
   CK(cudaSetDevice(h->p.device));
   launch_record(h->e, 1, h->stream);
   if (h->e.ess_ring) launch_ess_stream(h->e, h->stream);
-  if (h->e.pred_m > 0) {
+  if (h->e.pred.base) {
     launch_pred_product(h->e, h->stream);
     launch_pred_record(h->e, 1, h->stream);
   }
-  if (h->e.ll) {
+  if (h->e.ll.base) {
     if (!h->xg_valid) refresh_xg(h);
     launch_loglik_record(h->e, h->stream);
   }
@@ -1371,24 +1358,16 @@ extern "C" int bnr_summary(bnr_handle* h, int32_t chain, int64_t first_row, int6
   CK(cudaSetDevice(h->p.device));
   Engine& e = h->e;
   const Dims& d = e.d;
-  if (first_row + nrows > e.trace_rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
+  if (first_row + nrows > e.tr_full.rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
   if (rank_lo < 1 || rank_hi < 1 || rank_lo > nrows || rank_hi > nrows)
     return fail(BNR_EINVAL, "order-statistic ranks must lie in 1..nrows (the reference raises a BoundsError)");
   CK(cudaSetDevice(h->p.device));
-  const double* rows = nullptr;
-  size_t rowlen = 0;
   int off_g = 0, off_x = 0;
-  if (chain < e.trace_full_chains && e.tr_full) {
-    rowlen = e.rowlen_full;
-    rows = e.tr_full + (size_t)chain * e.trace_rows * rowlen;
-    off_g = row_offset(d, BNR_VAR_GAMMA); off_x = row_offset(d, BNR_VAR_XI);
-  } else if (e.tr_gx && chain < e.trace_gx_chains) {
-    rowlen = d.V + d.q;
-    rows = e.tr_gx + (size_t)chain * e.trace_rows * rowlen;
-    off_g = d.V; off_x = 0;
-  } else {
-    return fail(BNR_ESTATE, "gamma/xi of this chain are not traced");
-  }
+  const RowTable* t = traced(e, chain, BNR_VAR_GAMMA, &off_g);
+  if (!t) return fail(BNR_ESTATE, "gamma/xi of this chain are not traced");
+  traced(e, chain, BNR_VAR_XI, &off_x);     // (the same table)
+  const double* rows = t->row(chain, 0);
+  const size_t rowlen = t->width;
   if ((size_t)(3 * d.q + d.V) > h->tmp_doubles) return fail(BNR_EINVAL, "staging buffer too small");
   double* o = h->d_tmp;
   launch_summary_select(rows, rowlen, off_g, d.q, first_row, nrows, rank_lo, rank_hi, o, o + d.q, o + 2 * d.q, h->stream);
@@ -1412,9 +1391,9 @@ extern "C" int bnr_ess_accumulate(bnr_handle* h, int64_t first_row, int64_t nrow
   CK(cudaSetDevice(h->p.device));
   Engine& e = h->e;
   const Dims& d = e.d;
-  if (!e.tr_gx || e.trace_gx_chains < d.C)
+  if (!e.tr_gx.base || e.tr_gx.chains < d.C)
     return fail(BNR_ESTATE, "gamma/xi traces of every chain are not recorded (trace_gamma_xi_all = 0)");
-  if (first_row + nrows > e.trace_rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
+  if (first_row + nrows > e.tr_gx.rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
   if (max_lag > nrows - 1) max_lag = (int32_t)(nrows - 1);
   if (!(max_lag & 1)) max_lag -= 1;                  // Geyer pairs (2t, 2t+1): keep the last lag odd
   if (max_lag < 1) max_lag = 1;
@@ -1431,8 +1410,8 @@ extern "C" int bnr_ess_accumulate(bnr_handle* h, int64_t first_row, int64_t nrow
     h->acov_cap = need;
   }
   if (!h->d_cmean) DA(h->d_cmean, (size_t)d.C * P);
-  launch_chain_mean(e.tr_gx, e.trace_rows, P, d.C, first_row, nrows, h->d_cmean, h->stream);
-  launch_acov_sum(e.tr_gx, e.trace_rows, P, d.C, first_row, nrows, max_lag, h->d_cmean, h->d_acov, h->stream);
+  launch_chain_mean(e.tr_gx, first_row, nrows, h->d_cmean, h->stream);
+  launch_acov_sum(e.tr_gx, first_row, nrows, max_lag, h->d_cmean, h->d_acov, h->stream);
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
   h->ess_lag = max_lag;
@@ -1690,11 +1669,34 @@ extern "C" int bnr_profile_sweep(bnr_handle* h, float* ms) {
 static void drop_predictors(bnr_handle* h) {
   Engine& e = h->e;
   release_alloc(h, const_cast<double*>(e.Xp));
-  release_alloc(h, e.pred);
+  release_alloc(h, e.pred.base);
   release_alloc(h, e.pred_ws);
-  e.Xp = nullptr; e.pred = nullptr; e.pred_ws = nullptr;
-  e.pred_m = e.pred_mp = e.pred_mode = e.pred_splits = 0;
-  e.pred_rows = 0;
+  e.Xp = nullptr; e.pred = {}; e.pred_ws = nullptr;
+  e.pred_mp = e.pred_mode = e.pred_splits = 0;
+}
+
+// rows [first, last) of one chain of a row table into out[row + count * column] (iteration fastest, like the traces)
+static int get_table_rows(bnr_handle* h, const RowTable& t, int chain, int64_t first, int64_t last, double* out) {
+  CK(cudaSetDevice(h->p.device));
+  const size_t count = (size_t)(last - first), w = (size_t)t.width;
+  if (count == 0) return BNR_OK;
+  std::vector<double> tmp(count * w);
+  CK(cudaMemcpyAsync(tmp.data(), t.row(chain, first), sizeof(double) * tmp.size(), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  for (size_t r = 0; r < count; ++r)
+    for (size_t j = 0; j < w; ++j) out[r + count * j] = tmp[r * w + j];
+  return BNR_OK;
+}
+
+// rows [first_row, first_row + nrows) of every chain of a row table into dev_dst, [chain][nrows][width]
+static int export_table_rows(bnr_handle* h, const RowTable& t, int64_t first_row, int64_t nrows, double* dev_dst) {
+  CK(cudaSetDevice(h->p.device));
+  if (nrows == 0) return BNR_OK;
+  const size_t rowb = sizeof(double) * (size_t)t.width;
+  CK(cudaMemcpy2DAsync(dev_dst, rowb * nrows, t.row(0, first_row), rowb * t.rows, rowb * nrows, (size_t)t.chains,
+                       cudaMemcpyDeviceToDevice, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  return BNR_OK;
 }
 
 extern "C" int bnr_set_predictors(bnr_handle* h, int32_t m, const double* X_new, int64_t rows, int32_t mode) {
@@ -1712,56 +1714,38 @@ extern "C" int bnr_set_predictors(bnr_handle* h, int32_t m, const double* X_new,
   const Dims& d = e.d;
   const int mp = (m + TILE_N - 1) / TILE_N * TILE_N;
   const int ks = pred_splits(d, mp);
-  double *xp = nullptr, *pred = nullptr, *ws = nullptr;
+  RowTable pred = {nullptr, rows, m, d.C};
+  if (int r = alloc_table(h, pred, true, "prediction table")) return r;
+  double *xp = nullptr, *ws = nullptr;
   int r = dalloc(h, &xp, (size_t)d.qp * mp);
-  if (!r) r = dalloc(h, &pred, (size_t)d.C * rows * m, false);
   if (!r) r = dalloc(h, &ws, (size_t)ks * d.C * mp, false);
   if (r) {
     cudaGetLastError();                // a refused cudaMalloc must not surface in a later call
-    release_alloc(h, xp); release_alloc(h, pred); release_alloc(h, ws);
-    return fail(r, "prediction buffers (" + std::to_string(8.0 * ((double)d.qp * mp + (double)d.C * rows * m +
-                                                                   (double)ks * d.C * mp)) +
-                       " bytes): " + g_err);
+    release_alloc(h, pred.base); release_alloc(h, xp); release_alloc(h, ws);
+    return fail(r, "X_new and the split-K partials of the predictions (" +
+                       std::to_string(8.0 * ((double)d.qp * mp + (double)ks * d.C * mp)) + " bytes): " + g_err);
   }
   // X_new: m x q column-major host -> columns padded to mp rows (zeros beyond m and beyond q, like X)
   CK(cudaMemcpy2DAsync(xp, (size_t)mp * sizeof(double), X_new, (size_t)m * sizeof(double), (size_t)m * sizeof(double),
                        (size_t)d.q, cudaMemcpyHostToDevice, h->stream));
-  CK(cudaMemsetAsync(pred, 0xff, sizeof(double) * (size_t)d.C * rows * m, h->stream));   // NaN: rows never written
   CK(cudaStreamSynchronize(h->stream));
   e.Xp = xp; e.pred = pred; e.pred_ws = ws;
-  e.pred_m = m; e.pred_mp = mp; e.pred_mode = mode; e.pred_splits = ks; e.pred_rows = rows;
+  e.pred_mp = mp; e.pred_mode = mode; e.pred_splits = ks;
   return BNR_OK;
 }
 
 extern "C" int bnr_get_prediction_trace(bnr_handle* h, int32_t chain, int64_t first, int64_t last, double* out) {
   if (!h || !out || chain < 0 || chain >= h->e.d.C || first < 0 || last < first) return fail(BNR_EINVAL, "bad arguments");
-  const Engine& e = h->e;
-  if (e.pred_m == 0) return fail(BNR_ESTATE, "no predictors set (bnr_set_predictors)");
-  if (last > e.pred_rows) return fail(BNR_EINVAL, "rows beyond the prediction table");
-  CK(cudaSetDevice(h->p.device));
-  const size_t count = (size_t)(last - first), m = (size_t)e.pred_m;
-  if (count == 0) return BNR_OK;
-  std::vector<double> tmp(count * m);
-  CK(cudaMemcpyAsync(tmp.data(), e.pred + ((size_t)chain * e.pred_rows + first) * m, sizeof(double) * tmp.size(),
-                     cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  for (size_t r = 0; r < count; ++r)
-    for (size_t j = 0; j < m; ++j) out[r + count * j] = tmp[r * m + j];
-  return BNR_OK;
+  if (!h->e.pred.base) return fail(BNR_ESTATE, "no predictors set (bnr_set_predictors)");
+  if (last > h->e.pred.rows) return fail(BNR_EINVAL, "rows beyond the prediction table");
+  return get_table_rows(h, h->e.pred, chain, first, last, out);
 }
 
 extern "C" int bnr_export_predictions(bnr_handle* h, int64_t first_row, int64_t nrows, double* dev_dst) {
   if (!h || !dev_dst || first_row < 0 || nrows < 0) return fail(BNR_EINVAL, "bad arguments");
-  const Engine& e = h->e;
-  if (e.pred_m == 0) return fail(BNR_ESTATE, "no predictors set (bnr_set_predictors)");
-  if (first_row + nrows > e.pred_rows) return fail(BNR_EINVAL, "rows beyond the prediction table");
-  CK(cudaSetDevice(h->p.device));
-  if (nrows == 0) return BNR_OK;
-  const size_t rowb = sizeof(double) * (size_t)e.pred_m;
-  CK(cudaMemcpy2DAsync(dev_dst, rowb * nrows, e.pred + (size_t)first_row * e.pred_m, rowb * e.pred_rows, rowb * nrows,
-                       (size_t)e.d.C, cudaMemcpyDeviceToDevice, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  return BNR_OK;
+  if (!h->e.pred.base) return fail(BNR_ESTATE, "no predictors set (bnr_set_predictors)");
+  if (first_row + nrows > h->e.pred.rows) return fail(BNR_EINVAL, "rows beyond the prediction table");
+  return export_table_rows(h, h->e.pred, first_row, nrows, dev_dst);
 }
 
 extern "C" int bnr_prediction_summary(int device, const double* dev_rows, int64_t count, int32_t m, int64_t rank_lo,
@@ -1799,50 +1783,28 @@ extern "C" int bnr_set_loglik(bnr_handle* h, int64_t rows) {
   CK(cudaStreamSynchronize(h->stream));
   drop_graph(h);                       // the captured sweeps gain or lose the k_loglik_record node
   Engine& e = h->e;
-  release_alloc(h, e.ll);
-  e.ll = nullptr; e.ll_rows = 0;
+  release_alloc(h, e.ll.base);
+  e.ll = {};
   if (rows == 0) return BNR_OK;
-  const size_t count = (size_t)e.d.C * rows * e.d.n;
-  double* ll = nullptr;
-  if (int r = dalloc(h, &ll, count, false)) {
-    cudaGetLastError();                // a refused cudaMalloc must not surface in a later call
-    return fail(r, "log-likelihood table (" + std::to_string(8.0 * (double)count) + " bytes): " + g_err);
-  }
-  CK(cudaMemsetAsync(ll, 0xff, sizeof(double) * count, h->stream));   // NaN: rows never written
+  RowTable ll = {nullptr, rows, e.d.n, e.d.C};
+  if (int r = alloc_table(h, ll, true, "log-likelihood table")) return r;
   CK(cudaStreamSynchronize(h->stream));
-  e.ll = ll; e.ll_rows = rows;
+  e.ll = ll;
   return BNR_OK;
 }
 
 extern "C" int bnr_get_loglik_trace(bnr_handle* h, int32_t chain, int64_t first, int64_t last, double* out) {
   if (!h || !out || chain < 0 || chain >= h->e.d.C || first < 0 || last < first) return fail(BNR_EINVAL, "bad arguments");
-  const Engine& e = h->e;
-  if (!e.ll) return fail(BNR_ESTATE, "no log-likelihood table (bnr_set_loglik)");
-  if (last > e.ll_rows) return fail(BNR_EINVAL, "rows beyond the log-likelihood table");
-  CK(cudaSetDevice(h->p.device));
-  const size_t count = (size_t)(last - first), n = (size_t)e.d.n;
-  if (count == 0) return BNR_OK;
-  std::vector<double> tmp(count * n);
-  CK(cudaMemcpyAsync(tmp.data(), e.ll + ((size_t)chain * e.ll_rows + first) * n, sizeof(double) * tmp.size(),
-                     cudaMemcpyDeviceToHost, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  for (size_t r = 0; r < count; ++r)
-    for (size_t i = 0; i < n; ++i) out[r + count * i] = tmp[r * n + i];
-  return BNR_OK;
+  if (!h->e.ll.base) return fail(BNR_ESTATE, "no log-likelihood table (bnr_set_loglik)");
+  if (last > h->e.ll.rows) return fail(BNR_EINVAL, "rows beyond the log-likelihood table");
+  return get_table_rows(h, h->e.ll, chain, first, last, out);
 }
 
 extern "C" int bnr_export_loglik(bnr_handle* h, int64_t first_row, int64_t nrows, double* dev_dst) {
   if (!h || !dev_dst || first_row < 0 || nrows < 0) return fail(BNR_EINVAL, "bad arguments");
-  const Engine& e = h->e;
-  if (!e.ll) return fail(BNR_ESTATE, "no log-likelihood table (bnr_set_loglik)");
-  if (first_row + nrows > e.ll_rows) return fail(BNR_EINVAL, "rows beyond the log-likelihood table");
-  CK(cudaSetDevice(h->p.device));
-  if (nrows == 0) return BNR_OK;
-  const size_t rowb = sizeof(double) * (size_t)e.d.n;
-  CK(cudaMemcpy2DAsync(dev_dst, rowb * nrows, e.ll + (size_t)first_row * e.d.n, rowb * e.ll_rows, rowb * nrows,
-                       (size_t)e.d.C, cudaMemcpyDeviceToDevice, h->stream));
-  CK(cudaStreamSynchronize(h->stream));
-  return BNR_OK;
+  if (!h->e.ll.base) return fail(BNR_ESTATE, "no log-likelihood table (bnr_set_loglik)");
+  if (first_row + nrows > h->e.ll.rows) return fail(BNR_EINVAL, "rows beyond the log-likelihood table");
+  return export_table_rows(h, h->e.ll, first_row, nrows, dev_dst);
 }
 
 extern "C" int bnr_loo_summary(int device, const double* dev_rows, int64_t N, int32_t n, double* elpd_loo,

@@ -482,18 +482,17 @@ void launch_loo(const double* rows, long long N, int n, double* out, void* ws, c
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// ESS.  tr: [C][trace_rows][P] rows of (xi, gamma); window = rows [first, first + N).
+// ESS.  tr: the (xi, gamma) trace table, P = tr.width; window = rows [first, first + N).
 //   k_chain_mean : cmean[c][p]                       grid = (ceil(P/128), C), block = 128
 //   k_acov_sum   : acov[l][p] = sum_c 1/N sum_t (x_t - m_c)(x_{t+l} - m_c), l = 0 .. L (biased, per-chain centred)
 //                  grid = (ceil(P/32), ceil((L+1)/64)), block = 256 = 32 parameters x 8 lag groups of 8 lags;
 //                  row chunks of 128 are staged in shared memory, each thread slides an 8-lag register window.
 //   k_ess_finish : Geyer initial monotone sequence over the pooled autocorrelations -> ess[p], thread per parameter
 // ------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) k_chain_mean(const double* __restrict__ tr, long long trace_rows, int P,
-                                                    long long first, long long N, double* __restrict__ cmean) {
-  const int p = blockIdx.x * blockDim.x + threadIdx.x, c = blockIdx.y;
+__global__ void __launch_bounds__(128) k_chain_mean(RowTable tr, long long first, long long N, double* __restrict__ cmean) {
+  const int P = tr.width, p = blockIdx.x * blockDim.x + threadIdx.x, c = blockIdx.y;
   if (p >= P) return;
-  const double* b = tr + ((size_t)c * trace_rows + first) * P + p;
+  const double* __restrict__ b = tr.row(c, first) + p;
   double s = 0.0;
   for (long long r = 0; r < N; ++r) s += b[(size_t)r * P];
   cmean[(size_t)c * P + p] = s / (double)N;
@@ -503,9 +502,9 @@ constexpr int AC_TCH = 128;    // rows per staged chunk
 constexpr int AC_LB = 64;      // lags per block
 constexpr size_t ACOV_SMEM = sizeof(double) * ((size_t)AC_TCH * 32 + (size_t)(AC_TCH + AC_LB) * 32);
 
-__global__ void __launch_bounds__(256) k_acov_sum(const double* __restrict__ tr, long long trace_rows, int P, int C,
-                                                  long long first, long long N, int L,
+__global__ void __launch_bounds__(256) k_acov_sum(RowTable tr, long long first, long long N, int L,
                                                   const double* __restrict__ cmean, double* __restrict__ acov) {
+  const int P = tr.width, C = tr.chains;
   extern __shared__ double sm[];
   double* A = sm;                       // [AC_TCH][32]       x_t - m
   double* B = sm + AC_TCH * 32;         // [AC_TCH + 64][32]  x_{t + l0 + .} - m
@@ -516,18 +515,18 @@ __global__ void __launch_bounds__(256) k_acov_sum(const double* __restrict__ tr,
 #pragma unroll
   for (int k = 0; k < 8; ++k) acc[k] = 0.0;
   for (int c = 0; c < C; ++c) {
-    const double* base = tr + ((size_t)c * trace_rows + first) * P;
+    const double* base = tr.row(c, first);   // loaded through __ldg: a pointer taken from a struct is not __restrict__
     const double m = (p < P) ? cmean[(size_t)c * P + p] : 0.0;
     // every thread stages column pl of the tiles: its own parameter, so m is the right centre
     for (long long t0 = 0; t0 < N; t0 += AC_TCH) {
       __syncthreads();
       for (int r = g; r < AC_TCH; r += 8) {
         const long long t = t0 + r;
-        A[r * 32 + pl] = (p < P && t < N) ? base[(size_t)t * P + p] - m : 0.0;
+        A[r * 32 + pl] = (p < P && t < N) ? __ldg(base + (size_t)t * P + p) - m : 0.0;
       }
       for (int r = g; r < AC_TCH + AC_LB; r += 8) {
         const long long t = t0 + l0 + r;
-        B[r * 32 + pl] = (p < P && t < N) ? base[(size_t)t * P + p] - m : 0.0;
+        B[r * 32 + pl] = (p < P && t < N) ? __ldg(base + (size_t)t * P + p) - m : 0.0;
       }
       __syncthreads();
       // lags l0 + 8g + k, k = 0..7: acc[k] += A[t] * B[t + 8g + k]
@@ -694,18 +693,17 @@ void launch_ess_stream_finalize(const Engine& e, long long N, double* acov, doub
   ++g_launches; k_ess_stream_finalize<<<(e.d.V + e.d.q + 127) / 128, 128, 0, s>>>(e, N, acov, cmean);
 }
 
-void launch_chain_mean(const double* tr, long long trace_rows, int P, int C, long long first, long long N,
-                       double* cmean, cudaStream_t s) {
-  dim3 grid((P + 127) / 128, C);
-  ++g_launches; k_chain_mean<<<grid, 128, 0, s>>>(tr, trace_rows, P, first, N, cmean);
+void launch_chain_mean(const RowTable& tr, long long first, long long N, double* cmean, cudaStream_t s) {
+  dim3 grid((tr.width + 127) / 128, tr.chains);
+  ++g_launches; k_chain_mean<<<grid, 128, 0, s>>>(tr, first, N, cmean);
 }
 
-void launch_acov_sum(const double* tr, long long trace_rows, int P, int C, long long first, long long N, int L,
-                     const double* cmean, double* acov, cudaStream_t s) {
+void launch_acov_sum(const RowTable& tr, long long first, long long N, int L, const double* cmean, double* acov,
+                     cudaStream_t s) {
   static bool attr = false;
   if (!attr) { cudaFuncSetAttribute(k_acov_sum, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ACOV_SMEM); attr = true; }
-  dim3 grid((P + 31) / 32, (L + 1 + AC_LB - 1) / AC_LB);
-  ++g_launches; k_acov_sum<<<grid, 256, ACOV_SMEM, s>>>(tr, trace_rows, P, C, first, N, L, cmean, acov);
+  dim3 grid((tr.width + 31) / 32, (L + 1 + AC_LB - 1) / AC_LB);
+  ++g_launches; k_acov_sum<<<grid, 256, ACOV_SMEM, s>>>(tr, first, N, L, cmean, acov);
 }
 
 void launch_ess_finish(const double* acov_parts, int nparts, const double* cmeans, int chains, int P, long long N,

@@ -88,6 +88,22 @@ struct Aux {           // optional intermediate outputs for parity tests (nullpt
   double* G_copy;        // [C][gdim*gdim]  X D X' + I (n-form) or P (q-form) before factorisation
 };
 
+// One row of `width` doubles per chain and recorded sweep, chain-major: the layout of every table the record kernels
+// write at *trace_row (traces, predictions, log-likelihood) and bnr_copy_trace_rows moves.  base == nullptr: off
+struct RowTable {
+  double* base; long long rows; int width; int chains;
+  __host__ __device__ bool holds(int c, long long r) const { return base && c < chains && r < rows; }
+  __host__ __device__ double* row(int c, long long r) const { return base + ((size_t)c * rows + r) * width; }
+  // the chains [c0, c0 + Cg) of a chain group (only the leading `chains` chains have rows)
+  RowTable view(int c0, int Cg) const {
+    RowTable v = *this;
+    v.chains = chains - c0 < 0 ? 0 : (chains - c0 > Cg ? Cg : chains - c0);
+    v.base = base && v.chains > 0 ? row(c0, 0) : nullptr;
+    return v;
+  }
+  size_t doubles() const { return (size_t)chains * rows * width; }
+};
+
 struct Engine {
   Dims d;
   // data (read-only, shared by all chains)
@@ -129,23 +145,19 @@ struct Engine {
   double* ess_sum;        // [C][2][V+q]        x_first, sum_t y_t
   const long long* ess_win;  // device [4]: first sweep, draws N, max lag L, ring capacity ess_cap
   int ess_L, ess_cap;
-  // traces
-  int trace_full_chains; int trace_gx_chains; long long trace_rows;   // leading chains with full / (xi, gamma) rows
-  double* tr_full;  // [trace_full_chains][rows][rowlen_full]
-  double* tr_gx;    // [trace_gx_chains][rows][V+q]  (xi then gamma)
-  int rowlen_full;
-  // predictions for new networks (bnr_set_predictors; pred_m == 0: off).  Every recorded row r of chain c gets
-  // pred[c][r][j] = mu_c + X_new[j,:] gamma_c (+ sqrt(tau2_c) z_j in the predictive mode), written at *trace_row
+  // traces of the leading tr_full.chains / tr_gx.chains chains; both keep rows = the handle's trace capacity when off
+  RowTable tr_full;       // full state rows (state_elem order)
+  RowTable tr_gx;         // xi then gamma, width V+q
+  // predictions for new networks (bnr_set_predictors; pred.base == nullptr: off).  Every recorded row r of chain c gets
+  // pred.row(c, r)[j] = mu_c + X_new[j,:] gamma_c (+ sqrt(tau2_c) z_j in the predictive mode), width m
+  RowTable pred;
   const double* Xp;       // [qp][pred_mp] X_new columns padded to pred_mp rows (a multiple of 128; zeros beyond m, q)
-  int pred_m, pred_mp, pred_mode, pred_splits;   // m, padded m, BNR_PRED_*, k-splits of the product X_new gamma
-  long long pred_rows;    // rows of each chain's prediction table
-  double* pred;           // [C][pred_rows][pred_m]
+  int pred_mp, pred_mode, pred_splits;   // padded m, BNR_PRED_*, k-splits of the product X_new gamma
   double* pred_ws;        // split-K partials of X_new gamma, [pred_splits][C][pred_mp]; a chain group's view uses
                           // [pred_splits][Cg][pred_mp] at offset c0 * pred_splits * pred_mp
-  // pointwise log-likelihood (bnr_set_loglik; ll == nullptr: off).  Every recorded row r of chain c gets
-  // ll[c][r][i] = log N(y_i | mu_c + (X gamma_c)_i, tau2_c) of the row's own state, written at *trace_row
-  long long ll_rows;      // rows of each chain's log-likelihood table
-  double* ll;             // [C][ll_rows][n]
+  // pointwise log-likelihood (bnr_set_loglik; ll.base == nullptr: off).  Every recorded row r of chain c gets
+  // ll.row(c, r)[i] = log N(y_i | mu_c + (X gamma_c)_i, tau2_c) of the row's own state, width n
+  RowTable ll;
   // injection
   const double* inj;  // [C][inj_stride] or nullptr
   long long inj_stride;

@@ -286,16 +286,18 @@ struct bnr_fit_result {
   Outcome out;
   std::vector<double> rhat_xi, rhat_gamma, s_mean, s_lo, s_hi, s_xi, ess_xi, ess_gamma;
   bool summary_ok = false, ess_ok = false;
-  // predictions for new networks (bnr_fit_predict; pm == 0: none)
-  int pm = 0, pmode = 0;
-  std::vector<double*> pexp;           // per device: the retained rows of its chains, [chain][row][m]
+  // a per-row table pooled over all chains after the fit (width 0: not requested)
+  struct Pooled {
+    const char* what;
+    int width = 0;
+    std::vector<double*> exp;          // per device: the retained rows of its chains, [chain][row][width]
+    bool ok = false;                   // its summary was computed
+  };
+  Pooled pred = {"predictions"};       // predictions for new networks (bnr_fit_predict), width m
+  Pooled ll = {"log-likelihood"};      // pointwise log-likelihood for PSIS-LOO / WAIC (bnr_fit_loo), width n
+  int pmode = 0;
   std::vector<double> p_mean, p_lo, p_hi;
-  bool pred_ok = false;
-  // PSIS-LOO / WAIC (bnr_fit_loo)
-  bool loo = false;
-  std::vector<double*> lexp;           // per device: the retained log-likelihood rows of its chains, [chain][row][n]
   std::vector<double> l_pw[5];         // elpd_loo, p_loo, pareto_k, elpd_waic, p_waic per observation
-  bool loo_ok = false;
   int gamma_mode = 0;
   int status_or = 0;
   const char* exchange = "none";
@@ -303,8 +305,8 @@ struct bnr_fit_result {
     for (size_t d = 0; d < h.size(); ++d) {
       if (d < dev.size()) cudaSetDevice(dev[d]);
       if (d < gbuf.size() && gbuf[d]) cudaFree(gbuf[d]);
-      if (d < pexp.size() && pexp[d]) cudaFree(pexp[d]);
-      if (d < lexp.size() && lexp[d]) cudaFree(lexp[d]);
+      for (Pooled* t : {&pred, &ll})
+        if (d < t->exp.size() && t->exp[d]) cudaFree(t->exp[d]);
       if (d < xs.size() && xs[d]) cudaStreamDestroy(xs[d]);
     }
     if (xbuf) { cudaSetDevice(dev[0]); cudaFree(xbuf); }
@@ -377,7 +379,7 @@ struct DeviceOps : Ops {
         R.exchange = "peer-copy";
       }
     }
-    if (R.pm > 0 || R.loo) return create_tables(rows);
+    if (R.pred.width > 0 || R.ll.width > 0) return create_tables(rows);
     return 0;
   }
 
@@ -386,33 +388,29 @@ struct DeviceOps : Ops {
   // here, not after the sampling
   int create_tables(long long rows) {
     const int nd = (int)R.h.size(), world = R.p.ext_world > 1 ? R.p.ext_world : 1;
-    const char* what = "predictions";
-    auto refuse = [&](const char* buf, size_t doubles) {
+    auto refuse = [](const char* buf, const char* what, size_t doubles) {
       cudaGetLastError();
       return ffail(BNR_ENOMEM, std::string("cannot allocate the ") + buf + " of the " + what + " (" +
                                    std::to_string(doubles * sizeof(double)) + " bytes)");
     };
-    auto exports = [&](std::vector<double*>& buf, size_t local) -> int {
-      buf.assign(nd, nullptr);
+    if (R.pred.width > 0) for (auto* h : R.h) BN(bnr_set_predictors(h, R.pred.width, X_new, rows, R.pmode));
+    if (R.ll.width > 0) for (auto* h : R.h) BN(bnr_set_loglik(h, rows));
+    int width = 0;
+    for (bnr_fit_result::Pooled* t : {&R.pred, &R.ll}) {
+      if (t->width == 0) continue;
+      const size_t local = (size_t)R.C * rows * t->width;
+      t->exp.assign(nd, nullptr);
       for (int d = 0; d < nd; ++d) {
         CKF(cudaSetDevice(R.dev[d]));
-        if (cudaMalloc((void**)&buf[d], local * sizeof(double)) != cudaSuccess) { buf[d] = nullptr; return refuse("export buffer", local); }
+        if (cudaMalloc((void**)&t->exp[d], local * sizeof(double)) != cudaSuccess) {
+          t->exp[d] = nullptr;
+          return refuse("export buffer", t->what, local);
+        }
       }
-      return 0;
-    };
-    int width = 0;
-    if (R.pm > 0) {
-      for (auto* h : R.h) BN(bnr_set_predictors(h, R.pm, X_new, rows, R.pmode));
-      if (int r = exports(R.pexp, (size_t)R.C * rows * R.pm)) return r;
-      width = R.pm;
-    }
-    if (R.loo) {
-      what = "log-likelihood";
-      for (auto* h : R.h) BN(bnr_set_loglik(h, rows));
-      if (int r = exports(R.lexp, (size_t)R.C * rows * R.p.base.n)) return r;
-      if (R.p.base.n > width) width = R.p.base.n;
+      if (t->width > width) width = t->width;
     }
     const size_t local = (size_t)R.C * rows * width;
+    const char* what = (R.ll.width > 0 ? R.ll : R.pred).what;
     if (nd > 1 || world > 1) {
       // gather_local / gather_ext reuse these buffers (they only grow)
       for (int d = 0; d < nd; ++d) {
@@ -421,7 +419,7 @@ struct DeviceOps : Ops {
         R.gbuf[d] = nullptr;
         if (cudaMalloc((void**)&R.gbuf[d], local * nd * sizeof(double)) != cudaSuccess) {
           R.gbuf[d] = nullptr; R.gbuf_doubles = 0;
-          return refuse("pooled buffer", local * nd);
+          return refuse("pooled buffer", what, local * nd);
         }
       }
       R.gbuf_doubles = local * nd;
@@ -429,7 +427,7 @@ struct DeviceOps : Ops {
         CKF(cudaSetDevice(R.dev[0]));
         if (cudaMalloc((void**)&R.xbuf, local * nd * world * sizeof(double)) != cudaSuccess) {
           R.xbuf = nullptr;
-          return refuse("pooled buffer", local * nd * world);
+          return refuse("pooled buffer", what, local * nd * world);
         }
         R.xbuf_doubles = local * nd * world;
       }
@@ -437,44 +435,48 @@ struct DeviceOps : Ops {
     return 0;
   }
 
-  // the retained rows of every chain in global-chain order on device 0, then their pooled mean and order statistics
+  // the retained rows of every chain of a pooled table in global-chain order on device 0 (*all), each device's exported
+  // through export_rows
+  int pool(const Outcome& o, const bnr_fit_result::Pooled& t, int (*export_rows)(bnr_handle*, int64_t, int64_t, double*),
+           const double** all) {
+    const int nd = (int)R.h.size();
+    for (int d = 0; d < nd; ++d) BN(export_rows(R.h[d], o.burn_in, o.sampled, t.exp[d]));
+    *all = t.exp[0];
+    if (nd > 1 || R.p.ext_world > 1) {
+      const size_t cnt = (size_t)R.C * o.sampled * t.width;
+      std::vector<const double*> src(t.exp.begin(), t.exp.end());
+      if (int r = gather_local(src, cnt)) return r;
+      if (int r = gather_ext(cnt * nd, all)) return r;
+    }
+    return 0;
+  }
+
+  // pooled mean and order statistics of the predictions
   int predictions(const Outcome& o) {
     const long long N = (long long)total_chains() * o.sampled;
     const double lower = (100 - (R.p.interval > 0 ? R.p.interval : 95)) / 200.0;
     const long long lw = jround(N * lower), hi = jround(N * (1.0 - lower));
     if (o.sampled < 1 || lw < 1 || hi > N) return 0;
-    const int nd = (int)R.h.size();
-    for (int d = 0; d < nd; ++d) BN(bnr_export_predictions(R.h[d], o.burn_in, o.sampled, R.pexp[d]));
-    const size_t cnt = (size_t)R.C * o.sampled * R.pm;
-    const double* all = R.pexp[0];
-    if (nd > 1 || R.p.ext_world > 1) {
-      std::vector<const double*> src(R.pexp.begin(), R.pexp.end());
-      if (int r = gather_local(src, cnt)) return r;
-      if (int r = gather_ext(cnt * nd, &all)) return r;
-    }
-    R.p_mean.assign(R.pm, 0); R.p_lo.assign(R.pm, 0); R.p_hi.assign(R.pm, 0);
-    BN(bnr_prediction_summary(R.dev[0], all, N, R.pm, lw, hi, R.p_mean.data(), R.p_lo.data(), R.p_hi.data()));
-    R.pred_ok = true;
+    const double* all = nullptr;
+    if (int r = pool(o, R.pred, bnr_export_predictions, &all)) return r;
+    const int m = R.pred.width;
+    R.p_mean.assign(m, 0); R.p_lo.assign(m, 0); R.p_hi.assign(m, 0);
+    BN(bnr_prediction_summary(R.dev[0], all, N, m, lw, hi, R.p_mean.data(), R.p_lo.data(), R.p_hi.data()));
+    R.pred.ok = true;
     return 0;
   }
 
-  // the retained log-likelihood rows of every chain in global-chain order on device 0, then PSIS-LOO and WAIC
+  // pooled PSIS-LOO and WAIC of the log-likelihood
   int loo(const Outcome& o) {
     const long long N = (long long)total_chains() * o.sampled;
     if (N < 2) return 0;
-    const int nd = (int)R.h.size(), n = R.p.base.n;
-    for (int d = 0; d < nd; ++d) BN(bnr_export_loglik(R.h[d], o.burn_in, o.sampled, R.lexp[d]));
-    const size_t cnt = (size_t)R.C * o.sampled * n;
-    const double* all = R.lexp[0];
-    if (nd > 1 || R.p.ext_world > 1) {
-      std::vector<const double*> src(R.lexp.begin(), R.lexp.end());
-      if (int r = gather_local(src, cnt)) return r;
-      if (int r = gather_ext(cnt * nd, &all)) return r;
-    }
+    const double* all = nullptr;
+    if (int r = pool(o, R.ll, bnr_export_loglik, &all)) return r;
+    const int n = R.ll.width;
     for (auto& v : R.l_pw) v.assign(n, 0);
     BN(bnr_loo_summary(R.dev[0], all, N, n, R.l_pw[0].data(), R.l_pw[1].data(), R.l_pw[2].data(), R.l_pw[3].data(),
                        R.l_pw[4].data()));
-    R.loo_ok = true;
+    R.ll.ok = true;
     return 0;
   }
   int init() override { PhaseClock::Scope sc(clk, PH_INIT); for (auto* h : R.h) BN(bnr_init_state(h)); return 0; }
@@ -682,6 +684,9 @@ extern "C" int bnr_fit_plan(const bnr_fit_params* p, const double* psrf_max, int
 // bnr_fit, bnr_fit_predict (m > 0: predictions for the m rows of X_new) and bnr_fit_loo (loo: PSIS-LOO and WAIC)
 static int fit_body(const bnr_fit_params* p, const double* X, const double* y, int32_t m, const double* X_new,
                     int32_t mode, bool loo, bnr_fit_result** res_out) {
+  if (m < 0) return ffail(BNR_EINVAL, "m must be >= 0");
+  if (m > 0 && !X_new) return ffail(BNR_EINVAL, "null X_new");
+  if (mode != BNR_PRED_MEAN && mode != BNR_PRED_PREDICTIVE) return ffail(BNR_EINVAL, "unknown prediction mode");
   if (int r = check_params(p)) return r;
   if (!X || !y || !res_out) return ffail(BNR_EINVAL, "null argument");
   if (p->base.nu < p->base.R)
@@ -690,7 +695,7 @@ static int fit_body(const bnr_fit_params* p, const double* X, const double* y, i
     return ffail(BNR_EINVAL, "nu must not be smaller than R");
   bnr_fit_result* R = new bnr_fit_result();
   R->p = *p;
-  R->pm = m; R->pmode = mode; R->loo = loo;
+  R->pred.width = m; R->pmode = mode; R->ll.width = loo ? p->base.n : 0;
   DeviceOps o(*R, X, y, X_new);
   const double t_start = PhaseClock::now();
   int rc = fit_loops(o, *p, R->out);
@@ -737,26 +742,20 @@ extern "C" int bnr_fit(const bnr_fit_params* p, const double* X, const double* y
 
 extern "C" int bnr_fit_predict(const bnr_fit_params* p, const double* X, const double* y, int32_t m,
                                const double* X_new, int32_t mode, bnr_fit_result** res_out) {
-  if (m < 0) return ffail(BNR_EINVAL, "m must be >= 0");
-  if (m > 0 && !X_new) return ffail(BNR_EINVAL, "null X_new");
-  if (mode != BNR_PRED_MEAN && mode != BNR_PRED_PREDICTIVE) return ffail(BNR_EINVAL, "unknown prediction mode");
   return fit_body(p, X, y, m, X_new, mode, false, res_out);
 }
 
 extern "C" int bnr_fit_loo(const bnr_fit_params* p, const double* X, const double* y, int32_t m, const double* X_new,
                            int32_t pred_mode, bnr_fit_result** res_out) {
-  if (m < 0) return ffail(BNR_EINVAL, "m must be >= 0");
-  if (m > 0 && !X_new) return ffail(BNR_EINVAL, "null X_new");
-  if (pred_mode != BNR_PRED_MEAN && pred_mode != BNR_PRED_PREDICTIVE) return ffail(BNR_EINVAL, "unknown prediction mode");
   return fit_body(p, X, y, m, X_new, pred_mode, true, res_out);
 }
 
 extern "C" int bnr_fit_loo_pointwise(const bnr_fit_result* r, double* elpd_loo, double* p_loo, double* pareto_k,
                                      double* elpd_waic, double* p_waic) {
   if (!r) return ffail(BNR_EINVAL, "null result");
-  if (!r->loo_ok)
-    return ffail(BNR_ESTATE, r->loo ? "fewer than 2 retained draws for PSIS-LOO"
-                                    : "the fit was run without the log-likelihood (bnr_fit_loo)");
+  if (!r->ll.ok)
+    return ffail(BNR_ESTATE, r->ll.width > 0 ? "fewer than 2 retained draws for PSIS-LOO"
+                                             : "the fit was run without the log-likelihood (bnr_fit_loo)");
   double* dst[5] = {elpd_loo, p_loo, pareto_k, elpd_waic, p_waic};
   for (int k = 0; k < 5; ++k)
     if (dst[k]) memcpy(dst[k], r->l_pw[k].data(), sizeof(double) * r->l_pw[k].size());
@@ -765,12 +764,12 @@ extern "C" int bnr_fit_loo_pointwise(const bnr_fit_result* r, double* elpd_loo, 
 
 extern "C" int bnr_fit_prediction(const bnr_fit_result* r, double* mean, double* lo, double* hi) {
   if (!r) return ffail(BNR_EINVAL, "null result");
-  if (!r->pred_ok)
-    return ffail(BNR_ESTATE, r->pm > 0 ? "too few retained draws for the prediction interval"
-                                       : "the fit was run without X_new (bnr_fit_predict)");
-  if (mean) memcpy(mean, r->p_mean.data(), sizeof(double) * r->pm);
-  if (lo) memcpy(lo, r->p_lo.data(), sizeof(double) * r->pm);
-  if (hi) memcpy(hi, r->p_hi.data(), sizeof(double) * r->pm);
+  if (!r->pred.ok)
+    return ffail(BNR_ESTATE, r->pred.width > 0 ? "too few retained draws for the prediction interval"
+                                               : "the fit was run without X_new (bnr_fit_predict)");
+  if (mean) memcpy(mean, r->p_mean.data(), sizeof(double) * r->pred.width);
+  if (lo) memcpy(lo, r->p_lo.data(), sizeof(double) * r->pred.width);
+  if (hi) memcpy(hi, r->p_hi.data(), sizeof(double) * r->pred.width);
   return BNR_OK;
 }
 

@@ -89,10 +89,10 @@ void small_kernels_setup();
 void launch_summary_select(const double* rows, size_t rowlen, int off, int nelem, long long first, long long count,
                            long long rank_lo, long long rank_hi, double* mean_out, double* lo_out, double* hi_out,
                            cudaStream_t s);
-void launch_chain_mean(const double* tr, long long trace_rows, int P, int C, long long first, long long N,
-                       double* cmean, cudaStream_t s);
-void launch_acov_sum(const double* tr, long long trace_rows, int P, int C, long long first, long long N, int L,
-                     const double* cmean, double* acov, cudaStream_t s);
+// rows [first, first + N) of every chain of the (xi, gamma) trace table tr
+void launch_chain_mean(const RowTable& tr, long long first, long long N, double* cmean, cudaStream_t s);
+void launch_acov_sum(const RowTable& tr, long long first, long long N, int L, const double* cmean, double* acov,
+                     cudaStream_t s);
 // streaming ESS: per-sweep lagged-product accumulation (no all-chain trace) and its conversion into the statistics
 // launch_acov_sum / launch_chain_mean produce (acov [L+1][P] summed over the local chains, chain means [C][P])
 void launch_ess_stream(const Engine& e, cudaStream_t s);

@@ -770,7 +770,7 @@ __global__ void __launch_bounds__(256) k_record(Engine e, int sweep_done /* 1: s
   const int np_ = d.V + d.q;
   if (p < np_) {
     const double x = (p < d.V) ? e.xi[c * d.V + p] : e.gamma[(size_t)c * d.qp + (p - d.V)];
-    if (e.tr_gx && c < e.trace_gx_chains && row < e.trace_rows) e.tr_gx[((size_t)c * e.trace_rows + row) * np_ + p] = x;
+    if (e.tr_gx.holds(c, row)) e.tr_gx.row(c, row)[p] = x;
     const long long first = e.mom_window[0], len = e.mom_window[1];
     const long long h = len / 2, rel = sweep - first;
     if (len > 1 && rel >= 0 && rel < len) {
@@ -803,9 +803,10 @@ __global__ void __launch_bounds__(256) k_record(Engine e, int sweep_done /* 1: s
       }
     }
   }
-  if (c < e.trace_full_chains && e.tr_full && row < e.trace_rows) {
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < e.rowlen_full; i += gridDim.x * blockDim.x)
-      e.tr_full[((size_t)c * e.trace_rows + row) * e.rowlen_full + i] = state_elem(e, c, i);
+  if (e.tr_full.holds(c, row)) {
+    double* dst = e.tr_full.row(c, row);
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < e.tr_full.width; i += gridDim.x * blockDim.x)
+      dst[i] = state_elem(e, c, i);
   }
 }
 
@@ -814,7 +815,7 @@ __global__ void __launch_bounds__(256) k_record(Engine e, int sweep_done /* 1: s
 __global__ void __launch_bounds__(256) k_pred_record(Engine e, int sweep_done /* 1: state belongs to sweep iter+1 */) {
   const int c = blockIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x;
   const long long row = *e.trace_row;
-  if (j >= e.pred_m || row >= e.pred_rows) return;
+  if (j >= e.pred.width || !e.pred.holds(c, row)) return;
   const size_t stride = (size_t)e.d.C * e.pred_mp;
   const double* w = e.pred_ws + (size_t)c * e.pred_mp + j;
   double s = 0.0;
@@ -825,7 +826,7 @@ __global__ void __launch_bounds__(256) k_pred_record(Engine e, int sweep_done /*
     DrawStream st(chain_key(e.d, c), (uint32_t)sweep, SITE_PRED, (uint32_t)j);
     v += sqrt(e.tau2[c]) * st.normal();
   }
-  e.pred[((size_t)c * e.pred_rows + row) * e.pred_m + j] = v;
+  e.pred.row(c, row)[j] = v;
 }
 
 // one log-likelihood row per chain: ll[c][row][i] = -1/2 log(2 pi tau2_c) - (y_i - mu_c - (X gamma_c)_i)^2 / (2 tau2_c),
@@ -833,10 +834,10 @@ __global__ void __launch_bounds__(256) k_pred_record(Engine e, int sweep_done /*
 __global__ void __launch_bounds__(256) k_loglik_record(Engine e) {
   const int c = blockIdx.y, i = blockIdx.x * blockDim.x + threadIdx.x;
   const long long row = *e.trace_row;
-  if (i >= e.d.n || row >= e.ll_rows) return;
+  if (i >= e.ll.width || !e.ll.holds(c, row)) return;
   const double t2 = e.tau2[c];
   const double r = e.y[i] - e.mu[c] - e.xg[(size_t)c * e.d.np + i];
-  e.ll[((size_t)c * e.ll_rows + row) * e.d.n + i] = -0.5 * log(6.283185307179586 * t2) - r * r / (2.0 * t2);
+  e.ll.row(c, row)[i] = -0.5 * log(6.283185307179586 * t2) - r * r / (2.0 * t2);
 }
 
 __global__ void k_advance(Engine e, int inc_iter) {
@@ -938,11 +939,11 @@ void launch_record(const Engine& e, int sweep_done, cudaStream_t s) {
   ++g_launches; k_record<<<grid, 256, 0, s>>>(e, sweep_done);
 }
 void launch_pred_record(const Engine& e, int sweep_done, cudaStream_t s) {
-  dim3 grid((e.pred_m + 255) / 256, e.d.C);
+  dim3 grid((e.pred.width + 255) / 256, e.d.C);
   ++g_launches; k_pred_record<<<grid, 256, 0, s>>>(e, sweep_done);
 }
 void launch_loglik_record(const Engine& e, cudaStream_t s) {
-  dim3 grid((e.d.n + 255) / 256, e.d.C);
+  dim3 grid((e.ll.width + 255) / 256, e.d.C);
   ++g_launches; k_loglik_record<<<grid, 256, 0, s>>>(e);
 }
 void launch_advance(const Engine& e, int inc_iter, cudaStream_t s) { k_advance<<<1, 32, 0, s>>>(e, inc_iter); }

@@ -241,6 +241,31 @@ static int row_offset(const Dims& d, int var) {
   return o[var];
 }
 
+// the two branch streams of a stream (side at priority side_prio, side_hi at hi_prio), their fork / join events and the
+// event pool of the Cholesky's look-ahead schedule: 4 per panel (launch_cholesky)
+static int create_fork_join(ForkJoin& f, int panels, int side_prio, int hi_prio) {
+  CK(cudaStreamCreateWithPriority(&f.side, cudaStreamNonBlocking, side_prio));
+  CK(cudaStreamCreateWithPriority(&f.side_hi, cudaStreamNonBlocking, hi_prio));
+  CK(cudaEventCreateWithFlags(&f.fork, cudaEventDisableTiming));
+  CK(cudaEventCreateWithFlags(&f.join, cudaEventDisableTiming));
+  f.npool = 4 * panels;
+  f.pool = new cudaEvent_t[f.npool]();
+  for (int i = 0; i < f.npool; ++i) CK(cudaEventCreateWithFlags(&f.pool[i], cudaEventDisableTiming));
+  return BNR_OK;
+}
+
+// (also after a create_fork_join that failed part of the way)
+static void destroy_fork_join(ForkJoin& f) {
+  if (f.side) cudaStreamDestroy(f.side);
+  if (f.side_hi) cudaStreamDestroy(f.side_hi);
+  if (f.fork) cudaEventDestroy(f.fork);
+  if (f.join) cudaEventDestroy(f.join);
+  for (int i = 0; i < f.npool && f.pool; ++i)
+    if (f.pool[i]) cudaEventDestroy(f.pool[i]);
+  delete[] f.pool;
+  f = ForkJoin();
+}
+
 static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, const double* y);
 
 extern "C" int bnr_create(const bnr_params* p, const double* X, const double* y, bnr_handle** out) {
@@ -441,38 +466,19 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
     if (ng > d.C) ng = d.C;
     h->n_groups = ng;
     CK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-    const bool use_side = getenv("BNR_NO_SIDE") == nullptr;
-    // event pool of the Cholesky's lookahead schedule: 4 per panel (launch_cholesky)
-    auto make_pool = [&](ForkJoin& f) -> int {
-      f.npool = 4 * (d.gdim / TILE_N);
-      f.pool = new cudaEvent_t[f.npool]();
-      for (int i = 0; i < f.npool; ++i) CK(cudaEventCreateWithFlags(&f.pool[i], cudaEventDisableTiming));
-      return 0;
-    };
-    if (use_side) {
-      CK(cudaStreamCreateWithFlags(&h->fj.side, cudaStreamNonBlocking));
-      CK(cudaStreamCreateWithFlags(&h->fj.side_hi, cudaStreamNonBlocking));
-      CK(cudaEventCreateWithFlags(&h->fj.fork, cudaEventDisableTiming));
-      CK(cudaEventCreateWithFlags(&h->fj.join, cudaEventDisableTiming));
-      if (int r = make_pool(h->fj)) return r;
-    }
+    const int panels = d.gdim / TILE_N;
+    // eager sweeps on the whole chain set: both branches at the default priority
+    if (int r = create_fork_join(h->fj, panels, 0, 0)) return r;
+    // main stream: greatest priority (latency-bound kernels); side stream: least (SYRK, bulk panel updates)
+    int plo = 0, phi = 0;
+    CK(cudaDeviceGetStreamPriorityRange(&plo, &phi));       // plo = least, phi = greatest (numerically lower)
     for (int g = 0; g < ng; ++g) {
       ChainGroup& G = h->groups[g];
-      // main stream: greatest priority (latency-bound kernels); side stream: least (SYRK, bulk panel updates)
-      int plo = 0, phi = 0;
-      CK(cudaDeviceGetStreamPriorityRange(&plo, &phi));       // plo = least, phi = greatest (numerically lower)
-      const int prio = getenv("BNR_NO_PRIO") ? plo : phi;
-      CK(cudaStreamCreateWithPriority(&G.stream, cudaStreamNonBlocking, prio));
+      CK(cudaStreamCreateWithPriority(&G.stream, cudaStreamNonBlocking, phi));
       CK(cudaEventCreateWithFlags(&G.done, cudaEventDisableTiming));
-      if (use_side) {
-        CK(cudaStreamCreateWithPriority(&G.fj.side, cudaStreamNonBlocking, plo));
-        // look-ahead branch of the Cholesky: the priority of the main stream (one level lower was measured: config 3 at
-        // 8 chains 1.77 -> 1.81 ms, nothing gained elsewhere)
-        CK(cudaStreamCreateWithPriority(&G.fj.side_hi, cudaStreamNonBlocking, prio));
-        CK(cudaEventCreateWithFlags(&G.fj.fork, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&G.fj.join, cudaEventDisableTiming));
-        if (int r = make_pool(G.fj)) return r;
-      }
+      // look-ahead branch of the Cholesky: the priority of the main stream (one level lower was measured: config 3 at
+      // 8 chains 1.77 -> 1.81 ms, nothing gained elsewhere)
+      if (int r = create_fork_join(G.fj, panels, plo, phi)) return r;
       DA(G.ws, x_times_workspace_doubles(d));
       DA(G.counters, 2);
       DA(G.mom_window, 5);
@@ -489,13 +495,6 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
 }
 
 static void drop_graph(bnr_handle* h);
-static void drop_pool(ForkJoin& f) {
-  if (!f.pool) return;
-  for (int i = 0; i < f.npool; ++i)
-    if (f.pool[i]) cudaEventDestroy(f.pool[i]);
-  delete[] f.pool;
-  f.pool = nullptr; f.npool = 0;
-}
 
 extern "C" int bnr_trim_cache(void) {
   std::vector<CacheBlock> blocks;
@@ -527,17 +526,9 @@ extern "C" int bnr_destroy(bnr_handle* h) {
   for (int g = 0; g < h->n_groups; ++g) {
     if (h->groups[g].stream) { cudaStreamSynchronize(h->groups[g].stream); cudaStreamDestroy(h->groups[g].stream); }
     if (h->groups[g].done) cudaEventDestroy(h->groups[g].done);
-    if (h->groups[g].fj.side) cudaStreamDestroy(h->groups[g].fj.side);
-    if (h->groups[g].fj.side_hi) cudaStreamDestroy(h->groups[g].fj.side_hi);
-    if (h->groups[g].fj.fork) cudaEventDestroy(h->groups[g].fj.fork);
-    if (h->groups[g].fj.join) cudaEventDestroy(h->groups[g].fj.join);
-    drop_pool(h->groups[g].fj);
+    destroy_fork_join(h->groups[g].fj);
   }
-  drop_pool(h->fj);
-  if (h->fj.side) cudaStreamDestroy(h->fj.side);
-  if (h->fj.side_hi) cudaStreamDestroy(h->fj.side_hi);
-  if (h->fj.fork) cudaEventDestroy(h->fj.fork);
-  if (h->fj.join) cudaEventDestroy(h->fj.join);
+  destroy_fork_join(h->fj);
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
   for (auto& a : h->allocs) cache_give(h->p.device, a.first, a.second);
   if (h->ev0) cudaEventDestroy(h->ev0);
@@ -565,40 +556,77 @@ static void refresh_xg(bnr_handle* h) {
   h->xg_valid = true;
 }
 
+// phase boundary k of a profiled sweep (bnr_profile_sweep: marks holds its 9 events); nothing in any other sweep
+static void mark(cudaEvent_t* marks, int k, cudaStream_t s) {
+  if (marks) cudaEventRecord(marks[k], s);
+}
+
 // the gamma conditional: W, v, X v, rhs, G, Cholesky, solves, X' a4, gamma (and optionally S + lambda statistics).
 // syrk_forked: G = X D X' + I is already running on fj.side (enqueue_sweep forks it at the start of the sweep: it
 // depends on nothing but last sweep's S); wait for it just before the factorisation.
-static void run_gamma(Engine& e, double* ws, const ForkJoin& fj, cudaStream_t s, int gig_flags, bool syrk_forked = false) {
+static void run_gamma(Engine& e, double* ws, const ForkJoin& fj, cudaStream_t s, int gig_flags, bool syrk_forked = false,
+                      cudaEvent_t* marks = nullptr) {
   if (e.d.gmode == BNR_GAMMA_QFORM) {
     // P = (X'X + D^-1)/tau2 = L L';  L w = X'(y - mu - X W)/tau2;  L' beta = w + z;  gamma = W + beta
     launch_edge_prep(e, 2, s);                        // W, v = z
     launch_x_times(e, 0, e.W, e.xv, ws, s);           // X W
     launch_rhs(e, s);                                 // (y - mu - X W)/tau2
     launch_x_times(e, 1, e.rhs, e.t, ws, s);          // t = X' rhs
+    mark(marks, 3, s);
     launch_build_P(e, s);
+    mark(marks, 4, s);
     launch_cholesky(e, e.t, fj, s);
+    mark(marks, 5, s);
     launch_chol_solve(e, e.t, e.v, s);
+    mark(marks, 6, s);
     launch_gamma_gig(e, (gig_flags & ~1) | ((gig_flags & 1) ? 4 : 0), s);
     return;
   }
   launch_edge_prep(e, 1, s);
   launch_x_times(e, 0, e.v, e.xv, ws, s);
   launch_rhs(e, s);
+  mark(marks, 3, s);
   if (syrk_forked) cudaStreamWaitEvent(s, fj.join, 0);
   else launch_syrk_G(e, s);
+  mark(marks, 4, s);
   launch_cholesky(e, e.rhs, fj, s);
+  mark(marks, 5, s);
   launch_chol_solve(e, e.rhs, nullptr, s);
+  mark(marks, 6, s);
   launch_x_times(e, 1, e.rhs, e.t, ws, s);
   launch_gamma_gig(e, gig_flags, s);
+}
+
+// the record block of the initial state (row 0) or of a finished sweep (sweep_done: also the streamed ESS lags): the
+// trace rows, the prediction row, the log-likelihood row, then the row / iteration counters.  pred_forked: X_new gamma
+// already runs on fj.side (join it), else it is launched here.  xg_stale: e.xg does not hold X gamma of the state, which
+// the log-likelihood row reads.
+static void enqueue_record(Engine& e, double* ws, const ForkJoin& fj, cudaStream_t s, bool sweep_done, bool pred_forked,
+                           bool xg_stale) {
+  launch_record(e, sweep_done, s);
+  if (sweep_done && e.ess_ring) launch_ess_stream(e, s);
+  if (e.pred.base) {
+    if (pred_forked) cudaStreamWaitEvent(s, fj.join, 0);
+    else launch_pred_product(e, s);
+    launch_pred_record(e, sweep_done, s);
+  }
+  if (e.ll.base) {
+    if (xg_stale) launch_x_times(e, 0, e.gamma, e.xg, ws, s);
+    launch_loglik_record(e, s);
+  }
+  launch_advance(e, sweep_done, s);
 }
 
 // one full sweep in gibbs_sample! order (src/gibbs.jl:663-677).  The Gram SYRK (81 % of the sweep, pure throughput
 // work) goes to the low-priority side stream right away; the latency-bound kernels stay on the high-priority main
 // stream, so that they -- of this chain group and of the others -- get an SM as soon as any SYRK CTA retires instead
 // of queueing behind the SYRK's remaining CTAs.
-static void enqueue_sweep(Engine& e, double* ws, const ForkJoin& fj, cudaStream_t s) {
+// marks (bnr_profile_sweep): events recorded at the 8 phase boundaries; the Gram SYRK and X_new gamma then run on s,
+// so that each phase's events bracket its own kernels.
+static void enqueue_sweep(Engine& e, double* ws, const ForkJoin& fj, cudaStream_t s, cudaEvent_t* marks = nullptr) {
   NvtxRange sweep("bnr sweep");
-  const bool fork_syrk = fj.side != nullptr && e.d.gmode == BNR_GAMMA_NFORM && !e.aux.G_copy;
+  mark(marks, 0, s);
+  const bool fork_syrk = !marks && e.d.gmode == BNR_GAMMA_NFORM && !e.aux.G_copy;
   if (fork_syrk) {
     NvtxRange r("gamma: G = X D X' + I (forked)");
     cudaEventRecord(fj.fork, s);
@@ -607,22 +635,21 @@ static void enqueue_sweep(Engine& e, double* ws, const ForkJoin& fj, cudaStream_
     cudaEventRecord(fj.join, fj.side);
   }
   { NvtxRange r("tau2"); launch_tau2(e, s); }
+  mark(marks, 1, s);
   { NvtxRange r("u, xi"); launch_uxi(e, s); }
   std::swap(e.u, e.u_alt);          // u now holds the new draw (pointer swap is baked per captured sweep)
-  { NvtxRange r("gamma + D (GIG)"); run_gamma(e, ws, fj, s, 3, fork_syrk); }
+  mark(marks, 2, s);
+  { NvtxRange r("gamma + D (GIG)"); run_gamma(e, ws, fj, s, 3, fork_syrk, marks); }
+  mark(marks, 7, s);
   // predictions for new networks: X_new gamma depends on gamma only, so it runs on the side stream next to the scalar
   // conditionals and joins before k_pred_record, which needs the new mu (and tau2)
-  const bool fork_pred = e.pred.base && fj.side != nullptr;
-  if (e.pred.base) {
+  const bool fork_pred = !marks && e.pred.base;
+  if (fork_pred) {
     NvtxRange r("predictions: X_new gamma");
-    if (fork_pred) {
-      cudaEventRecord(fj.fork, s);
-      cudaStreamWaitEvent(fj.side, fj.fork, 0);
-      launch_pred_product(e, fj.side);
-      cudaEventRecord(fj.join, fj.side);
-    } else {
-      launch_pred_product(e, s);
-    }
+    cudaEventRecord(fj.fork, s);
+    cudaStreamWaitEvent(fj.side, fj.fork, 0);
+    launch_pred_product(e, fj.side);
+    cudaEventRecord(fj.join, fj.side);
   }
   {
     NvtxRange r("theta, Delta, M, mu, Lambda, pi");
@@ -631,14 +658,8 @@ static void enqueue_sweep(Engine& e, double* ws, const ForkJoin& fj, cudaStream_
                          (1 << BNR_COND_LAMBDA) | (1 << BNR_COND_PI), s);
   }
   NvtxRange r("record");
-  launch_record(e, 1, s);
-  if (e.ess_ring) launch_ess_stream(e, s);
-  if (e.pred.base) {
-    if (fork_pred) cudaStreamWaitEvent(s, fj.join, 0);
-    launch_pred_record(e, 1, s);
-  }
-  if (e.ll.base) launch_loglik_record(e, s);
-  launch_advance(e, 1, s);
+  enqueue_record(e, ws, fj, s, true, fork_pred, false);
+  mark(marks, 8, s);
 }
 
 // view of the handle's engine restricted to chains [c0, c0 + Cg): every per-chain array is chain-major, so the
@@ -693,7 +714,7 @@ static int build_graphs(bnr_handle* h) {
     enqueue_sweep(e, G.ws, G.fj, G.stream);
     CK(cudaStreamEndCapture(G.stream, &G.graph[par]));
     // node priorities = priorities of the streams the kernels were captured from (main: greatest, side: least)
-    CK(cudaGraphInstantiate(&G.gexec[par], G.graph[par], getenv("BNR_NO_PRIO") ? 0 : cudaGraphInstantiateFlagUseNodePriority));
+    CK(cudaGraphInstantiate(&G.gexec[par], G.graph[par], cudaGraphInstantiateFlagUseNodePriority));
   }
   h->graph_kernels = g_launches - before;
   h->graphs_ready[par] = true;
@@ -709,16 +730,7 @@ extern "C" int bnr_init_state(bnr_handle* h) {
   CK(cudaMemsetAsync(e.trace_row, 0, sizeof(long long), h->stream));
   CK(cudaMemsetAsync(e.status, 0, sizeof(int) * e.d.C, h->stream));
   launch_init(e, h->stream);
-  launch_record(e, 0, h->stream);
-  if (e.pred.base) {
-    launch_pred_product(e, h->stream);
-    launch_pred_record(e, 0, h->stream);
-  }
-  if (e.ll.base) {
-    refresh_xg(h);                     // X gamma_0: the cache is not valid after launch_init
-    launch_loglik_record(e, h->stream);
-  }
-  launch_advance(e, 0, h->stream);
+  enqueue_record(e, h->ws, h->fj, h->stream, false, false, true);     // X gamma_0: the cache is not valid after launch_init
   h->xg_valid = false;
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
@@ -1290,17 +1302,8 @@ extern "C" int bnr_step(bnr_handle* h, int32_t cond) {
 extern "C" int bnr_finish_sweep(bnr_handle* h) {
   if (!h) return fail(BNR_EINVAL, "null handle");
   CK(cudaSetDevice(h->p.device));
-  launch_record(h->e, 1, h->stream);
-  if (h->e.ess_ring) launch_ess_stream(h->e, h->stream);
-  if (h->e.pred.base) {
-    launch_pred_product(h->e, h->stream);
-    launch_pred_record(h->e, 1, h->stream);
-  }
-  if (h->e.ll.base) {
-    if (!h->xg_valid) refresh_xg(h);
-    launch_loglik_record(h->e, h->stream);
-  }
-  launch_advance(h->e, 1, h->stream);
+  enqueue_record(h->e, h->ws, h->fj, h->stream, true, false, !h->xg_valid);
+  if (h->e.ll.base) h->xg_valid = true;                       // (the log-likelihood row refreshed it)
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
   return BNR_OK;
@@ -1603,60 +1606,18 @@ extern "C" int bnr_export_moments(bnr_handle* h, double* dev_dst) {
   return BNR_OK;
 }
 
-// One eager sweep with CUDA events between its phases (on the handle's stream).  ms[8]:
-// 0 tau2, 1 (u,xi), 2 gamma prep (W, v, X v, rhs), 3 SYRK X D X' + I, 4 Cholesky, 5 triangular solves,
+// One eager sweep (enqueue_sweep, on the handle's stream) with CUDA events between its phases.  ms[8]:
+// 0 tau2, 1 (u,xi), 2 gamma prep (W, v, X v, rhs), 3 SYRK X D X' + I (q-form: P), 4 Cholesky, 5 triangular solves,
 // 6 X' a4 + gamma + GIG, 7 X gamma + theta/Delta/M/mu/lambda/pi + record.
 extern "C" int bnr_profile_sweep(bnr_handle* h, float* ms) {
   if (!h || !ms) return fail(BNR_EINVAL, "null argument");
   CK(cudaSetDevice(h->p.device));
   drop_graph(h);
-  Engine& e = h->e;
-  cudaStream_t s = h->stream;
   if (!h->xg_valid) refresh_xg(h);
   cudaEvent_t ev[9];
   for (int i = 0; i < 9; ++i) CK(cudaEventCreate(&ev[i]));
-  CK(cudaEventRecord(ev[0], s));
-  launch_tau2(e, s);
-  CK(cudaEventRecord(ev[1], s));
-  launch_uxi(e, s);
-  std::swap(e.u, e.u_alt);
-  CK(cudaEventRecord(ev[2], s));
-  if (e.d.gmode == BNR_GAMMA_QFORM) {
-    launch_edge_prep(e, 2, s);
-    launch_x_times(e, 0, e.W, e.xv, h->ws, s);
-    launch_rhs(e, s);
-    launch_x_times(e, 1, e.rhs, e.t, h->ws, s);
-    CK(cudaEventRecord(ev[3], s));
-    launch_build_P(e, s);
-    CK(cudaEventRecord(ev[4], s));
-    launch_cholesky(e, e.t, h->fj, s);
-    CK(cudaEventRecord(ev[5], s));
-    launch_chol_solve(e, e.t, e.v, s);
-    CK(cudaEventRecord(ev[6], s));
-    launch_gamma_gig(e, 6, s);
-  } else {
-    launch_edge_prep(e, 1, s);
-    launch_x_times(e, 0, e.v, e.xv, h->ws, s);
-    launch_rhs(e, s);
-    CK(cudaEventRecord(ev[3], s));
-    launch_syrk_G(e, s);
-    CK(cudaEventRecord(ev[4], s));
-    launch_cholesky(e, e.rhs, h->fj, s);
-    CK(cudaEventRecord(ev[5], s));
-    launch_chol_solve(e, e.rhs, nullptr, s);
-    CK(cudaEventRecord(ev[6], s));
-    launch_x_times(e, 1, e.rhs, e.t, h->ws, s);
-    launch_gamma_gig(e, 3, s);
-  }
-  CK(cudaEventRecord(ev[7], s));
-  launch_x_times(e, 0, e.gamma, e.xg, h->ws, s);
-  launch_finish(e, (1 << BNR_COND_THETA) | (1 << BNR_COND_DELTA) | (1 << BNR_COND_M) | (1 << BNR_COND_MU) |
-                       (1 << BNR_COND_LAMBDA) | (1 << BNR_COND_PI), s);
-  launch_record(e, 1, s);
-  if (e.ess_ring) launch_ess_stream(e, s);
-  launch_advance(e, 1, s);
-  CK(cudaEventRecord(ev[8], s));
-  CK(cudaStreamSynchronize(s));
+  enqueue_sweep(h->e, h->ws, h->fj, h->stream, ev);
+  CK(cudaStreamSynchronize(h->stream));
   for (int i = 0; i < 8; ++i) CK(cudaEventElapsedTime(&ms[i], ev[i], ev[i + 1]));
   for (int i = 0; i < 9; ++i) cudaEventDestroy(ev[i]);
   CK(cudaGetLastError());

@@ -61,8 +61,8 @@ constexpr int GRAM_I8_QP_MIN = 1024;
 constexpr int GRAM_I8_QP_MAX = 18724;     // 7 qp 2^14 < 2^31: the int32 accumulators of the digit products are exact
 bool gram_i8_selected(const Dims& d);
 size_t gram_i8_plane_bytes(const Dims& d);                    // digit planes of one chain
-// optional second stream + events that let launch_cholesky run the off-diagonal panel updates next to the panel
-// factorisation (works eagerly and under stream capture, where it becomes a fork/join of the graph)
+// branch streams + events that let launch_cholesky run the off-diagonal panel updates next to the panel factorisation
+// (works eagerly and under stream capture, where it becomes a fork/join of the graph)
 struct ForkJoin {
   cudaStream_t side = nullptr;   // low priority: throughput work (the Gram SYRK)
   cudaStream_t side_hi = nullptr;// same priority as the main stream: the Cholesky's look-ahead branch (it feeds the

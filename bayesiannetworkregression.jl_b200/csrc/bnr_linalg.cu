@@ -1743,11 +1743,6 @@ bool tmaps_check(const Engine& e) {
 
 int syrk_splits(const Dims& d, int C) {
   const int T = d.np / SY_BT, tiles = T * (T + 1) / 2, nk = d.qp / SY_BK;
-  if (const char* ov = getenv("BNR_SYRK_SPLITS")) {                       // tuning knob
-    int s = atoi(ov);
-    if (s > nk / 8) s = nk / 8;
-    return s < 1 ? 1 : (s > SYRK_MAX_SPLITS ? SYRK_MAX_SPLITS : s);
-  }
   // (measured: once chains x tiles reaches one wave, splitting only removes the natural stagger between chain groups)
   if (tiles * C >= 148) return 1;
   int s = (4 * 148 + tiles * C - 1) / (tiles * C);
@@ -2235,8 +2230,7 @@ void launch_build_P(const Engine& e, cudaStream_t s) {
 //     factorisation.  Tiles are cut into row strips (syrk_body) while the launch stays within one wave of CTAs.
 //       dependencies across the two streams:  T2(J) after PA(J);  Ulate(J) after T1(J);
 //                                             T1(J+1) after Ulate(J);  PA(J+2) after Uearly(J).
-// `side` is a forked branch of the graph with the priority of the main stream.  Without a side stream the same kernels
-// run in program order on `s` (identical results).
+// `side` is a forked branch of the graph with the priority of the main stream.
 void launch_cholesky(const Engine& e, double* rhs, const ForkJoin& fj, cudaStream_t s) {
   const Dims& d = e.d;
   const int N = d.gdim;
@@ -2244,9 +2238,7 @@ void launch_cholesky(const Engine& e, double* rhs, const ForkJoin& fj, cudaStrea
   const size_t cs = (size_t)N * N;
   const int T = N / PB;
   const size_t ls = (size_t)T * PB * PB;
-  static const bool serial = getenv("BNR_CHOL_SERIAL") != nullptr;        // debugging knob: program order on one stream
-  static const int forced = getenv("BNR_CHOL_SCHEDULE") ? atoi(getenv("BNR_CHOL_SCHEDULE")) : 0;   // 1 = (A), 2 = (B)
-  const bool latency = forced ? forced == 2 : (long long)d.C_total * (T - 1) <= 128;
+  const bool latency = (long long)d.C_total * (T - 1) <= 128;
   ++g_launches; k_augment<<<d.C, 256, 0, s>>>(e.G, cs, N, m, rhs, d.gmode == 2 ? d.qp : d.np, d.gmode == 2 ? e.S : nullptr, e.tau2);
   // operand maps of the ring-fed kernels: the chains' matrices stacked along the k axis (chain c, column k -> k-row
   // c N + k), boxes as wide as a tile / a half / a quarter tile (+ 4 rows of padding); the stacked panel inverses
@@ -2258,15 +2250,13 @@ void launch_cholesky(const Engine& e, double* rhs, const ForkJoin& fj, cudaStrea
 
   if (!latency) {
     // ---- (A) ----
-    const bool can_fork = !serial && fj.side != nullptr;
     // The forked updates run at the panel chain's priority.  With another chain group's SYRK resident (600 us CTAs that
     // give an SM back every ~4 us) every dependent kernel has to re-acquire its SMs one by one; on the SYRK's own
     // priority level they queued behind ALL its pending CTAs and the factorisation only ran in the SYRK's last wave
     // (timeline in profiles/r02_timeline_c3.txt: 1 ms per sweep without any SYRK CTA resident).
-    static const bool a_lo = getenv("BNR_CHOL_A_SIDE_LO") != nullptr;      // knob: the old low-priority branch
-    cudaStream_t sideA = (!a_lo && fj.side_hi) ? fj.side_hi : fj.side;
+    cudaStream_t sideA = fj.side_hi;
     for (int J = 0; J < T; ++J) {
-      const bool fork = can_fork && J > 0 && J + 1 < T;
+      const bool fork = J > 0 && J + 1 < T;
       if (J > 0) {
         const int nk = J * PB / SY_BK;
         if (fork) {
@@ -2293,57 +2283,51 @@ void launch_cholesky(const Engine& e, double* rhs, const ForkJoin& fj, cudaStrea
   }
 
   // ---- (B) ----
-  const bool fork = !serial && fj.side_hi != nullptr && fj.pool != nullptr && fj.npool >= 4 * T;
-  cudaStream_t side = fork ? fj.side_hi : s;
+  cudaStream_t side = fj.side_hi;
   cudaEvent_t* evP = fj.pool;                       // [T] each: after PA, after T1, after Ulate, after Uearly
   cudaEvent_t* evT = fj.pool + T;
   cudaEvent_t* evL = fj.pool + 2 * T;
   cudaEvent_t* evE = fj.pool + 3 * T;
   // row strips per tile (see syrk_body): as many as keep the launch within one wave of CTAs
   auto strips = [&](int tiles) {
-    static const int fs = getenv("BNR_STRIPS") ? atoi(getenv("BNR_STRIPS")) : 0;      // tuning knob (1, 2 or 4)
-    if (fs == 1 || fs == 2 || fs == 4) return fs;
     const int ctas = d.C_total * tiles;
     return ctas * 4 <= 148 ? 4 : (ctas * 2 <= 148 ? 2 : 1);
   };
   // panel solve of `rows` row blocks from ib_first of block column J: the shared-memory-resident kernel when the tiles
   // are cut into strips (few chains), else the ring-fed one
-  static const bool small_tiles = getenv("BNR_NO_SMALL_TILES") == nullptr;
   auto launch_trsm = [&](int J, int ib_first, int rows, int ns, cudaStream_t st) {
     dim3 g(d.C, rows * ns);
     const double* Lj = e.Linv + (size_t)J * PB * PB;
     ++g_launches;
-    if (small_tiles && ns == 8)
+    if (ns == 8)
       k_small_tile<2, 2><<<g, 256, small_tile_smem(16), st>>>(e.G, cs, N, J, ib_first, 8, Lj, ls, PB, J * PB, 0);
-    else if (small_tiles && ns == 4)
+    else if (ns == 4)
       k_small_tile<2, 4><<<g, 256, small_tile_smem(32), st>>>(e.G, cs, N, J, ib_first, 4, Lj, ls, PB, J * PB, 0);
-    else if (small_tiles && ns == 2)
+    else if (ns == 2)
       k_small_tile<2, 8><<<g, 256, small_tile_smem(64), st>>>(e.G, cs, N, J, ib_first, 2, Lj, ls, PB, J * PB, 0);
     else
-      k_trsm_dmma<<<g, SY_THREADS, SYRK_SMEM, st>>>(mL, mI(ns), e.G, cs, N, m + 1, J, ib_first, ns);
+      k_trsm_dmma<<<g, SY_THREADS, SYRK_SMEM, st>>>(mL, mG, e.G, cs, N, m + 1, J, ib_first, 1);
   };
   // The late part of the diagonal tile (J+1, J+1) -- the contribution of panel J -- either runs inside k_potf2_inv
   // (one SM: ~12 us of DMMA) or, when the chains are few enough for 4-8 CTAs per tile, as its own strip kernel Ud(J)
   // right after T1(J) (~5 us), with T1 itself cut into as many strips.
-  static const int ud_knob = getenv("BNR_CHOL_UD") ? atoi(getenv("BNR_CHOL_UD")) : -1;     // tuning knob: 0 off, 4 / 8 strips
   // (measured: config 2 0.320 -> 0.300 ms, config 4 1.684 -> 1.666 ms; with a chain group's SYRK competing for the SMs
   //  -- 8 / 16 chains of config 3 -- the extra CTAs wait for SMs and the in-kernel update stays ahead: 1.770 vs 1.782 ms)
   const bool quiet = d.gmode == 2 || e.syrk_ws != nullptr;          // no full-size SYRK CTAs of other groups around
-  int ud = (small_tiles && quiet) ? (d.C_total * 8 <= 148 ? 8 : (d.C_total * 4 <= 148 ? 4 : 0)) : 0;
-  if (ud_knob == 0 || ud_knob == 4 || ud_knob == 8) ud = small_tiles ? ud_knob : 0;
+  const int ud = quiet ? (d.C_total * 8 <= 148 ? 8 : (d.C_total * 4 <= 148 ? 4 : 0)) : 0;
   for (int J = 0; J < T; ++J) {
     const bool has_side = J + 2 < T;
-    if (fork && J >= 2 && !ud) cudaStreamWaitEvent(s, evE[J - 2], 0);
+    if (J >= 2 && !ud) cudaStreamWaitEvent(s, evE[J - 2], 0);
     ++g_launches; k_potf2_inv<<<d.C, 256, POTF2_SMEM, s>>>(e.G, cs, N, J, e.Linv, T, e.status, (J > 0 && !ud) ? 1 : 0);
-    if (fork && has_side) cudaEventRecord(evP[J], s);
+    if (has_side) cudaEventRecord(evP[J], s);
     if (J + 1 < T) {
-      if (fork && J >= 1 && J + 1 < T) cudaStreamWaitEvent(s, evL[J - 1], 0);
+      if (J >= 1) cudaStreamWaitEvent(s, evL[J - 1], 0);
       const int ns1 = ud ? ud : strips(1);
       launch_trsm(J, J + 1, 1, ns1, s);
-      if (fork && has_side) cudaEventRecord(evT[J], s);
+      if (has_side) cudaEventRecord(evT[J], s);
       if (ud) {
         // Ud(J): tile (J+1, J+1) -= L[J+1, J] L[J+1, J]' (lower triangle), after the early panels 0..J-1 (Uearly(J-1))
-        if (fork && J >= 1) cudaStreamWaitEvent(s, evE[J - 1], 0);
+        if (J >= 1) cudaStreamWaitEvent(s, evE[J - 1], 0);
         dim3 gd(d.C, ud);
         const double* Lt = e.G + (size_t)J * PB * N + (size_t)(J + 1) * PB;
         ++g_launches;
@@ -2353,22 +2337,22 @@ void launch_cholesky(const Engine& e, double* rhs, const ForkJoin& fj, cudaStrea
     }
     if (has_side) {
       const int rows = T - J - 2;                   // row blocks J+2 .. T-1
-      if (fork) cudaStreamWaitEvent(side, evP[J], 0);
+      cudaStreamWaitEvent(side, evP[J], 0);
       const int ns2 = strips(rows);
       dim3 g2(d.C, rows * ns2);
       launch_trsm(J, J + 2, rows, ns2, side);
-      if (fork) cudaStreamWaitEvent(side, evT[J], 0);
+      cudaStreamWaitEvent(side, evT[J], 0);
       ++g_launches;
-      if (small_tiles && ns2 == 4)
+      if (ns2 == 4)
         k_small_tile<1, 4><<<g2, 256, small_tile_smem(32), side>>>(e.G, cs, N, J + 1, J + 2, 4, e.G + (size_t)J * PB * N + (size_t)(J + 1) * PB, cs, N, J * PB, 0);
-      else if (small_tiles && ns2 == 2)
+      else if (ns2 == 2)
         k_small_tile<1, 8><<<g2, 256, small_tile_smem(64), side>>>(e.G, cs, N, J + 1, J + 2, 2, e.G + (size_t)J * PB * N + (size_t)(J + 1) * PB, cs, N, J * PB, 0);
       else
-        k_chol_update<<<g2, SY_THREADS, SYRK_SMEM, side>>>(mG, mI(ns2), J * PB, e.G, cs, N, m + 1, PB / SY_BK, J + 1, J + 2, ns2);
-      if (fork) cudaEventRecord(evL[J], side);
+        k_chol_update<<<g2, SY_THREADS, SYRK_SMEM, side>>>(mG, mG, J * PB, e.G, cs, N, m + 1, PB / SY_BK, J + 1, J + 2, 1);
+      cudaEventRecord(evL[J], side);
       ++g_launches; k_chol_update<<<g2, SY_THREADS, SYRK_SMEM, side>>>(mG, mI(ns2), 0, e.G, cs, N, m + 1, (J + 1) * PB / SY_BK,
                                                                    J + 2, J + 2, ns2);
-      if (fork) cudaEventRecord(evE[J], side);
+      cudaEventRecord(evE[J], side);
     }
   }
 }

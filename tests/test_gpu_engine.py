@@ -2,7 +2,6 @@
 drop-in surface, level-2 (posterior) agreement with the oracle chain and with the reference's golden run, and
 size-independent properties at the benchmark's full size (V=100, n=1000)."""
 import math
-import os
 
 import numpy as np
 import pytest
@@ -703,23 +702,3 @@ def test_unusual_shapes_factorisation_properties(bnr, V, n, R, mode):
         st = eng.get_state_dict(0)
         assert not (eng.status() & ~1).any()
         assert np.isfinite(st["gamma"]).all() and (st["S"] > 0).all() and st["tau2"] > 0
-
-
-@pytest.mark.parametrize("env", [{"BNR_CHOL_SCHEDULE": "1"}, {"BNR_CHOL_SCHEDULE": "1", "BNR_CHOL_A_SIDE_LO": "1"},
-                                 {"BNR_CHOL_SCHEDULE": "2", "BNR_CHOL_UD": "8"}, {"BNR_CHOL_SCHEDULE": "2", "BNR_CHOL_UD": "0"},
-                                 {"BNR_CHOL_SCHEDULE": "2", "BNR_CHOL_UD": "4", "BNR_STRIPS": "2"}, {"BNR_NO_SIDE": "1"},
-                                 {"BNR_NO_SMALL_TILES": "1"}])
-def test_every_cholesky_schedule_matches_the_oracle(env):
-    """The blocked Cholesky has two schedules and several launch variants that the library picks from the handle's chain
-    count; with two chains only one of them ever runs.  The knobs are read once per process, so a child process runs the
-    injected-sweep parity checks at the BASELINE shapes (configs 5, 4 and 2: n-form with and without a split SYRK, q-form)
-    under every variant."""
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    e = dict(os.environ)
-    e.update(env)
-    r = subprocess.run([sys.executable, "-m", "pytest", "tests/test_gpu_parity_edges.py", "-q", "-x", "-m", "gpu", "-k",
-                        "baseline_size_sweep_injected and (c5 or c4 or c2)"], cwd=root, env=e, capture_output=True, text=True,
-                       timeout=600)
-    assert r.returncode == 0, "%s\n%s\n%s" % (env, r.stdout[-2000:], r.stderr[-2000:])

@@ -54,7 +54,7 @@ def bwd_stages(N):
 
 
 def selection(V, n, mode, C):
-    """Everything (V, n, mode, C) selects for the eager sweep of a handle of C chains (no knobs set)."""
+    """Everything (V, n, mode, C) selects for the eager sweep of a handle of C chains."""
     q, np_, qp, N = padded(V, n, mode)
     T = N // TILE
     syrk = syrk_splits(np_, qp, C) if mode == "nform" else 1

@@ -7,8 +7,6 @@ power limit.
 
 Each arm is its own handle on the config's inputs (bench.synth) and chain count, warmed up with a few sweeps; every
 repetition times each arm over --sweeps sweeps with CUDA events (bnr_last_run_ms) and the median is reported.
---inline also runs the m = 100 arms with BNR_NO_SIDE set (no side streams: the product runs on the main stream, and so
-do the Gram SYRK and the Cholesky's look-ahead; its own baseline arm is timed alongside).
 """
 import argparse
 import os
@@ -28,7 +26,6 @@ def main():
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--configs", default="c2,c3,c5")
     ap.add_argument("--ms", default="100,1000")
-    ap.add_argument("--inline", action="store_true")
     args = ap.parse_args()
     import bench
     from __graft_entry__ import load_package
@@ -41,19 +38,13 @@ def main():
         X, y, info = bench.synth(cfg)
         C = bench.CONFIGS[cfg]["chains"]
         rng = np.random.default_rng(5)
-        arms = [("off", None, False, False)]
+        arms = [("off", None, False)]
         for m in ms:
             Xn = X[rng.integers(0, X.shape[0], size=m)]          # new networks drawn like the fitted ones
-            arms += [("m=%d mean" % m, Xn, False, False), ("m=%d predictive" % m, Xn, True, False)]
-        if args.inline:
-            Xn = X[rng.integers(0, X.shape[0], size=100)]
-            arms += [("off, no side streams", None, False, True), ("m=100 mean, no side streams", Xn, False, True)]
+            arms += [("m=%d mean" % m, Xn, False), ("m=%d predictive" % m, Xn, True)]
         engines = []
-        for name, Xn, pred, inline in arms:
-            if inline:
-                os.environ["BNR_NO_SIDE"] = "1"
+        for name, Xn, pred in arms:
             eng = bnr.Engine(X, y, info["R"], num_chains=C, seed=3)
-            os.environ.pop("BNR_NO_SIDE", None)
             if Xn is not None:
                 eng.set_predictors(Xn, args.sweeps + 8, predictive=pred)
             eng.init_state()
@@ -65,13 +56,11 @@ def main():
                 eng.trace_row = 0
                 eng.run(args.sweeps)
                 times[i].append(eng.last_run_ms() / args.sweeps)
-        base = {False: np.median(times[0])}
-        for i, (name, _, _, inline) in enumerate(arms):
+        base = float(np.median(times[0]))
+        for i, (name, _, _) in enumerate(arms):
             t = float(np.median(times[i]))
-            if name.startswith("off"):
-                base[inline] = t
             print("%s %-30s %.4f ms/sweep (spread %.4f-%.4f)  %+.2f %%" %
-                  (cfg, name, t, min(times[i]), max(times[i]), 100.0 * (t / base[inline] - 1.0)))
+                  (cfg, name, t, min(times[i]), max(times[i]), 100.0 * (t / base - 1.0)))
         for eng in engines:
             eng.close()
     lab = os.path.join(ROOT, "tools", "lab", "pred_select_lab")

@@ -124,7 +124,7 @@ struct bnr_handle {
   std::vector<std::pair<void*, size_t>> allocs;   // device buffers (pointer, bytes): returned to the cache on destroy
   double* ws = nullptr;          // split-K workspace
   double* d_inj = nullptr;       // injected variates
-  long long inj_len = 0;
+  size_t inj_len = 0;
   bool aux_on = false;
   Aux aux_saved = {};
   long long win[5] = {0, 0, 0, 1, 0};   // host copy of the device window record (bnr_set_moment_window / _blocks)
@@ -169,6 +169,19 @@ static void release_alloc(bnr_handle* h, void* p) {
       h->allocs.pop_back();
       return;
     }
+}
+
+// grow a handle-owned device buffer to `need` units of `unit` bytes; cap is its capacity in units.  The contents are not
+// kept.  A refused allocation leaves buf == nullptr and cap == 0
+template <typename T, typename N>
+static int grow_buffer(bnr_handle* h, T*& buf, N& cap, N need, size_t unit = sizeof(T)) {
+  if (need <= cap) return BNR_OK;
+  release_alloc(h, buf);
+  buf = nullptr; cap = 0;
+  void* p = nullptr;
+  if (int r = raw_alloc(h, &p, (size_t)need * unit)) return r;
+  buf = (T*)p; cap = need;
+  return BNR_OK;
 }
 
 // short-lived device scratch of the handle-less entry points (bnr_rhat_from_moments, bnr_ess_from_stats): taken from
@@ -424,11 +437,13 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
   DA(e.tau2_ticket, C);
   DA(e.status, C);
   DA(e.iter, 1); DA(e.trace_row, 1);
-  DA(e.moments, C * 2 * (d.V + d.q) * 2);
-  DA(e.mom_window, 5);
-  e.bmom = nullptr; e.bmom_nb = 0;
-  e.ess_ring = e.ess_head = e.ess_acc = e.ess_sum = nullptr; e.ess_win = nullptr; e.ess_L = e.ess_cap = 0;
-  DA(h->d_esswin, 4);
+  e.mom = {nullptr, nullptr, nullptr, 0, d.V + d.q};
+  DA(e.mom.halves, C * 2 * (d.V + d.q) * 2);
+  DA(e.mom.window, 5);
+  e.ess = {};
+  e.ess.P = d.V + d.q;
+  DA(h->d_esswin, 2);
+  e.ess.win = h->d_esswin;
   DA(h->ws, x_times_workspace_doubles(d));
   DA(h->d_rhat, (size_t)(d.V + d.q));
   const long long trace_rows = p->trace_rows > 0 ? p->trace_rows : 0;
@@ -604,7 +619,7 @@ static void run_gamma(Engine& e, double* ws, const ForkJoin& fj, cudaStream_t s,
 static void enqueue_record(Engine& e, double* ws, const ForkJoin& fj, cudaStream_t s, bool sweep_done, bool pred_forked,
                            bool xg_stale) {
   launch_record(e, sweep_done, s);
-  if (sweep_done && e.ess_ring) launch_ess_stream(e, s);
+  if (sweep_done && e.ess.on()) launch_ess_stream(e, s);
   if (e.pred.base) {
     if (pred_forked) cudaStreamWaitEvent(s, fj.join, 0);
     else launch_pred_product(e, s);
@@ -679,17 +694,11 @@ static Engine group_view(const bnr_handle* h, int c0, int Cg, long long* counter
   v.G += c * d.gdim * d.gdim; if (v.syrk_ws) v.syrk_ws += c * (size_t)v.syrk_ws_cap * d.gdim * d.gdim; v.Linv += c * (size_t)(d.gdim / TILE_N) * TILE_N * TILE_N;
   if (v.gram_planes) { v.gram_planes += c * gram_i8_plane_bytes(d); v.gram_rscale += c * d.np; }
   v.partials += c * d.nparts * (2 * MAX_R + 1);
-  v.moments += c * 2 * (d.V + d.q) * 2;
-  if (v.bmom) v.bmom += c * (size_t)v.bmom_nb * (d.V + d.q) * 2;
-  if (v.ess_ring) {
-    const size_t P = (size_t)d.V + d.q;
-    v.ess_ring += c * (size_t)v.ess_cap * P; v.ess_head += c * (size_t)v.ess_L * P;
-    v.ess_acc += c * (size_t)(v.ess_L + 1) * P; v.ess_sum += c * 2 * P;
-  }
+  v.mom = v.mom.view(c0, mom_window); v.ess = v.ess.view(c0);
   v.tr_full = v.tr_full.view(c0, Cg); v.tr_gx = v.tr_gx.view(c0, Cg);
   v.pred = v.pred.view(c0, Cg); v.ll = v.ll.view(c0, Cg);
   if (v.pred_ws) v.pred_ws += c * (size_t)v.pred_splits * v.pred_mp;
-  v.iter = counters; v.trace_row = counters + 1; v.mom_window = mom_window;
+  v.iter = counters; v.trace_row = counters + 1;
   v.inj = nullptr; v.inj_stride = 0;
   memset(&v.aux, 0, sizeof(v.aux));
   return v;
@@ -871,7 +880,7 @@ extern "C" int bnr_copy_trace_rows(bnr_handle* h, int64_t dst, int64_t src, int6
 
 // device copy of the 5-entry window record (split-half window + block-moment configuration) for the handle and groups
 static int push_windows(bnr_handle* h) {
-  CK(cudaMemcpyAsync(h->e.mom_window, h->win, sizeof(h->win), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(h->e.mom.window, h->win, sizeof(h->win), cudaMemcpyHostToDevice, h->stream));
   for (int g = 0; g < h->n_groups; ++g)
     CK(cudaMemcpyAsync(h->groups[g].mom_window, h->win, sizeof(h->win), cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
@@ -891,50 +900,23 @@ extern "C" int bnr_set_moment_window(bnr_handle* h, int64_t first, int64_t len) 
 extern "C" int bnr_set_moment_blocks(bnr_handle* h, int64_t first_sweep, int64_t block_len, int32_t nblocks) {
   if (!h || nblocks < 0 || (nblocks > 0 && block_len < 1)) return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
-  const Dims& d = h->e.d;
-  if (nblocks > h->e.bmom_nb) {
+  SplitMoments& m = h->e.mom;
+  if (nblocks > m.nblocks) {
     CK(cudaStreamSynchronize(h->stream));
     drop_graph(h);                       // the group views carry the buffer pointer and its block capacity
-    void* p = nullptr;
-    release_alloc(h, h->e.bmom);
-    h->e.bmom = nullptr; h->e.bmom_nb = 0;
-    int r = raw_alloc(h, &p, sizeof(double) * (size_t)d.C * nblocks * (d.V + d.q) * 2);
-    if (r) return r;
-    h->e.bmom = (double*)p;
-    h->e.bmom_nb = nblocks;
+    if (int r = grow_buffer(h, m.blocks, m.nblocks, (int)nblocks, sizeof(double) * h->e.d.C * m.P * 2)) return r;
   }
   h->win[2] = first_sweep; h->win[3] = block_len > 0 ? block_len : 1; h->win[4] = nblocks;
   h->blk_len = block_len;
   return push_windows(h);
 }
 
-// merge blocks [first_block, first_block + nblocks) (nblocks even) into the split-half moments: Chan's pairwise update
-// applied block after block in a fixed order.  grid = (ceil(P/128), C, 2)
-__global__ void k_merge_blocks(const double* __restrict__ bmom, int nb_cap, int nparam, int first_block, int per_half,
-                               long long blen, double* __restrict__ mom) {
-  const int p = blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= nparam) return;
-  const int c = blockIdx.y, half = blockIdx.z;
-  double n = 0.0, mean = 0.0, m2 = 0.0;
-  for (int b = 0; b < per_half; ++b) {
-    const double* m = bmom + (((size_t)c * nb_cap + first_block + half * per_half + b) * nparam + p) * 2;
-    const double nb_ = (double)blen, delta = m[0] - mean, tot = n + nb_;
-    mean += delta * nb_ / tot;
-    m2 += m[1] + delta * delta * n * nb_ / tot;
-    n = tot;
-  }
-  double* o = mom + (((size_t)c * 2 + half) * nparam + p) * 2;
-  o[0] = mean; o[1] = m2;
-}
-
+// merge blocks [first_block, first_block + nblocks) (nblocks even) into the split-half moments
 extern "C" int bnr_moments_from_blocks(bnr_handle* h, int32_t first_block, int32_t nblocks) {
   if (!h || first_block < 0 || nblocks < 2 || (nblocks & 1)) return fail(BNR_EINVAL, "need an even number of blocks >= 2");
   CK(cudaSetDevice(h->p.device));
-  if (!h->e.bmom || first_block + nblocks > (int)h->win[4]) return fail(BNR_ESTATE, "blocks not configured (bnr_set_moment_blocks)");
-  const Dims& d = h->e.d;
-  const int np_ = d.V + d.q;
-  dim3 grid((np_ + 127) / 128, d.C, 2);
-  k_merge_blocks<<<grid, 128, 0, h->stream>>>(h->e.bmom, h->e.bmom_nb, np_, first_block, nblocks / 2, h->blk_len, h->e.moments);
+  if (!h->e.mom.blocks || first_block + nblocks > (int)h->win[4]) return fail(BNR_ESTATE, "blocks not configured (bnr_set_moment_blocks)");
+  launch_merge_blocks(h->e.mom, h->e.d.C, first_block, nblocks / 2, h->blk_len, h->stream);
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
   h->mom_half = (long long)(nblocks / 2) * h->blk_len;
@@ -945,7 +927,7 @@ extern "C" int bnr_moments_device(bnr_handle* h, double** dev_ptr, int64_t* coun
   if (!h || !dev_ptr || !count) return fail(BNR_EINVAL, "null argument");
   CK(cudaSetDevice(h->p.device));
   CK(cudaStreamSynchronize(h->stream));
-  *dev_ptr = h->e.moments;
+  *dev_ptr = h->e.mom.halves;
   *count = (int64_t)h->e.d.C * 2 * (h->e.d.V + h->e.d.q) * 2;
   return BNR_OK;
 }
@@ -965,24 +947,7 @@ extern "C" int bnr_rhat_from_moments(int device, const double* dev_moments, int3
   return BNR_OK;
 }
 
-// two-pass split-half moments of rows [first_row, first_row + nrows) of the gamma/xi traces (what
-// return_psrf_VOI + rhat see, src/gibbs.jl:771-789).  grid = (ceil((V+q)/128), C, 2)
-__global__ void k_moments_from_trace(RowTable tr, long long first, long long nrows, double* __restrict__ mom) {
-  const int nparam = tr.width, p = blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= nparam) return;
-  const int c = blockIdx.y, half = blockIdx.z;
-  const long long h = nrows / 2;
-  const long long r0 = first + (half == 0 ? 0 : nrows - h);
-  const double* __restrict__ base = tr.row(c, r0) + p;
-  double s = 0.0;
-  for (long long r = 0; r < h; ++r) s += base[(size_t)r * nparam];
-  const double mean = s / (double)h;
-  double m2 = 0.0;
-  for (long long r = 0; r < h; ++r) { const double dl = base[(size_t)r * nparam] - mean; m2 += dl * dl; }
-  double* m = mom + (((size_t)c * 2 + half) * nparam + p) * 2;
-  m[0] = mean; m[1] = m2;
-}
-
+// two-pass split-half moments of rows [first_row, first_row + nrows) of the gamma/xi traces
 extern "C" int bnr_moments_from_trace(bnr_handle* h, int64_t first_row, int64_t nrows) {
   if (!h || first_row < 0 || nrows < 0) return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
@@ -992,8 +957,7 @@ extern "C" int bnr_moments_from_trace(bnr_handle* h, int64_t first_row, int64_t 
                             "moments of bnr_set_moment_window instead");
   if (first_row + nrows > e.tr_gx.rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
   if (nrows / 2 < 2) return fail(BNR_EINVAL, "need at least 4 rows");
-  dim3 grid((e.tr_gx.width + 127) / 128, e.d.C, 2);
-  k_moments_from_trace<<<grid, 128, 0, h->stream>>>(e.tr_gx, first_row, nrows, e.moments);
+  launch_moments_from_trace(e.tr_gx, first_row, nrows, e.mom, h->stream);
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
   h->mom_half = nrows / 2;
@@ -1012,7 +976,7 @@ extern "C" int bnr_rhat(bnr_handle* h, double* rhat_xi, double* rhat_gamma) {
   CK(cudaSetDevice(h->p.device));
   if (h->mom_half < 2) return fail(BNR_ESTATE, "moment window too short for R-hat");
   const Dims& d = h->e.d;
-  launch_rhat(h->e.moments, d.C, d.V + d.q, h->mom_half, h->d_rhat, h->stream);
+  launch_rhat(h->e.mom.halves, d.C, d.V + d.q, h->mom_half, h->d_rhat, h->stream);
   std::vector<double> host(d.V + d.q);
   CK(cudaMemcpyAsync(host.data(), h->d_rhat, sizeof(double) * (d.V + d.q), cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
@@ -1159,15 +1123,7 @@ extern "C" int bnr_set_injection(bnr_handle* h, const double* inj, int64_t per_c
   drop_graph(h);
   if (!inj) { h->e.inj = nullptr; h->e.inj_stride = 0; return BNR_OK; }
   const size_t total = (size_t)per_chain * h->e.d.C;
-  if ((long long)total > h->inj_len) {
-    void* p = nullptr;
-    release_alloc(h, h->d_inj);
-    h->d_inj = nullptr; h->inj_len = 0;
-    int r = raw_alloc(h, &p, total * sizeof(double));
-    if (r) return r;
-    h->d_inj = (double*)p;
-    h->inj_len = (long long)total;
-  }
+  if (int r = grow_buffer(h, h->d_inj, h->inj_len, total)) return r;
   CK(cudaMemcpy(h->d_inj, inj, total * sizeof(double), cudaMemcpyHostToDevice));
   h->e.inj = h->d_inj;
   h->e.inj_stride = per_chain;
@@ -1364,7 +1320,6 @@ extern "C" int bnr_summary(bnr_handle* h, int32_t chain, int64_t first_row, int6
   if (first_row + nrows > e.tr_full.rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
   if (rank_lo < 1 || rank_hi < 1 || rank_lo > nrows || rank_hi > nrows)
     return fail(BNR_EINVAL, "order-statistic ranks must lie in 1..nrows (the reference raises a BoundsError)");
-  CK(cudaSetDevice(h->p.device));
   int off_g = 0, off_x = 0;
   const RowTable* t = traced(e, chain, BNR_VAR_GAMMA, &off_g);
   if (!t) return fail(BNR_ESTATE, "gamma/xi of this chain are not traced");
@@ -1389,6 +1344,21 @@ extern "C" int bnr_summary(bnr_handle* h, int32_t chain, int64_t first_row, int6
 // ---------------------------------------------------------------------------------------------------------
 // Effective sample size of xi / gamma over rows [first_row, first_row + nrows) of every chain's trace
 // ---------------------------------------------------------------------------------------------------------
+// the lag budget of both ESS paths for n draws: at most n - 1, odd (Geyer pairs (2t, 2t+1) end on an odd lag), >= 1
+static int clamp_ess_lag(int max_lag, long long n) {
+  if (max_lag > n - 1) max_lag = (int)(n - 1);
+  if (!(max_lag & 1)) max_lag -= 1;
+  return max_lag < 1 ? 1 : max_lag;
+}
+
+// the statistics buffers both ESS paths fill: d_acov [L + 1][V + q] and d_cmean [C][V + q]
+static int size_ess_outputs(bnr_handle* h, int L) {
+  const size_t P = (size_t)h->e.d.V + h->e.d.q;
+  if (int r = grow_buffer(h, h->d_acov, h->acov_cap, (L + 1) * P)) return r;
+  if (!h->d_cmean) DA(h->d_cmean, h->e.d.C * P);
+  return BNR_OK;
+}
+
 extern "C" int bnr_ess_accumulate(bnr_handle* h, int64_t first_row, int64_t nrows, int32_t max_lag) {
   if (!h || first_row < 0 || nrows < 4 || max_lag < 1) return fail(BNR_EINVAL, "bad arguments (need nrows >= 4, max_lag >= 1)");
   CK(cudaSetDevice(h->p.device));
@@ -1397,22 +1367,8 @@ extern "C" int bnr_ess_accumulate(bnr_handle* h, int64_t first_row, int64_t nrow
   if (!e.tr_gx.base || e.tr_gx.chains < d.C)
     return fail(BNR_ESTATE, "gamma/xi traces of every chain are not recorded (trace_gamma_xi_all = 0)");
   if (first_row + nrows > e.tr_gx.rows) return fail(BNR_EINVAL, "rows beyond trace capacity");
-  if (max_lag > nrows - 1) max_lag = (int32_t)(nrows - 1);
-  if (!(max_lag & 1)) max_lag -= 1;                  // Geyer pairs (2t, 2t+1): keep the last lag odd
-  if (max_lag < 1) max_lag = 1;
-  CK(cudaSetDevice(h->p.device));
-  const int P = d.V + d.q;
-  const size_t need = (size_t)(max_lag + 1) * P;
-  if (need > h->acov_cap) {
-    void* pnew = nullptr;
-    release_alloc(h, h->d_acov);
-    h->d_acov = nullptr; h->acov_cap = 0;
-    int r = raw_alloc(h, &pnew, need * sizeof(double));
-    if (r) return r;
-    h->d_acov = (double*)pnew;
-    h->acov_cap = need;
-  }
-  if (!h->d_cmean) DA(h->d_cmean, (size_t)d.C * P);
+  max_lag = clamp_ess_lag(max_lag, nrows);
+  if (int r = size_ess_outputs(h, max_lag)) return r;
   launch_chain_mean(e.tr_gx, first_row, nrows, h->d_cmean, h->stream);
   launch_acov_sum(e.tr_gx, first_row, nrows, max_lag, h->d_cmean, h->d_acov, h->stream);
   CK(cudaGetLastError());
@@ -1428,57 +1384,30 @@ static int ess_stream_arm(bnr_handle* h, int32_t max_lag, int64_t first_sweep, i
   if (!h || ndraws < 4 || max_lag < 1) return fail(BNR_EINVAL, "bad arguments (need ndraws >= 4, max_lag >= 1)");
   CK(cudaSetDevice(h->p.device));
   Engine& e = h->e;
-  const Dims& d = e.d;
-  if (max_lag > ndraws - 1) max_lag = (int32_t)(ndraws - 1);
-  if (!(max_lag & 1)) max_lag -= 1;
-  if (max_lag < 1) max_lag = 1;
-  const int L = max_lag, cap = L + 8;
-  const size_t P = (size_t)d.V + d.q, C = d.C;
+  const int L = clamp_ess_lag(max_lag, ndraws);
   CK(cudaStreamSynchronize(h->stream));
   long long it = 0;
   CK(cudaMemcpyAsync(&it, e.iter, sizeof(it), cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   if (first_sweep < 0) first_sweep = it + 1;
   if (first_sweep <= it) return fail(BNR_EINVAL, "the window must start after the sweeps already run");
-  if (!e.ess_ring || e.ess_L != L) drop_graph(h);   // the sweep graphs gain the k_ess_stream node / its new geometry
-  const size_t need = C * P * ((size_t)cap + L + (L + 1) + 2);
-  if (need > h->ess_stream_cap) {
-    void* pnew = nullptr;
-    release_alloc(h, h->ess_stream_buf);
-    h->ess_stream_buf = nullptr; h->ess_stream_cap = 0;
-    int r = raw_alloc(h, &pnew, need * sizeof(double));
-    if (r) return r;
-    h->ess_stream_cap = need;
-    h->ess_stream_buf = (double*)pnew;
-    drop_graph(h);
-  }
-  e.ess_ring = h->ess_stream_buf;
-  e.ess_head = e.ess_ring + C * P * cap;
-  e.ess_acc = e.ess_head + C * P * L;
-  e.ess_sum = e.ess_acc + C * P * (L + 1);
-  e.ess_L = L; e.ess_cap = cap;
-  e.ess_win = h->d_esswin;
-  const long long win[4] = {first_sweep, ndraws, L, cap};
+  EssStream es = e.ess;
+  es.L = L; es.cap = L + 8;
+  const size_t need = es.doubles(e.d.C);
+  // the sweep graphs gain the k_ess_stream node, or bake its new geometry or buffer
+  if (!e.ess.on() || e.ess.L != L || need > h->ess_stream_cap) drop_graph(h);
+  if (int r = grow_buffer(h, h->ess_stream_buf, h->ess_stream_cap, need)) return r;
+  es.carve(h->ess_stream_buf, e.d.C);
+  e.ess = es;
+  const long long win[2] = {first_sweep, ndraws};
   CK(cudaMemcpyAsync(h->d_esswin, win, sizeof(win), cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
-  const size_t acov_need = (size_t)(L + 1) * P;
-  if (acov_need > h->acov_cap) {
-    void* pnew = nullptr;
-    release_alloc(h, h->d_acov);
-    h->d_acov = nullptr; h->acov_cap = 0;
-    int r = raw_alloc(h, &pnew, acov_need * sizeof(double));
-    if (r) return r;
-    h->d_acov = (double*)pnew;
-    h->acov_cap = acov_need;
-  }
-  if (!h->d_cmean) DA(h->d_cmean, C * P);
+  if (int r = size_ess_outputs(h, L)) return r;
   h->ess_stream_N = ndraws;
   h->ess_lag = -1;
   return BNR_OK;
 }
 
-// Streaming variant: the next `ndraws` sweeps contribute their lagged products while they run (k_ess_stream), so no
-// chain needs a trace.  bnr_ess_stream_finish turns the accumulators into the same two statistics buffers.
 extern "C" int bnr_ess_stream_begin(bnr_handle* h, int32_t max_lag, int64_t ndraws) {
   return ess_stream_arm(h, max_lag, -1, ndraws);
 }
@@ -1490,10 +1419,10 @@ extern "C" int bnr_ess_stream_window(bnr_handle* h, int32_t max_lag, int64_t fir
 
 extern "C" int bnr_ess_stream_finish(bnr_handle* h) {
   if (!h) return fail(BNR_EINVAL, "null handle");
-  if (h->ess_stream_N <= 0 || !h->e.ess_ring) return fail(BNR_ESTATE, "call bnr_ess_stream_begin first");
+  if (h->ess_stream_N <= 0 || !h->e.ess.on()) return fail(BNR_ESTATE, "call bnr_ess_stream_begin first");
   CK(cudaSetDevice(h->p.device));
   CK(cudaStreamSynchronize(h->stream));
-  long long it = 0, win[4];
+  long long it = 0, win[2];
   CK(cudaMemcpy(&it, h->e.iter, sizeof(it), cudaMemcpyDeviceToHost));
   CK(cudaMemcpy(win, h->d_esswin, sizeof(win), cudaMemcpyDeviceToHost));
   if (it < win[0] + win[1] - 1)
@@ -1501,11 +1430,12 @@ extern "C" int bnr_ess_stream_finish(bnr_handle* h) {
   launch_ess_stream_finalize(h->e, h->ess_stream_N, h->d_acov, h->d_cmean, h->stream);
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(h->stream));
-  h->ess_lag = h->e.ess_L;
+  EssStream& es = h->e.ess;
+  h->ess_lag = es.L;
   h->ess_rows = h->ess_stream_N;
   h->ess_stream_N = 0;
   drop_graph(h);                         // later sweeps run without the accumulation kernel
-  h->e.ess_ring = h->e.ess_head = h->e.ess_acc = h->e.ess_sum = nullptr;
+  es.ring_ = es.head_ = es.acc_ = es.sum_ = nullptr;
   // (the buffer stays with the handle and is reused by the next bnr_ess_stream_begin)
   return BNR_OK;
 }
@@ -1601,7 +1531,7 @@ extern "C" int bnr_export_moments(bnr_handle* h, double* dev_dst) {
   if (!h || !dev_dst) return fail(BNR_EINVAL, "null argument");
   CK(cudaSetDevice(h->p.device));
   const size_t n = (size_t)h->e.d.C * 2 * (h->e.d.V + h->e.d.q) * 2;
-  CK(cudaMemcpyAsync(dev_dst, h->e.moments, n * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+  CK(cudaMemcpyAsync(dev_dst, h->e.mom.halves, n * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   return BNR_OK;
 }

@@ -1,8 +1,12 @@
-// Posterior diagnostics computed on the device from the recorded traces (iteration-major rows):
+// Posterior diagnostics computed on the device from the recorded traces (iteration-major rows) or from the statistics
+// streamed while the chains run:
 //   * Summary (src/gibbs.jl:1214-1250): per-edge posterior mean and the two order statistics sort(gamma)[lw], [hi]
 //     that bound the credible interval, per-node mean xi            -> k_summary_select (radix select, no sort)
 //   * gamma / xi effective sample size (BASELINE metric "gamma ESS/sec"; not in the reference): multi-chain Geyer
-//     initial-monotone-sequence estimator on direct-lag autocovariances -> k_chain_mean, k_acov_sum, k_ess_finish
+//     initial-monotone-sequence estimator on direct-lag autocovariances -> k_chain_mean, k_acov_sum, k_ess_finish;
+//     streamed without traces (EssStream)                              -> k_ess_stream, k_ess_stream_finalize
+//   * split R-hat (src/convergence.jl:4-65)                            -> k_rhat, on the SplitMoments that k_record
+//     streams, k_moments_from_trace computes from a trace or k_merge_blocks from block moments
 // Everything is deterministic (fixed reduction orders, integer histograms).
 #include "bnr_engine.cuh"
 #include "bnr_kernels.h"
@@ -612,23 +616,24 @@ constexpr int ES_B = 8;
 
 __global__ void __launch_bounds__(128) k_ess_stream(Engine e) {
   const Dims& d = e.d;
+  const EssStream& es = e.ess;
   const int P = d.V + d.q;
   const int p = blockIdx.x * blockDim.x + threadIdx.x, c = blockIdx.y;
   if (p >= P) return;
-  const long long first = e.ess_win[0], N = e.ess_win[1];
-  const int L = (int)e.ess_win[2], cap = (int)e.ess_win[3];
+  const long long first = es.win[0], N = es.win[1];
+  const int L = es.L, cap = es.cap;
   const long long k = (*e.iter + 1) - first;        // index of this sweep's draw inside the window
   if (k < 0 || k >= N) return;
   const double x = (p < d.V) ? e.xi[c * d.V + p] : e.gamma[(size_t)c * d.qp + (p - d.V)];
-  double* sum = e.ess_sum + (size_t)c * 2 * P;
-  double* ring = e.ess_ring + (size_t)c * cap * P + p;
+  double* sum = es.sum(c);
+  double* ring = es.ring(c) + p;
   double ref, S;
   if (k == 0) { ref = x; S = 0.0; sum[p] = ref; }
   else { ref = sum[p]; S = sum[P + p]; }
   const double y = x - ref;
   sum[P + p] = S + y;
   ring[(size_t)(k % cap) * P] = y;
-  if (k < L) e.ess_head[((size_t)c * L + k) * P + p] = y;
+  if (k < L) es.head(c)[(size_t)k * P + p] = y;
   const int b = (int)(k % ES_B) + 1;
   if (b != ES_B && k != N - 1) return;
   // block of the b newest draws k0 .. k: A_l += sum_j y_(k0+j) y_(k0+j-l)
@@ -639,7 +644,7 @@ __global__ void __launch_bounds__(128) k_ess_stream(Engine e) {
     Y[j] = (j < b) ? ring[(size_t)((k0 + j) % cap) * P] : 0.0;
     w[j] = Y[j];
   }
-  double* A = e.ess_acc + (size_t)c * (L + 1) * P + p;
+  double* A = es.acc(c) + p;
   const int lmax = (long long)L < k ? L : (int)k;
   const bool fresh = (k0 == 0);                     // first block of the window: A starts from zero
   for (int l = 0; l <= L; ++l) {
@@ -661,17 +666,19 @@ __global__ void __launch_bounds__(128) k_ess_stream(Engine e) {
 __global__ void __launch_bounds__(128) k_ess_stream_finalize(Engine e, long long N, double* __restrict__ acov,
                                                              double* __restrict__ cmean) {
   const Dims& d = e.d;
-  const int P = d.V + d.q, L = e.ess_L, cap = e.ess_cap;
+  const EssStream& es = e.ess;
+  const int P = es.P, L = es.L, cap = es.cap;
   const int p = blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= P) return;
   const double n = (double)N;
   for (int c = 0; c < d.C; ++c) {
-    const double ref = e.ess_sum[(size_t)c * 2 * P + p], S = e.ess_sum[(size_t)c * 2 * P + P + p];
+    const double* sum = es.sum(c) + p;
+    const double ref = sum[0], S = sum[P];
     const double m = S / n;
     cmean[(size_t)c * P + p] = ref + m;
-    const double* A = e.ess_acc + (size_t)c * (L + 1) * P + p;
-    const double* head = e.ess_head + (size_t)c * L * P + p;
-    const double* ring = e.ess_ring + (size_t)c * cap * P + p;
+    const double* A = es.acc(c) + p;
+    const double* head = es.head(c) + p;
+    const double* ring = es.ring(c) + p;
     double H = 0.0, T = 0.0;
     for (int l = 0; l <= L; ++l) {
       if (l >= 1) {
@@ -682,6 +689,82 @@ __global__ void __launch_bounds__(128) k_ess_stream_finalize(Engine e, long long
       acov[(size_t)l * P + p] = (c == 0 ? 0.0 : acov[(size_t)l * P + p]) + v;
     }
   }
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Split R-hat, thread per parameter.  k_rhat: from [chains][2][P][2] split-half moments, of one handle or gathered.
+// k_moments_from_trace: two passes over trace rows [first, first + nrows) (return_psrf_VOI, src/gibbs.jl:771-789).
+// k_merge_blocks: Chan's pairwise update of blocks [first_block, first_block + 2 per_half), in block order.
+// ------------------------------------------------------------------------------------------------------------
+__global__ void k_rhat(const double* __restrict__ mom, int chains, int nparams, long long h, double* out) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= nparams) return;
+  const int ns = 2 * chains;
+  double W = 0.0, mm = 0.0;
+  for (int s = 0; s < ns; ++s) {
+    const double* m = mom + ((size_t)s * nparams + p) * 2;
+    W += m[1] / (double)(h - 1);
+    mm += m[0];
+  }
+  W /= ns; mm /= ns;
+  double B = 0.0;
+  for (int s = 0; s < ns; ++s) {
+    const double dm = mom[((size_t)s * nparams + p) * 2] - mm;
+    B += dm * dm;
+  }
+  B /= (ns - 1);
+  const double varp = (double)(h - 1) / (double)h * W + B;
+  double r;
+  if (varp == 0.0 && W == 0.0) r = 1.0;
+  else if (W == 0.0) r = INFINITY;
+  else r = sqrt(varp / W);
+  out[p] = r;
+}
+
+__global__ void k_moments_from_trace(RowTable tr, long long first, long long nrows, SplitMoments mom) {
+  const int nparam = tr.width, p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= nparam) return;
+  const int c = blockIdx.y, half = blockIdx.z;
+  const long long h = nrows / 2;
+  const long long r0 = first + (half == 0 ? 0 : nrows - h);
+  const double* __restrict__ base = tr.row(c, r0) + p;
+  double s = 0.0;
+  for (long long r = 0; r < h; ++r) s += base[(size_t)r * nparam];
+  const double mean = s / (double)h;
+  double m2 = 0.0;
+  for (long long r = 0; r < h; ++r) { const double dl = base[(size_t)r * nparam] - mean; m2 += dl * dl; }
+  double* m = mom.half(c, half, p);
+  m[0] = mean; m[1] = m2;
+}
+
+__global__ void k_merge_blocks(SplitMoments mom, int first_block, int per_half, long long blen) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= mom.P) return;
+  const int c = blockIdx.y, half = blockIdx.z;
+  double n = 0.0, mean = 0.0, m2 = 0.0;
+  for (int b = 0; b < per_half; ++b) {
+    const double* m = mom.block(c, first_block + half * per_half + b, p);   // (through __ldg: not __restrict__)
+    const double nb_ = (double)blen, delta = __ldg(m) - mean, tot = n + nb_;
+    mean += delta * nb_ / tot;
+    m2 += __ldg(m + 1) + delta * delta * n * nb_ / tot;
+    n = tot;
+  }
+  double* o = mom.half(c, half, p);
+  o[0] = mean; o[1] = m2;
+}
+
+void launch_rhat(const double* mom, int chains, int nparams, long long h, double* out, cudaStream_t s) {
+  ++g_launches; k_rhat<<<(nparams + 127) / 128, 128, 0, s>>>(mom, chains, nparams, h, out);
+}
+
+void launch_moments_from_trace(const RowTable& tr, long long first, long long nrows, const SplitMoments& mom,
+                               cudaStream_t s) {
+  k_moments_from_trace<<<dim3((tr.width + 127) / 128, tr.chains, 2), 128, 0, s>>>(tr, first, nrows, mom);
+}
+
+void launch_merge_blocks(const SplitMoments& mom, int chains, int first_block, int per_half, long long blen,
+                         cudaStream_t s) {
+  k_merge_blocks<<<dim3((mom.P + 127) / 128, chains, 2), 128, 0, s>>>(mom, first_block, per_half, blen);
 }
 
 void launch_ess_stream(const Engine& e, cudaStream_t s) {

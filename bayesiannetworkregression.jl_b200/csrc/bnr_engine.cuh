@@ -104,6 +104,75 @@ struct RowTable {
   size_t doubles() const { return (size_t)chains * rows * width; }
 };
 
+// Streamed (mean, M2) moments of the P = V + q parameters (xi then gamma) that R-hat reads: the split-half window
+// [C][2][P][2] and the per-block moments [C][nblocks][P][2] that bnr_moments_from_blocks merges into any window made of
+// whole blocks (the doubling scheme's growing window without all-chain traces).  blocks == nullptr: no block moments
+struct SplitMoments {
+  double* halves;
+  long long* window;   // device [5]: split-half window (first sweep, len), blocks (first sweep, block len, count)
+  double* blocks;
+  int nblocks;         // block capacity of `blocks`
+  int P;
+  __host__ __device__ double* half(int c, int h, int p) const { return halves + (((size_t)c * 2 + h) * P + p) * 2; }
+  __host__ __device__ double* block(int c, long long b, int p) const {
+    return blocks + (((size_t)c * nblocks + b) * P + p) * 2;
+  }
+  // Welford step of draw x of sweep `sweep` into the half window and the block that hold the sweep (if any)
+  __device__ void add(int c, int p, long long sweep, double x) const {
+    const long long first = window[0], len = window[1];
+    const long long h = len / 2, rel = sweep - first;
+    if (len > 1 && rel >= 0 && rel < len) {
+      int hf = -1;
+      long long cnt = 0;
+      if (rel < h) { hf = 0; cnt = rel + 1; }
+      else if (rel >= len - h) { hf = 1; cnt = rel - (len - h) + 1; }
+      if (hf >= 0) welford(half(c, hf, p), cnt, x);
+    }
+    const long long bfirst = window[2], blen = window[3], bcnt = window[4];
+    if (blocks && bcnt > 0 && sweep >= bfirst) {
+      const long long b = (sweep - bfirst) / blen;
+      if (b < bcnt && b < nblocks) welford(block(c, b, p), (sweep - bfirst) % blen + 1, x);
+    }
+  }
+  __device__ static void welford(double* m, long long cnt, double x) {
+    double mean = (cnt == 1) ? 0.0 : m[0], m2 = (cnt == 1) ? 0.0 : m[1];
+    const double dl = x - mean;
+    mean += dl / (double)cnt;
+    m2 += dl * (x - mean);
+    m[0] = mean; m[1] = m2;
+  }
+  // the chains from c0 on of a chain group, which keeps its own device window record
+  SplitMoments view(int c0, long long* group_window) const {
+    SplitMoments v = *this;
+    v.halves = half(c0, 0, 0);
+    if (blocks) v.blocks = block(c0, 0, 0);
+    v.window = group_window;
+    return v;
+  }
+};
+
+// Streamed ESS accumulators (bnr_ess_stream_begin; kernels in bnr_diagnostics.cu), per chain and parameter p < P with
+// y_t = x_t - x_first: ring [C][cap][P] of the last cap centred draws, head [C][L][P] the first L, acc [C][L+1][P] the
+// lagged products A_l = sum_t y_t y_(t-l), sum [C][2][P] x_first and sum_t y_t.  One allocation holds the four in this
+// order.  ring == nullptr: off
+struct EssStream {
+  double *ring_, *head_, *acc_, *sum_;
+  const long long* win;   // device [2]: first sweep, draws N
+  int L, cap, P;
+  __host__ __device__ bool on() const { return ring_ != nullptr; }
+  __host__ __device__ double* ring(int c) const { return ring_ + (size_t)c * cap * P; }
+  __host__ __device__ double* head(int c) const { return head_ + (size_t)c * L * P; }
+  __host__ __device__ double* acc(int c) const { return acc_ + (size_t)c * (L + 1) * P; }
+  __host__ __device__ double* sum(int c) const { return sum_ + (size_t)c * 2 * P; }
+  size_t doubles(int C) const { return (size_t)C * P * ((size_t)cap + L + (L + 1) + 2); }
+  void carve(double* base, int C) { ring_ = base; head_ = ring(C); acc_ = head(C); sum_ = acc(C); }
+  EssStream view(int c0) const {
+    EssStream v = *this;
+    if (on()) { v.ring_ = ring(c0); v.head_ = head(c0); v.acc_ = acc(c0); v.sum_ = sum(c0); }
+    return v;
+  }
+};
+
 struct Engine {
   Dims d;
   // data (read-only, shared by all chains)
@@ -133,18 +202,8 @@ struct Engine {
   int* status;      // [C]
   long long* iter;  // device scalar: completed sweeps
   long long* trace_row;   // device scalar: next trace row
-  // moments [C][2][V+q][2] and window
-  double* moments;
-  long long* mom_window;  // device [5]: split-half window (first sweep, len), block moments (first sweep, block len, blocks)
-  double* bmom;           // [C][bmom_nb][V+q][2] per-block (mean, M2): mergeable R-hat windows (doubling scheme)
-  int bmom_nb;
-  // streaming ESS statistics (bnr_ess_stream_begin; kernels in bnr_diagnostics.cu).  y_t = x_t - x_first per chain / parameter
-  double* ess_ring;       // [C][ess_cap][V+q]  ring of the last ess_cap centred draws
-  double* ess_head;       // [C][L][V+q]        the first L centred draws
-  double* ess_acc;        // [C][L+1][V+q]      lagged products A_l = sum_t y_t y_(t-l)
-  double* ess_sum;        // [C][2][V+q]        x_first, sum_t y_t
-  const long long* ess_win;  // device [4]: first sweep, draws N, max lag L, ring capacity ess_cap
-  int ess_L, ess_cap;
+  SplitMoments mom;
+  EssStream ess;
   // traces of the leading tr_full.chains / tr_gx.chains chains; both keep rows = the handle's trace capacity when off
   RowTable tr_full;       // full state rows (state_elem order)
   RowTable tr_gx;         // xi then gamma, width V+q

@@ -31,7 +31,6 @@ void launch_finish(const Engine& e, int mask, cudaStream_t s);
 void launch_init(const Engine& e, cudaStream_t s);
 void launch_record(const Engine& e, int sweep_done, cudaStream_t s);
 void launch_advance(const Engine& e, int inc_iter, cudaStream_t s);
-void launch_rhat(const double* mom, int chains, int nparams, long long h, double* out, cudaStream_t s);
 void launch_test_chol_jitter(int R, const double* Ain, double* Aused, double* Lout, int* status, cudaStream_t s);
 void launch_rng_dump(const Dims& d, int chain, long long iteration, int site, int element, int kind, double shape,
                      int count, double* out, cudaStream_t s);
@@ -110,5 +109,12 @@ size_t loo_ws_bytes(long long N, int n);
 void launch_loo(const double* rows, long long N, int n, double* out, void* ws, cudaStream_t s);
 void launch_ess_finish(const double* acov_parts, int nparts, const double* cmeans, int chains, int P, long long N,
                        int L, double* ess, double* lag_used, cudaStream_t s);
+// split R-hat of [chains][2][nparams][2] moments (h draws per half); the split-half moments of mom from trace rows
+// [first, first + nrows) of every chain of tr, or from blocks of blen sweeps (these two not counted in g_launches)
+void launch_rhat(const double* mom, int chains, int nparams, long long h, double* out, cudaStream_t s);
+void launch_moments_from_trace(const RowTable& tr, long long first, long long nrows, const SplitMoments& mom,
+                               cudaStream_t s);
+void launch_merge_blocks(const SplitMoments& mom, int chains, int first_block, int per_half, long long blen,
+                         cudaStream_t s);
 
 }  // namespace bnr

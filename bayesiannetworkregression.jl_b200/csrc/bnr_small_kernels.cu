@@ -771,37 +771,7 @@ __global__ void __launch_bounds__(256) k_record(Engine e, int sweep_done /* 1: s
   if (p < np_) {
     const double x = (p < d.V) ? e.xi[c * d.V + p] : e.gamma[(size_t)c * d.qp + (p - d.V)];
     if (e.tr_gx.holds(c, row)) e.tr_gx.row(c, row)[p] = x;
-    const long long first = e.mom_window[0], len = e.mom_window[1];
-    const long long h = len / 2, rel = sweep - first;
-    if (len > 1 && rel >= 0 && rel < len) {
-      int half = -1;
-      long long cnt = 0;
-      if (rel < h) { half = 0; cnt = rel + 1; }
-      else if (rel >= len - h) { half = 1; cnt = rel - (len - h) + 1; }
-      if (half >= 0) {
-        double* m = e.moments + (((size_t)c * 2 + half) * np_ + p) * 2;
-        double mean = (cnt == 1) ? 0.0 : m[0], m2 = (cnt == 1) ? 0.0 : m[1];
-        const double dl = x - mean;
-        mean += dl / (double)cnt;
-        m2 += dl * (x - mean);
-        m[0] = mean; m[1] = m2;
-      }
-    }
-    // block moments: sweep s belongs to block (s - first) / block_len; blocks are merged later into any window made
-    // of whole blocks (bnr_moments_from_blocks) -- the doubling scheme's growing window without all-chain traces
-    const long long bfirst = e.mom_window[2], blen = e.mom_window[3], bcnt = e.mom_window[4];
-    if (e.bmom && bcnt > 0 && sweep >= bfirst) {
-      const long long b = (sweep - bfirst) / blen;
-      if (b < bcnt && b < e.bmom_nb) {
-        const long long cnt = (sweep - bfirst) % blen + 1;
-        double* m = e.bmom + (((size_t)c * e.bmom_nb + b) * np_ + p) * 2;
-        double mean = (cnt == 1) ? 0.0 : m[0], m2 = (cnt == 1) ? 0.0 : m[1];
-        const double dl = x - mean;
-        mean += dl / (double)cnt;
-        m2 += dl * (x - mean);
-        m[0] = mean; m[1] = m2;
-      }
-    }
+    e.mom.add(c, p, sweep, x);
   }
   if (e.tr_full.holds(c, row)) {
     double* dst = e.tr_full.row(c, row);
@@ -845,33 +815,6 @@ __global__ void k_advance(Engine e, int inc_iter) {
     if (inc_iter) *e.iter += 1;
     *e.trace_row += 1;
   }
-}
-
-// R-hat from split-half moments (rhat, src/convergence.jl:4-65): one thread per parameter.
-// moments: [chains][2][nparams][2]
-__global__ void k_rhat(const double* __restrict__ mom, int chains, int nparams, long long h, double* out) {
-  const int p = blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= nparams) return;
-  const int ns = 2 * chains;
-  double W = 0.0, mm = 0.0;
-  for (int s = 0; s < ns; ++s) {
-    const double* m = mom + ((size_t)s * nparams + p) * 2;
-    W += m[1] / (double)(h - 1);
-    mm += m[0];
-  }
-  W /= ns; mm /= ns;
-  double B = 0.0;
-  for (int s = 0; s < ns; ++s) {
-    const double dm = mom[((size_t)s * nparams + p) * 2] - mm;
-    B += dm * dm;
-  }
-  B /= (ns - 1);
-  const double varp = (double)(h - 1) / (double)h * W + B;
-  double r;
-  if (varp == 0.0 && W == 0.0) r = 1.0;
-  else if (W == 0.0) r = INFINITY;
-  else r = sqrt(varp / W);
-  out[p] = r;
 }
 
 // raw streams for the parity tests (bnr_rng_stream / bnr_rng_gamma)
@@ -947,9 +890,6 @@ void launch_loglik_record(const Engine& e, cudaStream_t s) {
   ++g_launches; k_loglik_record<<<grid, 256, 0, s>>>(e);
 }
 void launch_advance(const Engine& e, int inc_iter, cudaStream_t s) { k_advance<<<1, 32, 0, s>>>(e, inc_iter); }
-void launch_rhat(const double* mom, int chains, int nparams, long long h, double* out, cudaStream_t s) {
-  ++g_launches; k_rhat<<<(nparams + 127) / 128, 128, 0, s>>>(mom, chains, nparams, h, out);
-}
 void launch_rng_dump(const Dims& d, int chain, long long iteration, int site, int element, int kind, double shape,
                      int count, double* out, cudaStream_t s) {
   ++g_launches; k_rng_dump<<<1, 32, 0, s>>>(d, chain, iteration, site, element, kind, shape, count, out);

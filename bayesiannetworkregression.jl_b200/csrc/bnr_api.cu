@@ -121,7 +121,9 @@ struct bnr_handle {
   cudaEvent_t ev_fork = nullptr;
   ForkJoin fj;                   // side stream for eager sweeps on the whole chain set
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  std::vector<std::pair<void*, size_t>> allocs;   // device buffers (pointer, bytes): returned to the cache on destroy
+  // device buffers, returned to the cache on destroy: pointer, block size, bytes asked for (a cached block can be larger)
+  struct Buffer { void* p; size_t bytes, asked; };
+  std::vector<Buffer> allocs;
   double* ws = nullptr;          // split-K workspace
   double* d_inj = nullptr;       // injected variates
   size_t inj_len = 0;
@@ -154,7 +156,7 @@ static int raw_alloc(bnr_handle* h, void** out, size_t bytes) {
   size_t got = bytes;
   void* p = cache_take(h->p.device, bytes, &got);
   if (!p) { CK(cudaMalloc(&p, bytes)); got = bytes; }
-  h->allocs.push_back({p, got});
+  h->allocs.push_back({p, got, bytes});
   *out = p;
   return 0;
 }
@@ -163,8 +165,8 @@ static int raw_alloc(bnr_handle* h, void** out, size_t bytes) {
 static void release_alloc(bnr_handle* h, void* p) {
   if (!p) return;
   for (size_t i = 0; i < h->allocs.size(); ++i)
-    if (h->allocs[i].first == p) {
-      cache_give(h->p.device, p, h->allocs[i].second);
+    if (h->allocs[i].p == p) {
+      cache_give(h->p.device, p, h->allocs[i].bytes);
       h->allocs[i] = h->allocs.back();
       h->allocs.pop_back();
       return;
@@ -233,25 +235,36 @@ extern "C" void bnr_default_params(bnr_params* p) {
   p->trace_full_chains = 1; p->trace_gamma_xi_all = 1; p->gig_inject_len = 64;
 }
 
-static int var_size(const Dims& d, int var) {
-  switch (var) {
-    case BNR_VAR_TAU2: case BNR_VAR_THETA: case BNR_VAR_DELTA: case BNR_VAR_MU: return 1;
-    case BNR_VAR_U: return d.R * d.V;
-    case BNR_VAR_XI: return d.V;
-    case BNR_VAR_GAMMA: case BNR_VAR_S: return d.q;
-    case BNR_VAR_M: return d.R * d.R;
-    case BNR_VAR_LAMBDA: return d.R;
-    case BNR_VAR_PI: return 3 * d.R;
+static_assert(BNR_NUM_VARS == NUM_STATE_VARS, "state variables out of sync");
+
+// Every chain-major array of an Engine with its per-chain element count (0: the array is absent in this handle) and
+// the elements that follow the last chain.  create_impl allocates through this list and group_view offsets through
+// it, so a chain group's view cannot miss an array.  The row tables, the streamed statistics (their own view types)
+// and the chain-group counters are not in it.
+template <class F>
+static void chain_arrays(Engine& e, F f) {
+  const Dims& d = e.d;
+  for (int v = 0; v < NUM_STATE_VARS; ++v) {
+    const StateVar s = state_var(d, v);
+    f(e.*s.at, (size_t)s.stride);
   }
-  return -1;
-}
-// offset of a variable inside a full trace row (k_record / state_elem order)
-static int row_offset(const Dims& d, int var) {
-  const int R = d.R, V = d.V, q = d.q;
-  const int o[BNR_NUM_VARS] = {0, 1, 1 + V * R, 1 + V * R + V, 1 + V * R + V + q, 1 + V * R + V + 2 * q,
-                               2 + V * R + V + 2 * q, 3 + V * R + V + 2 * q, 3 + V * R + V + 2 * q + R * R,
-                               4 + V * R + V + 2 * q + R * R, 4 + V * R + V + 2 * q + R * R + R};
-  return o[var];
+  const size_t qp = d.qp, np = d.np;
+  f(e.u_alt, (size_t)d.V * d.R);
+  f(e.W, qp); f(e.v, qp); f(e.t, qp);
+  f(e.xg, np); f(e.xv, np); f(e.rhs, np);
+  f(e.G, (size_t)d.gdim * d.gdim, (size_t)2048);
+  f(e.syrk_ws, (size_t)e.syrk_ws_cap * d.gdim * d.gdim);
+  // the blocks above the diagonal of every inverted panel are exact zeros that k_potf2_inv never writes: they come
+  // from the zero fill at allocation
+  f(e.Linv, (size_t)(d.gdim / TILE_N) * TILE_N * TILE_N);
+  const bool i8 = gram_i8_selected(d);
+  f(e.gram_planes, i8 ? gram_i8_plane_bytes(d) : 0);
+  f(e.gram_rscale, i8 ? np : 0);
+  f(e.partials, (size_t)d.nparts * (2 * MAX_R + 1));
+  f(e.status, (size_t)1);
+  f(e.pred_ws, (size_t)e.pred_splits * e.pred_mp);   // [pred_splits][C][pred_mp]: a view's chains sit at c0 * splits * mp
+  f(e.tau2_part, (size_t)2 * TAU2_MAX_BLOCKS);
+  f(e.tau2_ticket, (size_t)1);
 }
 
 // the two branch streams of a stream (side at priority side_prio, side_hi at hi_prio), their fork / join events and the
@@ -299,7 +312,11 @@ extern "C" int bnr_create(const bnr_params* p, const double* X, const double* y,
   h->p = *p;
   const double t0 = wall_ms();
   const int rc = create_impl(h, p, X, y);
-  if (g_timing) fprintf(stderr, "[bnr] bnr_create %.2f ms (%zu device buffers)\n", wall_ms() - t0, h->allocs.size());
+  if (g_timing) {
+    size_t asked = 0;
+    for (const auto& a : h->allocs) asked += a.asked;
+    fprintf(stderr, "[bnr] bnr_create %.2f ms (%zu device buffers, %zu bytes)\n", wall_ms() - t0, h->allocs.size(), asked);
+  }
   if (rc != BNR_OK) {
     const std::string msg = g_err;      // bnr_destroy must not clobber the reason
     bnr_destroy(h);
@@ -343,7 +360,6 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
   }
   d.nparts = (d.q + PART_BLOCK - 1) / PART_BLOCK;
   d.chain_offset = p->chain_offset;
-  d.chain_offset_local = 0;
   d.gigK = h->p.gig_inject_len;
   d.seed = p->seed;
   d.eta = p->eta; d.zeta = p->zeta; d.iota = p->iota; d.a_delta = p->a_delta; d.b_delta = p->b_delta; d.nu = p->nu;
@@ -390,30 +406,15 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
   CK(cudaStreamSynchronize(h->stream));
   e.edge_lk = dlk;
 
-  DA(e.tau2, C); DA(e.u, C * d.V * d.R); DA(e.u_alt, C * d.V * d.R); DA(e.xi, C * d.V);
+  // few chains x tiles: the FP64 SYRK splits its contraction (see launch_syrk_G).  The split count is fixed per handle
+  // from its total chain count, so the chain grouping never changes the summation order.
+  e.syrk_ws_cap = d.gmode == BNR_GAMMA_NFORM && !gram_i8_selected(d) ? syrk_splits(d, d.C) - 1 : 0;
+  int rc = BNR_OK;
+  chain_arrays(e, [&](auto*& a, size_t per_chain, size_t tail = 0) {   // zero-filled
+    if (per_chain > 0 && rc == BNR_OK) rc = dalloc(h, &a, C * per_chain + tail);
+  });
+  if (rc) return rc;
   h->u_first = e.u;
-  DA(e.gamma, C * d.qp); DA(e.S, C * d.qp); DA(e.theta, C); DA(e.Delta, C); DA(e.M, C * d.R * d.R);
-  DA(e.mu, C); DA(e.lambda, C * d.R); DA(e.pi, C * 3 * d.R);
-  DA(e.W, C * d.qp); DA(e.v, C * d.qp); DA(e.t, C * d.qp);
-  DA(e.xg, C * d.np); DA(e.xv, C * d.np); DA(e.rhs, C * d.np);
-  DA(e.G, C * d.gdim * d.gdim + 2048);
-  DA(e.Linv, C * (size_t)(d.gdim / TILE_N) * TILE_N * TILE_N);
-  // the blocks above the diagonal of every inverted panel are exact zeros that k_potf2_inv never writes
-  CK(cudaMemsetAsync(e.Linv, 0, sizeof(double) * C * (size_t)(d.gdim / TILE_N) * TILE_N * TILE_N, h->stream));
-  e.syrk_ws = nullptr; e.syrk_ws_cap = 0;
-  e.gram_planes = nullptr; e.gram_rscale = nullptr;
-  if (gram_i8_selected(d)) {
-    DA(e.gram_planes, C * gram_i8_plane_bytes(d));
-    DA(e.gram_rscale, C * d.np);
-  } else if (d.gmode == BNR_GAMMA_NFORM) {
-    // few chains x tiles: the SYRK splits its contraction (see launch_syrk_G).  The split count is fixed per handle
-    // from its total chain count, so the chain grouping never changes the summation order.
-    const int smax = syrk_splits(d, d.C);
-    if (smax > 1) {
-      e.syrk_ws_cap = smax - 1;
-      DA(e.syrk_ws, C * (size_t)e.syrk_ws_cap * d.gdim * d.gdim);
-    }
-  }
   e.XtX = nullptr;
   if (d.gmode == BNR_GAMMA_QFORM) {
     // X'X once: row-major copy of X as the SYRK operand (k-major over the n samples), unit scales, no identity
@@ -432,10 +433,6 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
     release_alloc(h, dOnes);
     e.XtX = dXtX;
   }
-  DA(e.partials, C * d.nparts * (2 * MAX_R + 1));
-  DA(e.tau2_part, C * 2 * TAU2_MAX_BLOCKS);
-  DA(e.tau2_ticket, C);
-  DA(e.status, C);
   DA(e.iter, 1); DA(e.trace_row, 1);
   e.mom = {nullptr, nullptr, nullptr, 0, d.V + d.q};
   DA(e.mom.halves, C * 2 * (d.V + d.q) * 2);
@@ -447,7 +444,7 @@ static int create_impl(bnr_handle* h, const bnr_params* p, const double* X, cons
   DA(h->ws, x_times_workspace_doubles(d));
   DA(h->d_rhat, (size_t)(d.V + d.q));
   const long long trace_rows = p->trace_rows > 0 ? p->trace_rows : 0;
-  e.tr_full = {nullptr, trace_rows, 4 + d.V * d.R + d.V + 2 * d.q + d.R * d.R + d.R + 3 * d.R, 0};
+  e.tr_full = {nullptr, trace_rows, state_offset(d, NUM_STATE_VARS), 0};
   e.tr_gx = {nullptr, trace_rows, d.V + d.q, 0};
   if (trace_rows > 0) {
     e.tr_full.chains = p->trace_full_chains < 0 ? 0 : (p->trace_full_chains < d.C ? p->trace_full_chains : d.C);
@@ -545,7 +542,7 @@ extern "C" int bnr_destroy(bnr_handle* h) {
   }
   destroy_fork_join(h->fj);
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-  for (auto& a : h->allocs) cache_give(h->p.device, a.first, a.second);
+  for (auto& a : h->allocs) cache_give(h->p.device, a.p, a.bytes);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->stream) cudaStreamDestroy(h->stream);
@@ -681,23 +678,12 @@ static void enqueue_sweep(Engine& e, double* ws, const ForkJoin& fj, cudaStream_
 // view is the same struct with offset pointers, a smaller C and a shifted global chain id
 static Engine group_view(const bnr_handle* h, int c0, int Cg, long long* counters, long long* mom_window) {
   Engine v = h->e;
-  const Dims& d = h->e.d;
-  const size_t c = (size_t)c0;
   v.d.C = Cg;
-  v.d.chain_offset = d.chain_offset + c0;
-  v.d.chain_offset_local = c0;
-  v.tau2 += c; v.theta += c; v.Delta += c; v.mu += c; v.status += c;
-  v.u += c * d.V * d.R; v.u_alt += c * d.V * d.R; v.xi += c * d.V;
-  v.gamma += c * d.qp; v.S += c * d.qp; v.W += c * d.qp; v.v += c * d.qp; v.t += c * d.qp;
-  v.M += c * d.R * d.R; v.lambda += c * d.R; v.pi += c * 3 * d.R;
-  v.xg += c * d.np; v.xv += c * d.np; v.rhs += c * d.np;
-  v.G += c * d.gdim * d.gdim; if (v.syrk_ws) v.syrk_ws += c * (size_t)v.syrk_ws_cap * d.gdim * d.gdim; v.Linv += c * (size_t)(d.gdim / TILE_N) * TILE_N * TILE_N;
-  if (v.gram_planes) { v.gram_planes += c * gram_i8_plane_bytes(d); v.gram_rscale += c * d.np; }
-  v.partials += c * d.nparts * (2 * MAX_R + 1);
+  v.d.chain_offset = h->e.d.chain_offset + c0;
+  chain_arrays(v, [&](auto*& a, size_t per_chain, size_t = 0) { if (a) a += (size_t)c0 * per_chain; });
   v.mom = v.mom.view(c0, mom_window); v.ess = v.ess.view(c0);
   v.tr_full = v.tr_full.view(c0, Cg); v.tr_gx = v.tr_gx.view(c0, Cg);
   v.pred = v.pred.view(c0, Cg); v.ll = v.ll.view(c0, Cg);
-  if (v.pred_ws) v.pred_ws += c * (size_t)v.pred_splits * v.pred_mp;
   v.iter = counters; v.trace_row = counters + 1;
   v.inj = nullptr; v.inj_stride = 0;
   memset(&v.aux, 0, sizeof(v.aux));
@@ -988,42 +974,20 @@ extern "C" int bnr_rhat(bnr_handle* h, double* rhat_xi, double* rhat_gamma) {
 extern "C" int bnr_var_size(bnr_handle* h, int32_t var, int64_t* n) {
   if (!h || !n || var < 0 || var >= BNR_NUM_VARS) return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
-  *n = var_size(h->e.d, var);
+  *n = state_var(h->e.d, var).count;
   return BNR_OK;
-}
-
-static double* var_ptr(Engine& e, int c, int var) {
-  const Dims& d = e.d;
-  switch (var) {
-    case BNR_VAR_TAU2: return e.tau2 + c;
-    case BNR_VAR_U: return e.u + (size_t)c * d.V * d.R;
-    case BNR_VAR_XI: return e.xi + (size_t)c * d.V;
-    case BNR_VAR_GAMMA: return e.gamma + (size_t)c * d.qp;
-    case BNR_VAR_S: return e.S + (size_t)c * d.qp;
-    case BNR_VAR_THETA: return e.theta + c;
-    case BNR_VAR_DELTA: return e.Delta + c;
-    case BNR_VAR_M: return e.M + (size_t)c * d.R * d.R;
-    case BNR_VAR_MU: return e.mu + c;
-    case BNR_VAR_LAMBDA: return e.lambda + (size_t)c * d.R;
-    case BNR_VAR_PI: return e.pi + (size_t)c * 3 * d.R;
-  }
-  return nullptr;
 }
 
 extern "C" int bnr_get_state(bnr_handle* h, int32_t chain, int32_t var, double* out) {
   if (!h || !out || chain < 0 || chain >= h->e.d.C || var < 0 || var >= BNR_NUM_VARS)
     return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
-  const int n = var_size(h->e.d, var), R = h->e.d.R;
-  std::vector<double> tmp(n);
-  CK(cudaMemcpyAsync(tmp.data(), var_ptr(h->e, chain, var), sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
+  const StateVar s = state_var(h->e.d, var);
+  std::vector<double> tmp(s.count);
+  CK(cudaMemcpyAsync(tmp.data(), (h->e.*s.at) + (size_t)chain * s.stride, sizeof(double) * s.count,
+                     cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
-  if (var == BNR_VAR_PI) {
-    for (int r = 0; r < R; ++r)
-      for (int c = 0; c < 3; ++c) out[r + R * c] = tmp[3 * r + c];
-  } else {
-    memcpy(out, tmp.data(), sizeof(double) * n);
-  }
+  for (int i = 0; i < s.count; ++i) out[i] = tmp[s.transposed ? pi_stored(i, h->e.d.R) : i];
   return BNR_OK;
 }
 
@@ -1031,12 +995,11 @@ extern "C" int bnr_set_state(bnr_handle* h, int32_t chain, int32_t var, const do
   if (!h || !in || chain < 0 || chain >= h->e.d.C || var < 0 || var >= BNR_NUM_VARS)
     return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
-  const int n = var_size(h->e.d, var), R = h->e.d.R;
-  std::vector<double> tmp(in, in + n);
-  if (var == BNR_VAR_PI)
-    for (int r = 0; r < R; ++r)
-      for (int c = 0; c < 3; ++c) tmp[3 * r + c] = in[r + R * c];
-  CK(cudaMemcpyAsync(var_ptr(h->e, chain, var), tmp.data(), sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
+  const StateVar s = state_var(h->e.d, var);
+  std::vector<double> tmp(s.count);
+  for (int i = 0; i < s.count; ++i) tmp[s.transposed ? pi_stored(i, h->e.d.R) : i] = in[i];
+  CK(cudaMemcpyAsync((h->e.*s.at) + (size_t)chain * s.stride, tmp.data(), sizeof(double) * s.count,
+                     cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   if (var == BNR_VAR_GAMMA) h->xg_valid = false;
   return BNR_OK;
@@ -1050,13 +1013,13 @@ __global__ void k_gather_trace(const double* __restrict__ rows, size_t rowlen, i
   const long long it = idx % count;
   const int el = (int)(idx / count);
   int src = el;
-  if (pi_R > 0) { const int r = el % pi_R, c = el / pi_R; src = 3 * r + c; }   // out is (R,3) column-major
+  if (pi_R > 0) src = pi_stored(el, pi_R);   // out is (R,3) column-major
   out[idx] = rows[(size_t)(first + it) * rowlen + off + src];
 }
 
 // the trace table that holds variable `var` of `chain` and the variable's offset in its rows (nullptr: not traced)
 static const RowTable* traced(const Engine& e, int chain, int var, int* off) {
-  if (e.tr_full.holds(chain, 0)) { *off = row_offset(e.d, var); return &e.tr_full; }
+  if (e.tr_full.holds(chain, 0)) { *off = state_offset(e.d, var); return &e.tr_full; }
   if (e.tr_gx.holds(chain, 0) && (var == BNR_VAR_XI || var == BNR_VAR_GAMMA)) {
     *off = var == BNR_VAR_XI ? 0 : e.d.V;
     return &e.tr_gx;
@@ -1076,7 +1039,8 @@ extern "C" int bnr_get_trace(bnr_handle* h, int32_t chain, int32_t var, int64_t 
   if (!t) return fail(BNR_ESTATE, "this variable of this chain is not traced (see trace_full_chains / trace_gamma_xi_all)");
   const double* rows = t->row(chain, 0);
   const size_t rowlen = t->width;
-  const int nelem = var_size(d, var);
+  const StateVar s = state_var(d, var);
+  const int nelem = s.count;
   const long long count = last - first;
   if (count == 0) return BNR_OK;
   // chunk over elements so the staging buffer suffices
@@ -1085,12 +1049,9 @@ extern "C" int bnr_get_trace(bnr_handle* h, int32_t chain, int32_t var, int64_t 
   for (int e0 = 0; e0 < nelem; e0 += (int)el_per_chunk) {
     const int ne = (int)((nelem - e0) < el_per_chunk ? (nelem - e0) : el_per_chunk);
     const long long tot = count * ne;
-    if (var == BNR_VAR_PI) {
-      if (ne != nelem) return fail(BNR_EINVAL, "row range too long for pi");
-      k_gather_trace<<<(unsigned)((tot + 255) / 256), 256, 0, h->stream>>>(rows, rowlen, off, ne, first, count, d.R, h->d_tmp);
-    } else {
-      k_gather_trace<<<(unsigned)((tot + 255) / 256), 256, 0, h->stream>>>(rows, rowlen, off + e0, ne, first, count, 0, h->d_tmp);
-    }
+    if (s.transposed && ne != nelem) return fail(BNR_EINVAL, "row range too long for pi");
+    k_gather_trace<<<(unsigned)((tot + 255) / 256), 256, 0, h->stream>>>(rows, rowlen, off + e0, ne, first, count,
+                                                                         s.transposed ? d.R : 0, h->d_tmp);
     CK(cudaMemcpyAsync(out + (size_t)e0 * count, h->d_tmp, sizeof(double) * tot, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
   }
@@ -1130,12 +1091,43 @@ extern "C" int bnr_set_injection(bnr_handle* h, const double* inj, int64_t per_c
   return BNR_OK;
 }
 
+// The array behind aux output `id`: chain c exports `count` doubles (the size include/bnr.h documents) at
+// *at + c * stride.  own: an Aux member, allocated by bnr_enable_aux; else one of the sweep's own buffers
+struct AuxArray { double** at; size_t count, stride; bool own; };
+static AuxArray aux_array(Engine& e, int id) {
+  const Dims& d = e.d;
+  Aux& x = e.aux;
+  const size_t R = d.R, V = d.V, q = d.q, qp = d.qp, N = (size_t)d.gdim * d.gdim;
+  const size_t m = d.gmode == BNR_GAMMA_QFORM ? q : d.n;   // G, G_CHOL: the leading m x m block of N
+  switch (id) {
+    case BNR_AUX_TAU2_PARAMS: return {&x.tau2_params, 2, 2, true};
+    case BNR_AUX_SIGMA_INV: return {&x.sigma_inv, V * R * R, V * R * R, true};
+    case BNR_AUX_SIGMA_CHOL: return {&x.sigma_chol, V * R * R, V * R * R, true};
+    case BNR_AUX_MU_T: return {&x.mu_t, V * R, V * R, true};
+    case BNR_AUX_LOG_ODDS: return {&x.log_odds, V, V, true};
+    case BNR_AUX_W: return {&e.W, q, qp, false};
+    case BNR_AUX_G: return {&x.G_copy, m * m, N, true};
+    case BNR_AUX_G_CHOL: return {&e.G, m * m, N, false};
+    case BNR_AUX_RHS: case BNR_AUX_A4:    // q-form: beta = gamma - W
+      if (d.gmode == BNR_GAMMA_QFORM) return {&e.t, q, qp, false};
+      return {&e.rhs, (size_t)d.n, (size_t)d.np, false};
+    case BNR_AUX_CHI: return {&x.chi, q, qp, true};
+    case BNR_AUX_THETA_PARAMS: return {&x.theta_params, 2, 2, true};
+    case BNR_AUX_DELTA_PARAMS: return {&x.delta_params, 2, 2, true};
+    case BNR_AUX_M_PARAMS: return {&x.m_params, 1 + 2 * R * R, 1 + 2 * R * R, true};
+    case BNR_AUX_MU_PARAMS: return {&x.mu_params, 2, 2, true};
+    case BNR_AUX_LAMBDA_LOGW: return {&x.lambda_logw, 3 * R, 3 * R, true};
+    case BNR_AUX_LAMBDA_WEIGHTS: return {&x.lambda_w, 3 * R, 3 * R, true};
+    case BNR_AUX_PI_ALPHA: return {&x.pi_alpha, 3 * R, 3 * R, true};
+    case BNR_AUX_GIG_USED: return {&x.gig_used, q, qp, true};
+  }
+  return {nullptr, 0, 0, false};
+}
+
 extern "C" int bnr_enable_aux(bnr_handle* h, int32_t on) {
   if (!h) return fail(BNR_EINVAL, "null handle");
   CK(cudaSetDevice(h->p.device));
   Engine& e = h->e;
-  const Dims& d = e.d;
-  const size_t C = d.C;
   CK(cudaStreamSynchronize(h->stream));
   drop_graph(h);
   if (!on) {
@@ -1147,11 +1139,10 @@ extern "C" int bnr_enable_aux(bnr_handle* h, int32_t on) {
   if (h->aux_saved.tau2_params) {
     e.aux = h->aux_saved;
   } else {
-    DA(e.aux.tau2_params, C * 2); DA(e.aux.sigma_inv, C * d.V * d.R * d.R); DA(e.aux.sigma_chol, C * d.V * d.R * d.R);
-    DA(e.aux.mu_t, C * d.V * d.R); DA(e.aux.log_odds, C * d.V); DA(e.aux.chi, C * d.qp);
-    DA(e.aux.theta_params, C * 2); DA(e.aux.delta_params, C * 2); DA(e.aux.m_params, C * (1 + 2 * d.R * d.R));
-    DA(e.aux.mu_params, C * 2); DA(e.aux.lambda_logw, C * 3 * d.R); DA(e.aux.lambda_w, C * 3 * d.R);
-    DA(e.aux.pi_alpha, C * 3 * d.R); DA(e.aux.gig_used, C * d.qp); DA(e.aux.G_copy, C * d.gdim * d.gdim);
+    for (int id = 0; id < BNR_NUM_AUX; ++id) {
+      const AuxArray a = aux_array(e, id);
+      if (a.own) DA(*a.at, (size_t)e.d.C * a.stride);
+    }
     CK(cudaStreamSynchronize(h->stream));
   }
   h->aux_on = true;
@@ -1162,52 +1153,25 @@ extern "C" int bnr_get_aux(bnr_handle* h, int32_t chain, int32_t aux_id, double*
   if (!h || !out || chain < 0 || chain >= h->e.d.C) return fail(BNR_EINVAL, "bad arguments");
   CK(cudaSetDevice(h->p.device));
   if (!h->aux_on) return fail(BNR_ESTATE, "call bnr_enable_aux first");
-  Engine& e = h->e;
-  const Dims& d = e.d;
-  const int R = d.R, V = d.V, RR = R * R;
-  const double* src = nullptr;
-  size_t n = 0;
-  std::vector<double> tmp;
-  switch (aux_id) {
-    case BNR_AUX_TAU2_PARAMS: src = e.aux.tau2_params + 2 * chain; n = 2; break;
-    case BNR_AUX_SIGMA_INV: src = e.aux.sigma_inv + (size_t)chain * V * RR; n = (size_t)V * RR; break;
-    case BNR_AUX_SIGMA_CHOL: src = e.aux.sigma_chol + (size_t)chain * V * RR; n = (size_t)V * RR; break;
-    case BNR_AUX_MU_T: src = e.aux.mu_t + (size_t)chain * V * R; n = (size_t)V * R; break;
-    case BNR_AUX_LOG_ODDS: src = e.aux.log_odds + (size_t)chain * V; n = V; break;
-    case BNR_AUX_W: src = e.W + (size_t)chain * d.qp; n = d.q; break;
-    case BNR_AUX_RHS: case BNR_AUX_A4:
-      if (d.gmode == BNR_GAMMA_QFORM) { src = e.t + (size_t)chain * d.qp; n = d.q; }   // beta = gamma - W
-      else { src = e.rhs + (size_t)chain * d.np; n = d.n; }
-      break;
-    case BNR_AUX_CHI: src = e.aux.chi + (size_t)chain * d.qp; n = d.q; break;
-    case BNR_AUX_THETA_PARAMS: src = e.aux.theta_params + 2 * chain; n = 2; break;
-    case BNR_AUX_DELTA_PARAMS: src = e.aux.delta_params + 2 * chain; n = 2; break;
-    case BNR_AUX_M_PARAMS: src = e.aux.m_params + (size_t)chain * (1 + 2 * RR); n = 1 + 2 * RR; break;
-    case BNR_AUX_MU_PARAMS: src = e.aux.mu_params + 2 * chain; n = 2; break;
-    case BNR_AUX_LAMBDA_LOGW: src = e.aux.lambda_logw + (size_t)chain * 3 * R; n = 3 * R; break;
-    case BNR_AUX_LAMBDA_WEIGHTS: src = e.aux.lambda_w + (size_t)chain * 3 * R; n = 3 * R; break;
-    case BNR_AUX_PI_ALPHA: src = e.aux.pi_alpha + (size_t)chain * 3 * R; n = 3 * R; break;
-    case BNR_AUX_GIG_USED: src = e.aux.gig_used + (size_t)chain * d.qp; n = d.q; break;
-    case BNR_AUX_G: case BNR_AUX_G_CHOL: {
-      // m x m sub-block of the padded gdim x gdim matrix (m = n in the n-form, q in the q-form)
-      const int m = d.gmode == BNR_GAMMA_QFORM ? d.q : d.n, N = d.gdim;
-      const double* base = (aux_id == BNR_AUX_G ? e.aux.G_copy : e.G) + (size_t)chain * N * N;
-      if (capacity < (int64_t)m * m) return fail(BNR_EINVAL, "capacity too small");
-      tmp.resize((size_t)N * N);
-      CK(cudaMemcpyAsync(tmp.data(), base, sizeof(double) * tmp.size(), cudaMemcpyDeviceToHost, h->stream));
-      CK(cudaStreamSynchronize(h->stream));
-      for (int j = 0; j < m; ++j)
-        for (int i = 0; i < m; ++i) {
-          double v = tmp[(size_t)j * N + i];
-          if (aux_id == BNR_AUX_G_CHOL && i < j) v = 0.0;
-          out[(size_t)j * m + i] = v;
-        }
-      return BNR_OK;
-    }
-    default: return fail(BNR_EINVAL, "unknown aux id");
+  const AuxArray a = aux_array(h->e, aux_id);
+  if (!a.at) return fail(BNR_EINVAL, "unknown aux id");
+  if ((int64_t)a.count > capacity) return fail(BNR_EINVAL, "capacity too small");
+  const double* src = *a.at + (size_t)chain * a.stride;
+  if (aux_id == BNR_AUX_G || aux_id == BNR_AUX_G_CHOL) {
+    // m x m sub-block of the padded gdim x gdim matrix (m = n in the n-form, q in the q-form)
+    const int N = h->e.d.gdim, m = h->e.d.gmode == BNR_GAMMA_QFORM ? h->e.d.q : h->e.d.n;
+    std::vector<double> tmp((size_t)N * N);
+    CK(cudaMemcpyAsync(tmp.data(), src, sizeof(double) * tmp.size(), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    for (int j = 0; j < m; ++j)
+      for (int i = 0; i < m; ++i) {
+        double v = tmp[(size_t)j * N + i];
+        if (aux_id == BNR_AUX_G_CHOL && i < j) v = 0.0;
+        out[(size_t)j * m + i] = v;
+      }
+    return BNR_OK;
   }
-  if ((int64_t)n > capacity) return fail(BNR_EINVAL, "capacity too small");
-  CK(cudaMemcpyAsync(out, src, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(out, src, sizeof(double) * a.count, cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   return BNR_OK;
 }

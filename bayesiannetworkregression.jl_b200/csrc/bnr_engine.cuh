@@ -22,7 +22,6 @@ struct Dims {
                       // > n resp. q: the first padding row carries the right-hand side of the forward solve
   int nparts;         // edge-kernel blocks per chain = ceil(q / PART_BLOCK)
   int chain_offset;
-  int chain_offset_local;   // index of this view's first chain inside the handle (0 for the handle itself)
   int gigK;           // injected uniforms per edge
   uint64_t seed;
   double eta, zeta, iota, a_delta, b_delta, nu;
@@ -197,15 +196,15 @@ struct Engine {
   double* gram_rscale;       // [C][np] power-of-two row scales of the digit planes
   double* Linv;     // [C][gdim/128][128*128]  inverses of the 128 x 128 diagonal blocks of the factor (column-major)
   double* partials; // [C][nparts][2*MAX_R+1]  block partial sums: A_r, B_r (lambda), sum S
-  double* tau2_part;      // [handle chains][2 * TAU2_MAX_BLOCKS] partial sums of the tau2 reduction (NOT offset per view)
-  unsigned* tau2_ticket;  // [handle chains] arrival counters of its blocks
+  double* tau2_part;      // [C][2 * TAU2_MAX_BLOCKS] partial sums of the tau2 reduction
+  unsigned* tau2_ticket;  // [C] arrival counters of its blocks
   int* status;      // [C]
   long long* iter;  // device scalar: completed sweeps
   long long* trace_row;   // device scalar: next trace row
   SplitMoments mom;
   EssStream ess;
   // traces of the leading tr_full.chains / tr_gx.chains chains; both keep rows = the handle's trace capacity when off
-  RowTable tr_full;       // full state rows (state_elem order)
+  RowTable tr_full;       // full state rows (state_var order)
   RowTable tr_gx;         // xi then gamma, width V+q
   // predictions for new networks (bnr_set_predictors; pred.base == nullptr: off).  Every recorded row r of chain c gets
   // pred.row(c, r)[j] = mu_c + X_new[j,:] gamma_c (+ sqrt(tau2_c) z_j in the predictive mode), width m
@@ -222,6 +221,42 @@ struct Engine {
   long long inj_stride;
   Aux aux;
 };
+
+// The state variables in BNR_VAR_* order, which is also their order in a full trace row: tau2, u[V*R], xi[V],
+// gamma[q], S[q], theta, Delta, M[R*R], mu, lambda[R], pi[R*3].  Chain c holds `count` doubles of a variable at
+// (e.*at) + c * stride.
+constexpr int NUM_STATE_VARS = 11;
+using EngineArray = double* Engine::*;
+struct StateVar {
+  EngineArray at;        // the member that holds the variable
+  int count;             // elements per chain
+  int stride;            // doubles between chains (qp for gamma and S)
+  bool transposed;       // stored [r][3], the transpose of the reference's column-major (R, 3) order (pi): pi_stored
+};
+__host__ __device__ inline StateVar state_var(const Dims& d, int var) {
+  const int R = d.R, V = d.V;
+  switch (var) {
+    case 0: return {&Engine::tau2, 1, 1, false};
+    case 1: return {&Engine::u, V * R, V * R, false};
+    case 2: return {&Engine::xi, V, V, false};
+    case 3: return {&Engine::gamma, d.q, d.qp, false};
+    case 4: return {&Engine::S, d.q, d.qp, false};
+    case 5: return {&Engine::theta, 1, 1, false};
+    case 6: return {&Engine::Delta, 1, 1, false};
+    case 7: return {&Engine::M, R * R, R * R, false};
+    case 8: return {&Engine::mu, 1, 1, false};
+    case 9: return {&Engine::lambda, R, R, false};
+    default: return {&Engine::pi, 3 * R, 3 * R, true};
+  }
+}
+// offset of a variable in a full trace row; state_offset(d, NUM_STATE_VARS) is the row's width
+__host__ __device__ inline int state_offset(const Dims& d, int var) {
+  int o = 0;
+  for (int v = 0; v < var; ++v) o += state_var(d, v).count;
+  return o;
+}
+// where element el of the reference's (R, 3) order of pi is stored in the chain's [r][3]
+__host__ __device__ inline int pi_stored(int el, int R) { return 3 * (el % R) + el / R; }
 
 __device__ __forceinline__ RngKey chain_key(const Dims& d, int c) {
   return make_key(d.seed, (uint32_t)(d.chain_offset + c));

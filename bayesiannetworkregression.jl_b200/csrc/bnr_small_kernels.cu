@@ -147,17 +147,17 @@ __global__ void __launch_bounds__(256) k_tau2(Engine e) {
   }
   s1 = block_sum(s1, red);
   s2 = block_sum(s2, red);
-  double* part = e.tau2_part + (size_t)(d.chain_offset_local + c) * 2 * TAU2_MAX_BLOCKS;
+  double* part = e.tau2_part + (size_t)c * 2 * TAU2_MAX_BLOCKS;
   if (tid == 0) {
     part[2 * b] = s1; part[2 * b + 1] = s2;
     __threadfence();
-    ticket = atomicAdd(&e.tau2_ticket[d.chain_offset_local + c], 1u);
+    ticket = atomicAdd(&e.tau2_ticket[c], 1u);
   }
   __syncthreads();
   if (ticket != (unsigned)(nb - 1)) return;
   if (tid == 0) {
     __threadfence();
-    e.tau2_ticket[d.chain_offset_local + c] = 0u;      // ready for the next sweep
+    e.tau2_ticket[c] = 0u;      // ready for the next sweep
     const volatile double* vp = part;
     s1 = 0.0; s2 = 0.0;
     for (int k = 0; k < nb; ++k) { s1 += vp[2 * k]; s2 += vp[2 * k + 1]; }
@@ -733,34 +733,8 @@ __global__ void __launch_bounds__(256) k_init(Engine e) {
 // ------------------------------------------------------------------------------------------------------------
 // trace rows + streaming split-half moments (replaces the T-row state Table and return_psrf_VOI's copies,
 // src/gibbs.jl:835-841, 771-789).  grid = (ceil((V+q)/256), C), block = 256.
-// Row layout of a full trace row: tau2, u[V*R], xi[V], gamma[q], S[q], theta, Delta, M[R*R], mu, lambda[R], pi[R*3]
+// Full trace rows hold the state variables in state_var order (bnr_engine.cuh)
 // ------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ double state_elem(const Engine& e, int c, int idx) {
-  const Dims& d = e.d;
-  const int R = d.R, V = d.V, q = d.q;
-  if (idx < 1) return e.tau2[c];
-  idx -= 1;
-  if (idx < V * R) return e.u[(size_t)c * V * R + idx];
-  idx -= V * R;
-  if (idx < V) return e.xi[c * V + idx];
-  idx -= V;
-  if (idx < q) return e.gamma[(size_t)c * d.qp + idx];
-  idx -= q;
-  if (idx < q) return e.S[(size_t)c * d.qp + idx];
-  idx -= q;
-  if (idx < 1) return e.theta[c];
-  idx -= 1;
-  if (idx < 1) return e.Delta[c];
-  idx -= 1;
-  if (idx < R * R) return e.M[(size_t)c * R * R + idx];
-  idx -= R * R;
-  if (idx < 1) return e.mu[c];
-  idx -= 1;
-  if (idx < R) return e.lambda[c * R + idx];
-  idx -= R;
-  return e.pi[(size_t)c * 3 * R + idx];   // stored [r][3]
-}
-
 __global__ void __launch_bounds__(256) k_record(Engine e, int sweep_done /* 1: state belongs to sweep iter+1 */) {
   const Dims& d = e.d;
   const int c = blockIdx.y;
@@ -775,8 +749,15 @@ __global__ void __launch_bounds__(256) k_record(Engine e, int sweep_done /* 1: s
   }
   if (e.tr_full.holds(c, row)) {
     double* dst = e.tr_full.row(c, row);
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < e.tr_full.width; i += gridDim.x * blockDim.x)
-      dst[i] = state_elem(e, c, i);
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < e.tr_full.width; i += gridDim.x * blockDim.x) {
+      int j = i;               // walk the state table to the variable that holds element i of the row
+#pragma unroll
+      for (int v = 0; v < NUM_STATE_VARS; ++v) {
+        const StateVar s = state_var(d, v);
+        if (j >= 0 && j < s.count) dst[i] = (e.*s.at)[(size_t)c * s.stride + j];
+        j -= s.count;
+      }
+    }
   }
 }
 

@@ -15,6 +15,12 @@ def _dp(a):
 LOO_FIELDS = ("elpd_loo", "p_loo", "pareto_k", "elpd_waic", "p_waic")
 
 
+def var_shape(var, R, V, q):
+    """Shape of one draw of a state variable in the reference's layout (column-major, like its state.<var>)."""
+    return {"tau2": (1, 1), "u": (R, V), "xi": (V, 1), "gamma": (q, 1), "S": (q, 1), "theta": (1, 1),
+            "Delta": (1, 1), "M": (R, R), "mu": (1, 1), "lam": (R, 1), "pi": (R, 3)}[var]
+
+
 def loo_summary(device, dev_ptr, N, n):
     """bnr_loo_summary on a device table of N draws x n observations: dict of the five pointwise [n] arrays."""
     out = [np.empty(int(n)) for _ in LOO_FIELDS]
@@ -294,9 +300,7 @@ class Engine:
 
     # -- state / traces in reference layout ------------------------------------------------------------
     def var_shape(self, var):
-        R, V, q = self.R, self.V, self.q
-        return {"tau2": (1, 1), "u": (R, V), "xi": (V, 1), "gamma": (q, 1), "S": (q, 1), "theta": (1, 1),
-                "Delta": (1, 1), "M": (R, R), "mu": (1, 1), "lam": (R, 1), "pi": (R, 3)}[var]
+        return var_shape(var, self.R, self.V, self.q)
 
     def get_state(self, chain, var):
         shp = self.var_shape(var)

@@ -15,7 +15,7 @@ import numpy as np
 
 from .capi import lib, check, check_fit, FitParams, FitInfo, ALLGATHER_FN, STATE, VAR, GAMMA_MODE, PRED_MEAN, \
     PRED_PREDICTIVE
-from .engine import LOO_FIELDS
+from .engine import LOO_FIELDS, var_shape
 
 _DP = C.POINTER(C.c_double)
 
@@ -280,11 +280,9 @@ def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsa
                            draws=int(info.total_chains) * int(info.sampled), y=y.copy())
         st = Table()
         rows = int(info.rows)
-        shapes = {"tau2": (1, 1), "u": (R, V), "xi": (V, 1), "gamma": (q, 1), "S": (q, 1), "theta": (1, 1),
-                  "Delta": (1, 1), "M": (R, R), "mu": (1, 1), "lam": (R, 1), "pi": (R, 3)}
         names = list(_UNI) if return_state == "full" else (["xi", "gamma"] if return_state == "gamma_xi" else [])
         for k in names:
-            shp = shapes[k]
+            shp = var_shape(k, R, V, q)
             out = np.empty(rows * shp[0] * shp[1])
             check_fit(L.bnr_fit_state(res, VAR[k], out.ctypes.data_as(_DP)))
             st[k] = out.reshape((rows,) + shp, order="F")

@@ -12,9 +12,9 @@ __graft_entry__.load_package) and registered as module `bnr_b200`.
 from .capi import lib, BnrError, check, Params, VAR, COND, AUX, STATUS_BITS  # noqa: F401
 from .engine import Engine  # noqa: F401
 from .io import read_matrix_networks, read_adjacency_csvs, read_responses  # noqa: F401
-from .fit import Fit, Summary, Predict, Loo, Compare, Results, BNRSummary, BNRPrediction, BNRLoo, BNRCompare, Table, \
-    setup_X, lower_triangle, create_lower_tri  # noqa: F401
+from .fit import Fit, Summary, Predict, Loo, Compare, KFold, Results, BNRSummary, BNRPrediction, BNRLoo, BNRCompare, \
+    BNRKFold, Table, setup_X, lower_triangle, create_lower_tri, kfold_split  # noqa: F401
 
-__all__ = ["Fit", "Summary", "Predict", "Loo", "Compare", "Results", "BNRSummary", "BNRPrediction", "BNRLoo",
-           "BNRCompare", "Table", "Engine", "BnrError", "setup_X",
+__all__ = ["Fit", "Summary", "Predict", "Loo", "Compare", "KFold", "Results", "BNRSummary", "BNRPrediction", "BNRLoo",
+           "BNRCompare", "BNRKFold", "kfold_split", "Table", "Engine", "BnrError", "setup_X",
            "lower_triangle", "create_lower_tri", "lib", "read_matrix_networks", "read_adjacency_csvs", "read_responses"]

@@ -1526,7 +1526,8 @@ static void drop_predictors(bnr_handle* h) {
   release_alloc(h, const_cast<double*>(e.Xp));
   release_alloc(h, e.pred.base);
   release_alloc(h, e.pred_ws);
-  e.Xp = nullptr; e.pred = {}; e.pred_ws = nullptr;
+  release_alloc(h, const_cast<double*>(e.pred_y));
+  e.Xp = nullptr; e.pred = {}; e.pred_ws = nullptr; e.pred_y = nullptr;
   e.pred_mp = e.pred_mode = e.pred_splits = 0;
 }
 
@@ -1554,11 +1555,12 @@ static int export_table_rows(bnr_handle* h, const RowTable& t, int64_t first_row
   return BNR_OK;
 }
 
-extern "C" int bnr_set_predictors(bnr_handle* h, int32_t m, const double* X_new, int64_t rows, int32_t mode) {
-  if (!h) return fail(BNR_EINVAL, "null handle");
-  if (m < 0) return fail(BNR_EINVAL, "m must be >= 0");
-  if (mode != BNR_PRED_MEAN && mode != BNR_PRED_PREDICTIVE) return fail(BNR_EINVAL, "unknown prediction mode");
+// the prediction table of bnr_set_predictors and bnr_set_heldout: X_new (m x q), `rows` rows per chain, and for held-out
+// rows (mode BNR_PRED_LOGDENS) their responses y_held [m]
+static int set_pred_table(bnr_handle* h, int32_t m, const double* X_new, const double* y_held, int64_t rows,
+                          int32_t mode) {
   if (m > 0 && !X_new) return fail(BNR_EINVAL, "null X_new");
+  if (m > 0 && mode == BNR_PRED_LOGDENS && !y_held) return fail(BNR_EINVAL, "null y_held");
   if (m > 0 && rows < 1) return fail(BNR_EINVAL, "the prediction table needs rows >= 1");
   CK(cudaSetDevice(h->p.device));
   CK(cudaStreamSynchronize(h->stream));
@@ -1569,24 +1571,40 @@ extern "C" int bnr_set_predictors(bnr_handle* h, int32_t m, const double* X_new,
   const Dims& d = e.d;
   const int mp = (m + TILE_N - 1) / TILE_N * TILE_N;
   const int ks = pred_splits(d, mp);
+  const size_t ny = mode == BNR_PRED_LOGDENS ? (size_t)m : 0;
   RowTable pred = {nullptr, rows, m, d.C};
   if (int r = alloc_table(h, pred, true, "prediction table")) return r;
-  double *xp = nullptr, *ws = nullptr;
+  double *xp = nullptr, *ws = nullptr, *yh = nullptr;
   int r = dalloc(h, &xp, (size_t)d.qp * mp);
   if (!r) r = dalloc(h, &ws, (size_t)ks * d.C * mp, false);
+  if (!r && ny) r = dalloc(h, &yh, ny, false);
   if (r) {
     cudaGetLastError();                // a refused cudaMalloc must not surface in a later call
-    release_alloc(h, pred.base); release_alloc(h, xp); release_alloc(h, ws);
+    release_alloc(h, pred.base); release_alloc(h, xp); release_alloc(h, ws); release_alloc(h, yh);
     return fail(r, "X_new and the split-K partials of the predictions (" +
-                       std::to_string(8.0 * ((double)d.qp * mp + (double)ks * d.C * mp)) + " bytes): " + g_err);
+                       std::to_string(8.0 * ((double)d.qp * mp + (double)ks * d.C * mp + (double)ny)) + " bytes): " + g_err);
   }
   // X_new: m x q column-major host -> columns padded to mp rows (zeros beyond m and beyond q, like X)
   CK(cudaMemcpy2DAsync(xp, (size_t)mp * sizeof(double), X_new, (size_t)m * sizeof(double), (size_t)m * sizeof(double),
                        (size_t)d.q, cudaMemcpyHostToDevice, h->stream));
+  if (ny) CK(cudaMemcpyAsync(yh, y_held, ny * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
-  e.Xp = xp; e.pred = pred; e.pred_ws = ws;
+  e.Xp = xp; e.pred = pred; e.pred_ws = ws; e.pred_y = yh;
   e.pred_mp = mp; e.pred_mode = mode; e.pred_splits = ks;
   return BNR_OK;
+}
+
+extern "C" int bnr_set_predictors(bnr_handle* h, int32_t m, const double* X_new, int64_t rows, int32_t mode) {
+  if (!h) return fail(BNR_EINVAL, "null handle");
+  if (m < 0) return fail(BNR_EINVAL, "m must be >= 0");
+  if (mode != BNR_PRED_MEAN && mode != BNR_PRED_PREDICTIVE) return fail(BNR_EINVAL, "unknown prediction mode");
+  return set_pred_table(h, m, X_new, nullptr, rows, mode);
+}
+
+extern "C" int bnr_set_heldout(bnr_handle* h, int32_t m, const double* X_held, const double* y_held, int64_t rows) {
+  if (!h) return fail(BNR_EINVAL, "null handle");
+  if (m < 0) return fail(BNR_EINVAL, "m must be >= 0");
+  return set_pred_table(h, m, X_held, y_held, rows, BNR_PRED_LOGDENS);
 }
 
 extern "C" int bnr_get_prediction_trace(bnr_handle* h, int32_t chain, int64_t first, int64_t last, double* out) {
@@ -1687,5 +1705,22 @@ extern "C" int bnr_loo_summary(int device, const double* dev_rows, int64_t N, in
   double* dst[5] = {elpd_loo, p_loo, pareto_k, elpd_waic, p_waic};
   for (int k = 0; k < 5; ++k)
     if (dst[k]) memcpy(dst[k], host.data() + (size_t)k * n, sizeof(double) * n);
+  return BNR_OK;
+}
+
+extern "C" int bnr_lpd_summary(int device, const double* dev_rows, int64_t N, int32_t m, double* lpd) {
+  if (!dev_rows || !lpd || N < 1 || m < 1) return fail(BNR_EINVAL, "bad arguments (need rows, N >= 1 draws, m >= 1)");
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+    return fail(BNR_ENODEV, "no CUDA device visible: libbnr has no CPU fallback");
+  if (device < 0 || device >= ndev) return fail(BNR_EINVAL, "device ordinal out of range");
+  CK(cudaSetDevice(device));
+  const size_t outb = sizeof(double) * (size_t)m;
+  Scratch sc(device, outb + lpd_ws_bytes(N, m));
+  if (!sc.p) return fail(BNR_ENOMEM, "device scratch allocation failed");
+  double* o = (double*)sc.p;
+  launch_lpd(dev_rows, N, m, o, o + m, 0);
+  CK(cudaMemcpy(lpd, o, outb, cudaMemcpyDeviceToHost));
+  CK(cudaGetLastError());
   return BNR_OK;
 }

@@ -251,6 +251,20 @@ long long loo_tail_max() {
   return M;
 }
 
+// Streamed logsumexp of a column as a partial (m, s), lse = m + log(s): lse_add takes one value, lse_merge another partial
+// (an empty partial has s = 0).  k_loo_pass and k_lpd_pass build their per-block partials with them, k_loo_tail and
+// k_lpd_finish add the block partials in block order.
+__device__ __forceinline__ void lse_add(double& m, double& s, double x) {
+  if (x > m) { s = s * exp(m - x) + 1.0; m = x; }
+  else s += exp(x - m);
+}
+__device__ __forceinline__ void lse_merge(double& m, double& s, double m2, double s2) {
+  if (s2 > 0.0) {
+    if (m2 > m) { s = s * exp(m - m2) + s2; m = m2; }
+    else s += s2 * exp(m2 - m);
+  }
+}
+
 __global__ void __launch_bounds__(256) k_loo_pass(const double* __restrict__ rows, long long N, int n, long long per,
                                                   long long M, const double* __restrict__ mean,
                                                   const double* __restrict__ av, const double* __restrict__ bv,
@@ -268,8 +282,7 @@ __global__ void __launch_bounds__(256) k_loo_pass(const double* __restrict__ row
     double* tl = tail + (size_t)col * M;
     for (long long r = r0 + lane; r < r1; r += 32) {
       const double x = rows[(size_t)r * n + col];
-      if (x > mx) { se = se * exp(mx - x) + 1.0; mx = x; }
-      else se += exp(x - mx);
+      lse_add(mx, se, x);
       const double dv = x - mu;
       sq += dv * dv;
       if (x > a) w += exp(b - x);
@@ -283,11 +296,7 @@ __global__ void __launch_bounds__(256) k_loo_pass(const double* __restrict__ row
   if (tid < PS_EPB && blockIdx.x * PS_EPB + tid < n) {
     double m = -INFINITY, s = 0.0, q = 0.0, ww = 0.0;
     for (int l = 0; l < 32; ++l) {
-      const double m2 = red[0][l][tid], s2 = red[1][l][tid];
-      if (s2 > 0.0) {
-        if (m2 > m) { s = s * exp(m - m2) + s2; m = m2; }
-        else s += s2 * exp(m2 - m);
-      }
+      lse_merge(m, s, red[0][l][tid], red[1][l][tid]);
       q += red[2][l][tid];
       ww += red[3][l][tid];
     }
@@ -431,10 +440,7 @@ __global__ void __launch_bounds__(LOO_TB) k_loo_tail(long long N, int n, long lo
     double m = -INFINITY, se = 0.0, sq = 0.0, w = 0.0;
     for (int y = 0; y < rb; ++y) {
       const double* p = part + ((size_t)y * n + col) * 4;
-      if (p[1] > 0.0) {
-        if (p[0] > m) { se = se * exp(m - p[0]) + p[1]; m = p[0]; }
-        else se += p[1] * exp(p[0] - m);
-      }
+      lse_merge(m, se, p[0], p[1]);
       sq += p[2];
       w += p[3];
     }
@@ -483,6 +489,50 @@ void launch_loo(const double* rows, long long N, int n, double* out, void* ws, c
   cudaFuncSetAttribute(k_loo_tail, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   ++g_launches;
   k_loo_tail<<<n, LOO_TB, smem, s>>>(N, n, M, rb, part, cnt, av, bv, tail, out);
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Pooled log-mean-exp of every column j of rows[N][m] (the held-out log predictive density of K-fold cross-validation):
+//   k_lpd_pass   : rows split over blocks like k_loo_pass; per block and column the logsumexp partial (m, s)
+//   k_lpd_finish : thread per column: the block partials added in block order, lpd = m + log(s) - log(N)
+// No atomics and a fixed order: the same table gives bit-identical results.
+// ------------------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) k_lpd_pass(const double* __restrict__ rows, long long N, int m, long long per,
+                                                  double* __restrict__ part) {
+  __shared__ double red[2][32][PS_EPB];
+  const int tid = threadIdx.x, e = tid % PS_EPB, lane = tid / PS_EPB;
+  const int col = blockIdx.x * PS_EPB + e;
+  const long long r0 = (long long)blockIdx.y * per, r1 = min(N, r0 + per);
+  double mx = -INFINITY, se = 0.0;
+  if (col < m)
+    for (long long r = r0 + lane; r < r1; r += 32) lse_add(mx, se, rows[(size_t)r * m + col]);
+  red[0][lane][e] = mx; red[1][lane][e] = se;
+  __syncthreads();
+  if (tid < PS_EPB && blockIdx.x * PS_EPB + tid < m) {
+    double mm = -INFINITY, ss = 0.0;
+    for (int l = 0; l < 32; ++l) lse_merge(mm, ss, red[0][l][tid], red[1][l][tid]);
+    double* p = part + ((size_t)blockIdx.y * m + blockIdx.x * PS_EPB + tid) * 2;
+    p[0] = mm; p[1] = ss;
+  }
+}
+
+__global__ void k_lpd_finish(long long N, int m, int rb, const double* __restrict__ part, double* __restrict__ lpd) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= m) return;
+  double mm = -INFINITY, ss = 0.0;
+  for (int b = 0; b < rb; ++b) lse_merge(mm, ss, part[((size_t)b * m + j) * 2], part[((size_t)b * m + j) * 2 + 1]);
+  lpd[j] = mm + log(ss) - log((double)N);
+}
+
+// scratch: partials [RB][m][2]
+size_t lpd_ws_bytes(long long N, int m) { return sizeof(double) * (size_t)pred_select_row_blocks(N, m) * m * 2; }
+
+void launch_lpd(const double* rows, long long N, int m, double* lpd, void* ws, cudaStream_t s) {
+  const int rb = pred_select_row_blocks(N, m);
+  const long long per = (N + rb - 1) / rb;
+  double* part = (double*)ws;
+  ++g_launches; k_lpd_pass<<<dim3((m + PS_EPB - 1) / PS_EPB, rb), 256, 0, s>>>(rows, N, m, per, part);
+  ++g_launches; k_lpd_finish<<<(m + 127) / 128, 128, 0, s>>>(N, m, rb, part, lpd);
 }
 
 // ------------------------------------------------------------------------------------------------------------

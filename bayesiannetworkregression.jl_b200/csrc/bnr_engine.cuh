@@ -207,9 +207,11 @@ struct Engine {
   RowTable tr_full;       // full state rows (state_var order)
   RowTable tr_gx;         // xi then gamma, width V+q
   // predictions for new networks (bnr_set_predictors; pred.base == nullptr: off).  Every recorded row r of chain c gets
-  // pred.row(c, r)[j] = mu_c + X_new[j,:] gamma_c (+ sqrt(tau2_c) z_j in the predictive mode), width m
+  // pred.row(c, r)[j] = mu_c + X_new[j,:] gamma_c (+ sqrt(tau2_c) z_j in the predictive mode), width m; for held-out
+  // rows (bnr_set_heldout, BNR_PRED_LOGDENS) log N(y_held[j] | mu_c + X_new[j,:] gamma_c, tau2_c) instead
   RowTable pred;
   const double* Xp;       // [qp][pred_mp] X_new columns padded to pred_mp rows (a multiple of 128; zeros beyond m, q)
+  const double* pred_y;   // [m] held-out responses (BNR_PRED_LOGDENS only, else nullptr)
   int pred_mp, pred_mode, pred_splits;   // padded m, BNR_PRED_*, k-splits of the product X_new gamma
   double* pred_ws;        // split-K partials of X_new gamma, [pred_splits][C][pred_mp]; a chain group's view uses
                           // [pred_splits][Cg][pred_mp] at offset c0 * pred_splits * pred_mp

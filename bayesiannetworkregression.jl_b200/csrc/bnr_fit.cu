@@ -295,6 +295,15 @@ struct bnr_fit_result {
   };
   Pooled pred = {"predictions"};       // predictions for new networks (bnr_fit_predict), width m
   Pooled ll = {"log-likelihood"};      // pointwise log-likelihood for PSIS-LOO / WAIC (bnr_fit_loo), width n
+  Pooled held = {"held-out log densities"};   // K-fold (bnr_fit_kfold): exp[f] holds fold f's retained rows
+  // K-fold cross-validation (K == 0: an ordinary fit).  h[f], dev[f] are fold f's handle and device
+  struct KFold {
+    int K = 0, n_devices = 0;
+    std::vector<std::vector<int>> held;                   // per fold: its held-out observations, in original order
+    std::vector<std::vector<double>> rhat_xi, rhat_gamma; // per fold: the R-hat of the last PSRF step
+    std::vector<double> elpd;                             // [n] elpd_kfold in original order
+    bool ok = false;
+  } kf;
   int pmode = 0;
   std::vector<double> p_mean, p_lo, p_hi;
   std::vector<double> l_pw[5];         // elpd_loo, p_loo, pareto_k, elpd_waic, p_waic per observation
@@ -305,7 +314,7 @@ struct bnr_fit_result {
     for (size_t d = 0; d < h.size(); ++d) {
       if (d < dev.size()) cudaSetDevice(dev[d]);
       if (d < gbuf.size() && gbuf[d]) cudaFree(gbuf[d]);
-      for (Pooled* t : {&pred, &ll})
+      for (Pooled* t : {&pred, &ll, &held})
         if (d < t->exp.size() && t->exp[d]) cudaFree(t->exp[d]);
       if (d < xs.size() && xs[d]) cudaStreamDestroy(xs[d]);
     }
@@ -329,6 +338,13 @@ struct PhaseClock {
   };
 };
 enum { PH_CREATE = 0, PH_INIT, PH_RUN, PH_COPY, PH_PSRF, PH_SUMMARY, PH_ESS, PH_MISC };
+
+// Julia's maximum(v): NaN if any element is NaN
+double jmax(const std::vector<double>& v) {
+  double m = -INFINITY;
+  for (double x : v) { if (std::isnan(x)) return (double)NAN; if (x > m) m = x; }
+  return m;
+}
 
 struct DeviceOps : Ops {
   bnr_fit_result& R;
@@ -577,11 +593,6 @@ struct DeviceOps : Ops {
       if (int r = gather_ext((size_t)cnt * R.h.size(), &all)) return r;
       BN(bnr_rhat_from_moments(R.dev[0], all, total_chains(), R.V, R.q, half, R.rhat_xi.data(), R.rhat_gamma.data()));
     }
-    auto jmax = [](const std::vector<double>& v) {
-      double m = -INFINITY;
-      for (double x : v) { if (std::isnan(x)) return (double)NAN; if (x > m) m = x; }
-      return m;
-    };
     *mx = jmax(R.rhat_xi); *mg = jmax(R.rhat_gamma);
     return 0;
   }
@@ -632,6 +643,96 @@ struct DeviceOps : Ops {
       if (rc) return rc;
     }
     R.ess_ok = true;
+    return 0;
+  }
+};
+
+// K-fold cross-validation: one handle per fold (fold f on device base.device + f mod n_devices), every broadcast
+// operation of DeviceOps applied to all of them, R-hat taken per fold and the maximum handed to the control loop
+struct KFoldOps : DeviceOps {
+  struct Fold { std::vector<double> X, y, Xh, yh; int n = 0, m = 0; };
+  std::vector<Fold> folds;
+  explicit KFoldOps(bnr_fit_result& r) : DeviceOps(r, nullptr, nullptr, nullptr) {}
+
+  int create(long long rows, bool gx_all, int full) override {
+    PhaseClock::Scope sc(clk, PH_CREATE);
+    const int K = R.kf.K, nd = R.p.n_devices > 0 ? R.p.n_devices : 1;
+    R.kf.n_devices = K < nd ? K : nd;
+    R.h.assign(K, nullptr); R.dev.assign(K, 0); R.xs.assign(K, nullptr); R.gbuf.assign(K, nullptr);
+    R.held.exp.assign(K, nullptr);
+    R.V = R.p.base.V; R.q = R.V * (R.V + 1) / 2; R.C = R.p.base.num_chains;
+    for (int f = 0; f < K; ++f) {
+      Fold& fd = folds[f];
+      // the device-0 handle bnr_fit creates for these training rows, at this fold's chain offset
+      bnr_params bp = R.p.base;
+      bp.n = fd.n;
+      bp.device = R.p.base.device + f % nd;
+      bp.chain_offset = R.p.base.chain_offset + f * bp.num_chains;
+      bp.trace_rows = rows;
+      bp.trace_gamma_xi_all = gx_all ? 1 : 0;
+      bp.trace_full_chains = full;
+      bp.trace_gamma_xi_chains = 1;
+      R.dev[f] = bp.device;
+      BN(bnr_create(&bp, fd.X.data(), fd.y.data(), &R.h[f]));
+      BN(bnr_set_heldout(R.h[f], fd.m, fd.Xh.data(), fd.yh.data(), rows));
+      // the handle holds its own copies now
+      for (std::vector<double>* v : {&fd.X, &fd.y, &fd.Xh, &fd.yh}) std::vector<double>().swap(*v);
+      const size_t local = (size_t)R.C * rows * fd.m;
+      CKF(cudaSetDevice(R.dev[f]));
+      if (cudaMalloc((void**)&R.held.exp[f], local * sizeof(double)) != cudaSuccess) {
+        R.held.exp[f] = nullptr;
+        cudaGetLastError();
+        return ffail(BNR_ENOMEM, "cannot allocate the export buffer of fold " + std::to_string(f + 1) +
+                                     "'s held-out log densities (" + std::to_string(local * sizeof(double)) + " bytes)");
+      }
+    }
+    int32_t gm = 0;
+    BN(bnr_gamma_mode(R.h[0], &gm));
+    R.gamma_mode = gm;
+    return 0;
+  }
+
+  int psrf(int mode, long long a, long long b, double* mx, double* mg) override {
+    PhaseClock::Scope sc(clk, PH_PSRF);
+    const int K = R.kf.K;
+    R.rhat_xi.assign(R.V, NAN); R.rhat_gamma.assign(R.q, NAN);
+    R.kf.rhat_xi.assign(K, std::vector<double>(R.V, NAN));
+    R.kf.rhat_gamma.assign(K, std::vector<double>(R.q, NAN));
+    if (mode != 2 && b / 2 < 2) { *mx = NAN; *mg = NAN; return 0; }
+    for (auto* h : R.h) {
+      if (mode == 0) BN(bnr_moments_from_trace(h, a, b));
+      if (mode == 2) BN(bnr_moments_from_blocks(h, (int32_t)a, (int32_t)b));
+    }
+    int64_t half = 0;
+    BN(bnr_moment_half_len(R.h[0], &half));
+    if (half < 2) { *mx = NAN; *mg = NAN; return 0; }
+    // element-wise maximum over the folds; NaN wins, so that jmax of it is jmax over all folds' values
+    auto fold_max = [](std::vector<double>& acc, const std::vector<double>& v, bool first) {
+      for (size_t i = 0; i < v.size(); ++i)
+        if (first || std::isnan(v[i]) || (!std::isnan(acc[i]) && v[i] > acc[i])) acc[i] = v[i];
+    };
+    for (int f = 0; f < K; ++f) {
+      BN(bnr_rhat(R.h[f], R.kf.rhat_xi[f].data(), R.kf.rhat_gamma[f].data()));
+      fold_max(R.rhat_xi, R.kf.rhat_xi[f], f == 0);
+      fold_max(R.rhat_gamma, R.kf.rhat_gamma[f], f == 0);
+    }
+    *mx = jmax(R.rhat_xi); *mg = jmax(R.rhat_gamma);
+    return 0;
+  }
+
+  // elpd_kfold of every held-out observation: the log-mean-exp of its fold's retained rows of all chains
+  int pool(const Outcome& o) {
+    const long long N = (long long)R.C * o.sampled;
+    if (N < 1) return 0;
+    R.kf.elpd.assign(R.p.base.n, NAN);
+    for (int f = 0; f < R.kf.K; ++f) {
+      const Fold& fd = folds[f];
+      BN(bnr_export_predictions(R.h[f], o.burn_in, o.sampled, R.held.exp[f]));
+      std::vector<double> lpd(fd.m);
+      BN(bnr_lpd_summary(R.dev[f], R.held.exp[f], N, fd.m, lpd.data()));
+      for (int j = 0; j < fd.m; ++j) R.kf.elpd[R.kf.held[f][j]] = lpd[j];
+    }
+    R.kf.ok = true;
     return 0;
   }
 };
@@ -750,9 +851,107 @@ extern "C" int bnr_fit_loo(const bnr_fit_params* p, const double* X, const doubl
   return fit_body(p, X, y, m, X_new, pred_mode, true, res_out);
 }
 
+// the fold layout of bnr_fit_kfold: labels checked, training and held-out rows of every fold in original order
+static int kfold_split(const bnr_fit_params* p, const double* X, const double* y, int32_t K, const int32_t* fold,
+                       bnr_fit_result* R, KFoldOps& o) {
+  const int n = p->base.n, V = p->base.V;
+  const size_t q = (size_t)V * (V + 1) / 2;
+  std::vector<int> cnt(K, 0);
+  for (int i = 0; i < n; ++i) {
+    if (fold[i] < 1 || fold[i] > K)
+      return ffail(BNR_EINVAL, "fold label " + std::to_string(fold[i]) + " of observation " + std::to_string(i + 1) +
+                                   " lies outside 1.." + std::to_string(K));
+    ++cnt[fold[i] - 1];
+  }
+  for (int f = 0; f < K; ++f) {
+    if (cnt[f] == 0) return ffail(BNR_EINVAL, "fold " + std::to_string(f + 1) + " holds no observation");
+    if (cnt[f] == n) return ffail(BNR_EINVAL, "fold " + std::to_string(f + 1) + " leaves an empty training set");
+  }
+  R->kf.K = K;
+  R->kf.held.assign(K, {});
+  o.folds.assign(K, {});
+  for (int f = 0; f < K; ++f) {
+    KFoldOps::Fold& fd = o.folds[f];
+    fd.m = cnt[f]; fd.n = n - cnt[f];
+    for (int i = 0; i < n; ++i) {
+      const bool held = fold[i] == f + 1;
+      (held ? fd.yh : fd.y).push_back(y[i]);
+      if (held) R->kf.held[f].push_back(i);
+    }
+    // column by column: X is column-major, so both sides are read and written in order
+    fd.X.resize((size_t)fd.n * q); fd.Xh.resize((size_t)fd.m * q);
+    double *dt = fd.X.data(), *dh = fd.Xh.data();
+    for (size_t j = 0; j < q; ++j) {
+      const double* col = X + (size_t)n * j;
+      for (int i = 0; i < n; ++i) *(fold[i] == f + 1 ? dh++ : dt++) = col[i];
+    }
+  }
+  return 0;
+}
+
+extern "C" int bnr_fit_kfold(const bnr_fit_params* p, const double* X, const double* y, int32_t K, const int32_t* fold,
+                             bnr_fit_result** res_out) {
+  if (int r = check_params(p)) return r;
+  if (!X || !y || !fold || !res_out) return ffail(BNR_EINVAL, "null argument");
+  if (K < 2) return ffail(BNR_EINVAL, "K-fold cross-validation needs K >= 2 folds");
+  if (p->base.n < 2) return ffail(BNR_EINVAL, "K-fold cross-validation needs n >= 2 observations");
+  if (p->base.V < 1) return ffail(BNR_EINVAL, "V must be >= 1");
+  if (p->ext_world > 1) return ffail(BNR_EINVAL, "K-fold cross-validation runs in one process (ext_world must be <= 1)");
+  if (p->ess_max_lag > 0) return ffail(BNR_EINVAL, "K-fold cross-validation computes no ESS (ess_max_lag must be 0)");
+  if (p->base.nu < p->base.R) return ffail(BNR_EINVAL, "nu must not be smaller than R");
+  bnr_fit_result* R = new bnr_fit_result();
+  R->p = *p;
+  KFoldOps o(*R);
+  int rc = kfold_split(p, X, y, K, fold, R, o);
+  const double t_start = PhaseClock::now();
+  if (!rc) rc = fit_loops(o, *p, R->out);
+  if (!rc) rc = o.pool(R->out);
+  if (!rc) {
+    std::vector<int32_t> st(R->C);
+    for (auto* h : R->h) {
+      if (bnr_status(h, st.data()) != BNR_OK) { rc = ffail(BNR_ECUDA, bnr_last_error()); break; }
+      for (int v : st) R->status_or |= v;
+    }
+  }
+  if (getenv("BNR_FIT_TIMING"))
+    fprintf(stderr, "bnr_fit_kfold %.1f ms: create %.1f  init %.1f  run %.1f  row copies %.1f  psrf %.1f\n",
+            1e3 * (PhaseClock::now() - t_start), 1e3 * o.clk.t[PH_CREATE], 1e3 * o.clk.t[PH_INIT], 1e3 * o.clk.t[PH_RUN],
+            1e3 * o.clk.t[PH_COPY], 1e3 * o.clk.t[PH_PSRF]);
+  if (rc) {
+    const std::string msg = g_fit_err;
+    delete R;
+    g_fit_err = msg;
+    return rc;
+  }
+  *res_out = R;
+  return BNR_OK;
+}
+
+extern "C" int bnr_fit_kfold_pointwise(const bnr_fit_result* r, double* elpd_kfold) {
+  if (!r || !elpd_kfold) return ffail(BNR_EINVAL, "null argument");
+  if (!r->kf.K) return ffail(BNR_ESTATE, "not a K-fold result (bnr_fit_kfold)");
+  if (!r->kf.ok) return ffail(BNR_ESTATE, "no retained draws");
+  memcpy(elpd_kfold, r->kf.elpd.data(), sizeof(double) * r->kf.elpd.size());
+  return BNR_OK;
+}
+
+extern "C" int bnr_fit_kfold_rhat(const bnr_fit_result* r, int32_t f, double* rhat_xi, double* rhat_gamma) {
+  if (!r) return ffail(BNR_EINVAL, "null result");
+  if (!r->kf.K) return ffail(BNR_ESTATE, "not a K-fold result (bnr_fit_kfold)");
+  if (f < 0 || f >= r->kf.K) return ffail(BNR_EINVAL, "fold index outside 0..K-1");
+  if (rhat_xi) memcpy(rhat_xi, r->kf.rhat_xi[f].data(), sizeof(double) * r->V);
+  if (rhat_gamma) memcpy(rhat_gamma, r->kf.rhat_gamma[f].data(), sizeof(double) * r->q);
+  return BNR_OK;
+}
+
+static int not_kfold(const bnr_fit_result* r) {
+  return r->kf.K ? ffail(BNR_ESTATE, "not available on a K-fold result (bnr_fit_kfold)") : 0;
+}
+
 extern "C" int bnr_fit_loo_pointwise(const bnr_fit_result* r, double* elpd_loo, double* p_loo, double* pareto_k,
                                      double* elpd_waic, double* p_waic) {
   if (!r) return ffail(BNR_EINVAL, "null result");
+  if (int e = not_kfold(r)) return e;
   if (!r->ll.ok)
     return ffail(BNR_ESTATE, r->ll.width > 0 ? "fewer than 2 retained draws for PSIS-LOO"
                                              : "the fit was run without the log-likelihood (bnr_fit_loo)");
@@ -764,6 +963,7 @@ extern "C" int bnr_fit_loo_pointwise(const bnr_fit_result* r, double* elpd_loo, 
 
 extern "C" int bnr_fit_prediction(const bnr_fit_result* r, double* mean, double* lo, double* hi) {
   if (!r) return ffail(BNR_EINVAL, "null result");
+  if (int e = not_kfold(r)) return e;
   if (!r->pred.ok)
     return ffail(BNR_ESTATE, r->pred.width > 0 ? "too few retained draws for the prediction interval"
                                                : "the fit was run without X_new (bnr_fit_predict)");
@@ -781,7 +981,7 @@ extern "C" int bnr_fit_get_info(const bnr_fit_result* r, bnr_fit_info* info) {
   info->summary_ok = r->summary_ok ? 1 : 0; info->ess_ok = r->ess_ok ? 1 : 0;
   info->gamma_mode = r->gamma_mode; info->status_or = r->status_or;
   info->total_chains = r->C * (int)r->h.size() * (r->p.ext_world > 1 ? r->p.ext_world : 1);
-  info->n_devices = (int)r->h.size();
+  info->n_devices = r->kf.K ? r->kf.n_devices : (int)r->h.size();
   info->exchange = !strcmp(r->exchange, "nccl") ? 1 : (!strcmp(r->exchange, "peer-copy") ? 2 : 0);
   return BNR_OK;
 }
@@ -796,6 +996,7 @@ extern "C" int bnr_fit_rhat(const bnr_fit_result* r, double* rhat_xi, double* rh
 extern "C" int bnr_fit_summary(const bnr_fit_result* r, double* gamma_mean, double* gamma_lo, double* gamma_hi,
                                double* xi_mean) {
   if (!r) return ffail(BNR_EINVAL, "null result");
+  if (int e = not_kfold(r)) return e;
   if (!r->summary_ok)
     return ffail(BNR_ESTATE, "too few retained draws for the credible interval (the reference's Summary raises a BoundsError)");
   if (gamma_mean) memcpy(gamma_mean, r->s_mean.data(), sizeof(double) * r->q);
@@ -807,6 +1008,7 @@ extern "C" int bnr_fit_summary(const bnr_fit_result* r, double* gamma_mean, doub
 
 extern "C" int bnr_fit_ess(const bnr_fit_result* r, double* ess_xi, double* ess_gamma) {
   if (!r) return ffail(BNR_EINVAL, "null result");
+  if (int e = not_kfold(r)) return e;
   if (!r->ess_ok) return ffail(BNR_ESTATE, "no ESS statistics (ess_max_lag = 0, or the doubling scheme with block moments)");
   if (ess_xi) memcpy(ess_xi, r->ess_xi.data(), sizeof(double) * r->V);
   if (ess_gamma) memcpy(ess_gamma, r->ess_gamma.data(), sizeof(double) * r->q);
@@ -815,6 +1017,7 @@ extern "C" int bnr_fit_ess(const bnr_fit_result* r, double* ess_xi, double* ess_
 
 extern "C" int bnr_fit_state(bnr_fit_result* r, int32_t var, double* out) {
   if (!r || !out) return ffail(BNR_EINVAL, "null argument");
+  if (int e = not_kfold(r)) return e;
   if (r->p.return_state == BNR_STATE_NONE) return ffail(BNR_ESTATE, "the fit was run with return_state = BNR_STATE_NONE");
   if (r->p.return_state == BNR_STATE_GAMMA_XI && var != BNR_VAR_GAMMA && var != BNR_VAR_XI)
     return ffail(BNR_ESTATE, "only gamma and xi were recorded (return_state = BNR_STATE_GAMMA_XI)");
@@ -822,6 +1025,7 @@ extern "C" int bnr_fit_state(bnr_fit_result* r, int32_t var, double* out) {
   return BNR_OK;
 }
 
+// device_index: the device's place among the result's devices, or the fold (0-based) of a K-fold result
 extern "C" int bnr_fit_handle(bnr_fit_result* r, int32_t device_index, bnr_handle** h) {
   if (!r || !h || device_index < 0 || device_index >= (int)r->h.size()) return ffail(BNR_EINVAL, "bad arguments");
   *h = r->h[device_index];

@@ -107,6 +107,10 @@ long long loo_tail_len(long long N);
 long long loo_tail_max();
 size_t loo_ws_bytes(long long N, int n);
 void launch_loo(const double* rows, long long N, int n, double* out, void* ws, cudaStream_t s);
+// pooled log-mean-exp of each of the m columns of rows[N][m]: lpd[j] = logsumexp_s rows[s][j] - log N (fixed order);
+// ws: lpd_ws_bytes(N, m) bytes
+size_t lpd_ws_bytes(long long N, int m);
+void launch_lpd(const double* rows, long long N, int m, double* lpd, void* ws, cudaStream_t s);
 void launch_ess_finish(const double* acov_parts, int nparts, const double* cmeans, int chains, int P, long long N,
                        int L, double* ess, double* lag_used, cudaStream_t s);
 // split R-hat of [chains][2][nparams][2] moments (h draws per half); the split-half moments of mom from trace rows

@@ -762,7 +762,8 @@ __global__ void __launch_bounds__(256) k_record(Engine e, int sweep_done /* 1: s
 }
 
 // one prediction row per chain: pred[c][row][j] = mu_c + sum_z partial_z[c][j] (z in split order) (+ sqrt(tau2_c) z_j,
-// z_j from the SITE_PRED stream of element j at the row's sweep).  grid = (ceil(m / 256), C)
+// z_j from the SITE_PRED stream of element j at the row's sweep); held-out rows (mode 2) store
+// -1/2 log(2 pi tau2_c) - (y_j - mu_c - sum_z partial_z[c][j])^2 / (2 tau2_c) and draw nothing.  grid = (ceil(m / 256), C)
 __global__ void __launch_bounds__(256) k_pred_record(Engine e, int sweep_done /* 1: state belongs to sweep iter+1 */) {
   const int c = blockIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x;
   const long long row = *e.trace_row;
@@ -771,6 +772,12 @@ __global__ void __launch_bounds__(256) k_pred_record(Engine e, int sweep_done /*
   const double* w = e.pred_ws + (size_t)c * e.pred_mp + j;
   double s = 0.0;
   for (int z = 0; z < e.pred_splits; ++z) s += w[z * stride];
+  if (e.pred_mode == 2) {
+    const double t2 = e.tau2[c];
+    const double r = e.pred_y[j] - e.mu[c] - s;
+    e.pred.row(c, row)[j] = -0.5 * log(6.283185307179586 * t2) - r * r / (2.0 * t2);
+    return;
+  }
   double v = e.mu[c] + s;
   if (e.pred_mode == 1) {
     const long long sweep = *e.iter + (sweep_done ? 1 : 0);

@@ -21,6 +21,13 @@ def var_shape(var, R, V, q):
             "Delta": (1, 1), "M": (R, R), "mu": (1, 1), "lam": (R, 1), "pi": (R, 3)}[var]
 
 
+def lpd_summary(device, dev_ptr, N, m):
+    """bnr_lpd_summary on a device table of N draws x m columns: [m] log((1/N) sum_s exp(rows[s][j]))."""
+    out = np.empty(int(m))
+    check(lib().bnr_lpd_summary(int(device), C.c_void_p(dev_ptr), int(N), int(m), _dp(out)))
+    return out
+
+
 def loo_summary(device, dev_ptr, N, n):
     """bnr_loo_summary on a device table of N draws x n observations: dict of the five pointwise [n] arrays."""
     out = [np.empty(int(n)) for _ in LOO_FIELDS]
@@ -256,6 +263,25 @@ class Engine:
         check(self._L.bnr_set_predictors(self._h, Xn.shape[0], _dp(Xn), int(rows),
                                          PRED_PREDICTIVE if predictive else PRED_MEAN))
         self.pred_m = Xn.shape[0]
+
+    def set_heldout(self, X, y, rows):
+        """Record log N(y_j | mu + X[j,:] gamma, tau2) for the m held-out observations (X: m x q laid out like the
+        training X, y: m) at every recorded row of every chain, in the prediction table (`rows` >= 1 rows per chain;
+        it replaces any predictors).  X=None switches it off (y and rows are then ignored)."""
+        if X is None:
+            check(self._L.bnr_set_heldout(self._h, 0, None, None, 0))
+            self.pred_m = 0
+            return
+        Xh = np.asfortranarray(X, dtype=np.float64)
+        yh = np.ascontiguousarray(y, dtype=np.float64)
+        if Xh.ndim != 2 or Xh.shape[1] != self.q or yh.shape != (Xh.shape[0],):
+            raise ValueError("X must be m x q with q = %d and y of length m" % self.q)
+        check(self._L.bnr_set_heldout(self._h, Xh.shape[0], _dp(Xh), _dp(yh), int(rows)))
+        self.pred_m = Xh.shape[0]
+
+    def heldout_trace(self, chain, first, last):
+        """Rows [first, last) of one chain's held-out log densities as an array of shape (last - first, m)."""
+        return self.prediction_trace(chain, first, last)
 
     def prediction_trace(self, chain, first, last):
         """Rows [first, last) of one chain's prediction table as an array of shape (last - first, m)."""

@@ -14,7 +14,7 @@ import warnings
 import numpy as np
 
 from .capi import lib, check, check_fit, FitParams, FitInfo, ALLGATHER_FN, STATE, VAR, GAMMA_MODE, PRED_MEAN, \
-    PRED_PREDICTIVE
+    PRED_PREDICTIVE, STATUS_BITS
 from .engine import LOO_FIELDS, var_shape
 
 _DP = C.POINTER(C.c_double)
@@ -197,13 +197,10 @@ def _torch_allgather(ctx, device, send, recv, count):
 _ALLGATHER = ALLGATHER_FN(_torch_allgather)
 
 
-def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsamp=0, mingen=0, maxgen=0,
+def _fit_params(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsamp=0, mingen=0, maxgen=0,
                 psrf_cutoff=1.01, purge_burn=None, num_chains=2, seed=0, device=0, return_state="full", verbose=False,
-                chain_offset=0, n_devices=1, ess_max_lag=0, interval=95, gamma_mode="auto", chain_groups=0, X_new=None,
-                predictive=False, loo=False):
-    """One bnr_fit call (include/bnr.h): chain generation, purge ring, PSRF loop, R-hat, Summary statistics on the GPU.
-    With X_new (m x q, already vectorised) the call is bnr_fit_predict, which also pools the predictions; with loo=True
-    it is bnr_fit_loo, which also scores the fit by PSIS-LOO and WAIC."""
+                chain_offset=0, n_devices=1, ess_max_lag=0, interval=95, gamma_mode="auto", chain_groups=0):
+    """(X column-major, y, V, struct bnr_fit_params) of one native call."""
     L = lib()
     Xf = np.asfortranarray(Xn, dtype=np.float64)
     y = np.ascontiguousarray(y, dtype=np.float64)
@@ -224,6 +221,18 @@ def _native_fit(Xn, y, R, *, eta, zeta, iota, a_delta, b_delta, nu, nburn=0, nsa
     p.purge_burn = int(purge_burn) if purge_burn else 0
     p.return_state = STATE[return_state]
     p.n_devices, p.interval, p.ess_max_lag, p.verbose = int(n_devices), int(interval), int(ess_max_lag), 1 if verbose else 0
+    return Xf, y, V, p
+
+
+def _native_fit(Xn, y, R, *, X_new=None, predictive=False, loo=False, **kw):
+    """One bnr_fit call (include/bnr.h): chain generation, purge ring, PSRF loop, R-hat, Summary statistics on the GPU.
+    With X_new (m x q, already vectorised) the call is bnr_fit_predict, which also pools the predictions; with loo=True
+    it is bnr_fit_loo, which also scores the fit by PSIS-LOO and WAIC."""
+    L = lib()
+    Xf, y, V, p = _fit_params(Xn, y, R, **kw)
+    n, q = Xf.shape
+    num_chains, interval, ess_max_lag = p.base.num_chains, p.interval, p.ess_max_lag
+    return_state, seed = kw.get("return_state", "full"), kw.get("seed", 0)
     rank, world = _dist_world()
     if world > 1:
         p.ext_world, p.ext_rank, p.allgather = world, rank, _ALLGATHER
@@ -517,51 +526,178 @@ def Loo(results):
 
 
 class BNRCompare:
-    """Compare's table: one row per fit, best first (a dict of columns like BNRSummary.edge_coef)."""
+    """Compare's table: one row per fit, best first (a dict of columns like BNRSummary.edge_coef).  `columns` lists the
+    numeric columns: those of loo_compare for PSIS-LOO fits, the elpd_kfold / kfoldic ones for K-fold fits."""
 
     COLUMNS = ("elpd_diff", "se_diff", "elpd_loo", "se_elpd_loo", "p_loo", "se_p_loo", "looic", "se_looic")
 
-    def __init__(self, table):
+    def __init__(self, table, columns=COLUMNS):
         self.table = table
+        self.columns = tuple(columns)
 
     def __repr__(self):
         t = self.table
-        lines = ["", "%-10s" % "model" + "".join("%12s" % c for c in self.COLUMNS)]
+        lines = ["", "%-10s" % "model" + "".join("%14s" % c if len(c) > 11 else "%12s" % c for c in self.columns)]
         for i, name in enumerate(t["model"]):
-            lines.append("%-10s" % name + "".join("%12.1f" % t[c][i] for c in self.COLUMNS))
+            lines.append("%-10s" % name + "".join(("%14.1f" if len(c) > 11 else "%12.1f") % t[c][i]
+                                                   for c in self.columns))
         return "\n".join(lines)
 
 
 def Compare(*results, names=None):
     """loo_compare: the fits ranked by elpd_loo (best first); elpd_diff = elpd_loo - elpd_loo(best) and
     se_diff = sqrt(n) sd(pointwise elpd_loo differences to the best), both 0 for the best.  The fits must have been
-    run on the same responses y."""
+    run on the same responses y.  K-fold results (KFold) are ranked the same way by elpd_kfold; they must share their
+    folds, and cannot be mixed with PSIS-LOO fits."""
     if len(results) < 2:
         raise ValueError("Compare needs at least two fits")
     names = list(names) if names is not None else ["model%d" % (i + 1) for i in range(len(results))]
     if len(names) != len(results):
         raise ValueError("one name per fit")
-    los = [_loo_pointwise(r) for r in results]
-    y0 = los[0]["y"]
-    for lo in los[1:]:
-        if lo["y"].shape != y0.shape or not np.array_equal(lo["y"], y0):
-            raise ValueError("Compare needs fits of the same responses y")
-    loos = [BNRLoo(lo["pointwise"], lo["draws"]) for lo in los]
-    elpd = np.array([lo.estimates["elpd_loo"][0] for lo in loos])
-    order = sorted(range(len(loos)), key=lambda i: -elpd[i])
-    best = loos[order[0]].pointwise["elpd_loo"]
+    kfold = [isinstance(r, BNRKFold) for r in results]
+    if any(kfold) and not all(kfold):
+        raise ValueError("Compare cannot mix PSIS-LOO fits and K-fold results")
+    if all(kfold):
+        y0, f0 = results[0].y, results[0].folds
+        for r in results[1:]:
+            if r.y.shape != y0.shape or not np.array_equal(r.y, y0):
+                raise ValueError("Compare needs fits of the same responses y")
+            if not np.array_equal(r.folds, f0):
+                raise ValueError("Compare needs K-fold results with the same folds")
+        scored = results
+        key, stats = "elpd_kfold", ("elpd_kfold", "kfoldic")
+    else:
+        los = [_loo_pointwise(r) for r in results]
+        y0 = los[0]["y"]
+        for lo in los[1:]:
+            if lo["y"].shape != y0.shape or not np.array_equal(lo["y"], y0):
+                raise ValueError("Compare needs fits of the same responses y")
+        scored = [BNRLoo(lo["pointwise"], lo["draws"]) for lo in los]
+        key, stats = "elpd_loo", ("elpd_loo", "p_loo", "looic")
+    columns = ("elpd_diff", "se_diff") + tuple(c for k in stats for c in (k, "se_" + k))
+    elpd = np.array([r.estimates[key][0] for r in scored])
+    order = sorted(range(len(scored)), key=lambda i: -elpd[i])
+    best = scored[order[0]].pointwise[key]
     n = best.size
-    table = {c: [] for c in ("model",) + BNRCompare.COLUMNS}
+    table = {c: [] for c in ("model",) + columns}
     for i in order:
-        lo = loos[i]
-        d = lo.pointwise["elpd_loo"] - best
+        r = scored[i]
+        d = r.pointwise[key] - best
         table["model"].append(names[i])
         table["elpd_diff"].append(float(d.sum()))
         table["se_diff"].append(float(math.sqrt(n) * d.std(ddof=1)) if n > 1 else 0.0)
-        for k in ("elpd_loo", "p_loo", "looic"):
-            e, se = lo.estimates[k]
+        for k in stats:
+            e, se = r.estimates[k]
             table[k].append(e)
             table["se_" + k].append(se)
-    for c in BNRCompare.COLUMNS:
+    for c in columns:
         table[c] = np.asarray(table[c])
-    return BNRCompare(table)
+    return BNRCompare(table, columns)
+
+
+# -- K-fold cross-validation (the R package loo: kfold, print.kfold) -------------------------------------------------
+class BNRKFold:
+    """KFold's result: `estimates` maps elpd_kfold and kfoldic (= -2 elpd_kfold) to (estimate, SE) with
+    SE = sqrt(n var(pointwise)); `pointwise` holds the [n] arrays in the original observation order; `folds` the 1-based
+    fold of every observation; `draws` the pooled draws behind each held-out density (chains per fold x sampled);
+    `rhat_max` the largest R-hat of xi and gamma of each fold's last convergence check; `status` the OR of the status
+    bits (capi.STATUS_BITS: jitter, non-PD, NaN ...) of every chain of every fold, 0 when no chain raised one."""
+
+    NAMES = ("elpd_kfold", "kfoldic")
+
+    def __init__(self, elpd_kfold, folds, y, draws, rhat_max=None, burn_in=0, sampled=0, status=0):
+        e = np.asarray(elpd_kfold, dtype=np.float64)
+        self.pointwise = dict(elpd_kfold=e, kfoldic=-2.0 * e)
+        self.folds = np.asarray(folds, dtype=np.int64)
+        self.K = int(self.folds.max())
+        self.y = np.asarray(y, dtype=np.float64)
+        self.draws = int(draws)
+        self.rhat_max = None if rhat_max is None else np.asarray(rhat_max, dtype=np.float64)
+        self.burn_in, self.sampled = int(burn_in), int(sampled)
+        self.status = int(status)
+        self.n = int(e.size)
+        self.estimates = {k: _estimate(self.pointwise[k]) for k in self.NAMES}
+
+    def __repr__(self):
+        lines = ["", "Based on %d-fold cross-validation." % self.K, "", "           Estimate      SE"]
+        for k in self.NAMES:
+            e, se = self.estimates[k]
+            lines.append("%-10s %9.1f %7.1f" % (k, e, se))
+        return "\n".join(lines)
+
+
+def kfold_split(n, K, seed):
+    """Balanced random folds: a permutation of 0..n-1 from numpy's default_rng(seed) gets the labels 1..K in turn, so
+    fold sizes differ by at most one."""
+    if not 2 <= K <= n:
+        raise ValueError("K-fold cross-validation needs 2 <= K <= n (K = %d, n = %d)" % (K, n))
+    perm = np.random.default_rng(seed).permutation(n)
+    folds = np.empty(n, dtype=np.int32)
+    folds[perm] = np.arange(n) % K + 1
+    return folds
+
+
+def KFold(X, y, R, K=None, folds=None, fold_seed=None, *, η=None, ζ=None, ι=None, aΔ=None, bΔ=None, ν=None,
+          nburn=30000, nsamples=20000, mingen=0, maxgen=0, psrf_cutoff=1.01, x_transform=True, num_chains=2,
+          seed=None, purge_burn=None, eta=None, zeta=None, iota=None, a_delta=None, b_delta=None, nu=None, device=0,
+          return_state="none", verbose=False, chain_offset=0, n_devices=1, gamma_mode="auto", chain_groups=0, **kw):
+    """K-fold cross-validation of `Fit(X, y, R, ...)` on the GPU (loo::kfold): observation i is held out by fold
+    folds[i] in 1..K; every fold is the fit of the other observations with the same keywords (num_chains per fold),
+    all folds advancing together (fold f on device device + f mod n_devices).  Each held-out observation scores
+    log((1/S) sum_s N(y_i | mu_s + x_i gamma_s, tau2_s)) over the S retained draws of all chains of its fold.  folds
+    defaults to balanced random folds from default_rng(fold_seed or seed) (kfold_split) with K = 10 unless given; with
+    folds given, K may be omitted and must otherwise equal max(folds).  Warns when a chain raised a status bit.  The remedy the loo package
+    prescribes when PSIS-LOO's Pareto k diagnostic is too high.  Compare ranks K-fold results that share their folds."""
+    for bad in ("X_new", "predictive", "loo", "ess_max_lag"):
+        if kw.get(bad) is not None and kw.get(bad) is not False and not (bad == "ess_max_lag" and kw[bad] == 0):
+            raise ValueError("KFold does not take %s: a K-fold run scores only its held-out observations" % bad)
+    unknown = set(kw) - {"X_new", "predictive", "loo", "ess_max_lag", "V", "suppress_timer", "filename", "interval"}
+    if unknown:
+        raise TypeError("KFold got unexpected keyword arguments %s" % sorted(unknown))
+
+    def pick(greek, ascii_, default):
+        return default if (greek is None and ascii_ is None) else (greek if greek is not None else ascii_)
+
+    hyper = dict(eta=pick(η, eta, 1.01), zeta=pick(ζ, zeta, 1.0), iota=pick(ι, iota, 1.0),
+                 a_delta=pick(aΔ, a_delta, 1.0), b_delta=pick(bΔ, b_delta, 1.0), nu=pick(ν, nu, 10))
+    if seed is None:
+        seed = random.randint(1, 55555)
+    Xn, y = _prepare(X, y, R, hyper["nu"], x_transform)
+    n = y.size
+    if folds is None:
+        folds = kfold_split(n, 10 if K is None else int(K), fold_seed or seed)
+    folds = np.ascontiguousarray(folds, dtype=np.int32)
+    if folds.shape != (n,):
+        raise ValueError("folds must hold one label per observation")
+    if K is not None and int(K) != int(folds.max()):
+        raise ValueError("K = %d disagrees with the folds, whose largest label is %d" % (int(K), int(folds.max())))
+    K = int(folds.max())
+    sched = dict(nburn=nburn, nsamp=nsamples) if not (mingen > 0 and maxgen > 0) else dict(mingen=mingen, maxgen=maxgen)
+    L = lib()
+    Xf, y, V, p = _fit_params(Xn, y, R, psrf_cutoff=psrf_cutoff, purge_burn=purge_burn, num_chains=num_chains,
+                              seed=seed, device=device, return_state=return_state, verbose=verbose,
+                              chain_offset=chain_offset, n_devices=n_devices, gamma_mode=gamma_mode,
+                              chain_groups=chain_groups, **sched, **hyper)
+    q = Xf.shape[1]
+    res = C.c_void_p()
+    check_fit(L.bnr_fit_kfold(C.byref(p), Xf.ctypes.data_as(_DP), y.ctypes.data_as(_DP), K,
+                              folds.ctypes.data_as(C.POINTER(C.c_int32)), C.byref(res)))
+    try:
+        info = FitInfo()
+        check_fit(L.bnr_fit_get_info(res, C.byref(info)))
+        pw = np.empty(n)
+        check_fit(L.bnr_fit_kfold_pointwise(res, pw.ctypes.data_as(_DP)))
+        rmax = np.empty(K)
+        rx, rg = np.empty(V), np.empty(q)
+        for f in range(K):
+            check_fit(L.bnr_fit_kfold_rhat(res, f, rx.ctypes.data_as(_DP), rg.ctypes.data_as(_DP)))
+            v = np.concatenate([rx, rg])
+            rmax[f] = np.nan if np.isnan(v).any() else v.max()
+        if info.status_or:
+            bits = [k for k, v in STATUS_BITS.items() if info.status_or & v]
+            warnings.warn("chains of the K-fold run raised status bits %s (BNRKFold.status)" % ", ".join(bits),
+                          stacklevel=2)
+        return BNRKFold(pw, folds, y.copy(), int(num_chains) * int(info.sampled), rmax, int(info.burn_in),
+                        int(info.sampled), int(info.status_or))
+    finally:
+        L.bnr_fit_free(res)

@@ -256,8 +256,17 @@ int bnr_ess_stream_finish(bnr_handle* h);
  * Rows never written hold NaN.  The table has its own capacity, so handles without traces can predict too. */
 #define BNR_PRED_MEAN 0
 #define BNR_PRED_PREDICTIVE 1
-/* X_new: m x q column-major; rows: capacity of each chain's prediction table; m = 0 switches predictions off */
+/* X_new: m x q column-major; rows: capacity of each chain's prediction table; m = 0 switches predictions off.
+ * Only BNR_PRED_MEAN and BNR_PRED_PREDICTIVE are accepted here; BNR_PRED_LOGDENS is set by bnr_set_heldout. */
 int bnr_set_predictors(bnr_handle* h, int32_t m, const double* X_new, int64_t rows, int32_t mode);
+/* Held-out rows (K-fold cross-validation): the prediction table of m observations the chains do not train on, whose
+ * responses y_held are known.  Every recorded row then holds, in place of the prediction,
+ *   BNR_PRED_LOGDENS     -1/2 log(2 pi tau2) - (y_held[j] - mu - X_held[j,:] gamma)^2 / (2 tau2)
+ * with the row's own state; no random numbers are drawn.  X_held: m x q column-major, y_held: m.  It replaces any
+ * predictors the handle had (like a second bnr_set_predictors call); m = 0 switches it off.  The table is read with
+ * bnr_get_prediction_trace and bnr_export_predictions. */
+#define BNR_PRED_LOGDENS 2
+int bnr_set_heldout(bnr_handle* h, int32_t m, const double* X_held, const double* y_held, int64_t rows);
 /* rows [first, last) of one local chain, iteration-fastest: out[(r - first) + (last - first) * j] */
 int bnr_get_prediction_trace(bnr_handle* h, int32_t chain, int64_t first, int64_t last, double* out);
 /* rows [first_row, first_row + nrows) of every local chain into caller-owned DEVICE memory as [chain][row][m] */
@@ -284,6 +293,11 @@ int bnr_export_loglik(bnr_handle* h, int64_t first_row, int64_t nrows, double* d
  * BNR_EINVAL.  Deterministic: the same table gives bit-identical results. */
 int bnr_loo_summary(int device, const double* dev_rows, int64_t N, int32_t n, double* elpd_loo, double* p_loo,
                     double* pareto_k, double* elpd_waic, double* p_waic);
+/* Pooled log-mean-exp of N rows of m doubles at a DEVICE pointer (row-major [N][m]): lpd[j] = log((1/N) sum_s
+ * exp(rows[s][j])), a HOST array of m -- the held-out log predictive density of K-fold cross-validation.  The rows are
+ * split over blocks whose partials are added in a fixed order: the same table gives bit-identical results.  No size
+ * limit beyond the device memory of the input. */
+int bnr_lpd_summary(int device, const double* dev_rows, int64_t N, int32_t m, double* lpd);
 
 /* chain groups (independent streams / CUDA graphs) the handle runs */
 int bnr_chain_groups(bnr_handle* h, int32_t* groups);
@@ -381,6 +395,24 @@ int bnr_fit_loo(const bnr_fit_params* p, const double* X, const double* y, int32
  * BNR_ESTATE when the fit ran without bnr_fit_loo or kept fewer than 2 draws */
 int bnr_fit_loo_pointwise(const bnr_fit_result* r, double* elpd_loo, double* p_loo, double* pareto_k,
                           double* elpd_waic, double* p_waic);
+/* K-fold cross-validation (loo::kfold with r_eff = 1): observation i belongs to fold fold[i] in 1..K.  Fold f trains
+ * on the rows with fold != f, in their original order, and holds out the rows with fold == f (bnr_set_heldout).  Every
+ * fold is the fit bnr_fit makes of its training rows with chain_offset = base.chain_offset + f * num_chains (f 0-based)
+ * on device base.device + f mod n_devices, bit for bit; all folds share one control loop, whose PSRF step sees the
+ * maximum R-hat over every fold (NaN if any is NaN), and every fold's sweeps are launched before any is waited for.
+ * Afterwards elpd_kfold[i] = log((1/S) sum_s N(y_i | mu_s + x_i gamma_s, tau2_s)) over the S = num_chains x sampled
+ * retained draws of i's fold.  The held-out tables and export buffers are allocated before the first sweep: a run that
+ * cannot hold them fails at once with BNR_ENOMEM.  Refused with BNR_EINVAL: K < 2, a label outside 1..K, an empty fold
+ * or training set, ext_world > 1, ess_max_lag > 0.  On the result: bnr_fit_get_info gives total_chains = K x
+ * num_chains and the devices used, bnr_fit_handle(r, f, ...) fold f's handle, bnr_fit_rhat the element-wise maximum
+ * over the folds; bnr_fit_summary, bnr_fit_state, bnr_fit_prediction, bnr_fit_ess and bnr_fit_loo_pointwise return
+ * BNR_ESTATE. */
+int bnr_fit_kfold(const bnr_fit_params* p, const double* X, const double* y, int32_t K, const int32_t* fold,
+                  bnr_fit_result** out);
+/* elpd_kfold of every observation [n], in the original order */
+int bnr_fit_kfold_pointwise(const bnr_fit_result* r, double* elpd_kfold);
+/* the last R-hat of fold f (0-based) alone: [V], [q] */
+int bnr_fit_kfold_rhat(const bnr_fit_result* r, int32_t f, double* rhat_xi, double* rhat_gamma);
 /* The control flow of bnr_fit as a pure host function (no GPU): the engine operations a fit would issue when its k-th
  * PSRF evaluation returns psrf_max[k] as the maximum R-hat of both xi and gamma (NaN allowed; 0 beyond n_psrf).
  * ops: [cap_ops][4] = (op, a, b, c) with op  0 create(trace rows, all chains traced, full-state chains)  1 init

@@ -125,4 +125,38 @@ function fit_b200(Xv::Matrix{Float64}, y::Vector{Float64}, R::Integer; η = 1.01
     end
 end
 
+"""
+    kfold_b200(Xv, y, R, folds; K = maximum(folds), the keywords of fit_b200 but X_new / predictive / loo)
+        -> (elpd_kfold::Vector, burn_in, sampled)
+
+K-fold cross-validation with ONE `ccall` of `bnr_fit_kfold`: observation i is held out by fold `folds[i]` in 1..K,
+every fold is the fit of the other rows (`num_chains` chains per fold, fold f on device `device + (f - 1) mod
+n_devices`), all folds advancing together.  `elpd_kfold[i]` is log((1/S) Σ_s N(y_i | μ_s + x_i γ_s, τ²_s)) over the S
+retained draws of all chains of i's fold; `sum(elpd_kfold)` and `sqrt(n * var(elpd_kfold))` are the estimate and
+its standard error.
+"""
+function kfold_b200(Xv::Matrix{Float64}, y::Vector{Float64}, R::Integer, folds::Vector{<:Integer};
+                    K = maximum(folds), η = 1.01, ζ = 1.0, ι = 1.0, aΔ = 1.0, bΔ = 1.0, ν = 10, nburn = 30000,
+                    nsamp = 20000, mingen = 0, maxgen = 0, psrf_cutoff = 1.01, num_chains = 2, seed = 1,
+                    purge_burn = nothing, n_devices = 1, device = 0, verbose = false)
+    n, q = size(Xv)
+    V = Int((-1 + sqrt(1 + 8q)) / 2)
+    base = BnrParams(n, V, R, num_chains, 0, device, 1, 0, 0, UInt64(seed), η, ζ, ι, aΔ, bΔ, Float64(ν), 64, 0, 0, 1)
+    p = Ref(BnrFitParams(base, nburn, nsamp, mingen, maxgen, psrf_cutoff, isnothing(purge_burn) ? 0 : purge_burn,
+                         Int32(0), n_devices, 95, 0, verbose ? 1 : 0, 0, 0, C_NULL, C_NULL))
+    res = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall((:bnr_fit_kfold, libbnr), Cint,
+                (Ref{BnrFitParams}, Ptr{Float64}, Ptr{Float64}, Int32, Ptr{Int32}, Ref{Ptr{Cvoid}}),
+                p, Xv, y, Int32(K), Vector{Int32}(folds), res))
+    try
+        info = Ref{BnrFitInfo}()
+        check(ccall((:bnr_fit_get_info, libbnr), Cint, (Ptr{Cvoid}, Ref{BnrFitInfo}), res[], info))
+        elpd = Vector{Float64}(undef, n)
+        check(ccall((:bnr_fit_kfold_pointwise, libbnr), Cint, (Ptr{Cvoid}, Ptr{Float64}), res[], elpd))
+        return elpd, Int(info[].burn_in), Int(info[].sampled)
+    finally
+        ccall((:bnr_fit_free, libbnr), Cint, (Ptr{Cvoid},), res[])
+    end
+end
+
 end # module

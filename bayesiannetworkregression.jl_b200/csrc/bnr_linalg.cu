@@ -1838,6 +1838,9 @@ __device__ __forceinline__ void gs_roots(double (*sq)[GS_TKP], const double* __r
   }
 }
 
+// max(m, a) that keeps a NaN once it has met one (fmax drops it): a row with a non-finite entry must not slice as finite
+__device__ __forceinline__ double gs_max(double m, double a) { return a > m || a != a ? a : m; }
+
 __device__ __forceinline__ void gs_load_x(double (&x)[16], const double* __restrict__ X, int np, int q, int row, int k0) {
   const bool full = k0 + 16 <= q;
 #pragma unroll
@@ -1876,8 +1879,8 @@ __global__ void __launch_bounds__(GS_THREADS, 2) k_gram_slice(const double* __re
 #pragma unroll
         for (int j = 0; j < 16; j += 2) {
           const double2 s2 = *reinterpret_cast<const double2*>(&sq[cb][gs_tidx(kk + j)]);
-          m[cb] = fmax(m[cb], fabs(x[j] * s2.x));
-          m[cb] = fmax(m[cb], fabs(x[j + 1] * s2.y));
+          m[cb] = gs_max(m[cb], fabs(x[j] * s2.x));
+          m[cb] = gs_max(m[cb], fabs(x[j + 1] * s2.y));
         }
       }
     }
@@ -1885,21 +1888,24 @@ __global__ void __launch_bounds__(GS_THREADS, 2) k_gram_slice(const double* __re
 #pragma unroll
   for (int cb = 0; cb < GS_CB; ++cb) {
     const double o = __shfl_xor_sync(0xffffffffu, m[cb], 16);
-    if (h == 0) red[warp][cb][rr] = fmax(m[cb], o);
+    if (h == 0) red[warp][cb][rr] = gs_max(m[cb], o);
   }
   __syncthreads();
   if (threadIdx.x < GS_CB * GS_ROWS) {
     const int cb = threadIdx.x / GS_ROWS, i = threadIdx.x % GS_ROWS;
     double mx = 0.0;
 #pragma unroll
-    for (int w = 0; w < NW; ++w) mx = fmax(mx, red[w][cb][i]);
-    // 2^p m in [2^53 * 126/64, 2^54) or [2^54, 2^54 * 126/64]: the top digit stays within [-127, 127]
+    for (int w = 0; w < NW; ++w) mx = gs_max(mx, red[w][cb][i]);
+    // 2^p m in [2^53 * 126/64, 2^54) or [2^54, 2^54 * 126/64]: the top digit stays within [-127, 127].  A row with a
+    // NaN or infinite entry (a NaN, infinite or negative S_k, a non-finite X) gets the scale NaN: its row and column of
+    // G are NaN and the factorisation flags the chain, as the FP64 SYRK's G would (its digits are never used).
+    const bool finite = mx <= 0x1.fffffffffffffp1023;
     int p = 0;
-    if (mx > 0.0) {
+    if (finite && mx > 0.0) {
       p = 54 - ilogb(mx);
       if (ldexp(mx, p) > 126.0 * 0x1p48) --p;
     }
-    if (cb < ncb) rscale[(size_t)(c0 + cb) * np + r0 + i] = ldexp(1.0, -p);
+    if (cb < ncb) rscale[(size_t)(c0 + cb) * np + r0 + i] = finite ? ldexp(1.0, -p) : __longlong_as_double(0x7ff8000000000000ll);
     const int p1 = p > 1000 ? 1000 : p;
     scl[cb][i] = make_double2(ldexp(1.0, p1), ldexp(1.0, p - p1));
   }

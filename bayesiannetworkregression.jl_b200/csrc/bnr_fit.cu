@@ -3,14 +3,17 @@
 // (822-864) and return_psrf_VOI (771-789), plus the statistics Summary needs (1214-1250).
 //
 // The control flow is host code written against a small operations interface (Ops), implemented twice:
-//   * DeviceOps  drives one libbnr handle per GPU through the public entry points of include/bnr.h (chains are sharded
-//                over n_devices GPUs of this process; the split-half moments -- and the ESS statistics -- are exchanged
-//                with ncclAllGather, then optionally across processes through a caller-supplied all-gather);
+//   * DeviceOps  drives a flat list of libbnr handles through the public entry points of include/bnr.h.  The handles
+//                are grouped into folds, a fold being the handles whose chains pool their statistics: bnr_fit shards
+//                its chains over one fold of n_devices GPUs of this process (the split-half moments -- and the ESS
+//                statistics -- are exchanged with ncclAllGather, then optionally across processes through a
+//                caller-supplied all-gather); bnr_fit_kfold makes K folds of one handle each;
 //   * PlanOps    records the operations and takes the PSRF maxima from the caller: bnr_fit_plan, a pure host function
 //                that lets the control flow be tested without a GPU against the restated reference loops
 //                (oracle/psrf_loops.py).
 // Row / sweep conventions: table rows are 0-based here (the reference's row r is row r - 1), sweep s = 1, 2, ... is the
 // s-th Gibbs sweep of a chain, row 0 holds the prior draw (sweep 0).
+#include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -274,8 +277,8 @@ constexpr int NCCL_DOUBLE = 8;     // ncclFloat64
 // ------------------------------------------------------------------------------------------------------------------
 struct bnr_fit_result {
   bnr_fit_params p;
-  std::vector<bnr_handle*> h;          // one handle per device; h[0] holds chain 1
-  std::vector<int> dev;
+  std::vector<bnr_handle*> h;          // the handles of every fold, fold by fold; h[0] holds chain 1
+  std::vector<int> dev;                // the device of each handle
   std::vector<cudaStream_t> xs;        // exchange streams
   std::vector<void*> comms;            // NCCL communicators (empty: single device or peer-copy exchange)
   std::vector<double*> gbuf;           // per device: gathered buffer
@@ -284,32 +287,35 @@ struct bnr_fit_result {
   size_t xbuf_doubles = 0;
   int V = 0, q = 0, C = 0;
   Outcome out;
+  // the handles whose chains pool their statistics: an ordinary fit is one fold over all its handles that holds
+  // nothing out; bnr_fit_kfold makes one fold of one handle per held-out set
+  struct Fold {
+    int first = 0, handles = 1;        // its handles h[first .. first + handles)
+    std::vector<int> held;             // the observations it holds out, in original order
+    std::vector<double> rhat_xi, rhat_gamma;   // the R-hat of the last PSRF step over its chains
+  };
+  std::vector<Fold> folds;
+  // rhat_*: the element-wise maximum over the folds (NaN wins)
   std::vector<double> rhat_xi, rhat_gamma, s_mean, s_lo, s_hi, s_xi, ess_xi, ess_gamma;
   bool summary_ok = false, ess_ok = false;
-  // a per-row table pooled over all chains after the fit (width 0: not requested)
+  // a per-row table pooled over the chains of each fold after the fit
   struct Pooled {
     const char* what;
-    int width = 0;
-    std::vector<double*> exp;          // per device: the retained rows of its chains, [chain][row][width]
+    std::vector<int> width;            // per handle: doubles per row (empty: not requested)
+    std::vector<double*> exp;          // per handle: the retained rows of its chains, [chain][row][width]
     bool ok = false;                   // its summary was computed
   };
   Pooled pred = {"predictions"};       // predictions for new networks (bnr_fit_predict), width m
   Pooled ll = {"log-likelihood"};      // pointwise log-likelihood for PSIS-LOO / WAIC (bnr_fit_loo), width n
-  Pooled held = {"held-out log densities"};   // K-fold (bnr_fit_kfold): exp[f] holds fold f's retained rows
-  // K-fold cross-validation (K == 0: an ordinary fit).  h[f], dev[f] are fold f's handle and device
-  struct KFold {
-    int K = 0, n_devices = 0;
-    std::vector<std::vector<int>> held;                   // per fold: its held-out observations, in original order
-    std::vector<std::vector<double>> rhat_xi, rhat_gamma; // per fold: the R-hat of the last PSRF step
-    std::vector<double> elpd;                             // [n] elpd_kfold in original order
-    bool ok = false;
-  } kf;
+  Pooled held = {"held-out log densities"};   // K-fold (bnr_fit_kfold): as wide as the fold holds out
+  std::vector<double> elpd;            // K-fold: [n] elpd_kfold in original order
+  bool kfold() const { return !held.width.empty(); }
   int pmode = 0;
   std::vector<double> p_mean, p_lo, p_hi;
   std::vector<double> l_pw[5];         // elpd_loo, p_loo, pareto_k, elpd_waic, p_waic per observation
   int gamma_mode = 0;
   int status_or = 0;
-  const char* exchange = "none";
+  int exchange = 0;                    // bnr_fit_info.exchange
   ~bnr_fit_result() {
     for (size_t d = 0; d < h.size(); ++d) {
       if (d < dev.size()) cudaSetDevice(dev[d]);
@@ -346,136 +352,182 @@ double jmax(const std::vector<double>& v) {
   return m;
 }
 
+// one handle of a fit: the rows it trains on and, in K-fold cross-validation, the rows its fold holds out
+struct Entry {
+  int fold = 0, n = 0;
+  const double* X = nullptr; const double* y = nullptr;   // training rows: the caller's X and y, or Xt and yt
+  std::vector<double> Xt, yt, Xh, yh;                     // K-fold: the fold's rows, freed once its handle holds them
+};
+
+// a refused cudaMalloc of one of the buffers of a pooled table
+int refuse(const char* buf, const char* what, size_t doubles) {
+  cudaGetLastError();
+  return ffail(BNR_ENOMEM, std::string("cannot allocate the ") + buf + " of the " + what + " (" +
+                               std::to_string(doubles * sizeof(double)) + " bytes)");
+}
+
 struct DeviceOps : Ops {
+  using Fold = bnr_fit_result::Fold;
+  using Pooled = bnr_fit_result::Pooled;
   bnr_fit_result& R;
-  const double* X; const double* y;
+  std::vector<Entry> E;                // one per handle of R.h
   const double* X_new;
   PhaseClock clk;
-  explicit DeviceOps(bnr_fit_result& r, const double* X_, const double* y_, const double* X_new_)
-      : R(r), X(X_), y(y_), X_new(X_new_) {}
-  int total_chains() const { return R.C * (int)R.h.size() * (R.p.ext_world > 1 ? R.p.ext_world : 1); }
+  explicit DeviceOps(bnr_fit_result& r, const double* X_new_) : R(r), X_new(X_new_) {}
+  int chains(const Fold& f) const { return R.C * f.handles * (R.p.ext_world > 1 ? R.p.ext_world : 1); }
+  // the chains of some fold meet in gathers: it spans several handles (only an ordinary fit's one fold can), or the
+  // fit spans several processes
+  bool gathers() const { return R.h.size() > R.folds.size() || R.p.ext_world > 1; }
 
   int create(long long rows, bool gx_all, int full) override {
     PhaseClock::Scope sc(clk, PH_CREATE);
-    const int nd = R.p.n_devices > 0 ? R.p.n_devices : 1;
-    R.h.assign(nd, nullptr); R.dev.assign(nd, 0); R.xs.assign(nd, nullptr); R.gbuf.assign(nd, nullptr);
+    const int H = (int)E.size(), nd = R.p.n_devices > 0 ? R.p.n_devices : 1;
+    R.h.assign(H, nullptr); R.dev.assign(H, 0); R.xs.assign(H, nullptr); R.gbuf.assign(H, nullptr);
+    for (Pooled* t : {&R.pred, &R.ll, &R.held}) t->exp.assign(t->width.size(), nullptr);
+    R.V = R.p.base.V; R.q = R.V * (R.V + 1) / 2; R.C = R.p.base.num_chains;
     const int rank = R.p.ext_world > 1 ? R.p.ext_rank : 0;
-    for (int d = 0; d < nd; ++d) {
+    for (int i = 0; i < H; ++i) {
+      Entry& e = E[i];
       bnr_params bp = R.p.base;
-      bp.device = R.p.base.device + d;
-      bp.chain_offset = R.p.base.chain_offset + (rank * nd + d) * bp.num_chains;
+      bp.n = e.n;
+      bp.device = R.p.base.device + i % nd;
+      bp.chain_offset = R.p.base.chain_offset + (rank * H + i) * bp.num_chains;
       bp.trace_rows = rows;
       bp.trace_gamma_xi_all = gx_all ? 1 : 0;
-      // chain 1 (first local chain of the first device of rank 0 ... every rank keeps its own first chain) is the one
-      // Results / Summary read; the other devices need traces only when R-hat is taken from trace rows
-      bp.trace_full_chains = d == 0 ? full : 0;
-      bp.trace_gamma_xi_chains = d == 0 ? 1 : 0;
-      if (d > 0 && !gx_all) bp.trace_rows = 0;
-      R.dev[d] = bp.device;
-      BN(bnr_create(&bp, X, y, &R.h[d]));
+      // a fold's chain 1 (first local chain of its first handle on rank 0 ... every rank keeps its own first chain) is
+      // the one Results / Summary read; its other handles need traces only when R-hat is taken from trace rows
+      const bool first = i == R.folds[e.fold].first;
+      bp.trace_full_chains = first ? full : 0;
+      bp.trace_gamma_xi_chains = first ? 1 : 0;
+      if (!first && !gx_all) bp.trace_rows = 0;
+      R.dev[i] = bp.device;
+      BN(bnr_create(&bp, e.X, e.y, &R.h[i]));
+      for (std::vector<double>* v : {&e.Xt, &e.yt}) std::vector<double>().swap(*v);
+      // its tables before the next handle: creating every handle first made the create phase of a K-fold run with
+      // all folds on one device 10 - 20 % slower (B200, 1000 W power limit)
+      if (int r = create_tables(i, rows)) return r;
     }
-    R.V = R.p.base.V; R.q = R.V * (R.V + 1) / 2; R.C = R.p.base.num_chains;
     int32_t gm = 0;
     BN(bnr_gamma_mode(R.h[0], &gm));
     R.gamma_mode = gm;
-    if (nd > 1 || R.p.ext_world > 1) {
-      for (int d = 0; d < nd; ++d) {
-        CKF(cudaSetDevice(R.dev[d]));
-        CKF(cudaStreamCreateWithFlags(&R.xs[d], cudaStreamNonBlocking));
+    if (gathers()) {
+      for (int i = 0; i < H; ++i) {
+        CKF(cudaSetDevice(R.dev[i]));
+        CKF(cudaStreamCreateWithFlags(&R.xs[i], cudaStreamNonBlocking));
       }
-      if (nd > 1 && nccl().ok) {
-        R.comms.assign(nd, nullptr);
-        const int rc = nccl().CommInitAll(R.comms.data(), nd, R.dev.data());
+      if (H > 1 && nccl().ok) {
+        R.comms.assign(H, nullptr);
+        const int rc = nccl().CommInitAll(R.comms.data(), H, R.dev.data());
         if (rc != 0) {
           R.comms.clear();
           return ffail(BNR_ECUDA, std::string("ncclCommInitAll: ") + (nccl().GetErrorString ? nccl().GetErrorString(rc) : "error"));
         }
-        R.exchange = "nccl";
-      } else if (nd > 1) {
-        R.exchange = "peer-copy";
+        R.exchange = 1;                                 // NCCL
+      } else if (H > 1) {
+        R.exchange = 2;                                 // peer copies
       }
     }
-    if (R.pred.width > 0 || R.ll.width > 0) return create_tables(rows);
+    return create_pooled(rows);
+  }
+
+  // handle i's prediction, log-likelihood and held-out tables of `rows` rows and their export buffers.  With the
+  // pooled buffers of create_pooled they are all allocated before the first sweep: a fit that cannot hold them fails
+  // here, not after the sampling
+  int create_tables(int i, long long rows) {
+    if (!R.pred.width.empty()) BN(bnr_set_predictors(R.h[i], R.pred.width[i], X_new, rows, R.pmode));
+    if (!R.ll.width.empty()) BN(bnr_set_loglik(R.h[i], rows));
+    if (R.kfold()) {
+      Entry& e = E[i];
+      BN(bnr_set_heldout(R.h[i], R.held.width[i], e.Xh.data(), e.yh.data(), rows));
+      for (std::vector<double>* v : {&e.Xh, &e.yh}) std::vector<double>().swap(*v);
+    }
+    for (Pooled* t : {&R.pred, &R.ll, &R.held}) {
+      if (t->width.empty()) continue;
+      const size_t local = (size_t)R.C * rows * t->width[i];
+      CKF(cudaSetDevice(R.dev[i]));
+      if (cudaMalloc((void**)&t->exp[i], local * sizeof(double)) != cudaSuccess) {
+        t->exp[i] = nullptr;
+        return refuse("export buffer", t->what, local);
+      }
+    }
     return 0;
   }
 
-  // prediction and log-likelihood tables of `rows` rows on every handle, their export buffers and the pooled buffers
-  // of the all-gather (sized for the wider of the two), all before the first sweep: a fit that cannot hold them fails
-  // here, not after the sampling
-  int create_tables(long long rows) {
-    const int nd = (int)R.h.size(), world = R.p.ext_world > 1 ? R.p.ext_world : 1;
-    auto refuse = [](const char* buf, const char* what, size_t doubles) {
-      cudaGetLastError();
-      return ffail(BNR_ENOMEM, std::string("cannot allocate the ") + buf + " of the " + what + " (" +
-                                   std::to_string(doubles * sizeof(double)) + " bytes)");
-    };
-    if (R.pred.width > 0) for (auto* h : R.h) BN(bnr_set_predictors(h, R.pred.width, X_new, rows, R.pmode));
-    if (R.ll.width > 0) for (auto* h : R.h) BN(bnr_set_loglik(h, rows));
+  // the pooled buffers of the all-gather, sized for the widest table
+  int create_pooled(long long rows) {
+    const int H = (int)R.h.size(), world = R.p.ext_world > 1 ? R.p.ext_world : 1;
     int width = 0;
-    for (bnr_fit_result::Pooled* t : {&R.pred, &R.ll}) {
-      if (t->width == 0) continue;
-      const size_t local = (size_t)R.C * rows * t->width;
-      t->exp.assign(nd, nullptr);
-      for (int d = 0; d < nd; ++d) {
-        CKF(cudaSetDevice(R.dev[d]));
-        if (cudaMalloc((void**)&t->exp[d], local * sizeof(double)) != cudaSuccess) {
-          t->exp[d] = nullptr;
-          return refuse("export buffer", t->what, local);
-        }
-      }
-      if (t->width > width) width = t->width;
+    const char* what = nullptr;
+    for (Pooled* t : {&R.pred, &R.ll, &R.held}) {
+      if (t->width.empty()) continue;
+      width = std::max(width, *std::max_element(t->width.begin(), t->width.end()));
+      what = t->what;
     }
     const size_t local = (size_t)R.C * rows * width;
-    const char* what = (R.ll.width > 0 ? R.ll : R.pred).what;
-    if (nd > 1 || world > 1) {
+    if (width > 0 && gathers()) {
       // gather_local / gather_ext reuse these buffers (they only grow)
-      for (int d = 0; d < nd; ++d) {
-        CKF(cudaSetDevice(R.dev[d]));
-        if (R.gbuf[d]) CKF(cudaFree(R.gbuf[d]));
-        R.gbuf[d] = nullptr;
-        if (cudaMalloc((void**)&R.gbuf[d], local * nd * sizeof(double)) != cudaSuccess) {
-          R.gbuf[d] = nullptr; R.gbuf_doubles = 0;
-          return refuse("pooled buffer", what, local * nd);
+      for (int i = 0; i < H; ++i) {
+        CKF(cudaSetDevice(R.dev[i]));
+        if (R.gbuf[i]) CKF(cudaFree(R.gbuf[i]));
+        R.gbuf[i] = nullptr;
+        if (cudaMalloc((void**)&R.gbuf[i], local * H * sizeof(double)) != cudaSuccess) {
+          R.gbuf[i] = nullptr; R.gbuf_doubles = 0;
+          return refuse("pooled buffer", what, local * H);
         }
       }
-      R.gbuf_doubles = local * nd;
+      R.gbuf_doubles = local * H;
       if (world > 1) {
         CKF(cudaSetDevice(R.dev[0]));
-        if (cudaMalloc((void**)&R.xbuf, local * nd * world * sizeof(double)) != cudaSuccess) {
+        if (cudaMalloc((void**)&R.xbuf, local * H * world * sizeof(double)) != cudaSuccess) {
           R.xbuf = nullptr;
-          return refuse("pooled buffer", what, local * nd * world);
+          return refuse("pooled buffer", what, local * H * world);
         }
-        R.xbuf_doubles = local * nd * world;
+        R.xbuf_doubles = local * H * world;
       }
     }
     return 0;
   }
 
-  // the retained rows of every chain of a pooled table in global-chain order on device 0 (*all), each device's exported
-  // through export_rows
-  int pool(const Outcome& o, const bnr_fit_result::Pooled& t, int (*export_rows)(bnr_handle*, int64_t, int64_t, double*),
+  // the retained rows of every chain of fold f in a pooled table, in global-chain order on the fold's first device
+  // (*all), each handle's exported through export_rows
+  int pool(const Outcome& o, const Fold& f, const Pooled& t, int (*export_rows)(bnr_handle*, int64_t, int64_t, double*),
            const double** all) {
-    const int nd = (int)R.h.size();
-    for (int d = 0; d < nd; ++d) BN(export_rows(R.h[d], o.burn_in, o.sampled, t.exp[d]));
-    *all = t.exp[0];
-    if (nd > 1 || R.p.ext_world > 1) {
-      const size_t cnt = (size_t)R.C * o.sampled * t.width;
-      std::vector<const double*> src(t.exp.begin(), t.exp.end());
+    for (int i = f.first; i < f.first + f.handles; ++i) BN(export_rows(R.h[i], o.burn_in, o.sampled, t.exp[i]));
+    *all = t.exp[f.first];
+    if (f.handles > 1 || R.p.ext_world > 1) {
+      const size_t cnt = (size_t)R.C * o.sampled * t.width[f.first];
+      std::vector<const double*> src(t.exp.begin() + f.first, t.exp.begin() + f.first + f.handles);
       if (int r = gather_local(src, cnt)) return r;
-      if (int r = gather_ext(cnt * nd, all)) return r;
+      if (int r = gather_ext(cnt * f.handles, all)) return r;
     }
+    return 0;
+  }
+
+  // Summary statistics of chain 1 on the device (src/gibbs.jl:1221-1236: lw / hi with Julia's round)
+  int summary(const Outcome& o) {
+    PhaseClock::Scope sc(clk, PH_SUMMARY);
+    const long long nsamp = o.sampled;
+    const double lower = (100 - (R.p.interval > 0 ? R.p.interval : 95)) / 200.0;
+    const long long lw = jround(nsamp * lower), hi = jround(nsamp * (1.0 - lower));
+    if (lw < 1 || hi > nsamp) return 0;
+    R.s_mean.assign(R.q, 0); R.s_lo.assign(R.q, 0); R.s_hi.assign(R.q, 0); R.s_xi.assign(R.V, 0);
+    if (bnr_summary(R.h[0], 0, o.burn_in, nsamp, lw, hi, R.s_mean.data(), R.s_lo.data(), R.s_hi.data(),
+                    R.s_xi.data()) != BNR_OK)
+      return ffail(BNR_ECUDA, std::string("bnr_summary: ") + bnr_last_error());
+    R.summary_ok = true;
     return 0;
   }
 
   // pooled mean and order statistics of the predictions
   int predictions(const Outcome& o) {
-    const long long N = (long long)total_chains() * o.sampled;
+    const Fold& f = R.folds[0];
+    const long long N = (long long)chains(f) * o.sampled;
     const double lower = (100 - (R.p.interval > 0 ? R.p.interval : 95)) / 200.0;
     const long long lw = jround(N * lower), hi = jround(N * (1.0 - lower));
     if (o.sampled < 1 || lw < 1 || hi > N) return 0;
     const double* all = nullptr;
-    if (int r = pool(o, R.pred, bnr_export_predictions, &all)) return r;
-    const int m = R.pred.width;
+    if (int r = pool(o, f, R.pred, bnr_export_predictions, &all)) return r;
+    const int m = R.pred.width[0];
     R.p_mean.assign(m, 0); R.p_lo.assign(m, 0); R.p_hi.assign(m, 0);
     BN(bnr_prediction_summary(R.dev[0], all, N, m, lw, hi, R.p_mean.data(), R.p_lo.data(), R.p_hi.data()));
     R.pred.ok = true;
@@ -484,15 +536,32 @@ struct DeviceOps : Ops {
 
   // pooled PSIS-LOO and WAIC of the log-likelihood
   int loo(const Outcome& o) {
-    const long long N = (long long)total_chains() * o.sampled;
+    const Fold& f = R.folds[0];
+    const long long N = (long long)chains(f) * o.sampled;
     if (N < 2) return 0;
     const double* all = nullptr;
-    if (int r = pool(o, R.ll, bnr_export_loglik, &all)) return r;
-    const int n = R.ll.width;
+    if (int r = pool(o, f, R.ll, bnr_export_loglik, &all)) return r;
+    const int n = R.ll.width[0];
     for (auto& v : R.l_pw) v.assign(n, 0);
     BN(bnr_loo_summary(R.dev[0], all, N, n, R.l_pw[0].data(), R.l_pw[1].data(), R.l_pw[2].data(), R.l_pw[3].data(),
                        R.l_pw[4].data()));
     R.ll.ok = true;
+    return 0;
+  }
+
+  // elpd_kfold of every held-out observation: the log-mean-exp of its fold's retained rows of all chains
+  int heldout(const Outcome& o) {
+    R.elpd.assign(R.p.base.n, NAN);
+    for (const Fold& f : R.folds) {
+      const long long N = (long long)chains(f) * o.sampled;
+      if (N < 1) return 0;
+      const double* all = nullptr;
+      if (int r = pool(o, f, R.held, bnr_export_predictions, &all)) return r;
+      std::vector<double> lpd(f.held.size());
+      BN(bnr_lpd_summary(R.dev[f.first], all, N, (int32_t)lpd.size(), lpd.data()));
+      for (size_t j = 0; j < lpd.size(); ++j) R.elpd[f.held[j]] = lpd[j];
+    }
+    R.held.ok = true;
     return 0;
   }
   int init() override { PhaseClock::Scope sc(clk, PH_INIT); for (auto* h : R.h) BN(bnr_init_state(h)); return 0; }
@@ -527,8 +596,8 @@ struct DeviceOps : Ops {
     R.gbuf_doubles = doubles;
     return 0;
   }
-  // every device contributes src[d] (cnt doubles, device memory); afterwards gbuf[0] holds [n_devices][cnt] in device
-  // order (with NCCL every device holds it)
+  // every handle contributes src[d] (cnt doubles, device memory); afterwards gbuf[0] holds [handles][cnt] in handle
+  // order (with NCCL every device holds it).  A fold that gathers spans every handle: see gathers()
   int gather_local(const std::vector<const double*>& src, size_t cnt) {
     const int nd = (int)R.h.size();
     if (int r = ensure_gbuf(cnt * nd)) return r;
@@ -569,8 +638,8 @@ struct DeviceOps : Ops {
   int psrf(int mode, long long a, long long b, double* mx, double* mg) override {
     PhaseClock::Scope sc(clk, PH_PSRF);
     R.rhat_xi.assign(R.V, NAN); R.rhat_gamma.assign(R.q, NAN);
-    const long long len = mode == 2 ? 0 : b;
-    if (mode != 2 && len / 2 < 2) { *mx = NAN; *mg = NAN; return 0; }
+    for (Fold& f : R.folds) { f.rhat_xi.assign(R.V, NAN); f.rhat_gamma.assign(R.q, NAN); }
+    if (mode != 2 && b / 2 < 2) { *mx = NAN; *mg = NAN; return 0; }
     for (auto* h : R.h) {
       if (mode == 0) BN(bnr_moments_from_trace(h, a, b));
       if (mode == 2) BN(bnr_moments_from_blocks(h, (int32_t)a, (int32_t)b));
@@ -578,20 +647,31 @@ struct DeviceOps : Ops {
     int64_t half = 0;
     BN(bnr_moment_half_len(R.h[0], &half));
     if (half < 2) { *mx = NAN; *mg = NAN; return 0; }
-    if (R.h.size() == 1 && R.p.ext_world <= 1) {
-      BN(bnr_rhat(R.h[0], R.rhat_xi.data(), R.rhat_gamma.data()));
-    } else {
-      std::vector<const double*> src(R.h.size());
-      int64_t cnt = 0;
-      for (size_t d = 0; d < R.h.size(); ++d) {
-        double* ptr = nullptr;
-        BN(bnr_moments_device(R.h[d], &ptr, &cnt));
-        src[d] = ptr;
+    // element-wise maximum over the folds; NaN wins, so that jmax of it is jmax over all folds' values
+    auto fold_max = [](std::vector<double>& acc, const std::vector<double>& v, bool first) {
+      for (size_t i = 0; i < v.size(); ++i)
+        if (first || std::isnan(v[i]) || (!std::isnan(acc[i]) && v[i] > acc[i])) acc[i] = v[i];
+    };
+    for (size_t k = 0; k < R.folds.size(); ++k) {
+      Fold& f = R.folds[k];
+      if (f.handles == 1 && R.p.ext_world <= 1) {
+        BN(bnr_rhat(R.h[f.first], f.rhat_xi.data(), f.rhat_gamma.data()));
+      } else {
+        std::vector<const double*> src(f.handles);
+        int64_t cnt = 0;
+        for (int d = 0; d < f.handles; ++d) {
+          double* ptr = nullptr;
+          BN(bnr_moments_device(R.h[f.first + d], &ptr, &cnt));
+          src[d] = ptr;
+        }
+        if (int r = gather_local(src, (size_t)cnt)) return r;
+        const double* all = nullptr;
+        if (int r = gather_ext((size_t)cnt * f.handles, &all)) return r;
+        BN(bnr_rhat_from_moments(R.dev[f.first], all, chains(f), R.V, R.q, half, f.rhat_xi.data(),
+                                 f.rhat_gamma.data()));
       }
-      if (int r = gather_local(src, (size_t)cnt)) return r;
-      const double* all = nullptr;
-      if (int r = gather_ext((size_t)cnt * R.h.size(), &all)) return r;
-      BN(bnr_rhat_from_moments(R.dev[0], all, total_chains(), R.V, R.q, half, R.rhat_xi.data(), R.rhat_gamma.data()));
+      fold_max(R.rhat_xi, f.rhat_xi, k == 0);
+      fold_max(R.rhat_gamma, f.rhat_gamma, k == 0);
     }
     *mx = jmax(R.rhat_xi); *mg = jmax(R.rhat_gamma);
     return 0;
@@ -635,7 +715,7 @@ struct DeviceOps : Ops {
       int rc = gather_local(sm, (size_t)nm);
       const double* all_m = nullptr;
       if (!rc) rc = gather_ext((size_t)nm * R.h.size(), &all_m);
-      if (!rc && bnr_ess_from_stats(R.dev[0], keep, parts, all_m, total_chains(), R.V, R.q, o.sampled, lag,
+      if (!rc && bnr_ess_from_stats(R.dev[0], keep, parts, all_m, chains(R.folds[0]), R.V, R.q, o.sampled, lag,
                                     R.ess_xi.data(), R.ess_gamma.data()) != BNR_OK)
         rc = ffail(BNR_ECUDA, std::string("bnr_ess_from_stats: ") + bnr_last_error());
       cudaSetDevice(R.dev[0]);
@@ -643,96 +723,6 @@ struct DeviceOps : Ops {
       if (rc) return rc;
     }
     R.ess_ok = true;
-    return 0;
-  }
-};
-
-// K-fold cross-validation: one handle per fold (fold f on device base.device + f mod n_devices), every broadcast
-// operation of DeviceOps applied to all of them, R-hat taken per fold and the maximum handed to the control loop
-struct KFoldOps : DeviceOps {
-  struct Fold { std::vector<double> X, y, Xh, yh; int n = 0, m = 0; };
-  std::vector<Fold> folds;
-  explicit KFoldOps(bnr_fit_result& r) : DeviceOps(r, nullptr, nullptr, nullptr) {}
-
-  int create(long long rows, bool gx_all, int full) override {
-    PhaseClock::Scope sc(clk, PH_CREATE);
-    const int K = R.kf.K, nd = R.p.n_devices > 0 ? R.p.n_devices : 1;
-    R.kf.n_devices = K < nd ? K : nd;
-    R.h.assign(K, nullptr); R.dev.assign(K, 0); R.xs.assign(K, nullptr); R.gbuf.assign(K, nullptr);
-    R.held.exp.assign(K, nullptr);
-    R.V = R.p.base.V; R.q = R.V * (R.V + 1) / 2; R.C = R.p.base.num_chains;
-    for (int f = 0; f < K; ++f) {
-      Fold& fd = folds[f];
-      // the device-0 handle bnr_fit creates for these training rows, at this fold's chain offset
-      bnr_params bp = R.p.base;
-      bp.n = fd.n;
-      bp.device = R.p.base.device + f % nd;
-      bp.chain_offset = R.p.base.chain_offset + f * bp.num_chains;
-      bp.trace_rows = rows;
-      bp.trace_gamma_xi_all = gx_all ? 1 : 0;
-      bp.trace_full_chains = full;
-      bp.trace_gamma_xi_chains = 1;
-      R.dev[f] = bp.device;
-      BN(bnr_create(&bp, fd.X.data(), fd.y.data(), &R.h[f]));
-      BN(bnr_set_heldout(R.h[f], fd.m, fd.Xh.data(), fd.yh.data(), rows));
-      // the handle holds its own copies now
-      for (std::vector<double>* v : {&fd.X, &fd.y, &fd.Xh, &fd.yh}) std::vector<double>().swap(*v);
-      const size_t local = (size_t)R.C * rows * fd.m;
-      CKF(cudaSetDevice(R.dev[f]));
-      if (cudaMalloc((void**)&R.held.exp[f], local * sizeof(double)) != cudaSuccess) {
-        R.held.exp[f] = nullptr;
-        cudaGetLastError();
-        return ffail(BNR_ENOMEM, "cannot allocate the export buffer of fold " + std::to_string(f + 1) +
-                                     "'s held-out log densities (" + std::to_string(local * sizeof(double)) + " bytes)");
-      }
-    }
-    int32_t gm = 0;
-    BN(bnr_gamma_mode(R.h[0], &gm));
-    R.gamma_mode = gm;
-    return 0;
-  }
-
-  int psrf(int mode, long long a, long long b, double* mx, double* mg) override {
-    PhaseClock::Scope sc(clk, PH_PSRF);
-    const int K = R.kf.K;
-    R.rhat_xi.assign(R.V, NAN); R.rhat_gamma.assign(R.q, NAN);
-    R.kf.rhat_xi.assign(K, std::vector<double>(R.V, NAN));
-    R.kf.rhat_gamma.assign(K, std::vector<double>(R.q, NAN));
-    if (mode != 2 && b / 2 < 2) { *mx = NAN; *mg = NAN; return 0; }
-    for (auto* h : R.h) {
-      if (mode == 0) BN(bnr_moments_from_trace(h, a, b));
-      if (mode == 2) BN(bnr_moments_from_blocks(h, (int32_t)a, (int32_t)b));
-    }
-    int64_t half = 0;
-    BN(bnr_moment_half_len(R.h[0], &half));
-    if (half < 2) { *mx = NAN; *mg = NAN; return 0; }
-    // element-wise maximum over the folds; NaN wins, so that jmax of it is jmax over all folds' values
-    auto fold_max = [](std::vector<double>& acc, const std::vector<double>& v, bool first) {
-      for (size_t i = 0; i < v.size(); ++i)
-        if (first || std::isnan(v[i]) || (!std::isnan(acc[i]) && v[i] > acc[i])) acc[i] = v[i];
-    };
-    for (int f = 0; f < K; ++f) {
-      BN(bnr_rhat(R.h[f], R.kf.rhat_xi[f].data(), R.kf.rhat_gamma[f].data()));
-      fold_max(R.rhat_xi, R.kf.rhat_xi[f], f == 0);
-      fold_max(R.rhat_gamma, R.kf.rhat_gamma[f], f == 0);
-    }
-    *mx = jmax(R.rhat_xi); *mg = jmax(R.rhat_gamma);
-    return 0;
-  }
-
-  // elpd_kfold of every held-out observation: the log-mean-exp of its fold's retained rows of all chains
-  int pool(const Outcome& o) {
-    const long long N = (long long)R.C * o.sampled;
-    if (N < 1) return 0;
-    R.kf.elpd.assign(R.p.base.n, NAN);
-    for (int f = 0; f < R.kf.K; ++f) {
-      const Fold& fd = folds[f];
-      BN(bnr_export_predictions(R.h[f], o.burn_in, o.sampled, R.held.exp[f]));
-      std::vector<double> lpd(fd.m);
-      BN(bnr_lpd_summary(R.dev[f], R.held.exp[f], N, fd.m, lpd.data()));
-      for (int j = 0; j < fd.m; ++j) R.kf.elpd[R.kf.held[f][j]] = lpd[j];
-    }
-    R.kf.ok = true;
     return 0;
   }
 };
@@ -782,78 +772,10 @@ extern "C" int bnr_fit_plan(const bnr_fit_params* p, const double* psrf_max, int
   return BNR_OK;
 }
 
-// bnr_fit, bnr_fit_predict (m > 0: predictions for the m rows of X_new) and bnr_fit_loo (loo: PSIS-LOO and WAIC)
-static int fit_body(const bnr_fit_params* p, const double* X, const double* y, int32_t m, const double* X_new,
-                    int32_t mode, bool loo, bnr_fit_result** res_out) {
-  if (m < 0) return ffail(BNR_EINVAL, "m must be >= 0");
-  if (m > 0 && !X_new) return ffail(BNR_EINVAL, "null X_new");
-  if (mode != BNR_PRED_MEAN && mode != BNR_PRED_PREDICTIVE) return ffail(BNR_EINVAL, "unknown prediction mode");
-  if (int r = check_params(p)) return r;
-  if (!X || !y || !res_out) return ffail(BNR_EINVAL, "null argument");
-  if (p->base.nu < p->base.R)
-    // the reference builds this ArgumentError without throwing it (src/gibbs.jl:901-902); the InverseWishart draw is
-    // undefined for nu <= R - 1, so the engine refuses
-    return ffail(BNR_EINVAL, "nu must not be smaller than R");
-  bnr_fit_result* R = new bnr_fit_result();
-  R->p = *p;
-  R->pred.width = m; R->pmode = mode; R->ll.width = loo ? p->base.n : 0;
-  DeviceOps o(*R, X, y, X_new);
-  const double t_start = PhaseClock::now();
-  int rc = fit_loops(o, *p, R->out);
-  if (!rc) {
-    PhaseClock::Scope sc(o.clk, PH_SUMMARY);
-    // Summary statistics of chain 1 on the device (src/gibbs.jl:1221-1236: lw / hi with Julia's round)
-    const long long nsamp = R->out.sampled;
-    const double lower = (100 - (p->interval > 0 ? p->interval : 95)) / 200.0;
-    const long long lw = jround(nsamp * lower), hi = jround(nsamp * (1.0 - lower));
-    if (lw >= 1 && hi <= nsamp) {
-      R->s_mean.assign(R->q, 0); R->s_lo.assign(R->q, 0); R->s_hi.assign(R->q, 0); R->s_xi.assign(R->V, 0);
-      if (bnr_summary(R->h[0], 0, R->out.burn_in, nsamp, lw, hi, R->s_mean.data(), R->s_lo.data(), R->s_hi.data(),
-                      R->s_xi.data()) == BNR_OK) R->summary_ok = true;
-      else rc = ffail(BNR_ECUDA, std::string("bnr_summary: ") + bnr_last_error());
-    }
-  }
-  if (!rc && m > 0) rc = o.predictions(R->out);
-  if (!rc && loo) rc = o.loo(R->out);
-  if (!rc) rc = o.ess(R->out);
-  if (!rc) {
-    std::vector<int32_t> st(R->C);
-    for (auto* h : R->h) {
-      if (bnr_status(h, st.data()) != BNR_OK) { rc = ffail(BNR_ECUDA, bnr_last_error()); break; }
-      for (int v : st) R->status_or |= v;
-    }
-  }
-  if (getenv("BNR_FIT_TIMING"))
-    fprintf(stderr, "bnr_fit %.1f ms: create %.1f  init %.1f  run %.1f  row copies %.1f  psrf %.1f  summary %.1f  ess %.1f\n",
-            1e3 * (PhaseClock::now() - t_start), 1e3 * o.clk.t[PH_CREATE], 1e3 * o.clk.t[PH_INIT], 1e3 * o.clk.t[PH_RUN],
-            1e3 * o.clk.t[PH_COPY], 1e3 * o.clk.t[PH_PSRF], 1e3 * o.clk.t[PH_SUMMARY], 1e3 * o.clk.t[PH_ESS]);
-  if (rc) {
-    const std::string msg = g_fit_err;
-    delete R;
-    g_fit_err = msg;
-    return rc;
-  }
-  *res_out = R;
-  return BNR_OK;
-}
-
-extern "C" int bnr_fit(const bnr_fit_params* p, const double* X, const double* y, bnr_fit_result** res_out) {
-  return fit_body(p, X, y, 0, nullptr, BNR_PRED_MEAN, false, res_out);
-}
-
-extern "C" int bnr_fit_predict(const bnr_fit_params* p, const double* X, const double* y, int32_t m,
-                               const double* X_new, int32_t mode, bnr_fit_result** res_out) {
-  return fit_body(p, X, y, m, X_new, mode, false, res_out);
-}
-
-extern "C" int bnr_fit_loo(const bnr_fit_params* p, const double* X, const double* y, int32_t m, const double* X_new,
-                           int32_t pred_mode, bnr_fit_result** res_out) {
-  return fit_body(p, X, y, m, X_new, pred_mode, true, res_out);
-}
-
-// the fold layout of bnr_fit_kfold: labels checked, training and held-out rows of every fold in original order
+// the folds of bnr_fit_kfold: labels checked, training and held-out rows of every fold in original order, one handle
+// per fold
 static int kfold_split(const bnr_fit_params* p, const double* X, const double* y, int32_t K, const int32_t* fold,
-                       bnr_fit_result* R, KFoldOps& o) {
+                       bnr_fit_result* R, std::vector<Entry>& E) {
   const int n = p->base.n, V = p->base.V;
   const size_t q = (size_t)V * (V + 1) / 2;
   std::vector<int> cnt(K, 0);
@@ -867,45 +789,67 @@ static int kfold_split(const bnr_fit_params* p, const double* X, const double* y
     if (cnt[f] == 0) return ffail(BNR_EINVAL, "fold " + std::to_string(f + 1) + " holds no observation");
     if (cnt[f] == n) return ffail(BNR_EINVAL, "fold " + std::to_string(f + 1) + " leaves an empty training set");
   }
-  R->kf.K = K;
-  R->kf.held.assign(K, {});
-  o.folds.assign(K, {});
+  R->folds.assign(K, {});
+  R->held.width = cnt;
+  E.assign(K, {});
   for (int f = 0; f < K; ++f) {
-    KFoldOps::Fold& fd = o.folds[f];
-    fd.m = cnt[f]; fd.n = n - cnt[f];
+    Entry& e = E[f];
+    R->folds[f].first = e.fold = f;
+    e.n = n - cnt[f];
     for (int i = 0; i < n; ++i) {
       const bool held = fold[i] == f + 1;
-      (held ? fd.yh : fd.y).push_back(y[i]);
-      if (held) R->kf.held[f].push_back(i);
+      (held ? e.yh : e.yt).push_back(y[i]);
+      if (held) R->folds[f].held.push_back(i);
     }
     // column by column: X is column-major, so both sides are read and written in order
-    fd.X.resize((size_t)fd.n * q); fd.Xh.resize((size_t)fd.m * q);
-    double *dt = fd.X.data(), *dh = fd.Xh.data();
+    e.Xt.resize((size_t)e.n * q); e.Xh.resize((size_t)cnt[f] * q);
+    double *dt = e.Xt.data(), *dh = e.Xh.data();
     for (size_t j = 0; j < q; ++j) {
       const double* col = X + (size_t)n * j;
       for (int i = 0; i < n; ++i) *(fold[i] == f + 1 ? dh++ : dt++) = col[i];
     }
+    e.X = e.Xt.data(); e.y = e.yt.data();
   }
   return 0;
 }
 
-extern "C" int bnr_fit_kfold(const bnr_fit_params* p, const double* X, const double* y, int32_t K, const int32_t* fold,
-                             bnr_fit_result** res_out) {
+// bnr_fit, bnr_fit_predict (m > 0: predictions for the m rows of X_new), bnr_fit_loo (loo: PSIS-LOO and WAIC) and
+// bnr_fit_kfold (K > 0: the folds of `fold`, each scored on the observations it holds out)
+static int fit_entry(const char* name, const bnr_fit_params* p, const double* X, const double* y, int32_t m,
+                     const double* X_new, int32_t mode, bool loo, int32_t K, const int32_t* fold,
+                     bnr_fit_result** res_out) {
+  if (m < 0) return ffail(BNR_EINVAL, "m must be >= 0");
+  if (m > 0 && !X_new) return ffail(BNR_EINVAL, "null X_new");
+  if (mode != BNR_PRED_MEAN && mode != BNR_PRED_PREDICTIVE) return ffail(BNR_EINVAL, "unknown prediction mode");
   if (int r = check_params(p)) return r;
-  if (!X || !y || !fold || !res_out) return ffail(BNR_EINVAL, "null argument");
-  if (K < 2) return ffail(BNR_EINVAL, "K-fold cross-validation needs K >= 2 folds");
-  if (p->base.n < 2) return ffail(BNR_EINVAL, "K-fold cross-validation needs n >= 2 observations");
-  if (p->base.V < 1) return ffail(BNR_EINVAL, "V must be >= 1");
-  if (p->ext_world > 1) return ffail(BNR_EINVAL, "K-fold cross-validation runs in one process (ext_world must be <= 1)");
-  if (p->ess_max_lag > 0) return ffail(BNR_EINVAL, "K-fold cross-validation computes no ESS (ess_max_lag must be 0)");
-  if (p->base.nu < p->base.R) return ffail(BNR_EINVAL, "nu must not be smaller than R");
+  if (!X || !y || !res_out) return ffail(BNR_EINVAL, "null argument");
+  if (p->base.nu < p->base.R)
+    // the reference builds this ArgumentError without throwing it (src/gibbs.jl:901-902); the InverseWishart draw is
+    // undefined for nu <= R - 1, so the engine refuses
+    return ffail(BNR_EINVAL, "nu must not be smaller than R");
   bnr_fit_result* R = new bnr_fit_result();
   R->p = *p;
-  KFoldOps o(*R);
-  int rc = kfold_split(p, X, y, K, fold, R, o);
+  R->pmode = mode;
+  DeviceOps o(*R, X_new);
+  int rc = 0;
+  if (K > 0) {
+    rc = kfold_split(p, X, y, K, fold, R, o.E);
+  } else {
+    // one fold over n_devices handles that share the caller's rows and hold nothing out
+    const int nd = p->n_devices > 0 ? p->n_devices : 1;
+    R->folds.assign(1, {});
+    R->folds[0].handles = nd;
+    o.E.assign(nd, {0, p->base.n, X, y});
+    if (m > 0) R->pred.width.assign(nd, m);
+    if (loo) R->ll.width.assign(nd, p->base.n);
+  }
   const double t_start = PhaseClock::now();
   if (!rc) rc = fit_loops(o, *p, R->out);
-  if (!rc) rc = o.pool(R->out);
+  if (!rc && K == 0) rc = o.summary(R->out);
+  if (!rc && m > 0) rc = o.predictions(R->out);
+  if (!rc && loo) rc = o.loo(R->out);
+  if (!rc && K > 0) rc = o.heldout(R->out);
+  if (!rc) rc = o.ess(R->out);
   if (!rc) {
     std::vector<int32_t> st(R->C);
     for (auto* h : R->h) {
@@ -914,9 +858,10 @@ extern "C" int bnr_fit_kfold(const bnr_fit_params* p, const double* X, const dou
     }
   }
   if (getenv("BNR_FIT_TIMING"))
-    fprintf(stderr, "bnr_fit_kfold %.1f ms: create %.1f  init %.1f  run %.1f  row copies %.1f  psrf %.1f\n",
-            1e3 * (PhaseClock::now() - t_start), 1e3 * o.clk.t[PH_CREATE], 1e3 * o.clk.t[PH_INIT], 1e3 * o.clk.t[PH_RUN],
-            1e3 * o.clk.t[PH_COPY], 1e3 * o.clk.t[PH_PSRF]);
+    fprintf(stderr, "%s %.1f ms: create %.1f  init %.1f  run %.1f  row copies %.1f  psrf %.1f  summary %.1f  ess %.1f\n",
+            name, 1e3 * (PhaseClock::now() - t_start), 1e3 * o.clk.t[PH_CREATE], 1e3 * o.clk.t[PH_INIT],
+            1e3 * o.clk.t[PH_RUN], 1e3 * o.clk.t[PH_COPY], 1e3 * o.clk.t[PH_PSRF], 1e3 * o.clk.t[PH_SUMMARY],
+            1e3 * o.clk.t[PH_ESS]);
   if (rc) {
     const std::string msg = g_fit_err;
     delete R;
@@ -927,25 +872,51 @@ extern "C" int bnr_fit_kfold(const bnr_fit_params* p, const double* X, const dou
   return BNR_OK;
 }
 
+extern "C" int bnr_fit(const bnr_fit_params* p, const double* X, const double* y, bnr_fit_result** res_out) {
+  return fit_entry("bnr_fit", p, X, y, 0, nullptr, BNR_PRED_MEAN, false, 0, nullptr, res_out);
+}
+
+extern "C" int bnr_fit_predict(const bnr_fit_params* p, const double* X, const double* y, int32_t m,
+                               const double* X_new, int32_t mode, bnr_fit_result** res_out) {
+  return fit_entry("bnr_fit_predict", p, X, y, m, X_new, mode, false, 0, nullptr, res_out);
+}
+
+extern "C" int bnr_fit_loo(const bnr_fit_params* p, const double* X, const double* y, int32_t m, const double* X_new,
+                           int32_t pred_mode, bnr_fit_result** res_out) {
+  return fit_entry("bnr_fit_loo", p, X, y, m, X_new, pred_mode, true, 0, nullptr, res_out);
+}
+
+extern "C" int bnr_fit_kfold(const bnr_fit_params* p, const double* X, const double* y, int32_t K, const int32_t* fold,
+                             bnr_fit_result** res_out) {
+  if (int r = check_params(p)) return r;             // before the K-fold rules read p
+  if (!fold) return ffail(BNR_EINVAL, "null argument");
+  if (K < 2) return ffail(BNR_EINVAL, "K-fold cross-validation needs K >= 2 folds");
+  if (p->base.n < 2) return ffail(BNR_EINVAL, "K-fold cross-validation needs n >= 2 observations");
+  if (p->base.V < 1) return ffail(BNR_EINVAL, "V must be >= 1");
+  if (p->ext_world > 1) return ffail(BNR_EINVAL, "K-fold cross-validation runs in one process (ext_world must be <= 1)");
+  if (p->ess_max_lag > 0) return ffail(BNR_EINVAL, "K-fold cross-validation computes no ESS (ess_max_lag must be 0)");
+  return fit_entry("bnr_fit_kfold", p, X, y, 0, nullptr, BNR_PRED_MEAN, false, K, fold, res_out);
+}
+
 extern "C" int bnr_fit_kfold_pointwise(const bnr_fit_result* r, double* elpd_kfold) {
   if (!r || !elpd_kfold) return ffail(BNR_EINVAL, "null argument");
-  if (!r->kf.K) return ffail(BNR_ESTATE, "not a K-fold result (bnr_fit_kfold)");
-  if (!r->kf.ok) return ffail(BNR_ESTATE, "no retained draws");
-  memcpy(elpd_kfold, r->kf.elpd.data(), sizeof(double) * r->kf.elpd.size());
+  if (!r->kfold()) return ffail(BNR_ESTATE, "not a K-fold result (bnr_fit_kfold)");
+  if (!r->held.ok) return ffail(BNR_ESTATE, "no retained draws");
+  memcpy(elpd_kfold, r->elpd.data(), sizeof(double) * r->elpd.size());
   return BNR_OK;
 }
 
 extern "C" int bnr_fit_kfold_rhat(const bnr_fit_result* r, int32_t f, double* rhat_xi, double* rhat_gamma) {
   if (!r) return ffail(BNR_EINVAL, "null result");
-  if (!r->kf.K) return ffail(BNR_ESTATE, "not a K-fold result (bnr_fit_kfold)");
-  if (f < 0 || f >= r->kf.K) return ffail(BNR_EINVAL, "fold index outside 0..K-1");
-  if (rhat_xi) memcpy(rhat_xi, r->kf.rhat_xi[f].data(), sizeof(double) * r->V);
-  if (rhat_gamma) memcpy(rhat_gamma, r->kf.rhat_gamma[f].data(), sizeof(double) * r->q);
+  if (!r->kfold()) return ffail(BNR_ESTATE, "not a K-fold result (bnr_fit_kfold)");
+  if (f < 0 || f >= (int)r->folds.size()) return ffail(BNR_EINVAL, "fold index outside 0..K-1");
+  if (rhat_xi) memcpy(rhat_xi, r->folds[f].rhat_xi.data(), sizeof(double) * r->V);
+  if (rhat_gamma) memcpy(rhat_gamma, r->folds[f].rhat_gamma.data(), sizeof(double) * r->q);
   return BNR_OK;
 }
 
 static int not_kfold(const bnr_fit_result* r) {
-  return r->kf.K ? ffail(BNR_ESTATE, "not available on a K-fold result (bnr_fit_kfold)") : 0;
+  return r->kfold() ? ffail(BNR_ESTATE, "not available on a K-fold result (bnr_fit_kfold)") : 0;
 }
 
 extern "C" int bnr_fit_loo_pointwise(const bnr_fit_result* r, double* elpd_loo, double* p_loo, double* pareto_k,
@@ -953,7 +924,7 @@ extern "C" int bnr_fit_loo_pointwise(const bnr_fit_result* r, double* elpd_loo, 
   if (!r) return ffail(BNR_EINVAL, "null result");
   if (int e = not_kfold(r)) return e;
   if (!r->ll.ok)
-    return ffail(BNR_ESTATE, r->ll.width > 0 ? "fewer than 2 retained draws for PSIS-LOO"
+    return ffail(BNR_ESTATE, !r->ll.width.empty() ? "fewer than 2 retained draws for PSIS-LOO"
                                              : "the fit was run without the log-likelihood (bnr_fit_loo)");
   double* dst[5] = {elpd_loo, p_loo, pareto_k, elpd_waic, p_waic};
   for (int k = 0; k < 5; ++k)
@@ -965,11 +936,11 @@ extern "C" int bnr_fit_prediction(const bnr_fit_result* r, double* mean, double*
   if (!r) return ffail(BNR_EINVAL, "null result");
   if (int e = not_kfold(r)) return e;
   if (!r->pred.ok)
-    return ffail(BNR_ESTATE, r->pred.width > 0 ? "too few retained draws for the prediction interval"
+    return ffail(BNR_ESTATE, !r->pred.width.empty() ? "too few retained draws for the prediction interval"
                                                : "the fit was run without X_new (bnr_fit_predict)");
-  if (mean) memcpy(mean, r->p_mean.data(), sizeof(double) * r->pred.width);
-  if (lo) memcpy(lo, r->p_lo.data(), sizeof(double) * r->pred.width);
-  if (hi) memcpy(hi, r->p_hi.data(), sizeof(double) * r->pred.width);
+  if (mean) memcpy(mean, r->p_mean.data(), sizeof(double) * r->p_mean.size());
+  if (lo) memcpy(lo, r->p_lo.data(), sizeof(double) * r->p_lo.size());
+  if (hi) memcpy(hi, r->p_hi.data(), sizeof(double) * r->p_hi.size());
   return BNR_OK;
 }
 
@@ -981,8 +952,10 @@ extern "C" int bnr_fit_get_info(const bnr_fit_result* r, bnr_fit_info* info) {
   info->summary_ok = r->summary_ok ? 1 : 0; info->ess_ok = r->ess_ok ? 1 : 0;
   info->gamma_mode = r->gamma_mode; info->status_or = r->status_or;
   info->total_chains = r->C * (int)r->h.size() * (r->p.ext_world > 1 ? r->p.ext_world : 1);
-  info->n_devices = r->kf.K ? r->kf.n_devices : (int)r->h.size();
-  info->exchange = !strcmp(r->exchange, "nccl") ? 1 : (!strcmp(r->exchange, "peer-copy") ? 2 : 0);
+  std::vector<int> devs(r->dev);
+  std::sort(devs.begin(), devs.end());
+  info->n_devices = (int)(std::unique(devs.begin(), devs.end()) - devs.begin());
+  info->exchange = r->exchange;
   return BNR_OK;
 }
 

@@ -316,6 +316,17 @@ def _native_fit(Xn, y, R, *, X_new=None, predictive=False, loo=False, **kw):
         L.bnr_fit_free(res)
 
 
+def _hyper_and_seed(greek, ascii_, seed):
+    """(hyper-parameters, seed) of Fit! (src/gibbs.jl:725): each of η, ζ, ι, aΔ, bΔ, ν from its Greek keyword, else
+    its ASCII alias (eta, zeta, iota, a_delta, b_delta, nu), else its default; a seed of None draws one in 1..55555."""
+    def pick(g, a, default):
+        return default if (g is None and a is None) else (g if g is not None else a)
+
+    defaults = dict(eta=1.01, zeta=1.0, iota=1.0, a_delta=1.0, b_delta=1.0, nu=10)
+    hyper = {k: pick(g, a, d) for (k, d), g, a in zip(defaults.items(), greek, ascii_)}
+    return hyper, random.randint(1, 55555) if seed is None else seed
+
+
 def Fit(X, y, R, *, η=None, V=30, ζ=None, ι=None, aΔ=None, bΔ=None, ν=None, nburn=30000, nsamples=20000,
         mingen=0, maxgen=0, psrf_cutoff=1.01, x_transform=True, suppress_timer=False, num_chains=2, seed=None,
         purge_burn=None, filename="parameters.log", eta=None, zeta=None, iota=None, a_delta=None, b_delta=None,
@@ -334,17 +345,7 @@ def Fit(X, y, R, *, η=None, V=30, ζ=None, ι=None, aΔ=None, bΔ=None, ν=None
     loo=True: every chain also records the pointwise log-likelihood log N(y_i | mu + (X gamma)_i, tau2) at every sweep,
     and PSIS-LOO and WAIC of the retained draws of all chains are computed on the GPU into res.extra["loo"] (see Loo
     and Compare)."""
-    def pick(greek, ascii_, default):
-        return default if (greek is None and ascii_ is None) else (greek if greek is not None else ascii_)
-
-    eta = pick(η, eta, 1.01)
-    zeta = pick(ζ, zeta, 1.0)
-    iota = pick(ι, iota, 1.0)
-    a_delta = pick(aΔ, a_delta, 1.0)
-    b_delta = pick(bΔ, b_delta, 1.0)
-    nu = pick(ν, nu, 10)
-    if seed is None:
-        seed = random.randint(1, 55555)
+    hyper, seed = _hyper_and_seed((η, ζ, ι, aΔ, bΔ, ν), (eta, zeta, iota, a_delta, b_delta, nu), seed)
     rank, world = _dist_world()
     if world > 1 and rank != 0:
         filename = None                  # one parameters.log per job
@@ -355,13 +356,12 @@ def Fit(X, y, R, *, η=None, V=30, ζ=None, ι=None, aΔ=None, bΔ=None, ν=None
             fh.write(_citation())
             fh.write("\n\nParameters:\n")
             fh.write("R=%s, η=%s, ζ=%s, ι=%s, aΔ=%s, bΔ=%s, ν=%s, nburn=%s, nsamples=%s, \n" %
-                     (R, eta, zeta, iota, a_delta, b_delta, nu, nburn, nsamples))
+                     (R, *hyper.values(), nburn, nsamples))
             fh.write("mingen=%s, maxgen=%s, psrf_cutoff=%s, \n" % (mingen, maxgen, psrf_cutoff))
             fh.write("x_transform=%s, suppress_timer=%s, num_chains=%s, purge_burn=%s \n" %
                      (str(x_transform).lower(), str(suppress_timer).lower(), num_chains, purge_burn))
             fh.write("seed=%s" % seed)
-    kw = dict(eta=eta, zeta=zeta, iota=iota, a_delta=a_delta, b_delta=b_delta, nu=nu,
-              psrf_cutoff=psrf_cutoff, x_transform=x_transform, num_chains=num_chains, seed=seed,
+    kw = dict(hyper, psrf_cutoff=psrf_cutoff, x_transform=x_transform, num_chains=num_chains, seed=seed,
               purge_burn=purge_burn, device=device, return_state=return_state, verbose=verbose,
               chain_offset=chain_offset, n_devices=n_devices, ess_max_lag=ess_max_lag, gamma_mode=gamma_mode,
               chain_groups=chain_groups, X_new=X_new, predictive=predictive, loo=loo)
@@ -386,27 +386,31 @@ def _prepare(X, y, R, nu, x_transform):
     return Xn, y
 
 
+def _generate(X, y, R, x_transform, kw):
+    """Either scheme, its schedule keywords in kw: setup_X of X (and X_new), then one native call."""
+    Xn, y = _prepare(X, y, R, kw["nu"], x_transform)
+    kw["X_new"] = _prepare_new(kw.get("X_new"), x_transform)
+    if kw["seed"] is None:
+        kw["seed"] = random.randint(1, 55555)
+    return _native_fit(Xn, y, R, **kw)
+
+
 def generate_samples(X, y, R, *, eta=1.01, zeta=1.0, iota=1.0, a_delta=1.0, b_delta=1.0, nu=10, nburn=30000,
                      nsamp=20000, psrf_cutoff=1.2, x_transform=True, num_chains=2, seed=None, purge_burn=None, **kw):
     """The "traditional" scheme (generate_samples!, src/gibbs.jl:897-1020; maxburn = nburn + nsamp as Fit! passes it):
     the control loop runs inside libbnr (bnr_fit)."""
-    Xn, y = _prepare(X, y, R, nu, x_transform)
-    kw["X_new"] = _prepare_new(kw.get("X_new"), x_transform)
-    seed = random.randint(1, 55555) if seed is None else seed
-    return _native_fit(Xn, y, R, eta=eta, zeta=zeta, iota=iota, a_delta=a_delta, b_delta=b_delta, nu=nu, nburn=nburn,
-                       nsamp=nsamp, psrf_cutoff=psrf_cutoff, purge_burn=purge_burn, num_chains=num_chains, seed=seed, **kw)
+    return _generate(X, y, R, x_transform, dict(kw, eta=eta, zeta=zeta, iota=iota, a_delta=a_delta, b_delta=b_delta,
+                                                nu=nu, nburn=nburn, nsamp=nsamp, psrf_cutoff=psrf_cutoff,
+                                                num_chains=num_chains, seed=seed, purge_burn=purge_burn))
 
 
 def generate_samples_dbl(X, y, R, *, eta=1.01, zeta=1.0, iota=1.0, a_delta=1.0, b_delta=1.0, nu=10, mingen=10000,
                          maxgen=100000, psrf_cutoff=1.01, x_transform=True, num_chains=2, seed=None,
                          purge_burn=None, **kw):
     """The "doubling generation" scheme (generate_samples_dbl!, src/gibbs.jl:1051-1198), inside libbnr (bnr_fit)."""
-    Xn, y = _prepare(X, y, R, nu, x_transform)
-    kw["X_new"] = _prepare_new(kw.get("X_new"), x_transform)
-    seed = random.randint(1, 55555) if seed is None else seed
-    return _native_fit(Xn, y, R, eta=eta, zeta=zeta, iota=iota, a_delta=a_delta, b_delta=b_delta, nu=nu, mingen=mingen,
-                       maxgen=maxgen, psrf_cutoff=psrf_cutoff, purge_burn=purge_burn, num_chains=num_chains, seed=seed,
-                       **kw)
+    return _generate(X, y, R, x_transform, dict(kw, eta=eta, zeta=zeta, iota=iota, a_delta=a_delta, b_delta=b_delta,
+                                                nu=nu, mingen=mingen, maxgen=maxgen, psrf_cutoff=psrf_cutoff,
+                                                num_chains=num_chains, seed=seed, purge_burn=purge_burn))
 
 
 def _summary_ranks(nsamp, interval):
@@ -654,14 +658,7 @@ def KFold(X, y, R, K=None, folds=None, fold_seed=None, *, η=None, ζ=None, ι=N
     unknown = set(kw) - {"X_new", "predictive", "loo", "ess_max_lag", "V", "suppress_timer", "filename", "interval"}
     if unknown:
         raise TypeError("KFold got unexpected keyword arguments %s" % sorted(unknown))
-
-    def pick(greek, ascii_, default):
-        return default if (greek is None and ascii_ is None) else (greek if greek is not None else ascii_)
-
-    hyper = dict(eta=pick(η, eta, 1.01), zeta=pick(ζ, zeta, 1.0), iota=pick(ι, iota, 1.0),
-                 a_delta=pick(aΔ, a_delta, 1.0), b_delta=pick(bΔ, b_delta, 1.0), nu=pick(ν, nu, 10))
-    if seed is None:
-        seed = random.randint(1, 55555)
+    hyper, seed = _hyper_and_seed((η, ζ, ι, aΔ, bΔ, ν), (eta, zeta, iota, a_delta, b_delta, nu), seed)
     Xn, y = _prepare(X, y, R, hyper["nu"], x_transform)
     n = y.size
     if folds is None:
